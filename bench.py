@@ -4,9 +4,11 @@ through edm_tts_b200.runner.ShardedDecoder: no collective on the decode path, th
 NCCL). Also in the line: the same global batch 512 split over the N GPUs (BASELINE config 3, `fixed_global_batch`), the eager-torch
 bf16-autocast incumbent on the same GPU (`gpu_incumbent`), single-utterance latency, and the secondary kernels.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
-Prints ONE JSON line (rank 0). See DESIGN.md "Measurement" for the definition of every field.
+Prints ONE JSON line (rank 0). See DESIGN.md "Measurement" for the definition of every field. --dump-outputs DIR writes the codes the
+last timed step returned to DIR/s2a_codes.npy (float32 [N*64, 12, 500]; [1, 12, 500] with --impl reference); the inputs are seeded,
+so two builds run with the same arguments can be compared output for output. bench_outputs/<name> inside the tree is ignored by git.
 """
 from __future__ import annotations
 
@@ -20,6 +22,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ in the tree the benchmark runs from, which may be read-only
 
 B_PER_GPU, T_FRAMES, P_PROMPT, DECODE_STEPS = 64, 500, 0, 8
 WORKLOAD = "S2A decode: batch 64 x 10 s (500 frames) per GPU, 8 first-level steps + full pass, no prompt (BASELINE config 2)"
@@ -146,6 +149,16 @@ def gpu_incumbent_fps(dev, B, T, steps):
     return B * T / (times[-1] * 1e-3), times
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor of `arrays` as out_dir/<name>.npy in float32."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().to("cpu", torch.float32).numpy())
+
+
 def run_reference(args):
     """--impl reference: the reference's algorithm on the host CPU (oracle port; the Python reference itself cannot
     travel to the GPU box), all host threads, one bounded sample per step: 1 utterance x 500 frames x 8 steps."""
@@ -165,15 +178,17 @@ def run_reference(args):
 
     def step():
         with torch.inference_mode():
-            os2a.infer_special(sd, cfg, inp["semantic_tokens"], None, None, steps=DECODE_STEPS, cat_gumbel=inp["cat_gumbel"],
-                               remask_gumbel=inp["remask_gumbel"], mode="fp32")
+            return os2a.infer_special(sd, cfg, inp["semantic_tokens"], None, None, steps=DECODE_STEPS, cat_gumbel=inp["cat_gumbel"],
+                                      remask_gumbel=inp["remask_gumbel"], mode="fp32")
 
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        codes = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"s2a_codes": codes})
     fps = args.steps * T_FRAMES / dt
     sample = (f"bounded sample of the workload: 1 utterance x {T_FRAMES} frames x {DECODE_STEPS} steps per timed step (1/64 of the 64-utterance batch the "
               f"GPU arm decodes per step; the full batch takes ~70 s per step on these cores), oracle port of the reference in fp32 torch, {threads} threads")
@@ -193,7 +208,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the codes of the last timed step to DIR/s2a_codes.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -258,7 +276,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(k):
-            fn()
+            out = fn()
         e1.record()
         sync_all()
         ms = e0.elapsed_time(e1)
@@ -266,7 +284,7 @@ def main():
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return t.item(), launches
+        return t.item(), launches, out
 
     first = None
     for _ in range(args.warmup):
@@ -283,10 +301,10 @@ def main():
     del first
     sampler = ClockSampler(local)
     sampler.start()
-    ms_total, launches = timed(step_resident, args.steps)          # the headline: no per-kernel instrumentation inside
+    ms_total, launches, codes = timed(step_resident, args.steps)   # the headline: no per-kernel instrumentation inside
     # same K steps again with every GEMM / attention / LayerNorm / conv launch bracketed by CUDA events (roofline numbers);
     # the event records add a few % of gaps between kernels, so this pass is reported separately as instrumented_ms_per_step
-    ms_prof, _ = timed(step_resident, args.steps, profile=True)
+    ms_prof, _, _ = timed(step_resident, args.steps, profile=True)
     sampler.stop_flag = True
     sampler.join()
     pm, pw, pc = (C.c_double * 5)(), (C.c_double * 5)(), (C.c_int * 5)()
@@ -294,7 +312,7 @@ def main():
     lib.edm_prof_enable(0)
     for _ in range(2):
         step_e2e()
-    ms_e2e, _ = timed(step_e2e, args.steps)
+    ms_e2e, _, _ = timed(step_e2e, args.steps)
 
     frames = world * B * T * args.steps
     value = frames / (ms_total * 1e-3)
@@ -309,7 +327,7 @@ def main():
         return sharded(sem512, None, None, steps=DECODE_STEPS, temperature=1.0, seed=SEED)
 
     step_fixed()
-    ms_fixed, _ = timed(step_fixed, fixed_steps)
+    ms_fixed, _, _ = timed(step_fixed, fixed_steps)
     del sem512
 
     # single-utterance latency (the reference's own call site, inference.py:43-48): B = 1, 150 frames, 8 steps, device time per decode
@@ -559,6 +577,8 @@ def main():
                                                    "sample": "oracle conv encoder (fp32 torch CPU) on 1 x 10 s of audio, best of 2 (RVQ not included)"}
         out["secondary_decode"]["cpu_baseline"] = {"value": 500 / t_dec, "unit": "frames/s", "cores": threads, "kind": "port",
                                                    "sample": "oracle conv decoder (fp32 torch CPU) on 1 x 500 frames of latent, best of 2"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"s2a_codes": codes})
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()
