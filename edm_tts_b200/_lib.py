@@ -46,9 +46,11 @@ _SIGNATURES = {
     "edm_prof_collect": (_i, [C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int)]),
     "edm_gemm_bf16": (_i, [_vp, _ll, _vp, _ll, _i, _i, _i, _i, _vp, _vp, _ll, _f, _vp, _vp, _i, _i, _vp]),
     "edm_attention": (_i, [_vp, _i, _i, _i, _vp, _vp]),
+    "edm_attention_varlen": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
     "edm_layernorm": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp]),
     "edm_gemm_resid_layernorm": (_i, [_vp, _ll, _vp, _ll, _i, _i, _vp, _vp, _f, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp, _i, _vp]),
     "edm_conv_module": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _vp]),
+    "edm_conv_module_varlen": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
     "edm_sample": (_i, [_vp, _ll, _i, _vp, _i, _ull, _u, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "edm_remask": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _f, _f, _ull, _u, _vp]),
     "edm_rvq_encode_tc": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -64,6 +66,8 @@ _SIGNATURES = {
     "edm_s2a_destroy": (None, [_vp]),
     "edm_s2a_workspace_bytes": (_sz, [_vp, _i, _i, _i]),
     "edm_s2a_bind": (_i, [_vp, _vp, _sz, _i, _i, _i]),
+    "edm_s2a_workspace_bytes_varlen": (_sz, [_vp, _i, _vp, _vp]),
+    "edm_s2a_bind_varlen": (_i, [_vp, _vp, _sz, _i, _vp, _vp, _vp]),
     "edm_s2a_buffer": (_vp, [_vp, C.c_char_p, C.POINTER(_sz)]),
     "edm_s2a_set_batch_offset": (_i, [_vp, _ll]),
     "edm_s2a_set_seed_buffer": (_i, [_vp, _vp]),

@@ -7,6 +7,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <algorithm>
 #include <utility>
 #include <vector>
 
@@ -215,20 +216,6 @@ int make_tmap_2d(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, 
   if (r != CUDA_SUCCESS) return fail(EDM_ERR_CUDA, "cuTensorMapEncodeTiled(2d rows=%llu cols=%llu ld=%llu) failed: %d", (unsigned long long)rows, (unsigned long long)cols, (unsigned long long)ld, (int)r);
   return 0;
 }
-// bf16 [B, N, cols]: box = 64 cols x 128 rows x 1 batch; rows past N are zero-filled instead of reading the next sequence
-int make_tmap_3d(CUtensorMap* m, const void* ptr, uint64_t B, uint64_t N, uint64_t cols) {
-  PFN_tmapEncodeTiled enc = get_encode();
-  if (enc == nullptr) return fail(EDM_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-  cuuint64_t dims[3] = {cols, N, B};
-  cuuint64_t strides[2] = {cols * 2, N * cols * 2};
-  cuuint32_t box[3] = {64, 128, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(EDM_ERR_CUDA, "cuTensorMapEncodeTiled(3d) failed: %d", (int)r);
-  return 0;
-}
-
 // fp32 row-major [rows, cols] with row pitch ld (elements); box = 32 columns (128 B, swizzle-128B) x box_rows
 int make_tmap_f32_2d(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows,
                      CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
@@ -350,14 +337,18 @@ int launch_gemm(int epi, const CUtensorMap& ma, const WMap& mb, const GemmParams
 #ifdef EDM_ATTN_TRACE
 unsigned long long* g_attn_trace = nullptr;
 #endif
-int launch_attention(const CUtensorMap& mqkv, int B, int N, int H, void* out, uint32_t lbo, uint32_t sbo, uint32_t kstep, cudaStream_t st, float scale = 0.125f) {
+// qkv map: make_tmap_2d over all rows, 128-row boxes. pairs: the packed layout's (sequence << 16 | query pair) list, longest first
+// (nullptr for a uniform layout); flops: the algorithmic work, for the measurement hooks.
+int launch_attention(const CUtensorMap& mqkv, const SeqLayout& lay, const int* pairs, int n_pairs, double flops, int H, void* out, uint32_t lbo,
+                     uint32_t sbo, uint32_t kstep, cudaStream_t st, float scale = 0.125f) {
   static DeviceOnce attr_once;
   if (attr_once.needed()) {
     EDM_CUDA(cudaFuncSetAttribute(attention_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kAttnSmemBytes));
     attr_once.done();
   }
   AttnParams p;
-  p.B = B; p.N = N; p.H = H;
+  p.lay = lay; p.H = H; p.pairs = pairs;
+  p.n_items = (pairs != nullptr ? n_pairs : lay.n_seq * ((lay.N + 255) / 256)) * H;
   p.q_col0 = 0; p.k_col0 = H * 64; p.v_col0 = 2 * H * 64;
   p.out = static_cast<__nv_bfloat16*>(out);
   p.ldo = static_cast<long long>(H) * 64;
@@ -366,9 +357,9 @@ int launch_attention(const CUtensorMap& mqkv, int B, int N, int H, void* out, ui
 #ifdef EDM_ATTN_TRACE
   p.trace = g_attn_trace;
 #endif
-  const int items = ((N + 255) / 256) * H * B;
-  dim3 grid(items < num_sms() ? items : num_sms());
-  ProfScope prof(PK_ATTN, 4.0 * B * H * static_cast<double>(N) * N * 64, st);
+  if (p.n_items <= 0) return 0;
+  dim3 grid(p.n_items < num_sms() ? p.n_items : num_sms());
+  ProfScope prof(PK_ATTN, flops, st);
   launch_pdl(attention_fwd_kernel, dim3(grid), dim3(kAttnThreads), kAttnSmemBytes, st, mqkv, p);
   EDM_LAUNCH_CHECK("attention_fwd");
   return 0;
@@ -380,7 +371,7 @@ int launch_ln(const LnParams& p_in, cudaStream_t st) {
   p.reverse = next_direction();
   // algorithmic bytes: one read of the row + each requested output
   ProfScope prof(PK_LN, static_cast<double>(p.rows) * kD * ((p.in_is_bf16 ? 2 : 4) + (p.y_out ? 4 : 0)) +
-                            (p.z_out ? static_cast<double>(p.rows) * (p.z_skip > 0 ? static_cast<double>(p.seq_len - p.z_skip) / p.seq_len : 1.0) * kD * 2 : 0.0), st);
+                            (p.z_out ? static_cast<double>(p.compact ? p.lay.t_rows : p.rows) * kD * 2 : 0.0), st);
   launch_pdl(layernorm_kernel, dim3((p.rows + 7) / 8), dim3(256), 0, st, p);
   EDM_LAUNCH_CHECK("layernorm");
   return 0;
@@ -435,9 +426,48 @@ int launch_gemm_resid_ln(const CUtensorMap& ma, const WMap& wm, const GemmParams
   return 0;
 }
 
-// glu_input: the kernel reads [B*N, 4096] and applies the GLU itself; otherwise the input is the already gated [B*N, 2048]
+// Run length of the streaming conv kernel: every sequence is split into runs so that the persistent CTAs are evenly loaded and few
+// halo rows are re-read (run lengths are multiples of the 16-token statistics group, so only a sequence's last run has a partial
+// group). lens: the n_seq sequence lengths, or nullptr when every sequence has n rows.
+int conv_run_len(int n_seq, const int* lens, int n, int sms) {
+  long long rows = 0;
+  int max_n = n;
+  if (lens != nullptr) {
+    max_n = 0;
+    for (int i = 0; i < n_seq; ++i) {
+      rows += lens[i];
+      max_n = std::max(max_n, lens[i]);
+    }
+  } else {
+    rows = static_cast<long long>(n_seq) * n;
+  }
+  int best_len = (max_n + 15) / 16 * 16;
+  double best = -1.0;
+  for (int len = 16; len <= (max_n + 15) / 16 * 16; len += 16) {
+    long long units = 0;
+    if (lens != nullptr)
+      for (int i = 0; i < n_seq; ++i) units += (lens[i] + len - 1) / len;
+    else
+      units = static_cast<long long>(n_seq) * ((n + len - 1) / len);
+    const long long rounds = (units + sms - 1) / sms;
+    const double eff = static_cast<double>(rows) / (static_cast<double>(rounds * sms) * len) * len / (len + 4.0);
+    if (eff > best + 1e-9) {
+      best = eff;
+      best_len = len;
+    }
+  }
+  return best_len;
+}
+// Runs of a packed layout (built once at bind: the run length and the first run of every sequence)
+struct ConvRuns {
+  int run_len = 0, num_units = 0;
+  const int* cu_runs = nullptr;  // device [n_seq + 1]
+};
+
+// glu_input: the kernel reads [rows, 4096] and applies the GLU itself; otherwise the input is the already gated [rows, 2048]
 // (the decoder's path: the GLU runs in the pointwise-conv GEMM epilogue) and the streaming kernel of conv_stream.cuh is used.
-int launch_conv(const ConvModParams& p, bool glu_input, cudaStream_t st) {
+// runs: required for a packed layout on the streaming kernel.
+int launch_conv(const ConvModParams& p, bool glu_input, cudaStream_t st, const ConvRuns* runs = nullptr) {
   static DeviceOnce attr_once;
   if (attr_once.needed()) {
     EDM_CUDA(cudaFuncSetAttribute(conv_module_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemBytes));
@@ -445,36 +475,28 @@ int launch_conv(const ConvModParams& p, bool glu_input, cudaStream_t st) {
     EDM_CUDA(cudaFuncSetAttribute(conv_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCsSmemBytes));
     attr_once.done();
   }
-  if (p.B <= 0 || p.N <= 0) return 0;
-  ProfScope prof(PK_CONV, static_cast<double>(p.B) * p.N * (glu_input ? 12288.0 : 8192.0), st);
+  if (p.lay.n_seq <= 0 || p.max_n <= 0) return 0;
+  ProfScope prof(PK_CONV, static_cast<double>(p.lay.rows) * (glu_input ? 12288.0 : 8192.0), st);
   static const bool legacy = env_switch("EDM_CONV_LEGACY", false);  // bring-up switch: tiled kernel on the gated input as well
   if (glu_input || legacy) {
-    dim3 grid((p.N + kConvTT - 1) / kConvTT, p.B);
+    dim3 grid((p.max_n + kConvTT - 1) / kConvTT, p.lay.n_seq);
     if (glu_input)
       launch_pdl(conv_module_kernel<true>, dim3(grid), dim3(kConvThreads), kConvSmemBytes, st, p);
     else
       launch_pdl(conv_module_kernel<false>, dim3(grid), dim3(kConvThreads), kConvSmemBytes, st, p);
   } else {
-    // split every sequence into runs so that the persistent CTAs are evenly loaded and few halo rows are re-read
-    // (run lengths are multiples of the 16-token statistics group, so only a sequence's last run has a partial group)
     const int sms = num_sms();
-    int best_len = (p.N + 15) / 16 * 16;
-    double best = -1.0;
-    for (int len = 16; len <= (p.N + 15) / 16 * 16; len += 16) {
-      const long long units = static_cast<long long>(p.B) * ((p.N + len - 1) / len);
-      const long long rounds = (units + sms - 1) / sms;
-      const double eff = static_cast<double>(p.B) * p.N / (static_cast<double>(rounds * sms) * len) * len / (len + 4.0);
-      if (eff > best + 1e-9) {
-        best = eff;
-        best_len = len;
-      }
-    }
     ConvStreamParams q;
-    q.in = p.in; q.out = p.out; q.dw_w = p.dw_w; q.dw_b = p.dw_b; q.cln_w = p.cln_w; q.B = p.B; q.N = p.N;
-    q.run_len = best_len;
+    q.in = p.in; q.out = p.out; q.dw_w = p.dw_w; q.dw_b = p.dw_b; q.cln_w = p.cln_w; q.lay = p.lay;
     q.reverse = next_direction();
-    q.runs_per_seq = (p.N + q.run_len - 1) / q.run_len;
-    const long long units = static_cast<long long>(p.B) * q.runs_per_seq;
+    if (p.lay.cu_n != nullptr) {
+      if (runs == nullptr || runs->cu_runs == nullptr) return fail(EDM_ERR_INVALID, "conv module: a packed layout needs its runs");
+      q.run_len = runs->run_len; q.runs_per_seq = 0; q.cu_runs = runs->cu_runs; q.num_units = runs->num_units;
+    } else {
+      q.run_len = conv_run_len(p.lay.n_seq, nullptr, p.lay.N, sms);
+      q.runs_per_seq = (p.lay.N + q.run_len - 1) / q.run_len; q.cu_runs = nullptr; q.num_units = p.lay.n_seq * q.runs_per_seq;
+    }
+    const long long units = q.num_units;
     launch_pdl(conv_stream_kernel, dim3(static_cast<unsigned>(units < sms ? units : sms)), dim3(kCsThreads), kCsSmemBytes, st, q);
   }
   EDM_LAUNCH_CHECK("conv_module");
@@ -493,15 +515,18 @@ __global__ void fill_u8_kernel(uint8_t* p, long long n, uint8_t v) {
   long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i < n) p[i] = v;
 }
-__global__ void assemble_codes_kernel(const int* coarse, int n_coarse, const int* fine, int n_fine, long long* out, int B, int T) {
+// codes of sequence b: [Q, T_b] at Q * t_start(b), from the coarse ids ([4, T_b] blocks) and the fine ids ([n_fine, T_b] blocks)
+__global__ void assemble_codes_kernel(const int* coarse, int n_coarse, const int* fine, int n_fine, long long* out, SeqLayout lay) {
   pdl_sync();
   const int Q = n_coarse + n_fine;
   long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i >= static_cast<long long>(B) * Q * T) return;
-  const int t = static_cast<int>(i % T);
-  const int q = static_cast<int>((i / T) % Q);
-  const int b = static_cast<int>(i / (static_cast<long long>(T) * Q));
-  out[i] = q < n_coarse ? coarse[(static_cast<long long>(b) * 4 + q) * T + t] : fine[(static_cast<long long>(b) * n_fine + (q - n_coarse)) * T + t];
+  if (i >= static_cast<long long>(lay.t_rows) * Q) return;
+  int b, t0;
+  lay.tgt_pos(static_cast<int>(i / Q), b, t0);  // Q t_start(b) <= i < Q t_start(b + 1)
+  const int tl = lay.t_len(b);
+  const int local = static_cast<int>(i - static_cast<long long>(Q) * lay.t_start(b));
+  const int q = local / tl, t = local - q * tl;
+  out[i] = q < n_coarse ? coarse[lay.out_offset(b, q, 4, t)] : fine[lay.out_offset(b, q - n_coarse, n_fine, t)];
 }
 
 }  // namespace
@@ -563,7 +588,9 @@ extern "C" int edm_gemm_bf16(const void* a, long long lda, const void* b, long l
   GemmParams p;
   p.M = M; p.N = N; p.K = K; p.a_k_offset = 0; p.b_row_offset = 0;
   p.bias = bias; p.out = out; p.ldo = ldo; p.scale = scale;
-  p.rope_cos = rope_cos; p.rope_sin = rope_sin; p.seq_len = seq_len > 0 ? seq_len : 1; p.rope_cols = rope_cols; p.reverse = 0; p.splits = 1; p.split_stride = 0;
+  seq_len = seq_len > 0 ? seq_len : 1;
+  p.rope_cos = rope_cos; p.rope_sin = rope_sin; p.rope_lay = uniform_layout((M + seq_len - 1) / seq_len, seq_len, seq_len); p.rope_cols = rope_cols;
+  p.reverse = 0; p.splits = 1; p.split_stride = 0;
   if (epilogue == EPI_QKV_ROPE && (rope_cos == nullptr || rope_sin == nullptr)) return fail(EDM_ERR_INVALID, "rope tables required");
   return launch_gemm(epilogue, ma, mb, p, static_cast<cudaStream_t>(stream));
 }
@@ -579,10 +606,12 @@ extern "C" int edm_gemm_resid_layernorm(const void* a, long long lda, const void
   if (int rc = make_wmap(&mb, b, kD, K, ldb)) return rc;
   GemmParams p;
   p.M = M; p.N = kD; p.K = K; p.a_k_offset = 0; p.b_row_offset = 0; p.bias = bias; p.out = x; p.ldo = kD; p.scale = scale;
-  p.rope_cos = nullptr; p.rope_sin = nullptr; p.seq_len = 1; p.rope_cols = 0; p.reverse = 0; p.splits = 1; p.split_stride = 0;
+  p.rope_cos = nullptr; p.rope_sin = nullptr; p.rope_lay = uniform_layout(M, 1, 1); p.rope_cols = 0; p.reverse = 0; p.splits = 1; p.split_stride = 0;
   LnParams ln;
   ln.in = x; ln.in_is_bf16 = 0; ln.rows = M; ln.w1 = w1; ln.b1 = b1; ln.w2 = w2; ln.b2 = b2; ln.y_out = y_out;
-  ln.z_out = static_cast<__nv_bfloat16*>(z_out); ln.seq_len = seq_len > 0 ? seq_len : 1; ln.z_skip = z_skip; ln.eps = eps; ln.reverse = 0;
+  ln.z_out = static_cast<__nv_bfloat16*>(z_out); ln.eps = eps; ln.reverse = 0;
+  seq_len = seq_len > 0 ? seq_len : 1;
+  ln.lay = uniform_layout(M / seq_len, seq_len, seq_len - z_skip); ln.compact = z_skip > 0;
   return launch_gemm_resid_ln(ma, mb, p, ln, scratch, splits, static_cast<cudaStream_t>(stream));
 }
 
@@ -594,8 +623,9 @@ int attention_entry(const void* qkv, int B, int N, int H, void* out, unsigned v_
   if (int rc = check_arch()) return rc;
   if (B <= 0 || N <= 0 || H <= 0) return fail(EDM_ERR_INVALID, "attention shape");
   CUtensorMap m;
-  if (int rc = make_tmap_3d(&m, qkv, B, N, 3ull * H * 64)) return rc;
-  return launch_attention(m, B, N, H, out, v_lbo, v_sbo, v_kstep, static_cast<cudaStream_t>(stream));
+  if (int rc = make_tmap_2d(&m, qkv, static_cast<uint64_t>(B) * N, 3ull * H * 64, 3ull * H * 64, 128)) return rc;
+  return launch_attention(m, uniform_layout(B, N, N), nullptr, 0, 4.0 * B * H * static_cast<double>(N) * N * 64, H, out, v_lbo, v_sbo, v_kstep,
+                          static_cast<cudaStream_t>(stream));
 }
 }  // namespace
 #ifdef EDM_BRINGUP
@@ -614,7 +644,9 @@ extern "C" int edm_layernorm(const void* in, int in_is_bf16, int rows, const flo
   if (int rc = check_arch()) return rc;
   LnParams p;
   p.in = in; p.in_is_bf16 = in_is_bf16; p.rows = rows; p.w1 = w1; p.b1 = b1; p.w2 = w2; p.b2 = b2;
-  p.y_out = y_out; p.z_out = static_cast<__nv_bfloat16*>(z_out); p.seq_len = seq_len > 0 ? seq_len : 1; p.z_skip = z_skip; p.eps = eps;
+  p.y_out = y_out; p.z_out = static_cast<__nv_bfloat16*>(z_out); p.eps = eps;
+  seq_len = seq_len > 0 ? seq_len : 1;
+  p.lay = uniform_layout(rows / seq_len, seq_len, seq_len - z_skip); p.compact = z_skip > 0;
   return launch_ln(p, static_cast<cudaStream_t>(stream));
 }
 
@@ -622,16 +654,102 @@ extern "C" int edm_conv_module(const void* in, int glu_input, void* out, const f
   if (int rc = check_arch()) return rc;
   ConvModParams p;
   p.in = static_cast<const __nv_bfloat16*>(in); p.out = static_cast<__nv_bfloat16*>(out);
-  p.dw_w = dw_w; p.dw_b = dw_b; p.cln_w = cln_w; p.B = B; p.N = N;
+  p.dw_w = dw_w; p.dw_b = dw_b; p.cln_w = cln_w; p.lay = uniform_layout(B, N, N); p.max_n = N;
   return launch_conv(p, glu_input != 0, static_cast<cudaStream_t>(stream));
+}
+
+// Op-level entry points of a packed batch (the context builds its layout once at bind; these build it per call).
+namespace {
+// reads the n_seq + 1 offsets back (the launch shapes depend on them) and checks them
+int read_offsets(const int* cu_dev, int n_seq, std::vector<int>* cu, cudaStream_t st) {
+  if (cu_dev == nullptr || n_seq <= 0 || n_seq >= (1 << 15)) return fail(EDM_ERR_INVALID, "varlen offsets (n_seq=%d)", n_seq);
+  cu->assign(n_seq + 1, 0);
+  EDM_CUDA(cudaMemcpyAsync(cu->data(), cu_dev, sizeof(int) * (n_seq + 1), cudaMemcpyDeviceToHost, st));
+  EDM_CUDA(cudaStreamSynchronize(st));
+  if ((*cu)[0] != 0) return fail(EDM_ERR_INVALID, "varlen offsets must start at 0");
+  for (int i = 0; i < n_seq; ++i)
+    if ((*cu)[i + 1] <= (*cu)[i]) return fail(EDM_ERR_INVALID, "varlen offsets: sequence %d is empty or negative", i);
+  return 0;
+}
+// a stream-ordered device copy of `h` that lives until the work enqueued after it on `st` has run
+struct StreamArray {
+  int* p = nullptr;
+  cudaStream_t st;
+  explicit StreamArray(cudaStream_t s) : st(s) {}
+  int put(const std::vector<int>& h) {
+    EDM_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&p), h.size() * sizeof(int), st));
+    EDM_CUDA(cudaMemcpyAsync(p, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    return 0;
+  }
+  ~StreamArray() {
+    if (p != nullptr) cudaFreeAsync(p, st);
+  }
+};
+SeqLayout packed_layout(int n_seq, const int* cu_dev, const std::vector<int>& cu) {
+  SeqLayout l;
+  l.n_seq = n_seq; l.N = 0; l.T = 0; l.cu_n = cu_dev; l.cu_t = cu_dev; l.rows = cu[n_seq]; l.t_rows = cu[n_seq];
+  return l;
+}
+}  // namespace
+
+extern "C" int edm_attention_varlen(const void* qkv, int n_seq, const int* cu_seqlens, int H, void* out, void* stream) {
+  if (int rc = check_arch()) return rc;
+  if (H <= 0) return fail(EDM_ERR_INVALID, "attention heads");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  std::vector<int> cu;
+  if (int rc = read_offsets(cu_seqlens, n_seq, &cu, st)) return rc;
+  std::vector<int> order(n_seq), pairs;
+  double flops = 0.0;
+  for (int i = 0; i < n_seq; ++i) {
+    order[i] = i;
+    flops += 4.0 * H * static_cast<double>(cu[i + 1] - cu[i]) * (cu[i + 1] - cu[i]) * 64;
+  }
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return cu[a + 1] - cu[a] > cu[b + 1] - cu[b]; });
+  for (int s : order)
+    for (int q2 = 0; q2 < (cu[s + 1] - cu[s] + 255) / 256; ++q2) pairs.push_back((s << 16) | q2);
+  CUtensorMap m;
+  if (int rc = make_tmap_2d(&m, qkv, cu[n_seq], 3ull * H * 64, 3ull * H * 64, 128)) return rc;
+  StreamArray dp(st);
+  if (int rc = dp.put(pairs)) return rc;
+  return launch_attention(m, packed_layout(n_seq, cu_seqlens, cu), dp.p, static_cast<int>(pairs.size()), flops, H, out, 1024, 1024, 2048, st);
+}
+
+extern "C" int edm_conv_module_varlen(const void* in, int glu_input, void* out, const float* dw_w, const float* dw_b, const float* cln_w, int n_seq,
+                                      const int* cu_seqlens, void* stream) {
+  if (int rc = check_arch()) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  std::vector<int> cu;
+  if (int rc = read_offsets(cu_seqlens, n_seq, &cu, st)) return rc;
+  std::vector<int> lens(n_seq);
+  int max_n = 0;
+  for (int i = 0; i < n_seq; ++i) {
+    lens[i] = cu[i + 1] - cu[i];
+    max_n = std::max(max_n, lens[i]);
+  }
+  ConvModParams p;
+  p.in = static_cast<const __nv_bfloat16*>(in); p.out = static_cast<__nv_bfloat16*>(out);
+  p.dw_w = dw_w; p.dw_b = dw_b; p.cln_w = cln_w; p.lay = packed_layout(n_seq, cu_seqlens, cu); p.max_n = max_n;
+  ConvRuns runs;
+  runs.run_len = conv_run_len(n_seq, lens.data(), 0, num_sms());
+  std::vector<int> cu_runs(n_seq + 1, 0);
+  for (int i = 0; i < n_seq; ++i) cu_runs[i + 1] = cu_runs[i] + (lens[i] + runs.run_len - 1) / runs.run_len;
+  runs.num_units = cu_runs[n_seq];
+  StreamArray dr(st);
+  if (!glu_input) {
+    if (int rc = dr.put(cu_runs)) return rc;
+    runs.cu_runs = dr.p;
+  }
+  return launch_conv(p, glu_input != 0, st, &runs);
 }
 
 extern "C" int edm_sample(const float* logits, long long ld, int rows, const float* noise, int use_philox, unsigned long long seed,
                           unsigned step, const int* forced_ids, int* ids, float* logp, int T, int Q, int out_q_stride, int out_q0, void* stream) {
   if (int rc = check_arch()) return rc;
   SampleParams p;
-  p.logits = logits; p.ld = ld; p.rows = rows; p.noise = noise; p.use_philox = use_philox; p.seed = seed; p.seed_dev = nullptr; p.step = step; p.row0 = 0;
-  p.forced_ids = forced_ids; p.ids = ids; p.ids_raw = nullptr; p.logp = logp; p.T = T; p.Q = Q; p.out_q_stride = out_q_stride; p.out_q0 = out_q0;
+  if (T <= 0 || Q <= 0) return fail(EDM_ERR_INVALID, "sample: T=%d Q=%d", T, Q);
+  p.logits = logits; p.ld = ld; p.rows = rows; p.noise = noise; p.use_philox = use_philox; p.seed = seed; p.seed_dev = nullptr; p.step = step; p.seq0 = 0;
+  p.forced_ids = forced_ids; p.ids = ids; p.ids_raw = nullptr; p.logp = logp; p.lay = uniform_layout(rows / (T * Q), T, T); p.Q = Q;
+  p.out_q_stride = out_q_stride; p.out_q0 = out_q0;
   return launch_sample(p, static_cast<cudaStream_t>(stream));
 }
 
@@ -641,7 +759,7 @@ extern "C" int edm_remask(const float* logp, const float* gumbel, const uint8_t*
   if (T > kRemaskMaxT) return fail(EDM_ERR_INVALID, "remask supports T <= %d", kRemaskMaxT);
   RemaskParams p;
   p.logp = logp; p.gumbel = gumbel; p.mask_old = mask_old; p.mask_new = mask_new; p.mask_raw = nullptr; p.forced_mask = forced_mask;
-  p.T = T; p.init_count = 0; p.ratio = ratio; p.temp_ratio = temp_ratio; p.seed = seed; p.seed_dev = nullptr; p.step = step; p.row0 = 0;
+  p.lay = uniform_layout(B, T, T); p.init_count = 0; p.ratio = ratio; p.temp_ratio = temp_ratio; p.seed = seed; p.seed_dev = nullptr; p.step = step; p.seq0 = 0;
   launch_pdl(remask_kernel, dim3(B), dim3(256), 0, static_cast<cudaStream_t>(stream), p);
   EDM_LAUNCH_CHECK("remask");
   return 0;
@@ -1002,9 +1120,17 @@ struct edm_s2a_ctx {
   WMap head_map, fine_map;
   int n_fine;
 
-  // bound shapes
+  // bound shapes. B = sequences; T / P / N: the common lengths of a uniform bind (0 after edm_s2a_bind_varlen)
   bool bound = false;
-  int B = 0, T = 0, P = 0, N = 0, M = 0, Mt = 0;
+  int B = 0, T = 0, P = 0, N = 0, M = 0, Mt = 0, Mp = 0, max_n = 0, min_t = 0;
+  bool varlen = false;
+  SeqLayout lay;                   // where the sequences are (device arrays in the workspace after a varlen bind)
+  const int* pairs = nullptr;      // varlen: attention (sequence, query pair) list in the workspace, longest first
+  int n_pairs = 0;
+  double attn_flops = 0.0;
+  ConvRuns conv_runs;              // varlen: runs of the streaming conv kernel
+  int* layout_dev = nullptr;       // varlen: the layout arrays in the workspace (cu_n | cu_t | cu_runs | pairs)
+  std::vector<int> host_layout;    // varlen: their host image
   uint8_t* ws = nullptr;
   size_t ws_bytes = 0;
   // workspace views
@@ -1056,7 +1182,7 @@ int injection_index(const edm_s2a_config& c, int layer) {
 GemmParams gp(int M, int N, int K, const float* bias, void* out, long long ldo, float scale = 1.0f) {
   GemmParams p;
   p.M = M; p.N = N; p.K = K; p.a_k_offset = 0; p.b_row_offset = 0; p.bias = bias; p.out = out; p.ldo = ldo; p.scale = scale;
-  p.rope_cos = nullptr; p.rope_sin = nullptr; p.seq_len = 1; p.rope_cols = 0; p.reverse = 0; p.splits = 1; p.split_stride = 0;
+  p.rope_cos = nullptr; p.rope_sin = nullptr; p.rope_lay = uniform_layout(M, 1, 1); p.rope_cols = 0; p.reverse = 0; p.splits = 1; p.split_stride = 0;
   return p;
 }
 
@@ -1068,7 +1194,7 @@ int run_block_body(edm_s2a_ctx* c, int l, const LnParams& post, cudaStream_t st)
   const float eps = 1e-5f;
   LnParams ln;
   ln.in = c->x; ln.in_is_bf16 = 0; ln.rows = M; ln.w2 = nullptr; ln.b2 = nullptr;
-  ln.y_out = nullptr; ln.z_out = c->z; ln.seq_len = 1; ln.z_skip = 0; ln.eps = eps;
+  ln.y_out = nullptr; ln.z_out = c->z; ln.lay = c->lay; ln.compact = 0; ln.eps = eps;
   // ff1: x += 0.5 * W2 swish(W1 z + b1) + b2; then the attention pre-norm
   if (int rc = launch_gemm(EPI_SWISH_BF16, c->m_z, c->bmaps[l].ff1_w1, gp(M, 4096, 1024, c->bwf(l, F_FF1_B1), c->h, 4096), st)) return rc;
   ln.w1 = c->bwf(l, F_ATTN_LN_W); ln.b1 = c->bwf(l, F_ATTN_LN_B);
@@ -1076,18 +1202,18 @@ int run_block_body(edm_s2a_ctx* c, int l, const LnParams& post, cudaStream_t st)
   // attention
   {
     GemmParams p = gp(M, 3072, 1024, nullptr, c->qkv, 3072);
-    p.rope_cos = c->gwf(G_ROPE_COS); p.rope_sin = c->gwf(G_ROPE_SIN); p.seq_len = c->N; p.rope_cols = 2048;
+    p.rope_cos = c->gwf(G_ROPE_COS); p.rope_sin = c->gwf(G_ROPE_SIN); p.rope_lay = c->lay; p.rope_cols = 2048;
     if (int rc = launch_gemm(EPI_QKV_ROPE, c->m_z, c->bmaps[l].wqkv, p, st)) return rc;
   }
-  if (int rc = launch_attention(c->m_qkv, c->B, c->N, 16, c->z, 1024, 1024, 2048, st)) return rc;
+  if (int rc = launch_attention(c->m_qkv, c->lay, c->pairs, c->n_pairs, c->attn_flops, 16, c->z, 1024, 1024, 2048, st)) return rc;
   ln.w1 = c->bwf(l, F_CONV_LN_W); ln.b1 = c->bwf(l, F_CONV_LN_B);
   if (int rc = launch_gemm_resid_ln(c->m_z, c->bmaps[l].wo, gp(M, 1024, 1024, c->bwf(l, F_BO), c->x, 1024, 1.0f), ln, c->part, c->low_latency ? choose_splits(M, 1024) : 1, st)) return rc;
   // conv module. pointwise conv 1 + GLU in one pass: the packed weight interleaves 32 value rows with their 32 gate rows
   if (int rc = launch_gemm(EPI_GLU_BF16, c->m_z, c->bmaps[l].pw1, gp(M, 4096, 1024, c->bwf(l, F_PW1_B), c->h, 2048), st)) return rc;
   {
     ConvModParams p;
-    p.in = c->h; p.out = c->g; p.dw_w = c->bwf(l, F_DW_W); p.dw_b = c->bwf(l, F_DW_B); p.cln_w = c->bwf(l, F_CLN_W); p.B = c->B; p.N = c->N;
-    if (int rc = launch_conv(p, false, st)) return rc;
+    p.in = c->h; p.out = c->g; p.dw_w = c->bwf(l, F_DW_W); p.dw_b = c->bwf(l, F_DW_B); p.cln_w = c->bwf(l, F_CLN_W); p.lay = c->lay; p.max_n = c->max_n;
+    if (int rc = launch_conv(p, false, st, &c->conv_runs)) return rc;
   }
   ln.w1 = c->bwf(l, F_FF2_LN_W); ln.b1 = c->bwf(l, F_FF2_LN_B);
   if (int rc = launch_gemm_resid_ln(c->m_g, c->bmaps[l].pw2, gp(M, 1024, 2048, c->bwf(l, F_PW2_B), c->x, 1024, 1.0f), ln, c->part, c->low_latency ? choose_splits(M, 2048) : 1, st)) return rc;
@@ -1101,7 +1227,7 @@ int pass_prologue(edm_s2a_ctx* c, const float* x_src, cudaStream_t st) {
   LnParams ln;
   ln.in = x_src; ln.in_is_bf16 = 0; ln.rows = c->M; ln.w1 = nullptr; ln.b1 = nullptr;
   ln.w2 = c->bwf(0, F_FF1_LN_W); ln.b2 = c->bwf(0, F_FF1_LN_B);
-  ln.y_out = c->x; ln.z_out = c->z; ln.seq_len = 1; ln.z_skip = 0; ln.eps = 1e-5f;
+  ln.y_out = c->x; ln.z_out = c->z; ln.lay = c->lay; ln.compact = 0; ln.eps = 1e-5f;
   return launch_ln(ln, st);
 }
 
@@ -1179,8 +1305,8 @@ struct Carver {
 };
 
 constexpr size_t kSplitMaxRows = 1024;  // choose_splits never splits beyond 4 row tiles (148 SMs / 16 column tiles / 2)
-size_t carve(edm_s2a_ctx* c, uint8_t* base, int B, int T, int P, bool assign) {
-  const size_t N = static_cast<size_t>(P) + T, M = static_cast<size_t>(B) * N, Mt = static_cast<size_t>(B) * T;
+// n_seq sequences, M encoder rows, Mt target rows, Mp prompt rows; layout_ints: ints of the varlen layout arrays (0 for a uniform bind)
+size_t carve(edm_s2a_ctx* c, uint8_t* base, int B, size_t M, size_t Mt, size_t Mp, size_t layout_ints, bool assign) {
   const int nf = c->n_fine;
   Carver k{base};
   float* x_in = k.take<float>(M * 1024);
@@ -1206,13 +1332,15 @@ size_t carve(edm_s2a_ctx* c, uint8_t* base, int B, int T, int P, bool assign) {
   int* pred_raw = k.take<int>(Mt * 4);
   int* fine_codes = k.take<int>(Mt * nf);
   int* sem_tokens = k.take<int>(Mt);
-  int* sem_prompt = k.take<int>(static_cast<size_t>(B) * (P > 0 ? P : 1));
-  int* ac_prompt = k.take<int>(static_cast<size_t>(B) * 12 * (P > 0 ? P : 1));
+  int* sem_prompt = k.take<int>(Mp > 0 ? Mp : static_cast<size_t>(B));
+  int* ac_prompt = k.take<int>(12 * (Mp > 0 ? Mp : static_cast<size_t>(B)));
   uint8_t* mask_a = k.take<uint8_t>(Mt);
   uint8_t* mask_b = k.take<uint8_t>(Mt);
   uint8_t* mask_raw = k.take<uint8_t>(Mt);
   float* part = M <= kSplitMaxRows ? k.take<float>(4 * M * 1024) : nullptr;
+  int* layout = layout_ints > 0 ? k.take<int>(layout_ints) : nullptr;
   if (assign) {
+    c->layout_dev = layout;
     c->part = part;
     c->x_in = x_in; c->x = x;
     for (int i = 0; i < 4; ++i) c->coarse_out[i] = co[i];
@@ -1223,11 +1351,40 @@ size_t carve(edm_s2a_ctx* c, uint8_t* base, int B, int T, int P, bool assign) {
   }
   return align_up(k.off, 1024);
 }
+
+
+// Lengths of a varlen bind: checked per sequence against the limits of a uniform bind; totals and the attention pair count out
+int varlen_shape(const edm_s2a_ctx* c, int n_seq, const int* T, const int* P, size_t* M, size_t* Mt, size_t* Mp, int* n_pairs) {
+  if (c == nullptr || n_seq <= 0 || n_seq >= (1 << 15) || T == nullptr) return fail(EDM_ERR_INVALID, "bind_varlen arguments (n_seq=%d)", n_seq);
+  size_t m = 0, mt = 0, mp = 0;
+  long long pairs = 0;
+  for (int i = 0; i < n_seq; ++i) {
+    const int t = T[i], pl = P != nullptr ? P[i] : 0;
+    if (t <= 0 || pl < 0) return fail(EDM_ERR_INVALID, "sequence %d: T=%d P=%d", i, t, pl);
+    if (t > kRemaskMaxT) return fail(EDM_ERR_INVALID, "sequence %d: T=%d exceeds %d", i, t, kRemaskMaxT);
+    if (static_cast<long long>(pl) + t > c->cfg.max_positions) return fail(EDM_ERR_INVALID, "sequence %d: P+T=%lld exceeds rotary table (%d)", i, static_cast<long long>(pl) + t, c->cfg.max_positions);
+    m += static_cast<size_t>(pl) + t;
+    mt += t;
+    mp += pl;
+    pairs += (pl + t + 255) / 256;
+  }
+  if (m > 0x7fffffffull / 16) return fail(EDM_ERR_INVALID, "bind_varlen: %zu rows", m);
+  *M = m; *Mt = mt; *Mp = mp; *n_pairs = static_cast<int>(pairs);
+  return 0;
+}
 }  // namespace
 
 extern "C" size_t edm_s2a_workspace_bytes(const edm_s2a_ctx* ctx, int B, int T, int P) {
   if (ctx == nullptr || B <= 0 || T <= 0 || P < 0) return 0;
-  return carve(const_cast<edm_s2a_ctx*>(ctx), nullptr, B, T, P, false);
+  const size_t N = static_cast<size_t>(P) + T;
+  return carve(const_cast<edm_s2a_ctx*>(ctx), nullptr, B, B * N, static_cast<size_t>(B) * T, static_cast<size_t>(B) * P, 0, false);
+}
+
+extern "C" size_t edm_s2a_workspace_bytes_varlen(const edm_s2a_ctx* ctx, int n_seq, const int* T, const int* P) {
+  size_t M, Mt, Mp;
+  int n_pairs;
+  if (varlen_shape(ctx, n_seq, T, P, &M, &Mt, &Mp, &n_pairs)) return 0;
+  return carve(const_cast<edm_s2a_ctx*>(ctx), nullptr, n_seq, M, Mt, Mp, 3 * (static_cast<size_t>(n_seq) + 1) + n_pairs, false);
 }
 
 extern "C" int edm_s2a_bind(edm_s2a_ctx* c, void* workspace, size_t bytes, int B, int T, int P) {
@@ -1235,11 +1392,15 @@ extern "C" int edm_s2a_bind(edm_s2a_ctx* c, void* workspace, size_t bytes, int B
   if (T > kRemaskMaxT) return fail(EDM_ERR_INVALID, "T=%d exceeds %d", T, kRemaskMaxT);
   if (P + T > c->cfg.max_positions) return fail(EDM_ERR_INVALID, "P+T=%d exceeds rotary table (%d)", P + T, c->cfg.max_positions);
   if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return fail(EDM_ERR_INVALID, "workspace must be 1024-byte aligned");
-  const size_t need = carve(c, nullptr, B, T, P, false);
+  const size_t N = static_cast<size_t>(P) + T;
+  const size_t need = carve(c, nullptr, B, B * N, static_cast<size_t>(B) * T, static_cast<size_t>(B) * P, 0, false);
   if (bytes < need) return fail(EDM_ERR_INVALID, "workspace too small: %zu < %zu", bytes, need);
-  carve(c, static_cast<uint8_t*>(workspace), B, T, P, true);
+  carve(c, static_cast<uint8_t*>(workspace), B, B * N, static_cast<size_t>(B) * T, static_cast<size_t>(B) * P, 0, true);
   c->ws = static_cast<uint8_t*>(workspace); c->ws_bytes = bytes;
-  c->B = B; c->T = T; c->P = P; c->N = P + T; c->M = B * (P + T); c->Mt = B * T;
+  c->B = B; c->T = T; c->P = P; c->N = P + T; c->M = B * (P + T); c->Mt = B * T; c->Mp = B * P; c->max_n = P + T; c->min_t = T;
+  c->varlen = false; c->lay = uniform_layout(B, P + T, T); c->pairs = nullptr; c->n_pairs = 0; c->conv_runs = ConvRuns();
+  c->attn_flops = 4.0 * B * 16 * static_cast<double>(c->N) * c->N * 64;
+  c->host_layout.clear();
   c->prompt_proj = nullptr;
   int rc = 0;
   rc = rc ? rc : make_tmap_2d(&c->m_z, c->z, c->M, 1024, 1024, kGemmBM);
@@ -1247,7 +1408,65 @@ extern "C" int edm_s2a_bind(edm_s2a_ctx* c, void* workspace, size_t bytes, int B
   rc = rc ? rc : make_tmap_2d(&c->m_g, c->g, c->M, 2048, 2048, kGemmBM);
   rc = rc ? rc : make_tmap_2d(&c->m_zt, c->zt, c->Mt, 1024, 1024, kGemmBM);
   rc = rc ? rc : make_tmap_2d(&c->m_fine_z, c->fine_z, c->Mt, static_cast<uint64_t>(c->n_fine) * 1024, static_cast<uint64_t>(c->n_fine) * 1024, kGemmBM);
-  rc = rc ? rc : make_tmap_3d(&c->m_qkv, c->qkv, B, c->N, 3072);
+  rc = rc ? rc : make_tmap_2d(&c->m_qkv, c->qkv, c->M, 3072, 3072, 128);
+  if (rc) return rc;
+  c->bound = true;
+  return 0;
+}
+
+extern "C" int edm_s2a_bind_varlen(edm_s2a_ctx* c, void* workspace, size_t bytes, int n_seq, const int* T, const int* P, void* stream) {
+  if (c == nullptr || workspace == nullptr) return fail(EDM_ERR_INVALID, "bind arguments");
+  if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return fail(EDM_ERR_INVALID, "workspace must be 1024-byte aligned");
+  size_t M, Mt, Mp;
+  int n_pairs;
+  if (int rc = varlen_shape(c, n_seq, T, P, &M, &Mt, &Mp, &n_pairs)) return rc;
+  const size_t n1 = static_cast<size_t>(n_seq) + 1, layout_ints = 3 * n1 + n_pairs;
+  const size_t need = carve(c, nullptr, n_seq, M, Mt, Mp, layout_ints, false);
+  if (bytes < need) return fail(EDM_ERR_INVALID, "workspace too small: %zu < %zu", bytes, need);
+  c->bound = false;
+  carve(c, static_cast<uint8_t*>(workspace), n_seq, M, Mt, Mp, layout_ints, true);
+  int* dev = c->layout_dev;
+  // host image of the layout arrays: cu_n | cu_t | cu_runs | pairs
+  std::vector<int> lens(n_seq);
+  std::vector<int>& h = c->host_layout;
+  h.assign(layout_ints, 0);
+  int max_n = 0, min_t = kRemaskMaxT;
+  double flops = 0.0;
+  for (int i = 0; i < n_seq; ++i) {
+    const int pl = P != nullptr ? P[i] : 0;
+    lens[i] = pl + T[i];
+    h[i + 1] = h[i] + lens[i];
+    h[n1 + i + 1] = h[n1 + i] + T[i];
+    max_n = std::max(max_n, lens[i]);
+    min_t = std::min(min_t, T[i]);
+    flops += 4.0 * 16 * static_cast<double>(lens[i]) * lens[i] * 64;
+  }
+  const int run_len = conv_run_len(n_seq, lens.data(), 0, num_sms());
+  for (int i = 0; i < n_seq; ++i) h[2 * n1 + i + 1] = h[2 * n1 + i] + (lens[i] + run_len - 1) / run_len;
+  // attention items, longest sequence first (ties in sequence order), so the static round-robin hands out the long items first
+  std::vector<int> order(n_seq);
+  for (int i = 0; i < n_seq; ++i) order[i] = i;
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return lens[a] > lens[b]; });
+  size_t k = 3 * n1;
+  for (int s : order)
+    for (int q2 = 0; q2 < (lens[s] + 255) / 256; ++q2) h[k++] = (s << 16) | q2;
+  EDM_CUDA(cudaMemcpyAsync(dev, h.data(), layout_ints * sizeof(int), cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream)));
+  c->ws = static_cast<uint8_t*>(workspace); c->ws_bytes = bytes;
+  c->B = n_seq; c->T = 0; c->P = 0; c->N = 0;
+  c->M = static_cast<int>(M); c->Mt = static_cast<int>(Mt); c->Mp = static_cast<int>(Mp); c->max_n = max_n; c->min_t = min_t;
+  c->varlen = true;
+  c->lay.n_seq = n_seq; c->lay.N = 0; c->lay.T = 0; c->lay.cu_n = dev; c->lay.cu_t = dev + n1; c->lay.rows = c->M; c->lay.t_rows = c->Mt;
+  c->conv_runs.run_len = run_len; c->conv_runs.cu_runs = dev + 2 * n1; c->conv_runs.num_units = h[2 * n1 + n_seq];
+  c->pairs = dev + 3 * n1; c->n_pairs = n_pairs;
+  c->attn_flops = flops;
+  c->prompt_proj = nullptr;
+  int rc = 0;
+  rc = rc ? rc : make_tmap_2d(&c->m_z, c->z, c->M, 1024, 1024, kGemmBM);
+  rc = rc ? rc : make_tmap_2d(&c->m_h, c->h, c->M, 4096, 4096, kGemmBM);
+  rc = rc ? rc : make_tmap_2d(&c->m_g, c->g, c->M, 2048, 2048, kGemmBM);
+  rc = rc ? rc : make_tmap_2d(&c->m_zt, c->zt, c->Mt, 1024, 1024, kGemmBM);
+  rc = rc ? rc : make_tmap_2d(&c->m_fine_z, c->fine_z, c->Mt, static_cast<uint64_t>(c->n_fine) * 1024, static_cast<uint64_t>(c->n_fine) * 1024, kGemmBM);
+  rc = rc ? rc : make_tmap_2d(&c->m_qkv, c->qkv, c->M, 3072, 3072, 128);
   if (rc) return rc;
   c->bound = true;
   return 0;
@@ -1278,18 +1497,18 @@ extern "C" int edm_s2a_build_input(edm_s2a_ctx* c, const int* sem_tokens, const 
   PdlScope pdl(c->M <= kPdlMaxRows);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (sem_tokens == nullptr) return fail(EDM_ERR_INVALID, "semantic tokens required");
-  if (c->P > 0) {
-    if (sem_prompt == nullptr || ac_prompt == nullptr) return fail(EDM_ERR_INVALID, "bound with P=%d but no prompt given", c->P);
+  if (c->Mp > 0) {
+    if (sem_prompt == nullptr || ac_prompt == nullptr) return fail(EDM_ERR_INVALID, "bound with %d prompt frames but no prompt given", c->Mp);
     if (ac_levels < c->cfg.n_injection || ac_levels > 12) return fail(EDM_ERR_INVALID, "acoustic prompt needs >= %d levels (got %d)", c->cfg.n_injection, ac_levels);
-    EDM_CUDA(cudaMemcpyAsync(c->sem_prompt, sem_prompt, sizeof(int) * c->B * c->P, cudaMemcpyDeviceToDevice, st));
-    EDM_CUDA(cudaMemcpyAsync(c->ac_prompt, ac_prompt, sizeof(int) * c->B * ac_levels * c->P, cudaMemcpyDeviceToDevice, st));
+    EDM_CUDA(cudaMemcpyAsync(c->sem_prompt, sem_prompt, sizeof(int) * c->Mp, cudaMemcpyDeviceToDevice, st));
+    EDM_CUDA(cudaMemcpyAsync(c->ac_prompt, ac_prompt, sizeof(int) * ac_levels * static_cast<size_t>(c->Mp), cudaMemcpyDeviceToDevice, st));
   }
   c->ac_levels = ac_levels;
   EDM_CUDA(cudaMemcpyAsync(c->sem_tokens, sem_tokens, sizeof(int) * c->Mt, cudaMemcpyDeviceToDevice, st));
   BuildInputParams p;
-  p.x = c->x_in; p.sem_tokens = c->sem_tokens; p.sem_prompt = c->P > 0 ? c->sem_prompt : nullptr; p.ac_prompt = c->P > 0 ? c->ac_prompt : nullptr;
+  p.x = c->x_in; p.sem_tokens = c->sem_tokens; p.sem_prompt = c->Mp > 0 ? c->sem_prompt : nullptr; p.ac_prompt = c->Mp > 0 ? c->ac_prompt : nullptr;
   p.ac_prompt_levels = ac_levels; p.sem_emb = c->gwf(G_SEM_EMB); p.mask_token = c->gwf(G_MASK_TOKEN); p.feat_table = c->gwf(G_FEAT_TABLE);
-  p.feat_const = c->gwf(G_FEAT_CONST); p.fp_ln_w = c->gwf(G_FP_LN_W); p.fp_ln_b = c->gwf(G_FP_LN_B); p.B = c->B; p.T = c->T; p.P = c->P; p.eps = 1e-5f;
+  p.feat_const = c->gwf(G_FEAT_CONST); p.fp_ln_w = c->gwf(G_FP_LN_W); p.fp_ln_b = c->gwf(G_FP_LN_B); p.lay = c->lay; p.rows = c->M; p.eps = 1e-5f;
   p.num_semantic = c->cfg.num_semantic;
   launch_pdl(build_input_kernel, dim3((c->M + 7) / 8), dim3(256), 0, st, p);
   EDM_LAUNCH_CHECK("build_input");
@@ -1310,10 +1529,10 @@ extern "C" int edm_s2a_first_level(edm_s2a_ctx* c, const float* x_in, void* stre
     ln.in = c->x; ln.in_is_bf16 = 0; ln.rows = c->M; ln.w1 = c->bwf(l, F_POST_LN_W); ln.b1 = c->bwf(l, F_POST_LN_B); ln.eps = 1e-5f;
     if (l < last) {
       ln.w2 = c->bwf(l + 1, F_FF1_LN_W); ln.b2 = c->bwf(l + 1, F_FF1_LN_B);
-      ln.y_out = c->x; ln.z_out = c->z; ln.seq_len = 1; ln.z_skip = 0;
+      ln.y_out = c->x; ln.z_out = c->z; ln.lay = c->lay; ln.compact = 0;
     } else {
       ln.w2 = c->gwf(G_TL_LN_W); ln.b2 = c->gwf(G_TL_LN_B);
-      ln.y_out = nullptr; ln.z_out = c->zt; ln.seq_len = c->N; ln.z_skip = c->P;
+      ln.y_out = nullptr; ln.z_out = c->zt; ln.lay = c->lay; ln.compact = c->Mp > 0;
     }
     if (int rc = run_block_body(c, l, ln, st)) return rc;
   }
@@ -1336,6 +1555,7 @@ extern "C" int edm_s2a_set_low_latency(edm_s2a_ctx* c, int on) {
 
 extern "C" int edm_s2a_set_prompt_injections(edm_s2a_ctx* c, const float* proj) {
   if (c == nullptr) return fail(EDM_ERR_INVALID, "null context");
+  if (c->varlen && proj != nullptr) return fail(EDM_ERR_STATE, "feature-valued prompt injections need a uniform bind (edm_s2a_bind)");
   c->prompt_proj = proj;
   return 0;
 }
@@ -1358,13 +1578,13 @@ extern "C" int edm_s2a_step(edm_s2a_ctx* c, int step, int steps, float temperatu
   if (steps < 2 || step < 0 || step >= steps) return fail(EDM_ERR_INVALID, "step %d of %d", step, steps);
   PdlScope pdl(c->M <= kPdlMaxRows);
   // the reference's take_along_dim(sorted_confidence, mask_len >= 1) is out of range for a single frame (utils/utils.py:56)
-  if (c->T < 2 && step < steps - 1 && forced_mask == nullptr) return fail(EDM_ERR_INVALID, "re-masking needs T >= 2 frames (T=%d, steps=%d)", c->T, steps);
+  if (c->min_t < 2 && step < steps - 1 && forced_mask == nullptr) return fail(EDM_ERR_INVALID, "re-masking needs T >= 2 frames (T=%d, steps=%d)", c->min_t, steps);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const bool last = step == steps - 1;
   SampleParams sp;
   sp.logits = c->logits; sp.ld = 1024; sp.rows = c->Mt; sp.noise = last ? nullptr : cat_noise; sp.use_philox = last ? 0 : 1; sp.seed = seed; sp.seed_dev = c->seed_dev;
-  sp.step = static_cast<unsigned>(step); sp.row0 = c->batch_offset * c->T; sp.forced_ids = forced_ids; sp.ids = c->ids; sp.ids_raw = c->ids_raw; sp.logp = last ? nullptr : c->logp;
-  sp.T = c->T; sp.Q = 1; sp.out_q_stride = 1; sp.out_q0 = 0;
+  sp.step = static_cast<unsigned>(step); sp.seq0 = c->batch_offset; sp.forced_ids = forced_ids; sp.ids = c->ids; sp.ids_raw = c->ids_raw; sp.logp = last ? nullptr : c->logp;
+  sp.lay = c->lay; sp.Q = 1; sp.out_q_stride = 1; sp.out_q0 = 0;
   if (int rc = launch_sample(sp, st)) return rc;
   uint8_t* m_old = c->mask_cur();
   uint8_t* m_new = nullptr;
@@ -1373,16 +1593,16 @@ extern "C" int edm_s2a_step(edm_s2a_ctx* c, int step, int steps, float temperatu
     const double ratio_d = std::cos(M_PI / 2.0 * (static_cast<double>(step + 1) / static_cast<double>(steps)));
     RemaskParams rp;
     rp.logp = c->logp; rp.gumbel = remask_noise; rp.mask_old = m_old; rp.mask_new = c->mask_next(); rp.mask_raw = c->mask_raw; rp.forced_mask = forced_mask;
-    rp.T = c->T; rp.init_count = 0; rp.ratio = static_cast<float>(ratio_d); rp.temp_ratio = static_cast<float>(static_cast<double>(temperature) * ratio_d);
-    rp.seed = seed; rp.seed_dev = c->seed_dev; rp.step = static_cast<unsigned>(step); rp.row0 = c->batch_offset * c->T;
-    launch_pdl(remask_kernel, dim3(c->B), dim3(256), 0, st, rp);
+    rp.lay = c->lay; rp.init_count = 0; rp.ratio = static_cast<float>(ratio_d); rp.temp_ratio = static_cast<float>(static_cast<double>(temperature) * ratio_d);
+    rp.seed = seed; rp.seed_dev = c->seed_dev; rp.step = static_cast<unsigned>(step); rp.seq0 = c->batch_offset;
+    launch_pdl(remask_kernel, dim3(c->lay.n_seq), dim3(256), 0, st, rp);
     EDM_LAUNCH_CHECK("remask");
     m_new = c->mask_next();
   }
   UpdateInputParams up;
   up.x = c->x_in; up.sem_tokens = c->sem_tokens; up.ids = c->ids; up.mask_old = m_old; up.mask_new = m_new; up.sem_emb = c->gwf(G_SEM_EMB);
   up.mask_token = c->gwf(G_MASK_TOKEN); up.feat_table = c->gwf(G_FEAT_TABLE); up.feat_const = c->gwf(G_FEAT_CONST);
-  up.fp_ln_w = c->gwf(G_FP_LN_W); up.fp_ln_b = c->gwf(G_FP_LN_B); up.B = c->B; up.T = c->T; up.P = c->P; up.eps = 1e-5f; up.num_semantic = c->cfg.num_semantic;
+  up.fp_ln_w = c->gwf(G_FP_LN_W); up.fp_ln_b = c->gwf(G_FP_LN_B); up.lay = c->lay; up.rows = c->Mt; up.eps = 1e-5f; up.num_semantic = c->cfg.num_semantic;
   launch_pdl(update_input_kernel, dim3((c->Mt + 7) / 8), dim3(256), 0, st, up);
   EDM_LAUNCH_CHECK("update_input");
   if (!last) c->mask_in_a = !c->mask_in_a;
@@ -1402,15 +1622,15 @@ extern "C" int edm_s2a_full_pass(edm_s2a_ctx* c, const float* x_in, const int* f
     ln.in = c->x; ln.in_is_bf16 = 0; ln.rows = c->M; ln.w1 = c->bwf(l, F_POST_LN_W); ln.b1 = c->bwf(l, F_POST_LN_B); ln.eps = 1e-5f;
     if (k < 0) {
       if (!is_last) {
-        ln.w2 = c->bwf(l + 1, F_FF1_LN_W); ln.b2 = c->bwf(l + 1, F_FF1_LN_B); ln.y_out = c->x; ln.z_out = c->z; ln.seq_len = 1; ln.z_skip = 0;
+        ln.w2 = c->bwf(l + 1, F_FF1_LN_W); ln.b2 = c->bwf(l + 1, F_FF1_LN_B); ln.y_out = c->x; ln.z_out = c->z; ln.lay = c->lay; ln.compact = 0;
       } else {
-        ln.w2 = nullptr; ln.b2 = nullptr; ln.y_out = nullptr; ln.z_out = c->zt; ln.seq_len = c->N; ln.z_skip = c->P;  // bf16 copy of the target rows
+        ln.w2 = nullptr; ln.b2 = nullptr; ln.y_out = nullptr; ln.z_out = c->zt; ln.lay = c->lay; ln.compact = c->Mp > 0;  // bf16 copy of the target rows
       }
       if (int rc = run_block_body(c, l, ln, st)) return rc;
       continue;
     }
     // injection layer k: keep the block output, predict level k on the target rows, inject
-    ln.w2 = c->gwf(G_TL_LN_W); ln.b2 = c->gwf(G_TL_LN_B); ln.y_out = c->coarse_out[k]; ln.z_out = c->zt; ln.seq_len = c->N; ln.z_skip = c->P;
+    ln.w2 = c->gwf(G_TL_LN_W); ln.b2 = c->gwf(G_TL_LN_B); ln.y_out = c->coarse_out[k]; ln.z_out = c->zt; ln.lay = c->lay; ln.compact = c->Mp > 0;
     if (int rc = run_block_body(c, l, ln, st)) return rc;
     if (c->keep_logits) {
       float* lk = c->coarse_logits + static_cast<size_t>(k) * c->Mt * 1024;
@@ -1418,8 +1638,8 @@ extern "C" int edm_s2a_full_pass(edm_s2a_ctx* c, const float* x_in, const int* f
       p.b_row_offset = k * 1024;
       if (int rc = launch_gemm(EPI_F32, c->m_zt, c->head_map, p, st)) return rc;
       SampleParams sp;
-      sp.logits = lk; sp.ld = 1024; sp.rows = c->Mt; sp.noise = nullptr; sp.use_philox = 0; sp.seed = 0; sp.seed_dev = nullptr; sp.step = 0; sp.row0 = 0; sp.forced_ids = forced_coarse;
-      sp.ids = c->pred_codes; sp.ids_raw = c->pred_raw; sp.logp = nullptr; sp.T = c->T; sp.Q = 1; sp.out_q_stride = 4; sp.out_q0 = k;
+      sp.logits = lk; sp.ld = 1024; sp.rows = c->Mt; sp.noise = nullptr; sp.use_philox = 0; sp.seed = 0; sp.seed_dev = nullptr; sp.step = 0; sp.seq0 = 0; sp.forced_ids = forced_coarse;
+      sp.ids = c->pred_codes; sp.ids_raw = c->pred_raw; sp.logp = nullptr; sp.lay = c->lay; sp.Q = 1; sp.out_q_stride = 4; sp.out_q0 = k;
       if (int rc = launch_sample(sp, st)) return rc;
     } else {
       // head k with the arg-max in the GEMM epilogue: 16 (max, index) partials per row instead of 1024 fp32 logits
@@ -1428,25 +1648,25 @@ extern "C" int edm_s2a_full_pass(edm_s2a_ctx* c, const float* x_in, const int* f
       if (int rc = launch_gemm(EPI_ARGMAX, c->m_zt, c->head_map, p, st)) return rc;
       ArgmaxCombineParams ap;
       ap.part = c->arg_part; ap.rows = c->Mt; ap.parts = 16; ap.forced_ids = forced_coarse; ap.ids = c->pred_codes; ap.ids_raw = c->pred_raw;
-      ap.T = c->T; ap.Q = 1; ap.out_q_stride = 4; ap.out_q0 = k;
+      ap.lay = c->lay; ap.Q = 1; ap.out_q_stride = 4; ap.out_q0 = k;
       launch_pdl(argmax_combine_kernel, dim3((c->Mt + 255) / 256), dim3(256), 0, st, ap);
       EDM_LAUNCH_CHECK("argmax_combine");
     }
     InjectParams ip;
     ip.x = c->x; ip.cur_out = c->coarse_out[k]; ip.prev_out = (k > 0 && cfg.residual) ? c->coarse_out[k - 1] : nullptr;
-    ip.pred_codes = c->pred_codes; ip.ac_prompt = c->P > 0 ? c->ac_prompt : nullptr; ip.ac_prompt_levels = c->ac_levels;
-    ip.prompt_proj = (c->P > 0 && c->prompt_proj != nullptr) ? c->prompt_proj + static_cast<size_t>(k) * c->B * c->P * 1024 : nullptr;
+    ip.pred_codes = c->pred_codes; ip.ac_prompt = c->Mp > 0 ? c->ac_prompt : nullptr; ip.ac_prompt_levels = c->ac_levels;
+    ip.prompt_proj = (c->Mp > 0 && c->prompt_proj != nullptr) ? c->prompt_proj + static_cast<size_t>(k) * c->Mp * 1024 : nullptr;
     for (int i = 0; i < 4; ++i) ip.tables[i] = c->gwf(G_INJ_TABLE) + (static_cast<size_t>(k) * 4 + i) * 1024 * 1024;
     ip.inj_const = c->gwf(G_INJ_CONST) + k * 1024; ip.ln_w = c->gwf(G_INJ_LN_W) + k * 1024; ip.ln_b = c->gwf(G_INJ_LN_B) + k * 1024;
-    ip.level = k; ip.B = c->B; ip.T = c->T; ip.P = c->P; ip.eps = 1e-5f;
+    ip.level = k; ip.lay = c->lay; ip.rows = c->M; ip.eps = 1e-5f;
     launch_pdl(inject_kernel, dim3((c->M + 7) / 8), dim3(256), 0, st, ip);
     EDM_LAUNCH_CHECK("inject");
     LnParams nx;
     nx.in = c->x; nx.in_is_bf16 = 0; nx.rows = c->M; nx.w1 = nullptr; nx.b1 = nullptr; nx.eps = 1e-5f; nx.y_out = nullptr;
     if (!is_last) {
-      nx.w2 = c->bwf(l + 1, F_FF1_LN_W); nx.b2 = c->bwf(l + 1, F_FF1_LN_B); nx.z_out = c->z; nx.seq_len = 1; nx.z_skip = 0;
+      nx.w2 = c->bwf(l + 1, F_FF1_LN_W); nx.b2 = c->bwf(l + 1, F_FF1_LN_B); nx.z_out = c->z; nx.lay = c->lay; nx.compact = 0;
     } else {
-      nx.w2 = nullptr; nx.b2 = nullptr; nx.z_out = c->zt; nx.seq_len = c->N; nx.z_skip = c->P;
+      nx.w2 = nullptr; nx.b2 = nullptr; nx.z_out = c->zt; nx.lay = c->lay; nx.compact = c->Mp > 0;
     }
     if (int rc = launch_ln(nx, st)) return rc;
   }
@@ -1456,7 +1676,7 @@ extern "C" int edm_s2a_full_pass(edm_s2a_ctx* c, const float* x_in, const int* f
   {
     LnParams ln;
     ln.in = c->fine_h; ln.in_is_bf16 = 1; ln.rows = c->Mt * nf; ln.w1 = c->gwf(G_TL_LN_W); ln.b1 = c->gwf(G_TL_LN_B); ln.w2 = nullptr; ln.b2 = nullptr;
-    ln.y_out = nullptr; ln.z_out = c->fine_z; ln.seq_len = 1; ln.z_skip = 0; ln.eps = 1e-5f;
+    ln.y_out = nullptr; ln.z_out = c->fine_z; ln.lay = c->lay; ln.compact = 0; ln.eps = 1e-5f;
     if (int rc = launch_ln(ln, st)) return rc;
   }
   for (int q = 0; q < nf; ++q) {
@@ -1474,19 +1694,19 @@ extern "C" int edm_s2a_full_pass(edm_s2a_ctx* c, const float* x_in, const int* f
   }
   if (c->keep_logits) {
     SampleParams sp;
-    sp.logits = c->fine_logits; sp.ld = 1024; sp.rows = c->Mt * nf; sp.noise = nullptr; sp.use_philox = 0; sp.seed = 0; sp.seed_dev = nullptr; sp.step = 0; sp.row0 = 0; sp.forced_ids = nullptr;
-    sp.ids = c->fine_codes; sp.ids_raw = nullptr; sp.logp = nullptr; sp.T = c->T; sp.Q = nf; sp.out_q_stride = nf; sp.out_q0 = 0;
+    sp.logits = c->fine_logits; sp.ld = 1024; sp.rows = c->Mt * nf; sp.noise = nullptr; sp.use_philox = 0; sp.seed = 0; sp.seed_dev = nullptr; sp.step = 0; sp.seq0 = 0; sp.forced_ids = nullptr;
+    sp.ids = c->fine_codes; sp.ids_raw = nullptr; sp.logp = nullptr; sp.lay = c->lay; sp.Q = nf; sp.out_q_stride = nf; sp.out_q0 = 0;
     if (int rc = launch_sample(sp, st)) return rc;
   } else {
     ArgmaxCombineParams ap;
     ap.part = c->arg_part; ap.rows = c->Mt * nf; ap.parts = 16; ap.forced_ids = nullptr; ap.ids = c->fine_codes; ap.ids_raw = nullptr;
-    ap.T = c->T; ap.Q = nf; ap.out_q_stride = nf; ap.out_q0 = 0;
+    ap.lay = c->lay; ap.Q = nf; ap.out_q_stride = nf; ap.out_q0 = 0;
     launch_pdl(argmax_combine_kernel, dim3((c->Mt * nf + 255) / 256), dim3(256), 0, st, ap);
     EDM_LAUNCH_CHECK("argmax_combine");
   }
   if (codes_out != nullptr) {
-    const long long total = static_cast<long long>(c->B) * cfg.num_quantizers * c->T;
-    launch_pdl(assemble_codes_kernel, dim3(static_cast<unsigned>((total + 255) / 256)), dim3(256), 0, st, c->pred_raw, cfg.n_injection, c->fine_codes, nf, codes_out, c->B, c->T);
+    const long long total = static_cast<long long>(c->Mt) * cfg.num_quantizers;
+    launch_pdl(assemble_codes_kernel, dim3(static_cast<unsigned>((total + 255) / 256)), dim3(256), 0, st, c->pred_raw, cfg.n_injection, c->fine_codes, nf, codes_out, c->lay);
     EDM_LAUNCH_CHECK("assemble_codes");
   }
   return 0;
@@ -1643,7 +1863,7 @@ int launch_conv_tiled_t(const ConvModParams& p, cudaStream_t st) {
     EDM_CUDA((cudaFuncSetAttribute(conv_module_kernel<false, kC>, cudaFuncAttributeMaxDynamicSharedMemorySize, conv_smem_bytes(kC))));
     attr_once.done();
   }
-  dim3 grid((p.N + kConvTT - 1) / kConvTT, p.B);
+  dim3 grid((p.max_n + kConvTT - 1) / kConvTT, p.lay.n_seq);
   launch_pdl(conv_module_kernel<false, kC>, dim3(grid), dim3(kC / 4), conv_smem_bytes(kC), st, p);
   EDM_LAUNCH_CHECK("conv_module");
   return 0;
@@ -1675,7 +1895,7 @@ int t2s_maps(edm_t2s_ctx* c, int M, int hp) {
   rc = rc ? rc : make_tmap_2d(&c->m_att, c->att, M, hp, hp, kGemmBM);
   rc = rc ? rc : make_tmap_2d(&c->m_g, c->g, M, c->C, c->C, kGemmBM);
   rc = rc ? rc : make_tmap_2d(&c->m_zt, c->zt, M, c->d, c->d, kGemmBM);
-  rc = rc ? rc : make_tmap_3d(&c->m_qkv, c->qkv, 1, M, 3ull * hp);
+  rc = rc ? rc : make_tmap_2d(&c->m_qkv, c->qkv, M, 3ull * hp, 3ull * hp, 128);
   return rc;
 }
 
@@ -1689,17 +1909,19 @@ int t2s_block_body(edm_t2s_ctx* c, int blk, int M, int H, int hp, const float* r
                                       lng(c->x, M, c->bwf(blk, F_ATTN_LN_W), c->bwf(blk, F_ATTN_LN_B), nullptr, nullptr, nullptr, c->z), c->part, st)) return rc;
   {
     GemmParams p = gp(M, 3 * hp, d, nullptr, c->qkv, 3 * hp);
-    p.rope_cos = rope_cos; p.rope_sin = rope_sin; p.seq_len = M; p.rope_cols = 2 * hp;
+    p.rope_cos = rope_cos; p.rope_sin = rope_sin; p.rope_lay = uniform_layout(1, M, M); p.rope_cols = 2 * hp;
     if (int rc = launch_gemm(EPI_QKV_ROPE, c->m_z, bm.wqkv, p, st)) return rc;
   }
   const float scale = 1.0f / sqrtf(static_cast<float>(d / H));
-  if (int rc = launch_attention(c->m_qkv, 1, M, H, c->att, 1024, 1024, 2048, st, scale)) return rc;
+  if (int rc = launch_attention(c->m_qkv, uniform_layout(1, M, M), nullptr, 0, 4.0 * H * static_cast<double>(M) * M * 64, H, c->att, 1024, 1024, 2048,
+                                st, scale))
+    return rc;
   if (int rc = launch_gemm_resid_ln_g(d, c->m_att, bm.wo, gp(M, d, hp, c->bwf(blk, F_BO), c->x, d, 1.0f),
                                       lng(c->x, M, c->bwf(blk, F_CONV_LN_W), c->bwf(blk, F_CONV_LN_B), nullptr, nullptr, nullptr, c->z), c->part, st)) return rc;
   if (int rc = launch_gemm(EPI_GLU_BF16, c->m_z, bm.pw1, gp(M, 2 * C, d, c->bwf(blk, F_PW1_B), c->h, C), st)) return rc;
   {
     ConvModParams p;
-    p.in = c->h; p.out = c->g; p.dw_w = c->bwf(blk, F_DW_W); p.dw_b = c->bwf(blk, F_DW_B); p.cln_w = c->bwf(blk, F_CLN_W); p.B = 1; p.N = M;
+    p.in = c->h; p.out = c->g; p.dw_w = c->bwf(blk, F_DW_W); p.dw_b = c->bwf(blk, F_DW_B); p.cln_w = c->bwf(blk, F_CLN_W); p.lay = uniform_layout(1, M, M); p.max_n = M;
     if (int rc = launch_conv_tiled(C, p, st)) return rc;
   }
   if (int rc = launch_gemm_resid_ln_g(d, c->m_g, bm.pw2, gp(M, d, C, c->bwf(blk, F_PW2_B), c->x, d, 1.0f),
@@ -1948,8 +2170,8 @@ extern "C" int edm_t2s_step(edm_t2s_ctx* c, int iter, int iters, float temperatu
   const int L = c->L;
   SampleParams sp;
   sp.logits = c->logits; sp.ld = 1024; sp.rows = L; sp.noise = last ? nullptr : cat_noise; sp.use_philox = last ? 0 : 1; sp.seed = seed; sp.seed_dev = nullptr;
-  sp.step = static_cast<unsigned>(iter); sp.row0 = 0; sp.forced_ids = forced_ids; sp.ids = c->ids; sp.ids_raw = c->ids_raw; sp.logp = last ? nullptr : c->logp;
-  sp.T = L; sp.Q = 1; sp.out_q_stride = 1; sp.out_q0 = 0;
+  sp.step = static_cast<unsigned>(iter); sp.seq0 = 0; sp.forced_ids = forced_ids; sp.ids = c->ids; sp.ids_raw = c->ids_raw; sp.logp = last ? nullptr : c->logp;
+  sp.lay = uniform_layout(1, L, L); sp.Q = 1; sp.out_q_stride = 1; sp.out_q0 = 0;
   if (int rc = launch_sample(sp, st)) return rc;
   T2sUpdateParams up;
   up.ids = c->ids; up.next_mask = nullptr; up.full_mask = c->full_mask; up.input_ids = c->input_ids; up.tokens = c->tokens; up.L = L;
@@ -1958,8 +2180,8 @@ extern "C" int edm_t2s_step(edm_t2s_ctx* c, int iter, int iters, float temperatu
     const double ratio_d = std::cos(M_PI / 2.0 * (static_cast<double>(iter + 1) / static_cast<double>(iters)));
     RemaskParams rp;
     rp.logp = c->logp; rp.gumbel = remask_noise; rp.mask_old = c->mask_cur(); rp.mask_new = c->mask_next(); rp.mask_raw = c->mask_raw; rp.forced_mask = forced_mask;
-    rp.T = L; rp.init_count = c->length; rp.ratio = static_cast<float>(ratio_d); rp.temp_ratio = static_cast<float>(static_cast<double>(temperature) * ratio_d);
-    rp.seed = seed; rp.seed_dev = nullptr; rp.step = static_cast<unsigned>(iter); rp.row0 = 0;
+    rp.lay = uniform_layout(1, L, L); rp.init_count = c->length; rp.ratio = static_cast<float>(ratio_d); rp.temp_ratio = static_cast<float>(static_cast<double>(temperature) * ratio_d);
+    rp.seed = seed; rp.seed_dev = nullptr; rp.step = static_cast<unsigned>(iter); rp.seq0 = 0;
     launch_pdl(remask_kernel, dim3(1), dim3(256), 0, st, rp);
     EDM_LAUNCH_CHECK("remask");
     up.next_mask = c->mask_next();

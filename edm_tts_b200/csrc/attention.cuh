@@ -1,8 +1,14 @@
 // Non-causal multi-head attention for the conformer block (reference: edm_tts/models/conformer/attend.py:63-115 via
 // conformer.py:128-146): softmax(q k^T / sqrt(64)) v, H heads of 64, no mask, one sequence = one batch element.
+// Sequences are placed by a SeqLayout (packed back to back, possibly of different lengths). qkv is read through a 2-D tensor map
+// over all rows: a key tile starts at the sequence's first row + 128 j, and the columns at or past the sequence's end (rows of the
+// next sequence, or TMA's zero fill after the last row) get -inf scores, so they add exact zeros to every sum; query rows past the
+// end are computed and not stored. Each query row is one lane with its own running max and rescale factor, so a row's result
+// does not depend on its neighbours.
 //
 // Persistent CTAs (one per SM) loop over work items; one item = 256 query rows (two 128-row tiles, "ping" and "pong")
-// of one (batch, head). The TMA producer runs one item ahead (Q is double-buffered, the K/V ring is continuous across
+// of one (sequence, head). A packed layout lists its (sequence, query pair) items longest sequence first (built at bind), so the
+// static round-robin hands out the long items first. The TMA producer runs one item ahead (Q is double-buffered, the K/V ring is continuous across
 // items), so the next item's first scores are issued while the current item's last tile is in its exp2 phase. Both contractions run on
 // tcgen05 with fp32 accumulators in TMEM (all 512 columns: S0 | S1 | O0 | O1):
 //   S_w = Q_w K^T : A = Q_w [128 x 64] K-major smem,  B = K tile [128 x 64] K-major smem        -> 128 TMEM columns
@@ -28,11 +34,15 @@
 //                       (setmaxnreg 88 / 208): a 128-wide fp32 score row per thread does not fit in 168 registers.
 #pragma once
 #include "ptx.cuh"
+#include "seq_layout.cuh"
 
 namespace edm {
 
 struct AttnParams {
-  int B, N, H;            // sequences, tokens per sequence, heads (head dim fixed at 64)
+  SeqLayout lay;          // where the sequences are
+  int H;                  // heads (head dim fixed at 64)
+  const int* pairs;       // packed layout: [n_pairs] (sequence << 16 | 256-row query pair), longest sequence first; nullptr: uniform
+  int n_items;            // work items = query pairs x heads
   int q_col0, k_col0, v_col0;  // first column of q / k / v inside the fused projection buffer
   __nv_bfloat16* out;     // [B*N, H*64]
   long long ldo;
@@ -74,6 +84,21 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
+// work item -> (sequence, query-tile pair, head)
+__device__ __forceinline__ void attn_item(const AttnParams& p, int it, int& b, int& qt2, int& h) {
+  if (p.pairs != nullptr) {
+    const int pr = __ldg(p.pairs + it / p.H);
+    b = pr >> 16;
+    qt2 = pr & 0xffff;
+    h = it % p.H;
+  } else {
+    const int n_q2 = (p.lay.N + 255) / 256;
+    qt2 = it % n_q2;
+    h = (it / n_q2) % p.H;
+    b = it / (n_q2 * p.H);
+  }
+}
+
 __global__ void __launch_bounds__(kAttnThreads, 1)
 attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -94,12 +119,19 @@ attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnPara
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const int n_kv = (p.N + 127) / 128;
-  const int n_q2 = (p.N + 255) / 256;
-  const int total_items = n_q2 * p.H * p.B;
-  // persistent: this CTA handles work items blockIdx.x, blockIdx.x + gridDim.x, ... ; item -> (query-tile pair, head, batch)
+  const int total_items = p.n_items;
+  // persistent: this CTA handles work items blockIdx.x, blockIdx.x + gridDim.x, ... ; item -> (query-tile pair, head, sequence).
+  // The kv iterations of this CTA are numbered g = 0, 1, ... across its items (n_kv of them per item, set by the item's sequence);
+  // ring stages and barrier phases follow g.
   const int my_items = (total_items - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
-  const int total_g = my_items * n_kv;  // kv iterations of this CTA, numbered g = item_index * n_kv + j
+  auto item_of = [&](int i) {
+    return p.reverse ? total_items - 1 - (static_cast<int>(blockIdx.x) + i * static_cast<int>(gridDim.x)) : static_cast<int>(blockIdx.x) + i * static_cast<int>(gridDim.x);
+  };
+  auto item_nkv = [&](int i) {
+    int b, qt2, h;
+    attn_item(p, item_of(i), b, qt2, h);
+    return (p.lay.n_len(b) + 127) >> 7;
+  };
 
   if (threadIdx.x == 0) {
     if ((smem_u32(smem) & 1023u) != 0) {
@@ -138,31 +170,34 @@ attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnPara
     asm volatile("setmaxnreg.dec.sync.aligned.u32 88;");
     if (warp == 8) {
       if (lane == 0) {
+        int g = 0;
         for (int i = 0; i < my_items; ++i) {
-          const int it = p.reverse ? total_items - 1 - (static_cast<int>(blockIdx.x) + i * static_cast<int>(gridDim.x)) : blockIdx.x + i * gridDim.x;
-          const int qt2 = it % n_q2, h = (it / n_q2) % p.H, b = it / (n_q2 * p.H);
+          int b, qt2, h;
+          attn_item(p, item_of(i), b, qt2, h);
+          const int row0 = p.lay.n_start(b), n_kv = (p.lay.n_len(b) + 127) >> 7;
           const int qs = i & 1;
           mbar_wait(&q_empty[qs], ((i >> 1) & 1) ^ 1);
           mbar_arrive_expect_tx(&q_full[qs], 2 * kAttnTile);
-          tma_load_3d(&tma_qkv, &q_full[qs], sQ + qs * 2 * kAttnTile, p.q_col0 + h * 64, qt2 * 256, b);
-          tma_load_3d(&tma_qkv, &q_full[qs], sQ + qs * 2 * kAttnTile + kAttnTile, p.q_col0 + h * 64, qt2 * 256 + 128, b);
-          for (int j = 0; j < n_kv; ++j) {
-            const int g = i * n_kv + j;
+          tma_load_2d(&tma_qkv, &q_full[qs], sQ + qs * 2 * kAttnTile, p.q_col0 + h * 64, row0 + qt2 * 256);
+          tma_load_2d(&tma_qkv, &q_full[qs], sQ + qs * 2 * kAttnTile + kAttnTile, p.q_col0 + h * 64, row0 + qt2 * 256 + 128);
+          for (int j = 0; j < n_kv; ++j, ++g) {
             const int s = g % kAttnKvStages;
             mbar_wait(&kv_empty[s], ((g / kAttnKvStages) & 1) ^ 1);
             mbar_arrive_expect_tx(&kv_full[s], 2 * kAttnTile);
-            tma_load_3d(&tma_qkv, &kv_full[s], sK + s * kAttnTile, p.k_col0 + h * 64, j * 128, b);
-            tma_load_3d(&tma_qkv, &kv_full[s], sV + s * kAttnTile, p.v_col0 + h * 64, j * 128, b);
+            tma_load_2d(&tma_qkv, &kv_full[s], sK + s * kAttnTile, p.k_col0 + h * 64, row0 + j * 128);
+            tma_load_2d(&tma_qkv, &kv_full[s], sV + s * kAttnTile, p.v_col0 + h * 64, row0 + j * 128);
           }
         }
       }
     } else if (warp == 9) {
+      int total_g = 0;
+      for (int i = 0; i < my_items; ++i) total_g += item_nkv(i);
       if (total_g > 0) {  // whole warp, warp-uniform control flow; one elected lane issues (umma_*_warp)
         constexpr uint32_t idesc_s = umma_idesc_bf16(128, 128, 0, 0);
         constexpr uint32_t idesc_o = umma_idesc_bf16(128, 64, 0, 1);  // B (= V) is MN-major
         // scores of kv iteration g for tile w (both tiles are issued back to back by the callers)
-        auto issue_s = [&](int w, int g) {
-          const int i = g / n_kv;
+        // scores of kv iteration g (of item i) for tile w
+        auto issue_s = [&](int w, int g, int i) {
           const uint64_t qdesc = umma_desc_sw128(smem_u32(sQ + (i & 1) * 2 * kAttnTile + w * kAttnTile), 16, 1024);
           const uint64_t kdesc = umma_desc_sw128(smem_u32(sK + (g % kAttnKvStages) * kAttnTile), 16, 1024);
 #pragma unroll
@@ -172,12 +207,11 @@ attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnPara
         // descriptor fields that do not change (layout, LBO / SBO) are built once; per tile only the 14-bit start address moves
         const uint64_t vdesc_fixed = umma_desc_sw128(0, p.v_lbo, p.v_sbo);
         const uint32_t v_kstep16 = p.v_kstep >> 4;
-        auto issue_pv = [&](int w, int g) {
+        auto issue_pv = [&](int w, int g, bool first) {  // first: the item's first kv tile overwrites O
           const uint32_t p_addr = smem_u32(sP + w * 2 * kAttnTile);
           const uint64_t pdesc0 = umma_desc_sw128(p_addr, 16, 1024);
           const uint64_t pdesc1 = pdesc0 + (kAttnTile >> 4);
           const uint64_t vdesc = vdesc_fixed + (smem_u32(sV + (g % kAttnKvStages) * kAttnTile) >> 4);
-          const bool first = (g % n_kv) == 0;  // first kv tile of an item overwrites O
 #pragma unroll
           for (int k = 0; k < 8; ++k) {
             const uint64_t adesc = (k < 4 ? pdesc0 : pdesc1) + 2 * (k & 3);
@@ -188,39 +222,48 @@ attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnPara
         mbar_wait_spin(&q_full[0], 0);
         mbar_wait_spin(&kv_full[0], 0);
         tc_fence_after();
-        issue_s(0, 0);
-        issue_s(1, 0);
+        // (item, kv tile, tiles of the item) of iteration g (P V) and of iteration g + 1 (scores)
+        int j = 0, n_kv = item_nkv(0), i1 = 0, j1 = 0, n_kv1 = n_kv;
+        issue_s(0, 0, 0);
+        issue_s(1, 0, 0);
         if (n_kv == 1) umma_commit_warp(&q_empty[0]);
         for (int g = 0; g < total_g; ++g) {
           if (g + 1 < total_g) {
             // next scores as soon as each warpgroup has drained S_w(g) into registers
             const int g1 = g + 1;
-            const int i1 = g1 / n_kv, j1 = g1 % n_kv;
+            if (++j1 == n_kv1) {
+              j1 = 0;
+              n_kv1 = item_nkv(++i1);
+            }
             if (j1 == 0) mbar_wait_spin(&q_full[i1 & 1], (i1 >> 1) & 1);
             mbar_wait_spin(&kv_full[g1 % kAttnKvStages], (g1 / kAttnKvStages) & 1);
             mbar_wait_spin(&s_free[0], g & 1);
             tc_fence_after();
             ATTN_TRACE(g1, 18);
-            issue_s(0, g1);
+            issue_s(0, g1, i1);
             ATTN_TRACE(g1, 8);
             mbar_wait_spin(&s_free[1], g & 1);
             tc_fence_after();
-            issue_s(1, g1);
+            issue_s(1, g1, i1);
             ATTN_TRACE(g1, 9);
-            if (j1 == n_kv - 1) umma_commit_warp(&q_empty[i1 & 1]);  // Q slot reusable once the item's last scores are done
+            if (j1 == n_kv1 - 1) umma_commit_warp(&q_empty[i1 & 1]);  // Q slot reusable once the item's last scores are done
           }
           // P_w(g) is in smem (and O_w rescaled if needed)
           mbar_wait_spin(&p_full[0], g & 1);
           tc_fence_after();
           ATTN_TRACE(g, 16);
-          issue_pv(0, g);
+          issue_pv(0, g, j == 0);
           ATTN_TRACE(g, 10);
           mbar_wait_spin(&p_full[1], g & 1);
           tc_fence_after();
           ATTN_TRACE(g, 17);
-          issue_pv(1, g);
+          issue_pv(1, g, j == 0);
           ATTN_TRACE(g, 11);
           umma_commit_warp(&kv_empty[g % kAttnKvStages]);  // K / V stage free once everything issued so far has completed
+          if (++j == n_kv) {  // iteration g + 1 opened the next item (the scores cursor is already there)
+            j = 0;
+            n_kv = n_kv1;
+          }
         }
       }
     }
@@ -237,14 +280,16 @@ attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnPara
     const int sw = row_in_tile & 7;
 
     if (w == 1) asm volatile("bar.arrive 2, 256;" ::: "memory");  // warpgroup 0 takes the first softmax phase
+    int g0 = 0;  // first kv iteration of the current item
     for (int i = 0; i < my_items; ++i) {
-      const int it = p.reverse ? total_items - 1 - (static_cast<int>(blockIdx.x) + i * static_cast<int>(gridDim.x)) : blockIdx.x + i * gridDim.x;
-      const int qt2 = it % n_q2, h = (it / n_q2) % p.H, b = it / (n_q2 * p.H);
+      int b, qt2, h;
+      attn_item(p, item_of(i), b, qt2, h);
+      const int row_b = p.lay.n_start(b), seq_n = p.lay.n_len(b), n_kv = (seq_n + 127) >> 7;
       float m_ref = -INFINITY;  // reference max in scaled log2 units
       float l_run = 0.f;
 
       for (int j = 0; j < n_kv; ++j) {
-        const int g = i * n_kv + j;
+        const int g = g0 + j;
         mbar_wait(&s_full[w], g & 1);
         tc_fence_after();
         if ((warp & 3) == 0 && lane == 0) ATTN_TRACE(g, 4 * w + 0);
@@ -260,8 +305,8 @@ attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnPara
         tc_fence_before();
         mbar_arrive(&s_free[w]);  // S_w may be overwritten by the next Q K^T
         if ((warp & 3) == 0 && lane == 0) ATTN_TRACE(g, 4 * w + 1);
-        const int kv_valid = p.N - j * 128;
-        if (kv_valid < 128) {  // only the last tile of a ragged sequence: padded key columns -> -inf
+        const int kv_valid = seq_n - j * 128;
+        if (kv_valid < 128) {  // only the last tile of a ragged sequence: key columns past its end -> -inf
 #pragma unroll
           for (int c = 0; c < 32; ++c) {
             if (c >= kv_valid) s0[c] = 0xff800000u;
@@ -349,16 +394,18 @@ attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnPara
         if ((warp & 3) == 3 && lane == 0) ATTN_TRACE(g, 22 + w);
       }
       // item epilogue: O_w / l
-      mbar_wait(&o_full[w], (i * n_kv + n_kv - 1) & 1);
+      const int g_last = g0 + n_kv - 1;
+      g0 += n_kv;
+      mbar_wait(&o_full[w], g_last & 1);
       tc_fence_after();
-      if ((warp & 3) == 0 && lane == 0) ATTN_TRACE(i * n_kv + n_kv - 1, 12 + 2 * w);
+      if ((warp & 3) == 0 && lane == 0) ATTN_TRACE(g_last, 12 + 2 * w);
       const float inv_l = 1.0f / l_run;
       uint32_t o0[32], o1[32];
       tmem_ld_32x32(tmem_O, o0);
       tmem_ld_32x32(tmem_O + 32, o1);
       tmem_ld_wait_dep(o0);
       tmem_ld_wait_dep(o1);
-      if ((warp & 3) == 0 && lane == 0) ATTN_TRACE(i * n_kv + n_kv - 1, 20 + w);
+      if ((warp & 3) == 0 && lane == 0) ATTN_TRACE(g_last, 20 + w);
       // Each thread holds one 128 B output row. Storing it directly costs 32 L1 wavefronts per STG (32 rows 2 KB apart per warp
       // instruction; measured 1.9 k cycles per item); instead the warp parks its 32 rows in its own slice of the (now idle) P_w
       // buffer and writes them back four full rows per instruction. Only this warp touches these smem rows: __syncwarp suffices.
@@ -380,17 +427,17 @@ attention_fwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const AttnPara
         const int r_sub = lane >> 3, ch = lane & 7;
         const int row0 = (warp & 3) * 32;                                    // this warp's first row in the tile
         const uint8_t* src = sP + w * 2 * kAttnTile;
-        __nv_bfloat16* dst = p.out + (static_cast<long long>(b) * p.N) * p.ldo + h * 64 + ch * 8;
+        __nv_bfloat16* dst = p.out + static_cast<long long>(row_b) * p.ldo + h * 64 + ch * 8;
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
           const int r = row0 + k * 4 + r_sub;
           const int qr = qt2 * 256 + w * 128 + r;
           const uint4 v = *reinterpret_cast<const uint4*>(src + r * 128 + ((ch ^ (r & 7)) * 16));
-          if (qr < p.N) *reinterpret_cast<uint4*>(dst + static_cast<long long>(qr) * p.ldo) = v;
+          if (qr < seq_n) *reinterpret_cast<uint4*>(dst + static_cast<long long>(qr) * p.ldo) = v;
         }
       }
       __syncwarp();   // the rows are overwritten by the next item's first P
-      if ((warp & 3) == 0 && lane == 0) ATTN_TRACE(i * n_kv + n_kv - 1, 13 + 2 * w);
+      if ((warp & 3) == 0 && lane == 0) ATTN_TRACE(g_last, 13 + 2 * w);
     }
   }
 

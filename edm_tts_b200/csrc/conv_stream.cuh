@@ -11,7 +11,8 @@
 //     (fma.rn.f32x2 and friends), which halves the FMA-pipe instruction count;
 //   * per-token statistics: every thread contributes one (sum, sum of squares) pair per token through shared memory, one warp
 //     per token reduces them; the Swish outputs themselves never leave registers.
-// in : [B*N, 2048] bf16 (GLU already applied by the pointwise-conv GEMM epilogue)     out : [B*N, 2048] bf16
+// in : [rows, 2048] bf16 (GLU already applied by the pointwise-conv GEMM epilogue)     out : [rows, 2048] bf16
+// Sequences are placed by a SeqLayout; a run never crosses the end of its sequence, so the zero padding is per sequence.
 #pragma once
 #include <type_traits>
 
@@ -32,9 +33,11 @@ struct ConvStreamParams {
   const float* dw_w;    // [2048, 5]
   const float* dw_b;    // [2048]
   const float* cln_w;   // [2048]
-  int B, N;
+  SeqLayout lay;
   int run_len;          // tokens per run
-  int runs_per_seq;
+  int runs_per_seq;     // uniform layout: runs of every sequence
+  const int* cu_runs;   // packed layout: [n_seq + 1] first run of each sequence (nullptr: uniform)
+  int num_units;        // runs in all
   int reverse;          // 1: the runs are walked from the last to the first
 };
 
@@ -63,16 +66,26 @@ __device__ __forceinline__ void cs_wait(uint32_t bar_addr, uint32_t parity) {
 }
 
 struct CsRun {
-  int b, t_begin, t_end, t_lo, t_hi;  // output tokens [t_begin, t_end), rows that exist in memory [t_lo, t_hi)
+  long long row0;                     // first row of the run's sequence
+  int t_begin, t_end, t_lo, t_hi;     // output tokens [t_begin, t_end), rows that exist in memory [t_lo, t_hi)
 };
 __device__ __forceinline__ CsRun cs_run(const ConvStreamParams& p, int unit) {
   CsRun r;
-  if (p.reverse) unit = p.B * p.runs_per_seq - 1 - unit;
-  r.b = unit / p.runs_per_seq;
-  r.t_begin = (unit % p.runs_per_seq) * p.run_len;
-  r.t_end = min(p.N, r.t_begin + p.run_len);
+  if (p.reverse) unit = p.num_units - 1 - unit;
+  int b, k;
+  if (p.cu_runs != nullptr) {
+    b = p.lay.search(p.cu_runs, unit);
+    k = unit - __ldg(p.cu_runs + b);
+  } else {
+    b = unit / p.runs_per_seq;
+    k = unit % p.runs_per_seq;
+  }
+  const int n = p.lay.n_len(b);
+  r.row0 = p.lay.n_start(b);
+  r.t_begin = k * p.run_len;
+  r.t_end = min(n, r.t_begin + p.run_len);
   r.t_lo = max(0, r.t_begin - 2);
-  r.t_hi = min(p.N, r.t_end + 2);
+  r.t_hi = min(n, r.t_end + 2);
   return r;
 }
 
@@ -85,7 +98,7 @@ __global__ void __launch_bounds__(kCsThreads, 1) conv_stream_kernel(const ConvSt
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int c0 = tid * 4;
-  const int num_units = p.B * p.runs_per_seq;
+  const int num_units = p.num_units;
 
   if (tid == 0) {
     for (int s = 0; s < kCsRing / kCsChunk; ++s) mbar_init(&s_bar[s], 1);
@@ -110,7 +123,7 @@ __global__ void __launch_bounds__(kCsThreads, 1) conv_stream_kernel(const ConvSt
       while (room > 0 && pu < num_units) {  // a chunk spans at most the tail of one run and the head of the next ones
         const int n = min(room, prun.t_hi - prun.t_lo - pr);
         asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(n * kCsRowBytes) : "memory");
-        bulk_load_row(s_ring + (q_issued % kCsRing) * kCsRowBytes, p.in + (static_cast<long long>(prun.b) * p.N + prun.t_lo + pr) * kConvC,
+        bulk_load_row(s_ring + (q_issued % kCsRing) * kCsRowBytes, p.in + (prun.row0 + prun.t_lo + pr) * kConvC,
                       n * kCsRowBytes, bar);
         q_issued += n;
         room -= n;
@@ -237,7 +250,7 @@ __global__ void __launch_bounds__(kCsThreads, 1) conv_stream_kernel(const ConvSt
       __syncthreads();
 
       // ---- phase 3: normalise from registers and store
-      __nv_bfloat16* orow = p.out + (static_cast<long long>(run.b) * p.N + tg) * kConvC + c0;
+      __nv_bfloat16* orow = p.out + (run.row0 + tg) * kConvC + c0;
 #pragma unroll
       for (int o = 0; o < kCsGroup; ++o) {
         if (kFull || tg + o < run.t_end) {

@@ -4,6 +4,7 @@
 // All rows are 1024 channels wide (hidden size); one warp owns one row, each lane 8 x 128-bit (fp32) accesses.
 #pragma once
 #include "ptx.cuh"
+#include "seq_layout.cuh"
 
 namespace edm {
 
@@ -127,7 +128,8 @@ struct LnParams {
   const float *w1, *b1, *w2, *b2;
   float* y_out;           // nullable
   __nv_bfloat16* z_out;   // nullable
-  int seq_len, z_skip;    // z row for input row (b*seq_len + n) is b*(seq_len - z_skip) + (n - z_skip); rows n < z_skip dropped
+  SeqLayout lay;          // compact != 0: the bf16 store keeps only target rows, encoder row of (s, P_s + t) -> target row of (s, t)
+  int compact;
   float eps;
   int reverse;            // 1: rows are walked from the last to the first (L2 reuse of the producer's most recent output)
   // layernorm_splitk_kernel only: the input row is the residual stream updated by a split-K GEMM whose K ranges left raw fp32 partial
@@ -168,10 +170,12 @@ __global__ void __launch_bounds__(256, 3) layernorm_kernel(const LnParams p) {
   if (p.y_out != nullptr) row_store_f32(p.y_out + static_cast<long long>(row) * kD, lane, v);
   if (p.z_out != nullptr) {
     long long zrow = row;
-    if (p.z_skip > 0) {
-      const int b = row / p.seq_len, n = row % p.seq_len;
-      if (n < p.z_skip) return;
-      zrow = static_cast<long long>(b) * (p.seq_len - p.z_skip) + (n - p.z_skip);
+    if (p.compact) {
+      int s, n;
+      p.lay.enc_pos(row, s, n);
+      const int np = p.lay.p_len(s);
+      if (n < np) return;
+      zrow = p.lay.t_start(s) + (n - np);
     }
     if (p.w2 != nullptr) row_layernorm(v, p.w2, p.b2, lane, p.eps);
     row_store_bf16(p.z_out + zrow * kD, lane, v);
@@ -232,10 +236,12 @@ __global__ void __launch_bounds__(256) layernorm_splitk_kernel(const LnParams p)
   if (p.y_out != nullptr) row_store_f32(p.y_out + static_cast<long long>(row) * kD, lane, v);
   if (p.z_out != nullptr) {
     long long zrow = row;
-    if (p.z_skip > 0) {
-      const int b = row / p.seq_len, n = row % p.seq_len;
-      if (n < p.z_skip) return;
-      zrow = static_cast<long long>(b) * (p.seq_len - p.z_skip) + (n - p.z_skip);
+    if (p.compact) {
+      int s, n;
+      p.lay.enc_pos(row, s, n);
+      const int np = p.lay.p_len(s);
+      if (n < np) return;
+      zrow = p.lay.t_start(s) + (n - np);
     }
     if (p.w2 != nullptr) row_layernorm(v, p.w2, p.b2, lane, p.eps);
     row_store_bf16(p.z_out + zrow * kD, lane, v);
@@ -258,7 +264,8 @@ struct ConvModParams {
   const float* dw_w;    // [2048, 5]
   const float* dw_b;    // [2048]
   const float* cln_w;   // [2048]
-  int B, N;
+  SeqLayout lay;        // rows of sequence s: [n_start(s), n_start(s) + n_len(s))
+  int max_n;            // longest sequence (grid size)
 };
 constexpr int kConvTT = 20;        // output tokens per CTA (4 halo rows are re-read: 20 % more loads, served by L2); 25 measured slower (wave quantisation)
 constexpr int kConvThreads = 512;  // 4 channels per thread at the S2A model's 2048 inner channels
@@ -283,8 +290,10 @@ __global__ void __launch_bounds__(kC / 4, 2) conv_module_kernel(const ConvModPar
   const int c0 = tid * 4;
   const int t0 = blockIdx.x * kConvTT;
   const int b = blockIdx.y;
+  const int seq_n = p.lay.n_len(b);
+  const long long row_b = p.lay.n_start(b);
   constexpr int kInW = kGlu ? 2 * kConvC : kConvC;  // input row width
-  const __nv_bfloat16* base = p.in + static_cast<long long>(b) * p.N * kInW + c0;
+  const __nv_bfloat16* base = p.in + row_b * kInW + c0;
 
   float wt[4][5], bias[4];
 #pragma unroll
@@ -301,6 +310,7 @@ __global__ void __launch_bounds__(kC / 4, 2) conv_module_kernel(const ConvModPar
     for (int c = 0; c < 4; ++c) win[j][c] = 0.f;
 
   pdl_sync();  // the depthwise weights above are constants; the rows below come from the previous kernel
+  if (t0 >= seq_n) return;  // tile past the end of a shorter sequence of a packed batch
 
   // two rows of loads in flight ahead of the arithmetic
   uint2 pa[2], pg[2] = {make_uint2(0, 0), make_uint2(0, 0)};
@@ -308,7 +318,7 @@ __global__ void __launch_bounds__(kC / 4, 2) conv_module_kernel(const ConvModPar
   for (int r = 0; r < 2; ++r) {
     const int t = t0 - 2 + r;
     pa[r] = make_uint2(0, 0);
-    if (t >= 0 && t < p.N) {
+    if (t >= 0 && t < seq_n) {
       pa[r] = *reinterpret_cast<const uint2*>(base + static_cast<long long>(t) * kInW);
       if constexpr (kGlu) pg[r] = *reinterpret_cast<const uint2*>(base + static_cast<long long>(t) * kInW + kConvC);
     }
@@ -320,7 +330,7 @@ __global__ void __launch_bounds__(kC / 4, 2) conv_module_kernel(const ConvModPar
     {
       const int tn = t0 + r;  // row r + 2
       pa[r & 1] = make_uint2(0, 0);
-      if (r + 2 < kConvTT + 4 && tn >= 0 && tn < p.N) {
+      if (r + 2 < kConvTT + 4 && tn >= 0 && tn < seq_n) {
         pa[r & 1] = *reinterpret_cast<const uint2*>(base + static_cast<long long>(tn) * kInW);
         if constexpr (kGlu) pg[r & 1] = *reinterpret_cast<const uint2*>(base + static_cast<long long>(tn) * kInW + kConvC);
       }
@@ -397,12 +407,12 @@ __global__ void __launch_bounds__(kC / 4, 2) conv_module_kernel(const ConvModPar
 #pragma unroll 4
   for (int o = 0; o < kConvTT; ++o) {
     const int t = t0 + o;
-    if (t >= p.N) break;
+    if (t >= seq_n) break;
     const uint32_t mean2 = s_mean2[o], rstd2 = s_rstd2[o];
     const uint2 k = s_keep[o * kConvThreads + tid];
     const uint32_t n0 = bf16x2_mul(bf16x2_sub(k.x, mean2), rstd2);
     const uint32_t n1 = bf16x2_mul(bf16x2_sub(k.y, mean2), rstd2);
-    *reinterpret_cast<uint2*>(p.out + (static_cast<long long>(b) * p.N + t) * kConvC + c0) =
+    *reinterpret_cast<uint2*>(p.out + (row_b + t) * kConvC + c0) =
         make_uint2(pack_bf16x2(bf16lo(n0) * cw[0], bf16hi(n0) * cw[1]), pack_bf16x2(bf16lo(n1) * cw[2], bf16hi(n1) * cw[3]));
   }
 }
@@ -412,17 +422,18 @@ __global__ void __launch_bounds__(kC / 4, 2) conv_module_kernel(const ConvModPar
 // semantic embedding + LayerNorm(Linear(level-0 DAC feature)), where Linear o codes_to_features collapses to a table
 // lookup (feat_table[code] = W_fp (W_out0 codebook0[code]) , feat_const = W_fp b_out0 + b_fp), exact algebra.
 struct BuildInputParams {
-  float* x;                        // [B, N, 1024]
-  const int* sem_tokens;           // [B, T]
-  const int* sem_prompt;           // [B, P] or nullptr
-  const int* ac_prompt;            // [B, Qp, P] (level 0 used here) or nullptr
+  float* x;                        // encoder rows [sum N_s, 1024]
+  const int* sem_tokens;           // target rows [sum T_s]
+  const int* sem_prompt;           // prompt rows [sum P_s] or nullptr
+  const int* ac_prompt;            // sequence s: [Qp, P_s] at Qp * p_start(s) (level 0 used here) or nullptr
   int ac_prompt_levels;            // Qp
   const float* sem_emb;            // [num_semantic, 1024]
   const float* mask_token;         // [1024]
   const float* feat_table;         // [1024 codes, 1024]
   const float* feat_const;         // [1024]
   const float *fp_ln_w, *fp_ln_b;  // acoustic_feat_proj.1
-  int B, T, P;
+  SeqLayout lay;
+  int rows;                        // sum N_s
   int num_semantic;                // rows of sem_emb
   float eps;
 };
@@ -430,22 +441,24 @@ struct BuildInputParams {
 __global__ void __launch_bounds__(256) build_input_kernel(const BuildInputParams p) {
   pdl_sync();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int N = p.P + p.T;
-  const long long row = static_cast<long long>(blockIdx.x) * 8 + warp;
-  if (row >= static_cast<long long>(p.B) * N) return;
-  const int b = static_cast<int>(row / N), n = static_cast<int>(row % N);
+  const int row = blockIdx.x * 8 + warp;
+  if (row >= p.rows) return;
+  int b, n;
+  p.lay.enc_pos(row, b, n);
+  const int np = p.lay.p_len(b);
   float v[32];
-  if (n < p.P) {
-    const int code = clamp_index(p.ac_prompt[(static_cast<long long>(b) * p.ac_prompt_levels + 0) * p.P + n], kV);
+  if (n < np) {
+    const long long pb = p.lay.p_start(b);
+    const int code = clamp_index(p.ac_prompt[static_cast<long long>(p.ac_prompt_levels) * pb + n], kV);  // level 0
     row_load_f32_ldg(p.feat_table + static_cast<long long>(code) * kD, lane, v);
     row_add_f32_ldg(p.feat_const, lane, v);
     row_layernorm(v, p.fp_ln_w, p.fp_ln_b, lane, p.eps);
-    row_add_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_prompt[static_cast<long long>(b) * p.P + n], p.num_semantic)) * kD, lane, v);
+    row_add_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_prompt[pb + n], p.num_semantic)) * kD, lane, v);
   } else {
-    row_load_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_tokens[static_cast<long long>(b) * p.T + (n - p.P)], p.num_semantic)) * kD, lane, v);
+    row_load_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_tokens[p.lay.t_start(b) + (n - np)], p.num_semantic)) * kD, lane, v);
     row_add_f32_ldg(p.mask_token, lane, v);
   }
-  row_store_f32(p.x + row * kD, lane, v);
+  row_store_f32(p.x + static_cast<long long>(row) * kD, lane, v);
 }
 
 // Per-step update of the target rows (modeling_injection_conformer.py:184-197, :214-218):
@@ -453,16 +466,17 @@ __global__ void __launch_bounds__(256) build_input_kernel(const BuildInputParams
 //   already unmasked earlier -> untouched.
 struct UpdateInputParams {
   float* x;
-  const int* sem_tokens;   // [B, T]
-  const int* ids;          // [B, T] sampled level-0 codes
-  const uint8_t* mask_old; // [B, T]
-  const uint8_t* mask_new; // [B, T] or nullptr (final step: nothing is re-masked)
+  const int* sem_tokens;   // target rows [sum T_s]
+  const int* ids;          // target rows: sampled level-0 codes
+  const uint8_t* mask_old; // target rows
+  const uint8_t* mask_new; // target rows or nullptr (final step: nothing is re-masked)
   const float* sem_emb;
   const float* mask_token;
   const float* feat_table;
   const float* feat_const;
   const float *fp_ln_w, *fp_ln_b;
-  int B, T, P;
+  SeqLayout lay;
+  int rows;                // sum T_s
   int num_semantic;
   float eps;
 };
@@ -470,9 +484,8 @@ struct UpdateInputParams {
 __global__ void __launch_bounds__(256) update_input_kernel(const UpdateInputParams p) {
   pdl_sync();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long r = static_cast<long long>(blockIdx.x) * 8 + warp;
-  if (r >= static_cast<long long>(p.B) * p.T) return;
-  const int b = static_cast<int>(r / p.T), t = static_cast<int>(r % p.T);
+  const int r = blockIdx.x * 8 + warp;
+  if (r >= p.rows) return;
   const bool was = p.mask_old[r] != 0;
   const bool now = p.mask_new != nullptr && p.mask_new[r] != 0;
   if (!was && !now) return;
@@ -485,7 +498,9 @@ __global__ void __launch_bounds__(256) update_input_kernel(const UpdateInputPara
     row_layernorm(v, p.fp_ln_w, p.fp_ln_b, lane, p.eps);
   }
   row_add_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_tokens[r], p.num_semantic)) * kD, lane, v);
-  row_store_f32(p.x + (static_cast<long long>(b) * (p.P + p.T) + p.P + t) * kD, lane, v);
+  int b, t;
+  p.lay.tgt_pos(r, b, t);
+  row_store_f32(p.x + p.lay.enc_row(b, t) * kD, lane, v);
 }
 
 // ------------------------------------------------------------------------------------------------ coarse injection
@@ -494,39 +509,41 @@ __global__ void __launch_bounds__(256) update_input_kernel(const UpdateInputPara
 //   x   = block_out + inj + (k > 0 ? previous coarse block_out : 0)
 // code_i comes from the arg-max of this pass for target rows and from the acoustic prompt for prompt rows.
 struct InjectParams {
-  float* x;                 // out: [B, N, 1024]
+  float* x;                 // out: encoder rows [sum N_s, 1024]
   const float* cur_out;     // block output at this injection layer (coarse_out[k])
   const float* prev_out;    // coarse_out[k-1] or nullptr
-  const int* pred_codes;    // [B, 4, T]
-  const int* ac_prompt;     // [B, Qp, P] or nullptr
+  const int* pred_codes;    // sequence s: [4, T_s] at 4 t_start(s)
+  const int* ac_prompt;     // sequence s: [Qp, P_s] at Qp p_start(s), or nullptr
   int ac_prompt_levels;
-  const float* prompt_proj; // [B, P, 1024] or nullptr: Linear_k(prompt feature) given by the caller (feature-valued injections)
+  const float* prompt_proj; // prompt rows [sum P_s, 1024] or nullptr: Linear_k(prompt feature) given by the caller (feature-valued injections)
   const float* tables[4];   // inj_table[k][i] : [1024 codes, 1024]
   const float* inj_const;   // [1024]
   const float *ln_w, *ln_b; // project_injection[k].1
   int level;                // k
-  int B, T, P;
+  SeqLayout lay;
+  int rows;                 // sum N_s
   float eps;
 };
 
 __global__ void __launch_bounds__(256) inject_kernel(const InjectParams p) {
   pdl_sync();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int N = p.P + p.T;
   const long long row = static_cast<long long>(blockIdx.x) * 8 + warp;
-  if (row >= static_cast<long long>(p.B) * N) return;
-  const int b = static_cast<int>(row / N), n = static_cast<int>(row % N);
+  if (row >= p.rows) return;
+  int b, n;
+  p.lay.enc_pos(static_cast<int>(row), b, n);
+  const int np = p.lay.p_len(b);
   float v[32];
-  if (n < p.P && p.prompt_proj != nullptr) {
-    row_load_f32_ldg(p.prompt_proj + (static_cast<long long>(b) * p.P + n) * kD, lane, v);
+  if (n < np && p.prompt_proj != nullptr) {
+    row_load_f32_ldg(p.prompt_proj + (p.lay.p_start(b) + static_cast<long long>(n)) * kD, lane, v);
   } else {
     row_load_f32_ldg(p.inj_const, lane, v);
     for (int i = 0; i <= p.level; ++i) {
       int code;
-      if (n < p.P)
-        code = p.ac_prompt[(static_cast<long long>(b) * p.ac_prompt_levels + i) * p.P + n];
+      if (n < np)
+        code = p.ac_prompt[static_cast<long long>(p.ac_prompt_levels) * p.lay.p_start(b) + static_cast<long long>(i) * np + n];
       else
-        code = p.pred_codes[(static_cast<long long>(b) * 4 + i) * p.T + (n - p.P)];
+        code = p.pred_codes[p.lay.out_offset(b, i, 4, n - np)];
       row_add_f32_ldg(p.tables[i] + static_cast<long long>(clamp_index(code, kV)) * kD, lane, v);
     }
   }
@@ -573,13 +590,15 @@ struct SampleParams {
   unsigned long long seed;
   const unsigned long long* seed_dev;  // when set, *seed_dev is added to seed (a captured CUDA graph draws fresh noise per replay)
   unsigned int step;
-  long long row0;           // global index of row 0 (keeps the Philox stream independent of batch chunking / sharding)
+  long long seq0;           // global index of sequence 0 (keeps the Philox stream independent of batch chunking / sharding)
   const int* forced_ids;    // teacher forcing (parity runs) or nullptr
   int* ids;                 // out (forced id when teacher forcing), element (row) lands at out_base(row)
   int* ids_raw;             // out, the model's own choice (nullable)
   float* logp;              // out [rows] or nullptr
-  // output index mapping: row r = (b, t, q) with r = (b*T + t)*Q + q  ->  ids[(b*out_q_stride + out_q0 + q)*T + t]
-  int T, Q, out_q_stride, out_q0;
+  // output index mapping: row r = (target row of (b, t)) * Q + q  ->  ids[lay.out_offset(b, out_q0 + q, out_q_stride, t)], i.e.
+  // (b*out_q_stride + out_q0 + q)*T + t for a uniform layout. Philox counter: lay.philox_row(seq0, b, t) * Q + q.
+  SeqLayout lay;
+  int Q, out_q_stride, out_q0;
 };
 
 __global__ void __launch_bounds__(256) sample_kernel(const SampleParams p) {
@@ -587,6 +606,9 @@ __global__ void __launch_bounds__(256) sample_kernel(const SampleParams p) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long row = static_cast<long long>(blockIdx.x) * 8 + warp;
   if (row >= p.rows) return;
+  int b, t;
+  p.lay.tgt_pos(static_cast<int>(row / p.Q), b, t);
+  const int q = static_cast<int>(row % p.Q);
   float v[32];
   row_load_f32(p.logits + row * p.ld, lane, v);
   float mx = -INFINITY;
@@ -614,10 +636,11 @@ __global__ void __launch_bounds__(256) sample_kernel(const SampleParams p) {
     }
   } else if (p.use_philox) {
     const unsigned long long seed = p.seed + (p.seed_dev != nullptr ? *p.seed_dev : 0ull);
+    const long long ctr = p.lay.philox_row(p.seq0, b, t) * p.Q + q;
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-      const uint4 bits = philox4x32_10(make_uint4(static_cast<uint32_t>(p.row0 + row), static_cast<uint32_t>(i * 32 + lane), p.step,
-                                                  static_cast<uint32_t>((p.row0 + row) >> 32)),
+      const uint4 bits = philox4x32_10(make_uint4(static_cast<uint32_t>(ctr), static_cast<uint32_t>(i * 32 + lane), p.step,
+                                                  static_cast<uint32_t>(ctr >> 32)),
                                        make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
       const uint32_t bb[4] = {bits.x, bits.y, bits.z, bits.w};
 #pragma unroll
@@ -653,10 +676,7 @@ __global__ void __launch_bounds__(256) sample_kernel(const SampleParams p) {
   // a row without any finite maximum (all NaN / all -inf) never updates best_idx: id 0, as torch.argmax gives for all -inf; ids index
   // the feature tables downstream, so they must stay inside [0, 1024)
   if (best_idx >= kV) best_idx = 0;
-  const long long bt = row / p.Q;
-  const int q = static_cast<int>(row % p.Q);
-  const int b = static_cast<int>(bt / p.T), t = static_cast<int>(bt % p.T);
-  const long long oidx = (static_cast<long long>(b) * p.out_q_stride + p.out_q0 + q) * p.T + t;
+  const long long oidx = p.lay.out_offset(b, p.out_q0 + q, p.out_q_stride, t);
   int id = best_idx;
   if (p.forced_ids != nullptr) id = min(max(p.forced_ids[oidx], 0), kV - 1);
   if (lane == 0) {
@@ -684,7 +704,8 @@ struct ArgmaxCombineParams {
   const int* forced_ids;
   int* ids;
   int* ids_raw;             // nullable
-  int T, Q, out_q_stride, out_q0;
+  SeqLayout lay;
+  int Q, out_q_stride, out_q0;
 };
 __global__ void __launch_bounds__(256) argmax_combine_kernel(const ArgmaxCombineParams p) {
   pdl_sync();
@@ -703,10 +724,10 @@ __global__ void __launch_bounds__(256) argmax_combine_kernel(const ArgmaxCombine
   }
   if (!(best == best)) idx = 0;      // NaN logits: no defined maximum; stay inside the tables
   idx = clamp_index(idx, kV);
-  const long long bt = row / p.Q;
+  int b, t;
+  p.lay.tgt_pos(static_cast<int>(row / p.Q), b, t);
   const int q = static_cast<int>(row % p.Q);
-  const int b = static_cast<int>(bt / p.T), t = static_cast<int>(bt % p.T);
-  const long long oidx = (static_cast<long long>(b) * p.out_q_stride + p.out_q0 + q) * p.T + t;
+  const long long oidx = p.lay.out_offset(b, p.out_q0 + q, p.out_q_stride, t);
   p.ids[oidx] = p.forced_ids != nullptr ? clamp_index(p.forced_ids[oidx], kV) : idx;
   if (p.ids_raw != nullptr) p.ids_raw[oidx] = idx;
 }
@@ -716,15 +737,16 @@ __global__ void __launch_bounds__(256) argmax_combine_kernel(const ArgmaxCombine
 //   mask_len = max(1, min(#masked - 1, floor(float32(T) * float32(ratio))))
 //   conf     = masked ? logp + float32(temperature * ratio) * gumbel : +inf
 //   cut      = sort(conf)[mask_len];  new_mask = conf < cut
-// One CTA per sequence; the k-th order statistic is found by rank counting in shared memory (T <= 4096).
+// One CTA per sequence over its T_s target rows (mask_len from T_s); the k-th order statistic is found by rank counting in shared
+// memory (T_s <= 4096). Every per-row buffer below is indexed by target row.
 struct RemaskParams {
-  const float* logp;        // [B, T]
-  const float* gumbel;      // [B, T] or nullptr (then Philox)
-  const uint8_t* mask_old;  // [B, T]
-  uint8_t* mask_new;        // [B, T]
-  uint8_t* mask_raw;        // [B, T] or nullptr: the kernel's own mask (before teacher forcing), for parity runs
+  const float* logp;
+  const float* gumbel;      // or nullptr (then Philox)
+  const uint8_t* mask_old;
+  uint8_t* mask_new;
+  uint8_t* mask_raw;        // or nullptr: the kernel's own mask (before teacher forcing), for parity runs
   const uint8_t* forced_mask;  // teacher forcing: copied to mask_new when given
-  int T;
+  SeqLayout lay;
   int init_count;    // 0: the S2A rule mask_len = max(1, min(#masked - 1, floor(T * ratio))) (modeling_injection_conformer.py:199-202);
                      // > 0: the text-to-semantic rule max(1, min(floor(init_count * ratio), init_count)) with init_count = number of
                      // speech positions (modeling_text_to_semantic.py:237-242)
@@ -733,7 +755,7 @@ struct RemaskParams {
   unsigned long long seed;
   const unsigned long long* seed_dev;  // see SampleParams
   unsigned int step;
-  long long row0;    // global index of element (0, 0)
+  long long seq0;    // global index of sequence 0 (Philox counter lay.philox_row(seq0, s, t))
 };
 constexpr int kRemaskMaxT = 4096;
 
@@ -743,7 +765,8 @@ __global__ void __launch_bounds__(256) remask_kernel(const RemaskParams p) {
   __shared__ int s_count;
   __shared__ float s_cut;
   const int b = blockIdx.x, tid = threadIdx.x;
-  const long long base = static_cast<long long>(b) * p.T;
+  const long long base = p.lay.t_start(b);
+  const int T = p.lay.t_len(b);
   if (tid == 0) {
     s_count = 0;
     s_cut = INFINITY;  // stays when mask_len >= T (the reference's take_along_dim raises there; the host rejects T < 2 with steps > 1)
@@ -751,7 +774,7 @@ __global__ void __launch_bounds__(256) remask_kernel(const RemaskParams p) {
   __syncthreads();
   const unsigned long long seed = p.seed + (p.seed_dev != nullptr ? *p.seed_dev : 0ull);
   int local = 0;
-  for (int t = tid; t < p.T; t += 256) {
+  for (int t = tid; t < T; t += 256) {
     const bool m = p.mask_old[base + t] != 0;
     float c = INFINITY;
     if (m) {
@@ -759,7 +782,8 @@ __global__ void __launch_bounds__(256) remask_kernel(const RemaskParams p) {
       if (p.gumbel != nullptr) {
         g = p.gumbel[base + t];
       } else {
-        const uint4 bits = philox4x32_10(make_uint4(static_cast<uint32_t>(p.row0 + base + t), 0x52454d41u, p.step, static_cast<uint32_t>((p.row0 + base + t) >> 32)),
+        const long long ctr = p.lay.philox_row(p.seq0, b, t);
+        const uint4 bits = philox4x32_10(make_uint4(static_cast<uint32_t>(ctr), 0x52454d41u, p.step, static_cast<uint32_t>(ctr >> 32)),
                                          make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
         g = gumbel_from_bits(bits.x);
       }
@@ -771,21 +795,21 @@ __global__ void __launch_bounds__(256) remask_kernel(const RemaskParams p) {
   atomicAdd(&s_count, local);
   __syncthreads();
   if (p.forced_mask != nullptr && p.mask_raw == nullptr) {
-    for (int t = tid; t < p.T; t += 256) p.mask_new[base + t] = p.forced_mask[base + t];
+    for (int t = tid; t < T; t += 256) p.mask_new[base + t] = p.forced_mask[base + t];
     return;
   }
   float ml;
   if (p.init_count > 0) {
     ml = fmaxf(1.0f, fminf(floorf(__fmul_rn(static_cast<float>(p.init_count), p.ratio)), static_cast<float>(p.init_count)));
   } else {
-    ml = floorf(__fmul_rn(static_cast<float>(p.T), p.ratio));
+    ml = floorf(__fmul_rn(static_cast<float>(T), p.ratio));
     ml = fmaxf(1.0f, fminf(static_cast<float>(s_count - 1), ml));
   }
   const int k = static_cast<int>(ml);
-  for (int t = tid; t < p.T; t += 256) {
+  for (int t = tid; t < T; t += 256) {
     const float c = conf[t];
     int less = 0, leq = 0;
-    for (int u = 0; u < p.T; ++u) {
+    for (int u = 0; u < T; ++u) {
       const float o = conf[u];
       less += (o < c);
       leq += (o <= c);
@@ -794,7 +818,7 @@ __global__ void __launch_bounds__(256) remask_kernel(const RemaskParams p) {
   }
   __syncthreads();
   const float cut = s_cut;
-  for (int t = tid; t < p.T; t += 256) {
+  for (int t = tid; t < T; t += 256) {
     const uint8_t own = conf[t] < cut ? 1 : 0;
     if (p.mask_raw != nullptr) p.mask_raw[base + t] = own;
     p.mask_new[base + t] = p.forced_mask != nullptr ? p.forced_mask[base + t] : own;

@@ -15,6 +15,7 @@
 // Linear/Conv outputs are rounded to bf16 before the activation / residual add, the residual stream stays fp32.
 #pragma once
 #include "ptx.cuh"
+#include "seq_layout.cuh"
 
 namespace edm {
 
@@ -48,13 +49,19 @@ struct GemmParams {
   const float* rope_sin;
   int reverse;    // 1: walk the output tiles from the last to the first (see edm_s2a_ctx::flip: each kernel of the decoder starts
                   // where its producer finished, so the most recently written ~100 MB of its input are still in L2)
-  int seq_len;    // rotary position = row % seq_len
+  SeqLayout rope_lay;  // rotary position of a row = its position inside its sequence
   int rope_cols;  // columns [0, rope_cols) get rotary (q and k parts of the fused QKV projection)
   // small-M kernel, EPI_F32 only: K is cut into `splits` equal ranges, one work item per (tile, range); range s writes its raw fp32
   // partial sums (no bias) to out + s * split_stride. The consumer adds them in range order (layernorm_kernel with LnParams::partials).
   int splits;
   long long split_stride;
 };
+
+__device__ __forceinline__ int rope_pos(const GemmParams& p, int row) {
+  int s, n;
+  p.rope_lay.enc_pos(row, s, n);
+  return n;
+}
 
 constexpr int kGemmBM = 128;
 constexpr int kGemmBN = 256;
@@ -161,7 +168,7 @@ __device__ __forceinline__ void gemm_epilogue_rope64(const GemmParams& p, int ro
     h2[i] = pack_bf16x2(__uint_as_float(hi[2 * i]), __uint_as_float(hi[2 * i + 1]));
   }
   if (col < p.rope_cols) {
-    const int pos = row % p.seq_len;
+    const int pos = rope_pos(p, row);
     const float4* c4 = reinterpret_cast<const float4*>(p.rope_cos + static_cast<long long>(pos) * 32);
     const float4* s4 = reinterpret_cast<const float4*>(p.rope_sin + static_cast<long long>(pos) * 32);
 #pragma unroll
@@ -335,8 +342,8 @@ gemm_bf16_tn_small_kernel(const __grid_constant__ CUtensorMap tma_a, const __gri
       float4 bias_v[16];
       if constexpr (EPI == EPI_QKV_ROPE) {
         if (col0 < p.rope_cols && row < p.M) {  // this row's cos | sin lines (constants): in L1 by the time the accumulator is ready
-          prefetch_l1(p.rope_cos + static_cast<long long>(row % p.seq_len) * 32);
-          prefetch_l1(p.rope_sin + static_cast<long long>(row % p.seq_len) * 32);
+          prefetch_l1(p.rope_cos + static_cast<long long>(rope_pos(p, row)) * 32);
+          prefetch_l1(p.rope_sin + static_cast<long long>(rope_pos(p, row)) * 32);
         }
       }
       if constexpr (EPI != EPI_QKV_ROPE) {
@@ -558,7 +565,7 @@ gemm_bf16_tn_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid
           for (int i = et; i < 128 * 16; i += 32 * kGemmEpiWarps) {
             const int r = i >> 4, c = i & 15;
             const int grow = m_blk * 2 * kGemmBM + static_cast<int>(rank) * kGemmBM + r;
-            const int pos = (grow < p.M ? grow : 0) % p.seq_len;
+            const int pos = rope_pos(p, grow < p.M ? grow : 0);
             const float* src = (c < 8 ? p.rope_cos : p.rope_sin) + static_cast<long long>(pos) * 32 + (c & 7) * 4;
             tab[r * 16 + (c ^ (r & 7))] = __ldg(reinterpret_cast<const float4*>(src));
           }

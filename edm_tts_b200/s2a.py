@@ -14,6 +14,7 @@ import os
 import torch
 
 from . import _lib as L
+from . import varlen
 from .config import InjectionConformerConfig
 from .weights import pack_rvq_weights, pack_s2a_weights
 
@@ -354,6 +355,25 @@ class InjectionConformerModel:
         L.check(lib.edm_s2a_bind(self._ctx, self._ws.data_ptr(), self._ws.numel(), B, T, P), "bind")
         self._bound = key
 
+    def _bind_varlen(self, T, P):
+        """Packed workspace for utterances of T[i] target / P[i] prompt frames (edm_s2a_bind_varlen); the arg-max stays in the head GEMMs."""
+        key = ("varlen", tuple(T), tuple(P))
+        if self._bound == key:
+            return
+        lib = L.lib()
+        L.check(lib.edm_s2a_set_keep_logits(self._ctx, 0), "set_keep_logits")
+        n = len(T)
+        t_arr, p_arr = (C.c_int * n)(*T), (C.c_int * n)(*P)
+        need = lib.edm_s2a_workspace_bytes_varlen(self._ctx, n, t_arr, p_arr)
+        if need == 0:
+            raise ValueError("invalid variable-length batch: " + lib.edm_last_error().decode("utf-8", "replace"))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = None
+            self._ws = torch.empty(need, device=self.device, dtype=torch.uint8)
+        self._bound = None
+        L.check(lib.edm_s2a_bind_varlen(self._ctx, self._ws.data_ptr(), self._ws.numel(), n, t_arr, p_arr, L.stream_ptr()), "bind_varlen")
+        self._bound = key
+
     def _view(self, name, shape, dtype):
         nbytes = C.c_size_t(0)
         p = L.lib().edm_s2a_buffer(self._ctx, name.encode(), C.byref(nbytes))
@@ -434,6 +454,91 @@ class InjectionConformerModel:
         return out
 
     generate = infer_special
+
+    @torch.no_grad()
+    @_on_device
+    def infer_batch(self, semantic_tokens, acoustic_prompt_tokens=None, semantic_prompt_tokens=None, steps=8, temperature=1.0, *,
+                    seed=0, batch_offset=0, cat_gumbel=None, remask_gumbel=None, forced_ids=None, forced_masks=None, forced_coarse=None):
+        """infer_special for utterances of different lengths, decoded together without padding.
+        semantic_tokens: list of LongTensor [T_i]; the prompts: None, or lists of acoustic [q, P_i] (one q for all; P_i may be 0) and
+        semantic [P_i] tokens. Returns a list of LongTensor [12, T_i], views of one packed output. Utterance i decodes to the bits of
+        infer_special(semantic_tokens[i][None], ..., batch_offset=batch_offset + i)[0] (outside low-latency mode). The keyword extras
+        are per-utterance lists shaped as infer_special's extras for one utterance: cat_gumbel[i] [S-1, T_i, codes], remask_gumbel[i]
+        [S-1, 1, T_i], forced_ids[i] [S, 1, T_i], forced_masks[i] [S-1, 1, T_i], forced_coarse[i] [1, 4, T_i]."""
+        dev, lib = self.device, L.lib()
+        if not isinstance(semantic_tokens, (list, tuple)) or len(semantic_tokens) == 0:
+            raise ValueError("semantic_tokens must be a non-empty list of [T_i] tensors")
+        n = len(semantic_tokens)
+        if any(not torch.is_tensor(t) or t.dim() != 1 for t in semantic_tokens):
+            raise ValueError("every semantic_tokens entry must be a 1-D tensor [T_i]")
+        T = [int(t.shape[0]) for t in semantic_tokens]
+        if min(T) < 1:
+            raise ValueError("every utterance needs at least one target frame")
+        if steps > 1 and min(T) < 2:
+            raise IndexError("re-masking needs at least 2 frames (the reference's take_along_dim is out of range for T = 1 with steps > 1)")
+        for t in semantic_tokens:
+            _check_range(t, self.config.num_semantic_tokens, "semantic_tokens")
+        has_prompt = acoustic_prompt_tokens is not None or semantic_prompt_tokens is not None
+        P = [0] * n
+        if has_prompt:
+            ap, sp = acoustic_prompt_tokens, semantic_prompt_tokens
+            if not isinstance(ap, (list, tuple)) or not isinstance(sp, (list, tuple)) or len(ap) != n or len(sp) != n:
+                raise ValueError("acoustic_prompt_tokens and semantic_prompt_tokens must both be lists with one entry per utterance")
+            if any(not torch.is_tensor(a) or a.dim() != 2 for a in ap) or any(not torch.is_tensor(x) or x.dim() != 1 for x in sp):
+                raise ValueError("prompt tokens must be acoustic [q, p_i] and semantic [p_i] tensors")
+            q = int(ap[0].shape[0])
+            if any(int(a.shape[0]) != q for a in ap):
+                raise ValueError("every acoustic prompt must have the same number of levels q")
+            if any(a.shape[1] != x.shape[0] for a, x in zip(ap, sp)):
+                raise ValueError("acoustic and semantic prompts of an utterance must have the same length")
+            if q < len(self.injection_layers):
+                raise IndexError("acoustic prompt needs at least one level per injection layer")  # reference: list index out of range
+            for a, x in zip(ap, sp):
+                _check_range(a, self.num_codevectors, "acoustic_prompt_tokens")
+                _check_range(x, self.config.num_semantic_tokens, "semantic_prompt_tokens")
+            P = [int(x.shape[0]) for x in sp]
+        S = int(steps)
+        V = self.num_codevectors
+        extras = dict(cat_gumbel=(cat_gumbel, lambda t: (S - 1, t, V)), remask_gumbel=(remask_gumbel, lambda t: (S - 1, 1, t)),
+                      forced_ids=(forced_ids, lambda t: (S, 1, t)), forced_masks=(forced_masks, lambda t: (S - 1, 1, t)),
+                      forced_coarse=(forced_coarse, lambda t: (1, 4, t)))
+        for name, (lst, shape) in extras.items():
+            if lst is None:
+                continue
+            if not isinstance(lst, (list, tuple)) or len(lst) != n:
+                raise ValueError(f"{name} must be a list with one entry per utterance")
+            for i, x in enumerate(lst):
+                if tuple(x.shape) != shape(T[i]):
+                    raise ValueError(f"{name}[{i}] must be {shape(T[i])}, got {tuple(x.shape)}")
+        if forced_ids is not None:
+            for x in forced_ids:
+                _check_range(x, V, "forced_ids")
+        if forced_coarse is not None:
+            for x in forced_coarse:
+                _check_range(x, V, "forced_coarse")
+        Q = self.num_quantizers
+        out = torch.empty(Q * sum(T), device=dev, dtype=torch.int64)
+
+        def cat(lst, sl, dim, dtype):
+            return None if lst is None else torch.cat([x.to(dev) for x in lst[sl]], dim).to(dtype).contiguous()
+
+        for ch in varlen.plan(T, P, MAX_CHUNK, batch_offset):
+            sl = slice(ch.start, ch.stop)
+            self._bind_varlen(ch.T, ch.P)
+            sem = cat(semantic_tokens, sl, 0, torch.int32)
+            spc = cat(semantic_prompt_tokens, sl, 0, torch.int32) if has_prompt else None
+            apc = torch.cat([a.to(dev).reshape(-1) for a in acoustic_prompt_tokens[sl]]).to(torch.int32).contiguous() if has_prompt else None
+            cg = cat(cat_gumbel, sl, 1, torch.float32)
+            rg = cat(remask_gumbel, sl, 2, torch.float32)
+            fi = cat(forced_ids, sl, 2, torch.int32)
+            fm = cat(forced_masks, sl, 2, torch.uint8)
+            fc = None if forced_coarse is None else torch.cat([x.to(dev).reshape(-1) for x in forced_coarse[sl]]).to(torch.int32).contiguous()
+            codes = out[Q * ch.t0:Q * (ch.t0 + sum(ch.T))]
+            L.check(lib.edm_s2a_set_batch_offset(self._ctx, ch.batch_offset), "set_batch_offset")
+            L.check(lib.edm_s2a_decode(self._ctx, L.ptr(sem), L.ptr(spc), L.ptr(apc), int(acoustic_prompt_tokens[0].shape[0]) if has_prompt else 0,
+                                       S, float(temperature), int(seed), L.ptr(cg), L.ptr(rg), L.ptr(fi), L.ptr(fm), L.ptr(fc), L.ptr(codes),
+                                       L.stream_ptr()), "decode")
+        return varlen.split_blocks(out, T, Q)
 
     @torch.no_grad()
     @_on_device

@@ -58,6 +58,11 @@ int edm_gemm_bf16(const void* a, long long lda, const void* b, long long ldb, in
  * Replaces Attend.flash_attn, attend.py:63-115 (non-causal, no mask, dropout 0). */
 int edm_attention(const void* qkv, int B, int N, int H, void* out, void* stream);
 
+/* edm_attention on a packed batch: n_seq sequences of different lengths back to back, sequence i = rows [cu_seqlens[i],
+ * cu_seqlens[i + 1]) of qkv [sum N_i, 3*H*64] and out [sum N_i, H*64]; cu_seqlens int32 [n_seq + 1] on the device, starting at 0.
+ * Each sequence attends only to itself. Reads the offsets back to size the launch (one synchronisation of `stream`). */
+int edm_attention_varlen(const void* qkv, int n_seq, const int* cu_seqlens, int H, void* out, void* stream);
+
 /* y = LN(in; w1,b1) [optional fp32 store], z = LN(y; w2,b2) or y [optional bf16 store, rows n < z_skip of every
  * seq_len-long sequence dropped]. 1024 channels. Replaces nn.LayerNorm at conformer.py:106,168,216 and wrapper :44. */
 int edm_layernorm(const void* in, int in_is_bf16, int rows, const float* w1, const float* b1, const float* w2,
@@ -78,6 +83,10 @@ int edm_gemm_resid_layernorm(const void* a, long long lda, const void* b, long l
  * Replaces conformer.py:171-174 (GLU :59-66, DepthWiseConv1d :69-77, Swish :54-56, ChanLayerNorm :90-99). */
 int edm_conv_module(const void* in, int glu_input, void* out, const float* dw_w, const float* dw_b, const float* cln_w,
                     int B, int N, void* stream);
+/* edm_conv_module on a packed batch (sequences as in edm_attention_varlen, zero padding at both ends of each sequence, any length
+ * >= 1). Reads the offsets back to size the launch (one synchronisation of `stream`). */
+int edm_conv_module_varlen(const void* in, int glu_input, void* out, const float* dw_w, const float* dw_b, const float* cln_w,
+                           int n_seq, const int* cu_seqlens, void* stream);
 
 /* Per-row arg-max / Gumbel-max sampling over 1024 logits + log-softmax of the chosen id.
  * rows = B*T*Q; ids land at ids[(b*out_q_stride + out_q0 + q)*T + t]. noise: [rows,1024] Gumbel or NULL;
@@ -182,6 +191,19 @@ void edm_s2a_destroy(edm_s2a_ctx* ctx);
 size_t edm_s2a_workspace_bytes(const edm_s2a_ctx* ctx, int B, int T, int P);
 /* workspace must be 1024-byte aligned; shapes stay bound until the next bind */
 int edm_s2a_bind(edm_s2a_ctx* ctx, void* workspace, size_t bytes, int B, int T, int P);
+
+/* Variable-length batch: n_seq utterances, utterance i with P[i] >= 0 prompt frames and T[i] >= 1 target frames (host arrays;
+ * P may be NULL = no prompts), each within the limits of edm_s2a_bind (T[i] <= 4096, P[i] + T[i] <= max_positions). The utterances
+ * are packed back to back without padding; every later call takes and returns its buffers in that layout:
+ *   semantic tokens [sum T_i] (utterance i at cu_t[i] = T_0 + .. + T_{i-1}), semantic prompt [sum P_i] (at cu_p[i]),
+ *   acoustic prompt: utterance i is [q, P_i] at q * cu_p[i], forced_coarse: [4, T_i] at 4 * cu_t[i],
+ *   codes out: [12, T_i] at 12 * cu_t[i], per-step noise / forcing [step][sum T_i (x 1024)], workspace buffers by packed rows.
+ * With equal lengths this is byte for byte the layout of edm_s2a_bind. Row t of utterance i draws the Philox counter
+ * (batch_offset + i) * T_i + t, what a single-utterance call with batch offset batch_offset + i draws, so utterance i decodes to the
+ * same bits as edm_s2a_bind(1, T_i, P_i) with that offset (outside low-latency mode). Copies the layout arrays into the workspace
+ * on `stream`. edm_s2a_set_prompt_injections(non-NULL) is refused (EDM_ERR_STATE) under this bind. */
+size_t edm_s2a_workspace_bytes_varlen(const edm_s2a_ctx* ctx, int n_seq, const int* T, const int* P);
+int edm_s2a_bind_varlen(edm_s2a_ctx* ctx, void* workspace, size_t bytes, int n_seq, const int* T, const int* P, void* stream);
 
 /* named views into the bound workspace (for parity tests / the Python mirror): returns device pointer or NULL */
 void* edm_s2a_buffer(edm_s2a_ctx* ctx, const char* name, size_t* bytes);
