@@ -85,13 +85,20 @@ _SIGNATURES = {
     "edm_t2s_destroy": (None, [_vp]),
     "edm_t2s_workspace_bytes": (_sz, [_vp, _i]),
     "edm_t2s_bind": (_i, [_vp, _vp, _sz, _i]),
+    "edm_t2s_workspace_bytes_batch": (_sz, [_vp, _i, _i]),
+    "edm_t2s_bind_batch": (_i, [_vp, _vp, _sz, _i, _i]),
+    "edm_t2s_set_low_latency": (_i, [_vp, _i]),
+    "edm_t2s_set_batch_offset": (_i, [_vp, _ll]),
     "edm_t2s_buffer": (_vp, [_vp, C.c_char_p, C.POINTER(_sz)]),
     "edm_t2s_predict_length": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "edm_t2s_predict_length_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "edm_t2s_begin": (_i, [_vp, _vp, _i, _i, _vp]),
+    "edm_t2s_begin_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "edm_t2s_logits": (_i, [_vp, _vp, _vp]),
     "edm_t2s_step": (_i, [_vp, _i, _i, _f, _ull, _vp, _vp, _vp, _vp, _vp]),
     "edm_t2s_result": (_i, [_vp, _vp, _vp]),
     "edm_t2s_decode": (_i, [_vp, _vp, _i, _i, _i, _f, _ull, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "edm_t2s_decode_batch": (_i, [_vp, _i, _vp, _vp, _vp, _i, _f, _ull, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -685,6 +685,16 @@ struct StreamArray {
     if (p != nullptr) cudaFreeAsync(p, st);
   }
 };
+// Work items of the attention kernel on a packed layout, appended to `out`: (sequence << 16 | query pair) for every 256-row query
+// pair of every sequence, longest sequence first (ties in sequence order), so that the static round-robin hands out the long items
+// first. lens: rows per sequence.
+void append_attention_pairs(const std::vector<int>& lens, std::vector<int>* out) {
+  std::vector<int> order(lens.size());
+  for (size_t i = 0; i < lens.size(); ++i) order[i] = static_cast<int>(i);
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return lens[a] > lens[b]; });
+  for (int s : order)
+    for (int q2 = 0; q2 < (lens[s] + 255) / 256; ++q2) out->push_back((s << 16) | q2);
+}
 SeqLayout packed_layout(int n_seq, const int* cu_dev, const std::vector<int>& cu) {
   SeqLayout l;
   l.n_seq = n_seq; l.N = 0; l.T = 0; l.cu_n = cu_dev; l.cu_t = cu_dev; l.rows = cu[n_seq]; l.t_rows = cu[n_seq];
@@ -698,15 +708,13 @@ extern "C" int edm_attention_varlen(const void* qkv, int n_seq, const int* cu_se
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   std::vector<int> cu;
   if (int rc = read_offsets(cu_seqlens, n_seq, &cu, st)) return rc;
-  std::vector<int> order(n_seq), pairs;
+  std::vector<int> lens(n_seq), pairs;
   double flops = 0.0;
   for (int i = 0; i < n_seq; ++i) {
-    order[i] = i;
-    flops += 4.0 * H * static_cast<double>(cu[i + 1] - cu[i]) * (cu[i + 1] - cu[i]) * 64;
+    lens[i] = cu[i + 1] - cu[i];
+    flops += 4.0 * H * static_cast<double>(lens[i]) * lens[i] * 64;
   }
-  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return cu[a + 1] - cu[a] > cu[b + 1] - cu[b]; });
-  for (int s : order)
-    for (int q2 = 0; q2 < (cu[s + 1] - cu[s] + 255) / 256; ++q2) pairs.push_back((s << 16) | q2);
+  append_attention_pairs(lens, &pairs);
   CUtensorMap m;
   if (int rc = make_tmap_2d(&m, qkv, cu[n_seq], 3ull * H * 64, 3ull * H * 64, 128)) return rc;
   StreamArray dp(st);
@@ -759,7 +767,7 @@ extern "C" int edm_remask(const float* logp, const float* gumbel, const uint8_t*
   if (T > kRemaskMaxT) return fail(EDM_ERR_INVALID, "remask supports T <= %d", kRemaskMaxT);
   RemaskParams p;
   p.logp = logp; p.gumbel = gumbel; p.mask_old = mask_old; p.mask_new = mask_new; p.mask_raw = nullptr; p.forced_mask = forced_mask;
-  p.lay = uniform_layout(B, T, T); p.init_count = 0; p.ratio = ratio; p.temp_ratio = temp_ratio; p.seed = seed; p.seed_dev = nullptr; p.step = step; p.seq0 = 0;
+  p.lay = uniform_layout(B, T, T); p.init_count = 0; p.init_counts = nullptr; p.ratio = ratio; p.temp_ratio = temp_ratio; p.seed = seed; p.seed_dev = nullptr; p.step = step; p.seq0 = 0;
   launch_pdl(remask_kernel, dim3(B), dim3(256), 0, static_cast<cudaStream_t>(stream), p);
   EDM_LAUNCH_CHECK("remask");
   return 0;
@@ -1429,7 +1437,7 @@ extern "C" int edm_s2a_bind_varlen(edm_s2a_ctx* c, void* workspace, size_t bytes
   // host image of the layout arrays: cu_n | cu_t | cu_runs | pairs
   std::vector<int> lens(n_seq);
   std::vector<int>& h = c->host_layout;
-  h.assign(layout_ints, 0);
+  h.assign(3 * n1, 0);
   int max_n = 0, min_t = kRemaskMaxT;
   double flops = 0.0;
   for (int i = 0; i < n_seq; ++i) {
@@ -1443,13 +1451,7 @@ extern "C" int edm_s2a_bind_varlen(edm_s2a_ctx* c, void* workspace, size_t bytes
   }
   const int run_len = conv_run_len(n_seq, lens.data(), 0, num_sms());
   for (int i = 0; i < n_seq; ++i) h[2 * n1 + i + 1] = h[2 * n1 + i] + (lens[i] + run_len - 1) / run_len;
-  // attention items, longest sequence first (ties in sequence order), so the static round-robin hands out the long items first
-  std::vector<int> order(n_seq);
-  for (int i = 0; i < n_seq; ++i) order[i] = i;
-  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return lens[a] > lens[b]; });
-  size_t k = 3 * n1;
-  for (int s : order)
-    for (int q2 = 0; q2 < (lens[s] + 255) / 256; ++q2) h[k++] = (s << 16) | q2;
+  append_attention_pairs(lens, &h);
   EDM_CUDA(cudaMemcpyAsync(dev, h.data(), layout_ints * sizeof(int), cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream)));
   c->ws = static_cast<uint8_t*>(workspace); c->ws_bytes = bytes;
   c->B = n_seq; c->T = 0; c->P = 0; c->N = 0;
@@ -1593,7 +1595,7 @@ extern "C" int edm_s2a_step(edm_s2a_ctx* c, int step, int steps, float temperatu
     const double ratio_d = std::cos(M_PI / 2.0 * (static_cast<double>(step + 1) / static_cast<double>(steps)));
     RemaskParams rp;
     rp.logp = c->logp; rp.gumbel = remask_noise; rp.mask_old = m_old; rp.mask_new = c->mask_next(); rp.mask_raw = c->mask_raw; rp.forced_mask = forced_mask;
-    rp.lay = c->lay; rp.init_count = 0; rp.ratio = static_cast<float>(ratio_d); rp.temp_ratio = static_cast<float>(static_cast<double>(temperature) * ratio_d);
+    rp.lay = c->lay; rp.init_count = 0; rp.init_counts = nullptr; rp.ratio = static_cast<float>(ratio_d); rp.temp_ratio = static_cast<float>(static_cast<double>(temperature) * ratio_d);
     rp.seed = seed; rp.seed_dev = c->seed_dev; rp.step = static_cast<unsigned>(step); rp.seq0 = c->batch_offset;
     launch_pdl(remask_kernel, dim3(c->lay.n_seq), dim3(256), 0, st, rp);
     EDM_LAUNCH_CHECK("remask");
@@ -1734,8 +1736,8 @@ extern "C" int edm_s2a_decode(edm_s2a_ctx* c, const int* sem_tokens, const int* 
 
 // ================================================================================================ text-to-semantic context
 // TextToSemanticWLen.infer (edm_tts/models/text_to_semantic/modeling_text_to_semantic.py:184-267): length predictor + `pred_iters`
-// iterations of (embed -> conformer -> pred_transform -> pred_head -> sample -> re-mask) on ONE sequence (the reference's infer is
-// batch-1). Hidden sizes 128..1024 in steps of 128, heads of <= 64 dims: the fused QKV projection is packed with every head
+// iterations of (embed -> conformer -> pred_transform -> pred_head -> sample -> re-mask). The reference's infer decodes one sequence;
+// edm_t2s_begin does the same, edm_t2s_begin_batch decodes several of different lengths packed back to back (SeqLayout). Hidden sizes 128..1024 in steps of 128, heads of <= 64 dims: the fused QKV projection is packed with every head
 // zero-padded to 64 columns (first half of the rotary pair in columns [0, dh/2), second half in [32, 32 + dh/2)), so the GEMM's
 // rotary epilogue and the tcgen05 attention kernel of the S2A path run unchanged; only the softmax scale dh^-1/2 differs.
 #include "t2s.cuh"
@@ -1753,16 +1755,25 @@ struct edm_t2s_ctx {
   std::vector<BlockMaps> bmaps;
   WMap pt_map, head_map;
   int d = 0, ff = 0, C = 0, hp = 0, lp_hp = 0, hp_max = 0, total_tokens = 0;
-  // bound workspace
+  bool low_latency = true;     // edm_t2s_set_low_latency
+  long long batch_offset = 0;  // edm_t2s_set_batch_offset
+  // bound workspace: max_len rows (all sequences of a request together), at most max_seq sequences
   bool bound = false;
-  int max_len = 0;
-  float *x, *y, *logits, *logp, *raw_len, *part = nullptr;
+  int max_len = 0, max_seq = 0;
+  size_t layout_cap = 0;       // ints of layout_dev
+  float *x, *y, *logits, *logp, *raw_len, *part = nullptr;  // part: split-K partial sums, carved by edm_t2s_bind only
   __nv_bfloat16 *z, *h, *qkv, *att, *g, *zt;
-  int *ids, *ids_raw, *tokens, *input_ids, *text;
+  int *ids, *ids_raw, *tokens, *input_ids, *text, *layout_dev;
   uint8_t *full_mask, *mask_a, *mask_b, *mask_raw;
-  // current request
+  std::vector<int> host_layout;
+  // current pass (length predictor or decode): where its sequences are. A single sequence is a uniform layout without arrays.
+  T2sSeqs seqs;
+  const int* pairs = nullptr;  // attention items of a packed layout
+  int n_pairs = 0, max_n = 0, out_len = 0;
+  double sum_sq = 0.0;         // sum of L_s^2 (attention work)
+  const int* init_counts = nullptr;  // packed decode: length_s per sequence (re-masking)
+  float* part_use = nullptr;   // split-K partials of this pass, nullptr: the unsplit launches
   bool begun = false, mask_in_a = true;
-  int L = 0, n_text = 0, length = 0;
   CUtensorMap m_z, m_h, m_att, m_g, m_zt, m_qkv;
 
   const void* bw(int blk, int f) const { return w[static_cast<size_t>(blk) * F_BLOCK_COUNT + f]; }
@@ -1810,7 +1821,8 @@ int launch_ln_g(int d, const LnGParams& p, cudaStream_t st) {
 
 // Residual GEMM + the LayerNorm that follows it, text-to-semantic form (any hidden size 128 * NV): with `part` and a K that divides into
 // 2 / 4 ranges of >= 4 k-blocks on few enough tiles, split-K partial sums reduced by layernorm_g_splitk_kernel (see launch_gemm_resid_ln);
-// otherwise the two plain launches. One sequence per decode, so there is no batch-invariance to keep: the split is always taken.
+// otherwise the two plain launches. `part` is given only to a single-sequence pass in low-latency mode (the default): the split changes
+// the fp32 summation order, so a packed batch never splits and a row's bits do not depend on the batch it is decoded in.
 int launch_gemm_resid_ln_g(int d, const CUtensorMap& ma, const WMap& wm, const GemmParams& p, const LnGParams& ln, float* part, cudaStream_t st) {
   const int sms = num_sms();
   const int tiles = ((p.M + kGemmBM - 1) / kGemmBM) * (p.N / kSmBN), num_kb = p.K / kGemmBK;
@@ -1818,7 +1830,7 @@ int launch_gemm_resid_ln_g(int d, const CUtensorMap& ma, const WMap& wm, const G
   const bool small = p.N % kGemmBN != 0 || (gemm_small_m() && pair_tiles * 4 <= sms);
   int splits = 1;
   if (small && part != nullptr && p.K % kGemmBK == 0 && p.N == d && p.ldo == d && ln.in == p.out && ln.rows == p.M && p.a_k_offset == 0 &&
-      ln.gather == nullptr && ln.row0_override == nullptr && !ln.pre_gelu && p.K >= 768)
+      ln.gather == nullptr && ln.override_row == nullptr && !ln.pre_gelu && p.K >= 768)
     for (int s = 4; s >= 2 && splits == 1; s >>= 1)
       if (tiles * s <= sms && num_kb % s == 0 && num_kb / s >= 3) splits = s;
   if (splits == 1) {
@@ -1882,7 +1894,7 @@ int launch_conv_tiled(int C, const ConvModParams& p, cudaStream_t st) {
 
 LnGParams lng(const void* in, int rows, const float* w1, const float* b1, const float* w2, const float* b2, float* y, __nv_bfloat16* z) {
   LnGParams p;
-  p.in = in; p.in_is_bf16 = 0; p.gather = nullptr; p.gather_rows = 0; p.row0_override = nullptr; p.rows = rows;
+  p.in = in; p.in_is_bf16 = 0; p.gather = nullptr; p.gather_rows = 0; p.override_row = nullptr; p.rows = rows;
   p.w1 = w1; p.b1 = b1; p.w2 = w2; p.b2 = b2; p.y_out = y; p.z_out = z; p.eps = 1e-5f; p.pre_gelu = 0;
   return p;
 }
@@ -1899,54 +1911,113 @@ int t2s_maps(edm_t2s_ctx* c, int M, int hp) {
   return rc;
 }
 
-// One ConformerBlock (conformer/conformer.py:219-235) on M rows of one sequence. In: x (fp32 stream), z = LN_ff1(x). Out: `post` applied
-// to the block's sum (post_norm + the next block's pre-norm), or x = pre-post_norm sum when post == nullptr (the last block of a stack).
-int t2s_block_body(edm_t2s_ctx* c, int blk, int M, int H, int hp, const float* rope_cos, const float* rope_sin, const LnGParams* post, cudaStream_t st) {
+// One ConformerBlock (conformer/conformer.py:219-235) on the rows of the current pass (c->seqs.lay). In: x (fp32 stream), z = LN_ff1(x).
+// Out: `post` applied to the block's sum (post_norm + the next block's pre-norm), or x = pre-post_norm sum when post == nullptr (the
+// last block of a stack).
+int t2s_block_body(edm_t2s_ctx* c, int blk, int H, int hp, const float* rope_cos, const float* rope_sin, const LnGParams* post, cudaStream_t st) {
   const int d = c->d, ff = c->ff, C = c->C;
+  const SeqLayout& lay = c->seqs.lay;
+  const int M = lay.rows;
   const BlockMaps& bm = c->bmaps[blk];
   if (int rc = launch_gemm(EPI_SWISH_BF16, c->m_z, bm.ff1_w1, gp(M, ff, d, c->bwf(blk, F_FF1_B1), c->h, ff), st)) return rc;
   if (int rc = launch_gemm_resid_ln_g(d, c->m_h, bm.ff1_w2, gp(M, d, ff, c->bwf(blk, F_FF1_B2), c->x, d, 0.5f),
-                                      lng(c->x, M, c->bwf(blk, F_ATTN_LN_W), c->bwf(blk, F_ATTN_LN_B), nullptr, nullptr, nullptr, c->z), c->part, st)) return rc;
+                                      lng(c->x, M, c->bwf(blk, F_ATTN_LN_W), c->bwf(blk, F_ATTN_LN_B), nullptr, nullptr, nullptr, c->z), c->part_use, st)) return rc;
   {
     GemmParams p = gp(M, 3 * hp, d, nullptr, c->qkv, 3 * hp);
-    p.rope_cos = rope_cos; p.rope_sin = rope_sin; p.rope_lay = uniform_layout(1, M, M); p.rope_cols = 2 * hp;
+    p.rope_cos = rope_cos; p.rope_sin = rope_sin; p.rope_lay = lay; p.rope_cols = 2 * hp;
     if (int rc = launch_gemm(EPI_QKV_ROPE, c->m_z, bm.wqkv, p, st)) return rc;
   }
   const float scale = 1.0f / sqrtf(static_cast<float>(d / H));
-  if (int rc = launch_attention(c->m_qkv, uniform_layout(1, M, M), nullptr, 0, 4.0 * H * static_cast<double>(M) * M * 64, H, c->att, 1024, 1024, 2048,
-                                st, scale))
-    return rc;
+  if (int rc = launch_attention(c->m_qkv, lay, c->pairs, c->n_pairs, 4.0 * H * c->sum_sq * 64, H, c->att, 1024, 1024, 2048, st, scale)) return rc;
   if (int rc = launch_gemm_resid_ln_g(d, c->m_att, bm.wo, gp(M, d, hp, c->bwf(blk, F_BO), c->x, d, 1.0f),
-                                      lng(c->x, M, c->bwf(blk, F_CONV_LN_W), c->bwf(blk, F_CONV_LN_B), nullptr, nullptr, nullptr, c->z), c->part, st)) return rc;
+                                      lng(c->x, M, c->bwf(blk, F_CONV_LN_W), c->bwf(blk, F_CONV_LN_B), nullptr, nullptr, nullptr, c->z), c->part_use, st)) return rc;
   if (int rc = launch_gemm(EPI_GLU_BF16, c->m_z, bm.pw1, gp(M, 2 * C, d, c->bwf(blk, F_PW1_B), c->h, C), st)) return rc;
   {
     ConvModParams p;
-    p.in = c->h; p.out = c->g; p.dw_w = c->bwf(blk, F_DW_W); p.dw_b = c->bwf(blk, F_DW_B); p.cln_w = c->bwf(blk, F_CLN_W); p.lay = uniform_layout(1, M, M); p.max_n = M;
+    p.in = c->h; p.out = c->g; p.dw_w = c->bwf(blk, F_DW_W); p.dw_b = c->bwf(blk, F_DW_B); p.cln_w = c->bwf(blk, F_CLN_W); p.lay = lay; p.max_n = c->max_n;
     if (int rc = launch_conv_tiled(C, p, st)) return rc;
   }
   if (int rc = launch_gemm_resid_ln_g(d, c->m_g, bm.pw2, gp(M, d, C, c->bwf(blk, F_PW2_B), c->x, d, 1.0f),
-                                      lng(c->x, M, c->bwf(blk, F_FF2_LN_W), c->bwf(blk, F_FF2_LN_B), nullptr, nullptr, nullptr, c->z), c->part, st)) return rc;
+                                      lng(c->x, M, c->bwf(blk, F_FF2_LN_W), c->bwf(blk, F_FF2_LN_B), nullptr, nullptr, nullptr, c->z), c->part_use, st)) return rc;
   if (int rc = launch_gemm(EPI_SWISH_BF16, c->m_z, bm.ff2_w1, gp(M, ff, d, c->bwf(blk, F_FF2_B1), c->h, ff), st)) return rc;
   if (post == nullptr) return launch_gemm(EPI_RESID_F32, c->m_h, bm.ff2_w2, gp(M, d, ff, c->bwf(blk, F_FF2_B2), c->x, d, 0.5f), st);
-  return launch_gemm_resid_ln_g(d, c->m_h, bm.ff2_w2, gp(M, d, ff, c->bwf(blk, F_FF2_B2), c->x, d, 0.5f), *post, c->part, st);
+  return launch_gemm_resid_ln_g(d, c->m_h, bm.ff2_w2, gp(M, d, ff, c->bwf(blk, F_FF2_B2), c->x, d, 0.5f), *post, c->part_use, st);
 }
 
-// blocks [blk0, blk0 + n) on M rows; x / z prepared by the caller; after the last block x holds the pre-post_norm sum
-int t2s_stack(edm_t2s_ctx* c, int blk0, int n, int M, int H, int hp, const float* rope_cos, const float* rope_sin, cudaStream_t st) {
+// blocks [blk0, blk0 + n) on the rows of the current pass; x / z prepared by the caller; after the last block x holds the pre-post_norm sum
+int t2s_stack(edm_t2s_ctx* c, int blk0, int n, int H, int hp, const float* rope_cos, const float* rope_sin, cudaStream_t st) {
+  const int M = c->seqs.lay.rows;
   for (int i = 0; i < n; ++i) {
     const int blk = blk0 + i;
     if (i + 1 < n) {
       // post_norm of this block fused with the first pre-norm of the next one
       const LnGParams post = lng(c->x, M, c->bwf(blk, F_POST_LN_W), c->bwf(blk, F_POST_LN_B), c->bwf(blk + 1, F_FF1_LN_W), c->bwf(blk + 1, F_FF1_LN_B), c->x, c->z);
-      if (int rc = t2s_block_body(c, blk, M, H, hp, rope_cos, rope_sin, &post, st)) return rc;
+      if (int rc = t2s_block_body(c, blk, H, hp, rope_cos, rope_sin, &post, st)) return rc;
     } else {
-      if (int rc = t2s_block_body(c, blk, M, H, hp, rope_cos, rope_sin, nullptr, st)) return rc;
+      if (int rc = t2s_block_body(c, blk, H, hp, rope_cos, rope_sin, nullptr, st)) return rc;
     }
   }
   return 0;
 }
 
-size_t t2s_carve(edm_t2s_ctx* c, uint8_t* base, int max_len, bool assign) {
+// The current pass is one sequence of `rows` rows (text n_text, speech `length`): the uniform layout, split-K in low-latency mode.
+void t2s_pass_single(edm_t2s_ctx* c, int rows, int n_text, int length) {
+  c->seqs.lay = uniform_layout(1, rows, rows);
+  c->seqs.cu_text = nullptr; c->seqs.cu_len = nullptr; c->seqs.n_text = n_text; c->seqs.length = length;
+  c->pairs = nullptr; c->n_pairs = 0; c->max_n = rows; c->out_len = length;
+  c->sum_sq = static_cast<double>(rows) * rows;
+  c->init_counts = nullptr;
+  c->part_use = c->low_latency ? c->part : nullptr;
+}
+
+// The current pass is n_seq packed sequences: n_text[s] + 1 rows each for the length predictor (length == nullptr), n_text[s] +
+// length[s] + 4 for the decode. Checks the lengths against the bound capacity and the rotary tables, then uploads the layout arrays
+// with one copy on `st`:  cu_n [n_seq + 1] | cu_text [n_seq + 1] | cu_len [n_seq + 1] | length [n_seq] | attention pairs.
+int t2s_pass_batch(edm_t2s_ctx* c, int n_seq, const int* n_text, const int* length, cudaStream_t st) {
+  if (n_seq < 1 || n_seq > c->max_seq) return fail(EDM_ERR_INVALID, "%d sequences for a workspace bound for %d", n_seq, c->max_seq);
+  if (n_text == nullptr) return fail(EDM_ERR_INVALID, "per-sequence text lengths required");
+  const size_t n1 = static_cast<size_t>(n_seq) + 1;
+  std::vector<int>& h = c->host_layout;
+  h.assign(3 * n1 + n_seq, 0);
+  std::vector<int> rows(n_seq);
+  long long total = 0;
+  int max_n = 0;
+  double sum_sq = 0.0;
+  for (int s = 0; s < n_seq; ++s) {
+    const int len = length != nullptr ? length[s] : 0;
+    if (n_text[s] < 0 || (length != nullptr && len < 1)) return fail(EDM_ERR_INVALID, "sequence %d: n_text=%d length=%d", s, n_text[s], len);
+    const long long r = length != nullptr ? static_cast<long long>(n_text[s]) + len + 4 : static_cast<long long>(n_text[s]) + 1;
+    if (r > c->cfg.max_positions) return fail(EDM_ERR_INVALID, "sequence %d of %lld tokens exceeds max_positions=%d", s, r, c->cfg.max_positions);
+    total += r;
+    if (total > c->max_len) return fail(EDM_ERR_INVALID, "sequences of %lld+ rows exceed the bound workspace (%d rows)", total, c->max_len);
+    rows[s] = static_cast<int>(r);
+    h[s + 1] = h[s] + rows[s];
+    h[n1 + s + 1] = h[n1 + s] + n_text[s];
+    h[2 * n1 + s + 1] = h[2 * n1 + s] + len;
+    h[3 * n1 + s] = len;
+    max_n = std::max(max_n, rows[s]);
+    sum_sq += static_cast<double>(r) * r;
+  }
+  append_attention_pairs(rows, &h);
+  if (h.size() > c->layout_cap) return fail(EDM_ERR_INVALID, "layout of %zu ints exceeds the bound workspace (%zu)", h.size(), c->layout_cap);
+  int* dev = c->layout_dev;
+  EDM_CUDA(cudaMemcpyAsync(dev, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  SeqLayout& l = c->seqs.lay;
+  l.n_seq = n_seq; l.N = 0; l.T = 0; l.cu_n = dev; l.cu_t = dev; l.rows = static_cast<int>(total); l.t_rows = l.rows;
+  c->seqs.cu_text = dev + n1; c->seqs.cu_len = dev + 2 * n1; c->seqs.n_text = 0; c->seqs.length = 0;
+  c->pairs = dev + 3 * n1 + n_seq; c->n_pairs = static_cast<int>(h.size() - (3 * n1 + n_seq));
+  c->max_n = max_n; c->out_len = h[3 * n1 - 1]; c->sum_sq = sum_sq;
+  c->init_counts = dev + 3 * n1;
+  c->part_use = nullptr;
+  return 0;
+}
+
+// ints of the layout arrays of t2s_pass_batch for max_seq sequences of max_len rows in all: 3 (max_seq + 1) offsets, max_seq lengths
+// and at most max_len / 256 + max_seq attention pairs
+size_t t2s_layout_ints(int max_len, int max_seq) { return 4 * (static_cast<size_t>(max_seq) + 1) + static_cast<size_t>(max_len) / 256 + max_seq; }
+
+// max_len rows, max_seq sequences; with_part: the split-K partial sums of a single-sequence bind
+size_t t2s_carve(edm_t2s_ctx* c, uint8_t* base, int max_len, int max_seq, bool with_part, bool assign) {
   const size_t M = static_cast<size_t>(max_len);
   Carver k{base};
   float* x = k.take<float>(M * c->d);
@@ -1959,7 +2030,7 @@ size_t t2s_carve(edm_t2s_ctx* c, uint8_t* base, int max_len, bool assign) {
   __nv_bfloat16* zt = k.take<__nv_bfloat16>(M * c->d);
   float* logits = k.take<float>(M * 1024);
   float* logp = k.take<float>(M);
-  float* raw_len = k.take<float>(4);
+  float* raw_len = k.take<float>(std::max(4, max_seq));
   int* ids = k.take<int>(M);
   int* ids_raw = k.take<int>(M);
   int* tokens = k.take<int>(M);
@@ -1969,9 +2040,11 @@ size_t t2s_carve(edm_t2s_ctx* c, uint8_t* base, int max_len, bool assign) {
   uint8_t* mask_a = k.take<uint8_t>(M);
   uint8_t* mask_b = k.take<uint8_t>(M);
   uint8_t* mask_raw = k.take<uint8_t>(M);
-  float* part = k.take<float>(4 * M * c->d);   // K-range partial sums of the split-K residual GEMMs
+  float* part = with_part ? k.take<float>(4 * M * c->d) : nullptr;   // K-range partial sums of the split-K residual GEMMs
+  int* layout = k.take<int>(t2s_layout_ints(max_len, max_seq));
   if (assign) {
     c->part = part;
+    c->layout_dev = layout; c->layout_cap = t2s_layout_ints(max_len, max_seq);
     c->x = x; c->y = y; c->z = z; c->h = h; c->qkv = qkv; c->att = att; c->g = g; c->zt = zt; c->logits = logits; c->logp = logp; c->raw_len = raw_len;
     c->ids = ids; c->ids_raw = ids_raw; c->tokens = tokens; c->input_ids = input_ids; c->text = text;
     c->full_mask = full_mask; c->mask_a = mask_a; c->mask_b = mask_b; c->mask_raw = mask_raw;
@@ -2048,21 +2121,51 @@ extern "C" edm_t2s_ctx* edm_t2s_create(const edm_t2s_config* cfg, const void* co
 
 extern "C" void edm_t2s_destroy(edm_t2s_ctx* ctx) { delete ctx; }
 
+namespace {
+int t2s_bind(edm_t2s_ctx* c, void* workspace, size_t bytes, int max_len, int max_seq, bool with_part) {
+  if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return fail(EDM_ERR_INVALID, "workspace must be 1024-byte aligned");
+  const size_t need = t2s_carve(c, nullptr, max_len, max_seq, with_part, false);
+  if (bytes < need) return fail(EDM_ERR_INVALID, "workspace too small: %zu < %zu", bytes, need);
+  t2s_carve(c, static_cast<uint8_t*>(workspace), max_len, max_seq, with_part, true);
+  c->max_len = max_len;
+  c->max_seq = max_seq;
+  c->bound = true;
+  c->begun = false;
+  return 0;
+}
+}  // namespace
+
 extern "C" size_t edm_t2s_workspace_bytes(const edm_t2s_ctx* ctx, int max_len) {
   if (ctx == nullptr || max_len <= 0) return 0;
-  return t2s_carve(const_cast<edm_t2s_ctx*>(ctx), nullptr, max_len, false);
+  return t2s_carve(const_cast<edm_t2s_ctx*>(ctx), nullptr, max_len, 1, true, false);
 }
 
 extern "C" int edm_t2s_bind(edm_t2s_ctx* c, void* workspace, size_t bytes, int max_len) {
   if (c == nullptr || workspace == nullptr || max_len <= 0) return fail(EDM_ERR_INVALID, "bind arguments");
   if (max_len > c->cfg.max_positions) return fail(EDM_ERR_INVALID, "max_len=%d exceeds the rotary tables (%d)", max_len, c->cfg.max_positions);
-  if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return fail(EDM_ERR_INVALID, "workspace must be 1024-byte aligned");
-  const size_t need = t2s_carve(c, nullptr, max_len, false);
-  if (bytes < need) return fail(EDM_ERR_INVALID, "workspace too small: %zu < %zu", bytes, need);
-  t2s_carve(c, static_cast<uint8_t*>(workspace), max_len, true);
-  c->max_len = max_len;
-  c->bound = true;
-  c->begun = false;
+  return t2s_bind(c, workspace, bytes, max_len, 1, true);
+}
+
+extern "C" size_t edm_t2s_workspace_bytes_batch(const edm_t2s_ctx* ctx, int max_rows, int max_seq) {
+  if (ctx == nullptr || max_rows <= 0 || max_seq <= 0 || max_seq >= (1 << 15)) return 0;
+  return t2s_carve(const_cast<edm_t2s_ctx*>(ctx), nullptr, max_rows, max_seq, false, false);
+}
+
+extern "C" int edm_t2s_bind_batch(edm_t2s_ctx* c, void* workspace, size_t bytes, int max_rows, int max_seq) {
+  if (c == nullptr || workspace == nullptr || max_rows <= 0 || max_seq <= 0 || max_seq >= (1 << 15)) return fail(EDM_ERR_INVALID, "bind arguments");
+  if (max_rows > 0x7fffffff / 1024) return fail(EDM_ERR_INVALID, "max_rows=%d", max_rows);
+  return t2s_bind(c, workspace, bytes, max_rows, max_seq, false);
+}
+
+extern "C" int edm_t2s_set_low_latency(edm_t2s_ctx* c, int on) {
+  if (c == nullptr) return fail(EDM_ERR_INVALID, "null context");
+  c->low_latency = on != 0;
+  return 0;
+}
+
+extern "C" int edm_t2s_set_batch_offset(edm_t2s_ctx* c, long long batch_offset) {
+  if (c == nullptr || batch_offset < 0) return fail(EDM_ERR_INVALID, "batch offset");
+  c->batch_offset = batch_offset;
   return 0;
 }
 
@@ -2070,7 +2173,8 @@ extern "C" void* edm_t2s_buffer(edm_t2s_ctx* c, const char* name, size_t* bytes)
   if (c == nullptr || !c->bound || name == nullptr) return nullptr;
   const size_t M = c->max_len;
   struct { const char* n; void* p; size_t b; } tab[] = {
-      {"x", c->x, M * c->d * 4}, {"logits", c->logits, M * 1024 * 4}, {"logp", c->logp, M * 4}, {"raw_len", c->raw_len, 4},
+      {"x", c->x, M * c->d * 4}, {"logits", c->logits, M * 1024 * 4}, {"logp", c->logp, M * 4},
+      {"raw_len", c->raw_len, static_cast<size_t>(std::max(4, c->max_seq)) * 4},
       {"ids", c->ids, M * 4}, {"ids_raw", c->ids_raw, M * 4}, {"tokens", c->tokens, M * 4}, {"input_ids", c->input_ids, M * 4},
       {"full_mask", c->full_mask, M}, {"mask", c->mask_cur(), M}, {"mask_raw", c->mask_raw, M}};
   for (auto& e : tab)
@@ -2081,37 +2185,71 @@ extern "C" void* edm_t2s_buffer(edm_t2s_ctx* c, const char* name, size_t* bytes)
   return nullptr;
 }
 
-// :198-203: length predictor on [length_token, text embeddings]; raw_out[0] (device) = log of the predicted length. The caller reads it
-// back (the sequence length decides every later shape), applies exp / ceil as the reference does, and passes `length` to edm_t2s_begin.
-extern "C" int edm_t2s_predict_length(edm_t2s_ctx* c, const int* text_tokens, int n_text, float* raw_out, void* stream) {
-  if (c == nullptr || !c->bound) return fail(EDM_ERR_STATE, "context not bound");
-  if (n_text < 0 || n_text + 1 > c->max_len) return fail(EDM_ERR_INVALID, "text of %d tokens does not fit the bound workspace (%d rows)", n_text, c->max_len);
-  if (n_text > 0 && text_tokens == nullptr) return fail(EDM_ERR_INVALID, "text tokens required");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int M = n_text + 1;
+namespace {
+// length predictor on the current pass (c->seqs.lay: n_text_s + 1 rows per sequence) over the packed text tokens
+int t2s_length_predictor(edm_t2s_ctx* c, const int* text_tokens, float* raw_out, cudaStream_t st) {
   const edm_t2s_config& cfg = c->cfg;
-  // gather indices: row 0 is the length token (row0_override), rows 1.. the text embeddings
-  EDM_CUDA(cudaMemsetAsync(c->text, 0, sizeof(int), st));
-  if (n_text > 0) EDM_CUDA(cudaMemcpyAsync(c->text + 1, text_tokens, sizeof(int) * n_text, cudaMemcpyDeviceToDevice, st));
+  const SeqLayout& lay = c->seqs.lay;
+  const int M = lay.rows;
+  launch_pdl(t2s_lp_gather_kernel, dim3((M + 255) / 256), dim3(256), 0, st, c->seqs, text_tokens, c->text);
+  EDM_LAUNCH_CHECK("t2s_lp_gather");
   if (int rc = t2s_maps(c, M, c->lp_hp)) return rc;
   const int b0 = cfg.depth;
   LnGParams p = lng(c->gw(TG_EMB), M, nullptr, nullptr, c->bwf(b0, F_FF1_LN_W), c->bwf(b0, F_FF1_LN_B), c->x, c->z);
-  p.gather = c->text; p.gather_rows = c->total_tokens; p.row0_override = c->gwf(TG_LENGTH_TOKEN);
+  p.gather = c->text; p.gather_rows = c->total_tokens; p.override_row = c->gwf(TG_LENGTH_TOKEN);
   if (int rc = launch_ln_g(c->d, p, st)) return rc;
-  if (int rc = t2s_stack(c, b0, cfg.lp_depth, M, cfg.lp_heads, c->lp_hp, c->gwf(TG_LP_ROPE_COS), c->gwf(TG_LP_ROPE_SIN), st)) return rc;
+  if (int rc = t2s_stack(c, b0, cfg.lp_depth, cfg.lp_heads, c->lp_hp, c->gwf(TG_LP_ROPE_COS), c->gwf(TG_LP_ROPE_SIN), st)) return rc;
   const int last = b0 + cfg.lp_depth - 1;
   float* out = raw_out != nullptr ? raw_out : c->raw_len;
+  const dim3 grid(lay.n_seq);
+  const float *lw = c->bwf(last, F_POST_LN_W), *lb = c->bwf(last, F_POST_LN_B), *w = c->gwf(TG_LEN_W), *b = c->gwf(TG_LEN_B);
   switch (c->d) {
-    case 128: launch_pdl(t2s_length_head_kernel<1>, dim3(1), dim3(32), 0, st, c->x, c->bwf(last, F_POST_LN_W), c->bwf(last, F_POST_LN_B), c->gwf(TG_LEN_W), c->gwf(TG_LEN_B), 1e-5f, out); break;
-    case 256: launch_pdl(t2s_length_head_kernel<2>, dim3(1), dim3(32), 0, st, c->x, c->bwf(last, F_POST_LN_W), c->bwf(last, F_POST_LN_B), c->gwf(TG_LEN_W), c->gwf(TG_LEN_B), 1e-5f, out); break;
-    case 384: launch_pdl(t2s_length_head_kernel<3>, dim3(1), dim3(32), 0, st, c->x, c->bwf(last, F_POST_LN_W), c->bwf(last, F_POST_LN_B), c->gwf(TG_LEN_W), c->gwf(TG_LEN_B), 1e-5f, out); break;
-    case 512: launch_pdl(t2s_length_head_kernel<4>, dim3(1), dim3(32), 0, st, c->x, c->bwf(last, F_POST_LN_W), c->bwf(last, F_POST_LN_B), c->gwf(TG_LEN_W), c->gwf(TG_LEN_B), 1e-5f, out); break;
-    default: launch_pdl(t2s_length_head_kernel<8>, dim3(1), dim3(32), 0, st, c->x, c->bwf(last, F_POST_LN_W), c->bwf(last, F_POST_LN_B), c->gwf(TG_LEN_W), c->gwf(TG_LEN_B), 1e-5f, out); break;
+    case 128: launch_pdl(t2s_length_head_kernel<1>, grid, dim3(32), 0, st, c->x, lay.cu_n, lw, lb, w, b, 1e-5f, out); break;
+    case 256: launch_pdl(t2s_length_head_kernel<2>, grid, dim3(32), 0, st, c->x, lay.cu_n, lw, lb, w, b, 1e-5f, out); break;
+    case 384: launch_pdl(t2s_length_head_kernel<3>, grid, dim3(32), 0, st, c->x, lay.cu_n, lw, lb, w, b, 1e-5f, out); break;
+    case 512: launch_pdl(t2s_length_head_kernel<4>, grid, dim3(32), 0, st, c->x, lay.cu_n, lw, lb, w, b, 1e-5f, out); break;
+    default: launch_pdl(t2s_length_head_kernel<8>, grid, dim3(32), 0, st, c->x, lay.cu_n, lw, lb, w, b, 1e-5f, out); break;
   }
   EDM_LAUNCH_CHECK("t2s_length_head");
   c->begun = false;  // the activation buffers were reused
   return 0;
 }
+}  // namespace
+
+// :198-203: length predictor on [length_token, text embeddings]; raw_out[0] (device) = log of the predicted length. The caller reads it
+// back (the sequence length decides every later shape), applies exp / ceil as the reference does, and passes `length` to edm_t2s_begin.
+extern "C" int edm_t2s_predict_length(edm_t2s_ctx* c, const int* text_tokens, int n_text, float* raw_out, void* stream) {
+  if (c == nullptr || !c->bound) return fail(EDM_ERR_STATE, "context not bound");
+  if (n_text < 0 || n_text + 1 > c->max_len) return fail(EDM_ERR_INVALID, "text of %d tokens does not fit the bound workspace (%d rows)", n_text, c->max_len);
+  if (n_text + 1 > c->cfg.max_positions) return fail(EDM_ERR_INVALID, "text of %d tokens exceeds max_positions=%d", n_text, c->cfg.max_positions);
+  if (n_text > 0 && text_tokens == nullptr) return fail(EDM_ERR_INVALID, "text tokens required");
+  t2s_pass_single(c, n_text + 1, n_text, 0);
+  return t2s_length_predictor(c, text_tokens, raw_out, static_cast<cudaStream_t>(stream));
+}
+
+// the length predictor on n_seq texts packed back to back (n_text_host[s] tokens each) in one pass: raw_out[s] = log length of text s
+extern "C" int edm_t2s_predict_length_batch(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, float* raw_out, void* stream) {
+  if (c == nullptr || !c->bound) return fail(EDM_ERR_STATE, "context not bound");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (int rc = t2s_pass_batch(c, n_seq, n_text_host, nullptr, st)) return rc;
+  if (c->seqs.lay.rows > n_seq && text_tokens == nullptr) return fail(EDM_ERR_INVALID, "text tokens required");
+  return t2s_length_predictor(c, text_tokens, raw_out, st);
+}
+
+namespace {
+// token sequences and mask state of the current pass (:205-222); text: the packed text tokens in c->text
+int t2s_begin_pass(edm_t2s_ctx* c, cudaStream_t st) {
+  c->mask_in_a = true;
+  T2sBeginParams p;
+  p.seqs = c->seqs; p.text_tokens = c->text; p.tok_text = 1; p.tok_sep = 3; p.tok_speech = 2; p.tok_mask = 4;
+  p.input_ids = c->input_ids; p.tokens = c->tokens; p.full_mask = c->full_mask; p.mask = c->mask_a;
+  launch_pdl(t2s_begin_kernel, dim3((c->seqs.lay.rows + 255) / 256), dim3(256), 0, st, p);
+  EDM_LAUNCH_CHECK("t2s_begin");
+  if (int rc = t2s_maps(c, c->seqs.lay.rows, c->hp)) return rc;
+  c->begun = true;
+  return 0;
+}
+}  // namespace
 
 // :205-222: the token sequence of one request and its mask state
 extern "C" int edm_t2s_begin(edm_t2s_ctx* c, const int* text_tokens, int n_text, int length, void* stream) {
@@ -2119,34 +2257,43 @@ extern "C" int edm_t2s_begin(edm_t2s_ctx* c, const int* text_tokens, int n_text,
   if (n_text < 0 || length < 1) return fail(EDM_ERR_INVALID, "n_text=%d length=%d", n_text, length);
   const long long L = static_cast<long long>(n_text) + length + 4;
   if (L > c->max_len) return fail(EDM_ERR_INVALID, "sequence of %lld tokens exceeds the bound workspace (%d rows)", L, c->max_len);
+  if (L > c->cfg.max_positions) return fail(EDM_ERR_INVALID, "sequence of %lld tokens exceeds max_positions=%d", L, c->cfg.max_positions);
   if (n_text > 0 && text_tokens == nullptr) return fail(EDM_ERR_INVALID, "text tokens required");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (n_text > 0) EDM_CUDA(cudaMemcpyAsync(c->text, text_tokens, sizeof(int) * n_text, cudaMemcpyDeviceToDevice, st));
-  c->L = static_cast<int>(L); c->n_text = n_text; c->length = length; c->mask_in_a = true;
-  T2sBeginParams p;
-  p.text_tokens = c->text; p.n_text = n_text; p.length = length; p.tok_text = 1; p.tok_sep = 3; p.tok_speech = 2; p.tok_mask = 4;
-  p.input_ids = c->input_ids; p.tokens = c->tokens; p.full_mask = c->full_mask; p.mask = c->mask_a;
-  launch_pdl(t2s_begin_kernel, dim3((c->L + 255) / 256), dim3(256), 0, st, p);
-  EDM_LAUNCH_CHECK("t2s_begin");
-  if (int rc = t2s_maps(c, c->L, c->hp)) return rc;
-  c->begun = true;
-  return 0;
+  t2s_pass_single(c, static_cast<int>(L), n_text, length);
+  return t2s_begin_pass(c, st);
 }
 
-// embeddings_to_logits (:135-152, mask = None) -> buffer "logits" [L, 1024] fp32. x_in: fp32 [L, hidden] embeddings, or NULL to embed
-// the context's running tokens (input_embedding lookup fused into the first LayerNorm pass).
+// n_seq requests packed back to back: text s has n_text_host[s] tokens (packed in text_tokens), length_host[s] speech positions
+extern "C" int edm_t2s_begin_batch(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, void* stream) {
+  if (c == nullptr || !c->bound) return fail(EDM_ERR_STATE, "context not bound");
+  if (length_host == nullptr) return fail(EDM_ERR_INVALID, "per-sequence lengths required");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  c->begun = false;
+  if (int rc = t2s_pass_batch(c, n_seq, n_text_host, length_host, st)) return rc;
+  const int total_text = c->host_layout[2 * (static_cast<size_t>(n_seq) + 1) - 1];
+  if (total_text > 0) {
+    if (text_tokens == nullptr) return fail(EDM_ERR_INVALID, "text tokens required");
+    EDM_CUDA(cudaMemcpyAsync(c->text, text_tokens, sizeof(int) * total_text, cudaMemcpyDeviceToDevice, st));
+  }
+  return t2s_begin_pass(c, st);
+}
+
+// embeddings_to_logits (:135-152, mask = None) -> buffer "logits" [rows, 1024] fp32 over the rows of what was begun. x_in: fp32
+// [rows, hidden] embeddings, or NULL to embed the context's running tokens (input_embedding lookup fused into the first LayerNorm pass).
 extern "C" int edm_t2s_logits(edm_t2s_ctx* c, const float* x_in, void* stream) {
   if (c == nullptr || !c->bound || !c->begun) return fail(EDM_ERR_STATE, "no sequence: call edm_t2s_begin first");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const edm_t2s_config& cfg = c->cfg;
-  const int M = c->L, d = c->d;
+  const int M = c->seqs.lay.rows, d = c->d;
   LnGParams p = lng(x_in != nullptr ? static_cast<const void*>(x_in) : c->gw(TG_EMB), M, nullptr, nullptr, c->bwf(0, F_FF1_LN_W), c->bwf(0, F_FF1_LN_B), c->x, c->z);
   if (x_in == nullptr) {
     p.gather = c->tokens;
     p.gather_rows = c->total_tokens;
   }
   if (int rc = launch_ln_g(d, p, st)) return rc;
-  if (int rc = t2s_stack(c, 0, cfg.depth, M, cfg.heads, c->hp, c->gwf(TG_ROPE_COS), c->gwf(TG_ROPE_SIN), st)) return rc;
+  if (int rc = t2s_stack(c, 0, cfg.depth, cfg.heads, c->hp, c->gwf(TG_ROPE_COS), c->gwf(TG_ROPE_SIN), st)) return rc;
   const int last = cfg.depth - 1;
   // post_norm -> bf16 operand of pred_transform.0; Linear -> fp32; GELU + LayerNorm -> bf16 operand of pred_head -> fp32 logits
   if (int rc = launch_ln_g(d, lng(c->x, M, c->bwf(last, F_POST_LN_W), c->bwf(last, F_POST_LN_B), nullptr, nullptr, nullptr, c->zt), st)) return rc;
@@ -2160,54 +2307,55 @@ extern "C" int edm_t2s_logits(edm_t2s_ctx* c, const float* x_in, void* stream) {
 }
 
 // one iteration's decisions (:229-260) on the logits of edm_t2s_logits: sample / arg-max, confidence re-masking over the speech
-// positions, token update. Noise / forcing arrays are those of this iteration ([L, 1024], [L], [L], [L]) or NULL.
+// positions of every sequence, token update. Noise / forcing arrays are those of this iteration ([rows, 1024], [rows], [rows], [rows])
+// or NULL. Row t of sequence s draws the Philox counter (batch_offset + s) * L_s + t.
 extern "C" int edm_t2s_step(edm_t2s_ctx* c, int iter, int iters, float temperature, unsigned long long seed, const float* cat_noise,
                             const float* remask_noise, const int* forced_ids, const uint8_t* forced_mask, void* stream) {
   if (c == nullptr || !c->bound || !c->begun) return fail(EDM_ERR_STATE, "no sequence: call edm_t2s_begin first");
   if (iters < 1 || iter < 0 || iter >= iters) return fail(EDM_ERR_INVALID, "iteration %d of %d", iter, iters);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const bool last = iter == iters - 1;
-  const int L = c->L;
+  const SeqLayout& lay = c->seqs.lay;
+  const int rows = lay.rows;
   SampleParams sp;
-  sp.logits = c->logits; sp.ld = 1024; sp.rows = L; sp.noise = last ? nullptr : cat_noise; sp.use_philox = last ? 0 : 1; sp.seed = seed; sp.seed_dev = nullptr;
-  sp.step = static_cast<unsigned>(iter); sp.seq0 = 0; sp.forced_ids = forced_ids; sp.ids = c->ids; sp.ids_raw = c->ids_raw; sp.logp = last ? nullptr : c->logp;
-  sp.lay = uniform_layout(1, L, L); sp.Q = 1; sp.out_q_stride = 1; sp.out_q0 = 0;
+  sp.logits = c->logits; sp.ld = 1024; sp.rows = rows; sp.noise = last ? nullptr : cat_noise; sp.use_philox = last ? 0 : 1; sp.seed = seed; sp.seed_dev = nullptr;
+  sp.step = static_cast<unsigned>(iter); sp.seq0 = c->batch_offset; sp.forced_ids = forced_ids; sp.ids = c->ids; sp.ids_raw = c->ids_raw; sp.logp = last ? nullptr : c->logp;
+  sp.lay = lay; sp.Q = 1; sp.out_q_stride = 1; sp.out_q0 = 0;
   if (int rc = launch_sample(sp, st)) return rc;
   T2sUpdateParams up;
-  up.ids = c->ids; up.next_mask = nullptr; up.full_mask = c->full_mask; up.input_ids = c->input_ids; up.tokens = c->tokens; up.L = L;
+  up.ids = c->ids; up.next_mask = nullptr; up.full_mask = c->full_mask; up.input_ids = c->input_ids; up.tokens = c->tokens; up.rows = rows;
   up.offset = c->cfg.num_special + c->cfg.text_vocab; up.tok_mask = 4;
   if (!last) {
     const double ratio_d = std::cos(M_PI / 2.0 * (static_cast<double>(iter + 1) / static_cast<double>(iters)));
     RemaskParams rp;
     rp.logp = c->logp; rp.gumbel = remask_noise; rp.mask_old = c->mask_cur(); rp.mask_new = c->mask_next(); rp.mask_raw = c->mask_raw; rp.forced_mask = forced_mask;
-    rp.lay = uniform_layout(1, L, L); rp.init_count = c->length; rp.ratio = static_cast<float>(ratio_d); rp.temp_ratio = static_cast<float>(static_cast<double>(temperature) * ratio_d);
-    rp.seed = seed; rp.seed_dev = nullptr; rp.step = static_cast<unsigned>(iter); rp.seq0 = 0;
-    launch_pdl(remask_kernel, dim3(1), dim3(256), 0, st, rp);
+    rp.lay = lay; rp.init_count = c->seqs.length; rp.init_counts = c->init_counts;
+    rp.ratio = static_cast<float>(ratio_d); rp.temp_ratio = static_cast<float>(static_cast<double>(temperature) * ratio_d);
+    rp.seed = seed; rp.seed_dev = nullptr; rp.step = static_cast<unsigned>(iter); rp.seq0 = c->batch_offset;
+    launch_pdl(remask_kernel, dim3(lay.n_seq), dim3(256), 0, st, rp);
     EDM_LAUNCH_CHECK("remask");
     up.next_mask = c->mask_next();
   }
-  launch_pdl(t2s_update_kernel, dim3((L + 255) / 256), dim3(256), 0, st, up);
+  launch_pdl(t2s_update_kernel, dim3((rows + 255) / 256), dim3(256), 0, st, up);
   EDM_LAUNCH_CHECK("t2s_update");
   if (!last) c->mask_in_a = !c->mask_in_a;
   return 0;
 }
 
-// speech_pred_tokens (:267): int64 [length], semantic vocabulary
+// speech_pred_tokens (:267): int64, semantic vocabulary; [length] of the one sequence, or [sum length_s] packed for a batch
 extern "C" int edm_t2s_result(edm_t2s_ctx* c, long long* tokens_out, void* stream) {
   if (c == nullptr || !c->bound || !c->begun) return fail(EDM_ERR_STATE, "no sequence: call edm_t2s_begin first");
   if (tokens_out == nullptr) return fail(EDM_ERR_INVALID, "output required");
-  launch_pdl(t2s_gather_out_kernel, dim3((c->length + 255) / 256), dim3(256), 0, static_cast<cudaStream_t>(stream), c->tokens, c->n_text + 3, c->length, tokens_out);
+  launch_pdl(t2s_gather_out_kernel, dim3((c->out_len + 255) / 256), dim3(256), 0, static_cast<cudaStream_t>(stream), c->seqs, c->tokens, c->out_len, tokens_out);
   EDM_LAUNCH_CHECK("t2s_gather_out");
   return 0;
 }
 
-// whole infer loop for a known length. Noise / forcing arrays are laid out [iteration][...] over L = n_text + length + 4 positions.
-extern "C" int edm_t2s_decode(edm_t2s_ctx* c, const int* text_tokens, int n_text, int length, int pred_iters, float temperature,
-                              unsigned long long seed, const float* cat_noise, const float* remask_noise, const int* forced_ids,
-                              const uint8_t* forced_masks, long long* tokens_out, void* stream) {
-  if (pred_iters < 1) return fail(EDM_ERR_INVALID, "pred_iters must be >= 1");
-  if (int rc = edm_t2s_begin(c, text_tokens, n_text, length, stream)) return rc;
-  const size_t L = c->L;
+namespace {
+// pred_iters x (logits, step) + result on what was begun. Noise / forcing arrays are laid out [iteration][rows (x 1024)].
+int t2s_iterate(edm_t2s_ctx* c, int pred_iters, float temperature, unsigned long long seed, const float* cat_noise, const float* remask_noise,
+                const int* forced_ids, const uint8_t* forced_masks, long long* tokens_out, void* stream) {
+  const size_t L = c->seqs.lay.rows;
   for (int i = 0; i < pred_iters; ++i) {
     const bool last = i == pred_iters - 1;
     if (int rc = edm_t2s_logits(c, nullptr, stream)) return rc;
@@ -2217,4 +2365,24 @@ extern "C" int edm_t2s_decode(edm_t2s_ctx* c, const int* text_tokens, int n_text
       return rc;
   }
   return edm_t2s_result(c, tokens_out, stream);
+}
+}  // namespace
+
+// whole infer loop for a known length. Noise / forcing arrays are laid out [iteration][...] over L = n_text + length + 4 positions.
+extern "C" int edm_t2s_decode(edm_t2s_ctx* c, const int* text_tokens, int n_text, int length, int pred_iters, float temperature,
+                              unsigned long long seed, const float* cat_noise, const float* remask_noise, const int* forced_ids,
+                              const uint8_t* forced_masks, long long* tokens_out, void* stream) {
+  if (pred_iters < 1) return fail(EDM_ERR_INVALID, "pred_iters must be >= 1");
+  if (int rc = edm_t2s_begin(c, text_tokens, n_text, length, stream)) return rc;
+  return t2s_iterate(c, pred_iters, temperature, seed, cat_noise, remask_noise, forced_ids, forced_masks, tokens_out, stream);
+}
+
+// edm_t2s_decode for n_seq packed requests (edm_t2s_begin_batch); noise / forcing arrays [iteration][sum L_s (x 1024)], tokens_out
+// [sum length_s]
+extern "C" int edm_t2s_decode_batch(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, int pred_iters,
+                                    float temperature, unsigned long long seed, const float* cat_noise, const float* remask_noise,
+                                    const int* forced_ids, const uint8_t* forced_masks, long long* tokens_out, void* stream) {
+  if (pred_iters < 1) return fail(EDM_ERR_INVALID, "pred_iters must be >= 1");
+  if (int rc = edm_t2s_begin_batch(c, n_seq, text_tokens, n_text_host, length_host, stream)) return rc;
+  return t2s_iterate(c, pred_iters, temperature, seed, cat_noise, remask_noise, forced_ids, forced_masks, tokens_out, stream);
 }

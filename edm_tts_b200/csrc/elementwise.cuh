@@ -750,6 +750,7 @@ struct RemaskParams {
   int init_count;    // 0: the S2A rule mask_len = max(1, min(#masked - 1, floor(T * ratio))) (modeling_injection_conformer.py:199-202);
                      // > 0: the text-to-semantic rule max(1, min(floor(init_count * ratio), init_count)) with init_count = number of
                      // speech positions (modeling_text_to_semantic.py:237-242)
+  const int* init_counts;  // nullable: init_count of sequence s is init_counts[s] (a text-to-semantic batch)
   float ratio;       // float32(cos(pi/2 (t+1)/S))
   float temp_ratio;  // float32(temperature * ratio)
   unsigned long long seed;
@@ -799,8 +800,9 @@ __global__ void __launch_bounds__(256) remask_kernel(const RemaskParams p) {
     return;
   }
   float ml;
-  if (p.init_count > 0) {
-    ml = fmaxf(1.0f, fminf(floorf(__fmul_rn(static_cast<float>(p.init_count), p.ratio)), static_cast<float>(p.init_count)));
+  const int init_count = p.init_counts != nullptr ? __ldg(p.init_counts + b) : p.init_count;
+  if (init_count > 0) {
+    ml = fmaxf(1.0f, fminf(floorf(__fmul_rn(static_cast<float>(init_count), p.ratio)), static_cast<float>(init_count)));
   } else {
     ml = floorf(__fmul_rn(static_cast<float>(T), p.ratio));
     ml = fmaxf(1.0f, fminf(static_cast<float>(s_count - 1), ml));

@@ -2,6 +2,7 @@
 // that the S2A path does not already provide: LayerNorm for hidden sizes 384 / 512 (+ embedding gather on load, + GELU on load for
 // pred_transform), the length head, and the token update of one decode iteration. GEMMs, attention, the conv module, sampling and
 // re-masking are the S2A kernels (gemm.cuh small-M kernel, attention.cuh with 64-wide zero-padded heads, elementwise.cuh).
+// Every kernel here takes one sequence or a batch of sequences packed back to back (T2sSeqs).
 #pragma once
 #include "elementwise.cuh"
 
@@ -63,13 +64,14 @@ __device__ __forceinline__ void rowg_layernorm(float (&v)[4 * NV], const float* 
 }
 
 // y = LN1(f(in)) (LN1 skipped when w1 == nullptr); optional fp32 store of y; z = LN2(y) when w2 != nullptr else y; optional bf16 store.
-// in row r is in[gather ? clamp(gather[r]) : r]; f = GELU(tanh) when pre_gelu (pred_transform: Linear -> GELU -> LayerNorm, :56-58).
+// in row r is in[gather ? clamp(gather[r]) : r], or override_row when gather[r] < 0; f = GELU(tanh) when pre_gelu (pred_transform:
+// Linear -> GELU -> LayerNorm, :56-58).
 struct LnGParams {
   const void* in;
   int in_is_bf16;
   const int* gather;     // nullable: embedding lookup (nn.Embedding, :47) fused into the load
   int gather_rows;       // rows of the table
-  const float* row0_override;  // nullable: row 0 is read from here instead (the length token in front of the text, :199)
+  const float* override_row;  // nullable: rows whose gather index is negative are read from here (the length token in front of every text, :199)
   int rows;
   const float *w1, *b1, *w2, *b2;
   float* y_out;
@@ -94,10 +96,14 @@ __global__ void __launch_bounds__(256) layernorm_g_kernel(const LnGParams p) {
   const int row = blockIdx.x * 8 + warp;
   if (row >= p.rows) return;
   long long src = row;
-  if (p.gather != nullptr) src = clamp_index(p.gather[row], p.gather_rows);
+  int gi = 0;
+  if (p.gather != nullptr) {
+    gi = p.gather[row];
+    src = clamp_index(gi, p.gather_rows);
+  }
   float v[4 * NV];
-  if (p.row0_override != nullptr && row == 0)
-    rowg_load_f32<NV>(p.row0_override, lane, v);
+  if (p.override_row != nullptr && gi < 0)
+    rowg_load_f32<NV>(p.override_row, lane, v);
   else if (p.in_is_bf16)
     rowg_load_bf16<NV>(static_cast<const __nv_bfloat16*>(p.in) + src * D, lane, v);
   else
@@ -164,46 +170,77 @@ __global__ void __launch_bounds__(256) layernorm_g_splitk_kernel(const LnGParams
   }
 }
 
-// length head (:201-203): raw = <LN_post(x[0, :]), w> + b on the length-token row of the length predictor's output. One warp.
-// x0 is the pre-post_norm residual row; the post_norm of the last block is applied here.
+// length head (:201-203): raw[s] = <LN_post(x[row_s, :]), w> + b on the length-token row of sequence s of the length predictor's
+// output, row_s = cu_rows[s] (0 when cu_rows == nullptr: one sequence). One warp per sequence. x is the pre-post_norm residual stream;
+// the post_norm of the last block is applied here.
 template <int NV>
-__global__ void __launch_bounds__(32) t2s_length_head_kernel(const float* x0, const float* ln_w, const float* ln_b, const float* w, const float* b,
-                                                             float eps, float* raw_out) {
+__global__ void __launch_bounds__(32) t2s_length_head_kernel(const float* x, const int* cu_rows, const float* ln_w, const float* ln_b, const float* w,
+                                                             const float* b, float eps, float* raw_out) {
   pdl_sync();
-  const int lane = threadIdx.x;
+  const int lane = threadIdx.x, s = blockIdx.x;
+  const long long row = cu_rows != nullptr ? __ldg(cu_rows + s) : 0;
   float v[4 * NV], ww[4 * NV];
-  rowg_load_f32<NV>(x0, lane, v);
+  rowg_load_f32<NV>(x + row * (128 * NV), lane, v);
   rowg_layernorm<NV>(v, ln_w, ln_b, lane, eps);
   rowg_load_f32<NV>(w, lane, ww);
-  float s = 0.f;
+  float acc = 0.f;
 #pragma unroll
-  for (int i = 0; i < 4 * NV; ++i) s = fmaf(v[i], ww[i], s);
-  s = warp_sum(s);
-  if (lane == 0) raw_out[0] = s + b[0];
+  for (int i = 0; i < 4 * NV; ++i) acc = fmaf(v[i], ww[i], acc);
+  acc = warp_sum(acc);
+  if (lane == 0) raw_out[s] = acc + b[0];
 }
 
-// sequence of one request (:205-217): [text] bytes [sep] [speech] [mask] * length [sep]; full_mask marks the speech positions.
+// The requests of a decode: sequence s is [text] bytes_s [sep] [speech] [mask] * length_s [sep] (:205-217), L_s = n_text_s + length_s + 4
+// rows of `lay` starting at lay.n_start(s). Its text bytes start at cu_text[s] of the packed text, its speech tokens at cu_len[s] of the
+// packed output. One sequence (cu_text == nullptr): n_text / length, both offsets 0.
+struct T2sSeqs {
+  SeqLayout lay;
+  const int* cu_text;  // [n_seq + 1] or nullptr
+  const int* cu_len;   // [n_seq + 1] or nullptr
+  int n_text, length;  // the single sequence's
+
+  __device__ __forceinline__ int text_start(int s) const { return cu_text != nullptr ? __ldg(cu_text + s) : 0; }
+  __device__ __forceinline__ int n_text_of(int s) const { return cu_text != nullptr ? __ldg(cu_text + s + 1) - __ldg(cu_text + s) : n_text; }
+  __device__ __forceinline__ int len_start(int s) const { return cu_len != nullptr ? __ldg(cu_len + s) : 0; }
+  // the speech positions (full_mask) of sequence s are the rows [speech_start(s), speech_start(s) + length_s)
+  __device__ __forceinline__ long long speech_start(int s) const { return static_cast<long long>(lay.n_start(s)) + n_text_of(s) + 3; }
+};
+
+// gather indices of the length predictor's input (:199): per sequence the length token (index -1, LnGParams::override_row), then the
+// text embeddings. lay: the predictor layout, n_text_s + 1 rows per sequence.
+__global__ void t2s_lp_gather_kernel(const T2sSeqs q, const int* text_tokens, int* gather) {
+  pdl_sync();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= q.lay.rows) return;
+  int s, n;
+  q.lay.enc_pos(i, s, n);
+  gather[i] = n == 0 ? -1 : text_tokens[q.text_start(s) + n - 1];
+}
+
+// token sequences of the requests (:205-222); full_mask marks the speech positions.
 struct T2sBeginParams {
-  const int* text_tokens;  // [n_text], already shifted past the special tokens
-  int n_text, length;
+  T2sSeqs seqs;
+  const int* text_tokens;  // packed [sum n_text_s], already shifted past the special tokens
   int tok_text, tok_sep, tok_speech, tok_mask;
-  int* input_ids;          // [L]
-  int* tokens;             // [L] the running "sampled_tokens"
-  uint8_t* full_mask;      // [L]
-  uint8_t* mask;           // [L] current mask = full_mask
+  int* input_ids;          // [rows]
+  int* tokens;             // [rows] the running "sampled_tokens"
+  uint8_t* full_mask;      // [rows]
+  uint8_t* mask;           // [rows] current mask = full_mask
 };
 __global__ void t2s_begin_kernel(const T2sBeginParams p) {
   pdl_sync();
-  const int L = p.n_text + p.length + 4;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= L) return;
+  if (i >= p.seqs.lay.rows) return;
+  int s, n;
+  p.seqs.lay.enc_pos(i, s, n);
+  const int n_text = p.seqs.n_text_of(s), L = p.seqs.lay.n_len(s);
   int tok;
   uint8_t m = 0;
-  if (i == 0) tok = p.tok_text;
-  else if (i <= p.n_text) tok = p.text_tokens[i - 1];
-  else if (i == p.n_text + 1) tok = p.tok_sep;
-  else if (i == p.n_text + 2) tok = p.tok_speech;
-  else if (i < L - 1) { tok = p.tok_mask; m = 1; }
+  if (n == 0) tok = p.tok_text;
+  else if (n <= n_text) tok = p.text_tokens[p.seqs.text_start(s) + n - 1];
+  else if (n == n_text + 1) tok = p.tok_sep;
+  else if (n == n_text + 2) tok = p.tok_speech;
+  else if (n < L - 1) { tok = p.tok_mask; m = 1; }
   else tok = p.tok_sep;
   p.input_ids[i] = tok;
   p.tokens[i] = tok;
@@ -211,21 +248,21 @@ __global__ void t2s_begin_kernel(const T2sBeginParams p) {
   p.mask[i] = m;
 }
 
-// end of one iteration (:231-233 last iteration, :256-258 otherwise):
+// end of one iteration (:231-233 last iteration, :256-258 otherwise), row-local over the rows of every sequence:
 //   last : tokens = full_mask ? id : input_ids
 //   else : tokens = full_mask ? (next_mask ? [mask] : id + offset) : input_ids
 struct T2sUpdateParams {
-  const int* ids;            // [L] sampled / arg-max ids (semantic vocabulary)
-  const uint8_t* next_mask;  // [L] or nullptr on the last iteration
+  const int* ids;            // [rows] sampled / arg-max ids (semantic vocabulary)
+  const uint8_t* next_mask;  // [rows] or nullptr on the last iteration
   const uint8_t* full_mask;
   const int* input_ids;
   int* tokens;
-  int L, offset, tok_mask;
+  int rows, offset, tok_mask;
 };
 __global__ void t2s_update_kernel(const T2sUpdateParams p) {
   pdl_sync();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= p.L) return;
+  if (i >= p.rows) return;
   int tok = p.input_ids[i];
   if (p.full_mask[i]) {
     if (p.next_mask == nullptr) tok = p.ids[i];
@@ -234,11 +271,13 @@ __global__ void t2s_update_kernel(const T2sUpdateParams p) {
   p.tokens[i] = tok;
 }
 
-// speech_pred_tokens = sampled_tokens[full_mask] (:267): the speech positions are the contiguous range [start, start + length)
-__global__ void t2s_gather_out_kernel(const int* tokens, int start, int length, long long* out) {
+// speech_pred_tokens = sampled_tokens[full_mask] (:267) of every sequence, packed: out[len_start(s) + k] = tokens[speech_start(s) + k]
+__global__ void t2s_gather_out_kernel(const T2sSeqs q, const int* tokens, int total, long long* out) {
   pdl_sync();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < length) out[i] = tokens[start + i];
+  if (i >= total) return;
+  const int s = q.cu_len != nullptr ? q.lay.search(q.cu_len, i) : 0;
+  out[i] = tokens[q.speech_start(s) + (i - q.len_start(s))];
 }
 
 }  // namespace edm

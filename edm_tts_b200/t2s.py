@@ -2,8 +2,10 @@
 
 Mirrors edm_tts/models/text_to_semantic/modeling_text_to_semantic.py:26-267 (TextToSemanticWLen): same constructor inputs (config +
 state dict / HF directory), `infer(text, pred_iters, temperature, gt_length)` with the reference's argument meaning and return type
-(`.speech_pred_tokens`), `embeddings_to_logits`. One sequence per call, as in the reference. All arithmetic runs in the CUDA
-kernels; the only host round trip is the predicted length (it fixes the shape of everything after it). No CPU fallback.
+(`.speech_pred_tokens`), `embeddings_to_logits`. `infer` decodes one sequence per call, as in the reference; `infer_batch` decodes
+a list of texts of different lengths together, packed back to back without padding. All arithmetic runs in the CUDA kernels; the only
+host round trip is the predicted length (it fixes the shape of everything after it): one read per call, or per chunk of a batch.
+No CPU fallback.
 """
 from __future__ import annotations
 
@@ -14,8 +16,9 @@ import os
 import torch
 
 from . import _lib as L
+from . import varlen
 from .config import TextToSemanticWLenConfig
-from .s2a import _check_range, _on_device
+from .s2a import MAX_CHUNK, _check_range, _on_device
 from .weights import glu_interleave
 
 
@@ -107,7 +110,8 @@ def pack_t2s_weights(sd: dict, cfg: TextToSemanticWLenConfig, device, max_positi
 
 
 class TextToSemanticWLen:
-    """Drop-in for the reference TextToSemanticWLen on the decode path (inference only, one utterance per call)."""
+    """Drop-in for the reference TextToSemanticWLen on the decode path (inference only): `infer` decodes one utterance per call as
+    the reference does, `infer_batch` a list of them in one packed decode."""
 
     def __init__(self, config, state_dict: dict, device="cuda", max_positions: int = 2048):
         if not torch.cuda.is_available():
@@ -131,17 +135,25 @@ class TextToSemanticWLen:
         n = lib.edm_t2s_num_weights(C.byref(c))
         if n <= 0:
             raise ValueError("unsupported text-to-semantic configuration: " + lib.edm_last_error().decode())
+        # the batch context (infer_batch / predict_length_batch) shares the weights; it is created and bound on first use
+        self._bctx, self._bws, self._bcap = None, None, (0, 0)
+        self.low_latency = True
         with torch.cuda.device(self.device):
             self._w = pack_t2s_weights(state_dict, cfg, self.device, self.max_positions)
             names = [lib.edm_t2s_weight_name(C.byref(c), i).decode() for i in range(n)]
-            ptrs = (C.c_void_p * n)(*[self._w[name].data_ptr() for name in names])
-            self._ctx = lib.edm_t2s_create(C.byref(c), ptrs, n)
-            if not self._ctx:
-                raise L.EdmError("edm_t2s_create failed: " + lib.edm_last_error().decode())
+            self._wptrs = (C.c_void_p * n)(*[self._w[name].data_ptr() for name in names])
+            self._ctx = self._create_ctx()
             need = lib.edm_t2s_workspace_bytes(self._ctx, self.max_positions)
             self._ws = torch.empty(need, device=self.device, dtype=torch.uint8)
             L.check(lib.edm_t2s_bind(self._ctx, self._ws.data_ptr(), need, self.max_positions), "bind")
         self.training = False
+
+    def _create_ctx(self):
+        lib = L.lib()
+        ctx = lib.edm_t2s_create(C.byref(self._cfg_c), self._wptrs, len(self._wptrs))
+        if not ctx:
+            raise L.EdmError("edm_t2s_create failed: " + lib.edm_last_error().decode())
+        return ctx
 
     @classmethod
     def from_pretrained(cls, path: str, device="cuda", **kw):
@@ -168,9 +180,10 @@ class TextToSemanticWLen:
 
     def __del__(self):
         try:
-            if getattr(self, "_ctx", None):
-                L.lib().edm_t2s_destroy(self._ctx)
-                self._ctx = None
+            for name in ("_ctx", "_bctx"):
+                if getattr(self, name, None):
+                    L.lib().edm_t2s_destroy(getattr(self, name))
+                    setattr(self, name, None)
         except Exception:
             pass
 
@@ -185,6 +198,31 @@ class TextToSemanticWLen:
         esz = torch.empty(0, dtype=dtype).element_size()
         assert numel * esz <= nbytes.value, (name, shape, nbytes.value)
         return self._ws[off:off + numel * esz].view(dtype).view(*shape)
+
+    def _bind_batch(self, rows, n_seq):
+        """The batch context with a workspace for n_seq sequences of `rows` rows in all (grown, never shrunk)."""
+        if self._bctx is None:
+            self._bctx = self._create_ctx()
+        if rows <= self._bcap[0] and n_seq <= self._bcap[1]:
+            return self._bctx
+        lib = L.lib()
+        cap = (max(rows, self._bcap[0]), max(n_seq, MAX_CHUNK))
+        need = lib.edm_t2s_workspace_bytes_batch(self._bctx, *cap)
+        if need == 0:
+            raise ValueError(f"invalid batch capacity {cap}")
+        self._bws, self._bcap = None, (0, 0)
+        self._bws = torch.empty(need, device=self.device, dtype=torch.uint8)
+        L.check(lib.edm_t2s_bind_batch(self._bctx, self._bws.data_ptr(), need, *cap), "bind_batch")
+        self._bcap = cap
+        return self._bctx
+
+    def set_low_latency(self, on=True):
+        """on (the default): `infer` splits its long-K residual GEMMs over K, faster for one utterance (edm_t2s_set_low_latency). The
+        split changes the fp32 summation order, so with it `infer` does not give the bits of the same utterance in `infer_batch`,
+        which never splits; off, it does (with batch_offset = the utterance's index in the batch)."""
+        L.check(L.lib().edm_t2s_set_low_latency(self._ctx, int(bool(on))), "set_low_latency")
+        self.low_latency = bool(on)
+        return self
 
     def text_tokens(self, text) -> torch.Tensor:
         """:193-194: utf-8 bytes shifted past the special tokens (int32 on the device). A LongTensor of already shifted tokens passes through."""
@@ -208,11 +246,13 @@ class TextToSemanticWLen:
 
     @torch.no_grad()
     @_on_device
-    def infer(self, text, pred_iters=10, temperature=1.0, gt_length=None, *, seed=0, cat_gumbel=None, remask_gumbel=None, forced_ids=None,
-              forced_masks=None, **kwargs):
+    def infer(self, text, pred_iters=10, temperature=1.0, gt_length=None, *, seed=0, batch_offset=0, cat_gumbel=None, remask_gumbel=None,
+              forced_ids=None, forced_masks=None, **kwargs):
         """modeling_text_to_semantic.py:184-267 -> TextToSemanticWLenOutput(speech_pred_tokens=LongTensor[length]).
-        Keyword-only extras are for parity runs: injected noise (cat_gumbel [iters-1, L, 1024], remask_gumbel [iters-1, 1, L] with
-        L = len(text bytes) + length + 4) and teacher forcing (forced_ids [iters, 1, L], forced_masks [iters-1, 1, L])."""
+        seed / batch_offset drive the in-kernel Philox noise: position t draws counter batch_offset * L + t, what the utterance at
+        index batch_offset of an infer_batch call draws. Keyword-only extras are for parity runs: injected noise (cat_gumbel
+        [iters-1, L, 1024], remask_gumbel [iters-1, 1, L] with L = len(text bytes) + length + 4) and teacher forcing (forced_ids
+        [iters, 1, L], forced_masks [iters-1, 1, L])."""
         tt = self.text_tokens(text)
         length = int(gt_length) if gt_length is not None else self.predict_length(tt)[0]
         if length < 1:
@@ -231,13 +271,14 @@ class TextToSemanticWLen:
         if cg is not None and cg.shape[0] < pred_iters - 1:
             raise ValueError("cat_gumbel must cover pred_iters - 1 iterations")
         out = torch.empty(length, device=dev, dtype=torch.int64)
+        L.check(L.lib().edm_t2s_set_batch_offset(self._ctx, int(batch_offset)), "set_batch_offset")
         L.check(L.lib().edm_t2s_decode(self._ctx, L.ptr(tt) if n_text else None, n_text, length, int(pred_iters), float(temperature), int(seed),
                                        L.ptr(cg), L.ptr(rg), L.ptr(fi), L.ptr(fm), L.ptr(out), L.stream_ptr()), "t2s_decode")
         return TextToSemanticWLenOutput(speech_pred_tokens=out)
 
     @torch.no_grad()
     @_on_device
-    def decode_trace(self, text, pred_iters=10, temperature=1.0, gt_length=None, *, seed=0, cat_gumbel=None, remask_gumbel=None,
+    def decode_trace(self, text, pred_iters=10, temperature=1.0, gt_length=None, *, seed=0, batch_offset=0, cat_gumbel=None, remask_gumbel=None,
                      forced_ids=None, forced_masks=None):
         """infer run stage by stage through the entry points edm_t2s_decode composes; returns every intermediate. Parity tests only."""
         lib, s_ = L.lib(), L.stream_ptr()
@@ -246,6 +287,7 @@ class TextToSemanticWLen:
         n_text = tt.numel()
         Lseq = n_text + length + 4
         dev = self.device
+        L.check(lib.edm_t2s_set_batch_offset(self._ctx, int(batch_offset)), "set_batch_offset")
         L.check(lib.edm_t2s_begin(self._ctx, L.ptr(tt) if n_text else None, n_text, length, s_), "begin")
         tr = dict(step_logits=[], step_ids=[], step_masks=[], step_masks_raw=[], length=length,
                   input_ids=self._view("input_ids", (1, Lseq), torch.int32).clone().long(),
@@ -267,6 +309,104 @@ class TextToSemanticWLen:
         L.check(lib.edm_t2s_result(self._ctx, L.ptr(out), s_), "result")
         tr["tokens"] = out
         return tr
+
+    def _batch_tokens(self, texts):
+        if not isinstance(texts, (list, tuple)) or len(texts) == 0:
+            raise ValueError("texts must be a non-empty list of str or 1-D token tensors")
+        for i, t in enumerate(texts):
+            if torch.is_tensor(t) and t.dim() != 1:
+                raise ValueError(f"texts[{i}] must be a str or a 1-D tensor of shifted tokens, got shape {tuple(t.shape)}")
+        return [self.text_tokens(t) for t in texts]
+
+    @staticmethod
+    def _packed(tokens):
+        """tokens of one chunk back to back (int32 on the device), or None when every text is empty"""
+        n = sum(t.numel() for t in tokens)
+        return torch.cat(tokens).contiguous() if n else None
+
+    @torch.no_grad()
+    @_on_device
+    def predict_length_batch(self, texts):
+        """predict_length for a list of texts in one pass per chunk of MAX_CHUNK -> (lengths, raw log-lengths), two lists. One
+        device->host read per chunk. The raw values are the bits of predict_length(texts[i]) with set_low_latency(False)."""
+        toks = self._batch_tokens(texts)
+        n_text = [t.numel() for t in toks]
+        for i, nt in enumerate(n_text):
+            if nt + 1 > self.max_positions:
+                raise ValueError(f"texts[{i}]: text of {nt} bytes exceeds max_positions={self.max_positions}")
+        lib, lengths, raws = L.lib(), [], []
+        for ch in varlen.plan(n_text, [0] * len(n_text), MAX_CHUNK):
+            n = ch.stop - ch.start
+            ctx = self._bind_batch(sum(ch.T) + n, n)
+            raw = torch.empty(n, device=self.device, dtype=torch.float32)
+            tt = self._packed(toks[ch.start:ch.stop])
+            L.check(lib.edm_t2s_predict_length_batch(ctx, n, L.ptr(tt), (C.c_int * n)(*ch.T), L.ptr(raw), L.stream_ptr()), "predict_length_batch")
+            # length as predict_length computes it (on the device), and the raw bits, in one read
+            both = torch.stack([raw.exp().ceil().long(), raw.view(torch.int32).long()]).cpu()
+            lengths += [int(x) for x in both[0]]
+            raws += [float(x) for x in both[1].to(torch.int32).view(torch.float32)]
+        return lengths, raws
+
+    @torch.no_grad()
+    @_on_device
+    def infer_batch(self, texts, pred_iters=10, temperature=1.0, gt_lengths=None, *, seed=0, batch_offset=0, cat_gumbel=None, remask_gumbel=None,
+                    forced_ids=None, forced_masks=None):
+        """infer for a list of texts (str, or 1-D tensors of shifted tokens) of different lengths, decoded together without padding,
+        in chunks of MAX_CHUNK utterances. Returns a list of LongTensor [length_i], views of one packed output. Without gt_lengths
+        the lengths come from predict_length_batch. Utterance i decodes to the bits of infer(texts[i], ..., batch_offset=batch_offset
+        + i) with set_low_latency(False). The keyword extras are per-utterance lists shaped as infer's extras for one utterance, with
+        L_i = len(text_i bytes) + length_i + 4: cat_gumbel[i] [iters-1, L_i, 1024], remask_gumbel[i] [iters-1, 1, L_i], forced_ids[i]
+        [iters, 1, L_i], forced_masks[i] [iters-1, 1, L_i]."""
+        toks = self._batch_tokens(texts)
+        n = len(toks)
+        iters = int(pred_iters)
+        if iters < 1:
+            raise ValueError(f"pred_iters must be >= 1, got {pred_iters}")
+        if gt_lengths is None:
+            lengths = self.predict_length_batch(toks)[0]
+        else:
+            if len(gt_lengths) != n:
+                raise ValueError(f"gt_lengths has {len(gt_lengths)} entries for {n} texts")
+            lengths = [int(x) for x in gt_lengths]
+        n_text = [t.numel() for t in toks]
+        Lseq = [nt + ln + 4 for nt, ln in zip(n_text, lengths)]
+        for i, ln in enumerate(lengths):
+            if ln < 1:
+                raise ValueError(f"utterance {i}: length {ln} < 1")
+            if Lseq[i] > self.max_positions:
+                raise ValueError(f"utterance {i}: sequence of {Lseq[i]} tokens exceeds max_positions={self.max_positions}")
+        V = self.config.semantic_vocab_size
+        extras = dict(cat_gumbel=(cat_gumbel, lambda l: (iters - 1, l, V)), remask_gumbel=(remask_gumbel, lambda l: (iters - 1, 1, l)),
+                      forced_ids=(forced_ids, lambda l: (iters, 1, l)), forced_masks=(forced_masks, lambda l: (iters - 1, 1, l)))
+        for name, (lst, shape) in extras.items():
+            if lst is None:
+                continue
+            if not isinstance(lst, (list, tuple)) or len(lst) != n:
+                raise ValueError(f"{name} must be a list with one entry per utterance")
+            for i, x in enumerate(lst):
+                if tuple(x.shape) != shape(Lseq[i]):
+                    raise ValueError(f"{name}[{i}] must be {shape(Lseq[i])}, got {tuple(x.shape)}")
+        dev, lib = self.device, L.lib()
+
+        def cat(lst, sl, dim, dtype):
+            if lst is None or lst[sl.start].shape[0] == 0:  # the [iters - 1, ...] extras of a 1-iteration decode are empty
+                return None
+            return torch.cat([x.to(dev) for x in lst[sl]], dim).to(dtype).contiguous()
+
+        out = torch.empty(sum(lengths), device=dev, dtype=torch.int64)
+        for ch in varlen.plan(lengths, [0] * n, MAX_CHUNK, batch_offset):
+            sl, m = slice(ch.start, ch.stop), ch.stop - ch.start
+            ctx = self._bind_batch(sum(Lseq[sl]), m)
+            cg = cat(cat_gumbel, sl, 1, torch.float32)
+            rg = cat(remask_gumbel, sl, 2, torch.float32)
+            fi = cat(forced_ids, sl, 2, torch.int32)
+            fm = cat(forced_masks, sl, 2, torch.uint8)
+            tt = self._packed(toks[sl])
+            L.check(lib.edm_t2s_set_batch_offset(ctx, ch.batch_offset), "set_batch_offset")
+            L.check(lib.edm_t2s_decode_batch(ctx, m, L.ptr(tt), (C.c_int * m)(*n_text[sl]), (C.c_int * m)(*ch.T), iters, float(temperature),
+                                             int(seed), L.ptr(cg), L.ptr(rg), L.ptr(fi), L.ptr(fm), L.ptr(out[ch.t0:ch.t0 + sum(ch.T)]),
+                                             L.stream_ptr()), "t2s_decode_batch")
+        return [b[0] for b in varlen.split_blocks(out, lengths, 1)]
 
     @torch.no_grad()
     @_on_device

@@ -260,9 +260,10 @@ int edm_s2a_decode(edm_s2a_ctx* ctx, const int* sem_tokens, const int* sem_promp
                    const float* remask_noise, const int* forced_ids, const uint8_t* forced_masks,
                    const int* forced_coarse, long long* codes_out, void* stream);
 /* ---------------------------------------------------------------------------------------------------------------
- * Text-to-semantic decoder context: TextToSemanticWLen.infer, edm_tts/models/text_to_semantic/modeling_text_to_semantic.py:184-267
- * (one sequence per call, as in the reference). Same conventions as the S2A context: weights by name, caller-owned workspace,
- * stream-ordered, no host synchronisation inside the library.
+ * Text-to-semantic decoder context: TextToSemanticWLen.infer, edm_tts/models/text_to_semantic/modeling_text_to_semantic.py:184-267.
+ * One sequence per call as in the reference (edm_t2s_begin / edm_t2s_decode), or several of different lengths packed back to back
+ * (the *_batch entry points). Same conventions as the S2A context: weights by name, caller-owned workspace, stream-ordered, no host
+ * synchronisation inside the library.
  * ------------------------------------------------------------------------------------------------------------- */
 typedef struct edm_t2s_ctx edm_t2s_ctx;
 
@@ -289,24 +290,47 @@ edm_t2s_ctx* edm_t2s_create(const edm_t2s_config* cfg, const void* const* weight
 void edm_t2s_destroy(edm_t2s_ctx* ctx);
 size_t edm_t2s_workspace_bytes(const edm_t2s_ctx* ctx, int max_len);
 int edm_t2s_bind(edm_t2s_ctx* ctx, void* workspace, size_t bytes, int max_len);
+/* Workspace of a packed batch: up to max_seq sequences of max_rows rows in all (each sequence still within max_positions, the
+ * rotary tables; the total is not). Such a workspace has no room for split-K partial sums, so nothing decoded on it splits. */
+size_t edm_t2s_workspace_bytes_batch(const edm_t2s_ctx* ctx, int max_rows, int max_seq);
+int edm_t2s_bind_batch(edm_t2s_ctx* ctx, void* workspace, size_t bytes, int max_rows, int max_seq);
 void* edm_t2s_buffer(edm_t2s_ctx* ctx, const char* name, size_t* bytes);
+/* on != 0 (the default): a single sequence decoded on an edm_t2s_bind workspace splits its long-K residual GEMMs over K, which is
+ * faster for one utterance but changes the fp32 summation order. on == 0: the unsplit launches a packed batch always takes, so an
+ * utterance decodes to the same bits alone (with batch offset b + s) as at index s of a batch with offset b. */
+int edm_t2s_set_low_latency(edm_t2s_ctx* ctx, int on);
+/* Global index of the first sequence of the next decodes (default 0): row t of sequence s draws the Philox counter
+ * (batch_offset + s) * L_s + t, so the tokens do not depend on how a batch is chunked. */
+int edm_t2s_set_batch_offset(edm_t2s_ctx* ctx, long long batch_offset);
 
 /* :198-203 length predictor; text_tokens int32 [n_text] on the device (bytes + num_special). raw_out[0] (device, or the buffer
  * "raw_len" when NULL) = log(length); the caller applies exp / ceil (the sequence length fixes every later shape). */
 int edm_t2s_predict_length(edm_t2s_ctx* ctx, const int* text_tokens, int n_text, float* raw_out, void* stream);
+/* The length predictor on n_seq texts in one pass: text s is n_text_host[s] tokens (host array) of the packed device array
+ * text_tokens; raw_out[s] (device, or the buffer "raw_len" when NULL) = log(length_s). */
+int edm_t2s_predict_length_batch(edm_t2s_ctx* ctx, int n_seq, const int* text_tokens, const int* n_text_host, float* raw_out, void* stream);
 /* :205-222 sequence [text] bytes [sep] [speech] [mask]*length [sep] + mask state. */
 int edm_t2s_begin(edm_t2s_ctx* ctx, const int* text_tokens, int n_text, int length, void* stream);
+/* n_seq sequences packed back to back: sequence s is text s (n_text_host[s] tokens of the packed text_tokens) with length_host[s]
+ * speech positions, L_s = n_text_s + length_s + 4 rows starting at L_0 + .. + L_{s-1}. edm_t2s_logits / step / result then work on
+ * all of them: buffers and per-iteration noise / forcing by packed rows, result [sum length_s] packed. Copies the layout arrays into
+ * the workspace on `stream`. */
+int edm_t2s_begin_batch(edm_t2s_ctx* ctx, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, void* stream);
 /* embeddings_to_logits :135-152 on the running tokens (x_in == NULL) or on given embeddings fp32 [L, hidden] -> buffer "logits". */
 int edm_t2s_logits(edm_t2s_ctx* ctx, const float* x_in, void* stream);
 /* :229-260 decisions of iteration `iter` of `iters`: sample (arg-max on the last), confidence re-masking, token update. */
 int edm_t2s_step(edm_t2s_ctx* ctx, int iter, int iters, float temperature, unsigned long long seed, const float* cat_noise,
                  const float* remask_noise, const int* forced_ids, const uint8_t* forced_mask, void* stream);
-/* :267 speech_pred_tokens int64 [length]. */
+/* :267 speech_pred_tokens int64 [length] ([sum length_s] after edm_t2s_begin_batch). */
 int edm_t2s_result(edm_t2s_ctx* ctx, long long* tokens_out, void* stream);
 /* begin + pred_iters x (logits, step) + result. */
 int edm_t2s_decode(edm_t2s_ctx* ctx, const int* text_tokens, int n_text, int length, int pred_iters, float temperature,
                    unsigned long long seed, const float* cat_noise, const float* remask_noise, const int* forced_ids,
                    const uint8_t* forced_masks, long long* tokens_out, void* stream);
+/* begin_batch + pred_iters x (logits, step) + result; noise / forcing arrays [iteration][sum L_s (x 1024)] or NULL. */
+int edm_t2s_decode_batch(edm_t2s_ctx* ctx, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, int pred_iters,
+                         float temperature, unsigned long long seed, const float* cat_noise, const float* remask_noise, const int* forced_ids,
+                         const uint8_t* forced_masks, long long* tokens_out, void* stream);
 
 /* number of kernels launched by this library since load (bench.py's gpu_launches) */
 unsigned long long edm_launch_count(void);
