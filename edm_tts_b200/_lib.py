@@ -59,6 +59,7 @@ _SIGNATURES = {
     "edm_dac_conv_last": (_i, [_vp, _ll, _i, _i, _i, _vp, C.c_float, _vp, _i, _vp]),
     "edm_dac_resunit": (_i, [_vp, _ll, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _ll, _i, _i, _vp]),
     "edm_dac_conv_first": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "edm_dac_zero_rows": (_i, [_vp, _ll, _vp, _i, _i, _vp]),
     "edm_codes_to_features": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "edm_s2a_num_weights": (_i, [C.POINTER(S2AConfig)]),
     "edm_s2a_weight_name": (C.c_char_p, [C.POINTER(S2AConfig), _i]),

@@ -1073,6 +1073,20 @@ extern "C" int edm_dac_conv_last(const void* a, long long a_batch_stride, int B,
   return 0;
 }
 
+extern "C" int edm_dac_zero_rows(void* buf, long long row_pitch_bytes, const int* ranges, int n_ranges, int max_range_rows, void* stream) {
+  if (int rc = check_arch()) return rc;
+  if (n_ranges <= 0 || max_range_rows <= 0) return 0;
+  if (buf == nullptr || ranges == nullptr || (reinterpret_cast<uintptr_t>(buf) & 15) != 0 || (reinterpret_cast<uintptr_t>(ranges) & 7) != 0 ||
+      row_pitch_bytes <= 0 || row_pitch_bytes % 16 != 0)
+    return fail(EDM_ERR_INVALID, "dac_zero_rows: buffer and row pitch must be 16-byte aligned, ranges 8-byte aligned");
+  const long long blocks = (static_cast<long long>(max_range_rows) * row_pitch_bytes / 16 + kZeroRowsThreads - 1) / kZeroRowsThreads;
+  const dim3 grid(static_cast<unsigned>(blocks < 1024 ? blocks : 1024), static_cast<unsigned>(n_ranges < 65535 ? n_ranges : 65535));
+  dac_zero_rows_kernel<<<grid, kZeroRowsThreads, 0, static_cast<cudaStream_t>(stream)>>>(static_cast<uint8_t*>(buf), row_pitch_bytes,
+                                                                                        reinterpret_cast<const int2*>(ranges), n_ranges);
+  EDM_LAUNCH_CHECK("dac_zero_rows");
+  return 0;
+}
+
 extern "C" int edm_dac_conv_first(const float* audio, int B, int L, const float* w, const float* bias, const float* alpha, int c0,
                                   float* y, void* s_out, void* stream) {
   if (int rc = check_arch()) return rc;

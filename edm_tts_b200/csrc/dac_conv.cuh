@@ -1268,4 +1268,21 @@ __global__ void __launch_bounds__(256) dac_conv_last_kernel(const DacConvLastPar
   }
 }
 
+// Gap rows of the packed decoder batch (DACDecoder.forward_batch, DESIGN §4a): every producer writes bias / Snake(bias) / junk view
+// rows into the rows between utterances, and the next multi-tap conv must read them as its zero padding. A [start, end) row range of
+// a channel-last buffer is one contiguous span of (end - start) * pitch bytes, so this is a memset over a list of spans: blockIdx.y
+// walks the ranges, the x blocks of a range stride over its 16-byte words.
+constexpr int kZeroRowsThreads = 256;
+
+__global__ void __launch_bounds__(kZeroRowsThreads) dac_zero_rows_kernel(uint8_t* buf, long long pitch, const int2* ranges, int n_ranges) {
+  for (int r = blockIdx.y; r < n_ranges; r += gridDim.y) {
+    const int2 rg = __ldg(ranges + r);
+    uint4* span = reinterpret_cast<uint4*>(buf + static_cast<long long>(rg.x) * pitch);
+    const long long words = static_cast<long long>(rg.y - rg.x) * pitch / 16;
+    for (long long w = static_cast<long long>(blockIdx.x) * kZeroRowsThreads + threadIdx.x; w < words;
+         w += static_cast<long long>(gridDim.x) * kZeroRowsThreads)
+      span[w] = make_uint4(0u, 0u, 0u, 0u);
+  }
+}
+
 }  // namespace edm

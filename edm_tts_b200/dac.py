@@ -101,3 +101,45 @@ class DAC:
     def decode_from_codes(self, codes: torch.Tensor, length=None) -> torch.Tensor:
         """codes [B, n, T] -> audio [B, 1, L] (modeling_dac.py:169-171; the step after the S2A decode in inference.py:49)."""
         return self.decode(self.quantizer.from_codes(codes)[0], length)["audio"]
+
+    def _decoder_or_raise(self):
+        if self.decoder is None:
+            raise RuntimeError("this DAC was built without decoder weights")
+        return self.decoder
+
+    @staticmethod
+    def _trim(audio: list, lengths) -> list:
+        return audio if lengths is None else [a[..., :n] for a, n in zip(audio, lengths)]
+
+    @torch.no_grad()
+    def decode_batch(self, zs, lengths=None) -> list:
+        """Latents of different lengths, [D, T_i] each, decoded together -> list of audio [1, L_i] (trimmed to lengths[i] when
+        given). Item i equals decode(zs[i][None], lengths[i])["audio"][0] bit for bit."""
+        dec = self._decoder_or_raise()
+        if lengths is not None and isinstance(zs, (list, tuple)) and len(lengths) != len(zs):
+            raise ValueError(f"{len(zs)} utterances but {len(lengths)} lengths")
+        return self._trim(dec.forward_batch(zs), lengths)
+
+    @torch.no_grad()
+    def decode_from_codes_batch(self, codes, lengths=None) -> list:
+        """codes: list of integer [n, T_i] tensors (one n for all, n <= n_codebooks), e.g. what the S2A infer_batch returns -> list of
+        audio [1, L_i], views of one packed output (trimmed to lengths[i] when given). Item i equals
+        decode_from_codes(codes[i][None], lengths[i])[0] bit for bit. The features of the whole list come from one codes_to_features
+        pass over the concatenated codes, which works frame by frame."""
+        dec = self._decoder_or_raise()
+        if not isinstance(codes, (list, tuple)) or len(codes) == 0:
+            raise ValueError("codes must be a non-empty list of [n, T_i] tensors")
+        if any(not torch.is_tensor(c) or c.dim() != 2 for c in codes):
+            raise ValueError("every codes entry must be a 2-D tensor [n, T_i]")
+        if any(c.dtype.is_floating_point or c.dtype.is_complex or c.dtype == torch.bool for c in codes):
+            raise ValueError("codes must be integer tensors")
+        n = int(codes[0].shape[0])
+        if any(int(c.shape[0]) != n for c in codes) or not 1 <= n <= self.n_codebooks:
+            raise ValueError(f"every codes entry must have the same number of levels n, 1 <= n <= {self.n_codebooks}")
+        T = [int(c.shape[1]) for c in codes]
+        if min(T) < 1:
+            raise ValueError("every utterance needs at least one frame")
+        if lengths is not None and len(lengths) != len(codes):
+            raise ValueError(f"{len(codes)} utterances but {len(lengths)} lengths")
+        z = self.quantizer.from_codes(torch.cat([c.to(self.device, torch.int64) for c in codes], dim=1)[None])[0][0]
+        return self._trim(dec._forward_packed(z.to(torch.bfloat16), T), lengths)

@@ -1,9 +1,11 @@
-"""Host-side layout of a variable-length S2A batch (plain Python, no GPU): where each utterance sits in the packed buffers of
-edm_s2a_bind_varlen, how a long list is cut into chunks, and the per-utterance views of the packed output.
+"""Host-side layout of variable-length batches (plain Python, no GPU): where each utterance sits in the packed buffers, how a long
+list is cut into chunks, and the per-utterance views of the packed output.
 
-Utterance i has T_i target and P_i prompt frames. Packed buffers hold the utterances back to back: per-frame data of utterance i
-starts at cu_t[i] (targets) or cu_p[i] (prompt), a per-utterance [Q, T_i] block at Q * cu_t[i]. With equal lengths this is the
-[B, ...] layout of a uniform batch.
+S2A (edm_s2a_bind_varlen): utterance i has T_i target and P_i prompt frames. Packed buffers hold the utterances back to back:
+per-frame data of utterance i starts at cu_t[i] (targets) or cu_p[i] (prompt), a per-utterance [Q, T_i] block at Q * cu_t[i]. With
+equal lengths this is the [B, ...] layout of a uniform batch.
+
+DAC decoder (DACDecoder.forward_batch): the utterances are packed along time with zero gap rows between them, see dac_pack.
 """
 from __future__ import annotations
 
@@ -42,3 +44,103 @@ def split_blocks(packed, T, Q: int) -> list:
     """Views [Q, T_i] of a flat packed buffer of per-utterance [Q, T_i] blocks."""
     cu = offsets(T)
     return [packed[Q * cu[i]:Q * cu[i + 1]].view(Q, T[i]) for i in range(len(T))]
+
+
+# ---------------------------------------------------------------------------------------------------------------------------------
+# DAC decoder batches: utterances packed along time with zero gap rows between them (DESIGN §4a). The conv kernels zero-fill only at
+# the two ends of a tensor, so every utterance gets its conv padding from gap rows that are exactly zero when a conv reads them.
+# Stage 0 is the latent (and the first conv's output, same rows); stage k follows the k-th transposed conv (stride r_k). Utterance i
+# starts at a[k][i] = r_k * a[k-1][i] and has L[k][i] = conv_transpose_length(L[k-1][i], r_k) rows, so the transposed conv's output
+# view (out_view[q] -> out[q r + phase - pad]) lands every utterance at its packed place without any new indexing.
+
+DAC_FIRST_READ = 3      # first conv k=7 (reads the latent)
+DAC_UNIT_READ = 27      # dilation-9 k=7 conv of the last ResidualUnit of every upsampled stage
+DAC_LAST_READ = 3       # last conv k=7
+DAC_UP_READ = 1         # transposed conv as a 2-tap conv: x[q - 1], x[q]
+
+
+def conv_transpose_length(L_in: int, stride: int) -> int:
+    """Output length of ConvTranspose1d(kernel 2s, stride s, padding floor(s/2), output_padding s % 2) (decoder.py:15-23)."""
+    return (L_in - 1) * stride - 2 * (stride // 2) + 2 * stride + stride % 2
+
+
+def dac_stage_reads(rates) -> list[int]:
+    """Widest one-sided read into each stage's bf16 operand: the first conv and the first transposed conv read stage 0, the
+    ResidualUnits, the next transposed conv (or the last conv) read stage k >= 1."""
+    K = len(rates)
+    return [max(DAC_FIRST_READ, DAC_UP_READ)] + [max(DAC_UNIT_READ, DAC_UP_READ if k < K else DAC_LAST_READ) for k in range(1, K + 1)]
+
+
+def dac_stage_gaps(g0: int, rates) -> list[int]:
+    """Rows between two neighbouring utterances (and after the last one) at each stage, for a latent gap of g0 rows:
+    g_k = r_k g_{k-1} - 2 (r_k % 2). The gap in front of the first utterance is prod(r) g0 >= g_k."""
+    out = [int(g0)]
+    for r in rates:
+        out.append(r * out[-1] - 2 * (r % 2))
+    return out
+
+
+def dac_min_gap(rates) -> int:
+    """Smallest latent gap G0 whose gaps cover every stage's widest one-sided read."""
+    if any(int(r) < 2 for r in rates):
+        raise ValueError(f"transposed-conv strides must be >= 2 (output_padding s % 2 < s), got {tuple(rates)}")
+    need = dac_stage_reads(rates)
+    g0 = 1
+    while any(g < n for g, n in zip(dac_stage_gaps(g0, rates), need)):
+        g0 += 1
+    return g0
+
+
+@dataclass(frozen=True)
+class DacChunk:
+    """Utterances [start, stop) of the caller's list, decoded by one packed pass. rows[k] packed rows of stage k, starts[k][i] /
+    lengths[k][i] where utterance start + i sits in them; t0 is the chunk's first frame in the concatenated latent."""
+    start: int
+    stop: int
+    t0: int
+    rows: tuple
+    starts: tuple
+    lengths: tuple
+
+    def gaps(self, k: int) -> list[tuple[int, int]]:
+        """[start, end) row ranges of stage k outside every utterance: exactly the complement of the valid ranges in [0, rows[k])."""
+        out, prev = [], 0
+        for a, n in zip(self.starts[k], self.lengths[k]):
+            out.append((prev, a))
+            prev = a + n
+        out.append((prev, self.rows[k]))
+        return out
+
+
+def dac_pack(T, rates, g0: int, start: int = 0, t0: int = 0) -> DacChunk:
+    """Packed geometry of utterances with T[i] latent frames, laid out as | g0 | T_0 | g0 | T_1 | ... | T_n-1 | g0 |."""
+    a, n = [], []
+    pos = g0
+    for t in T:
+        a.append(pos)
+        n.append(int(t))
+        pos += int(t) + g0
+    rows, starts, lengths = [pos], [tuple(a)], [tuple(n)]
+    for r in rates:
+        rows.append(r * rows[-1])
+        starts.append(tuple(r * x for x in starts[-1]))
+        lengths.append(tuple(conv_transpose_length(x, r) for x in lengths[-1]))
+    return DacChunk(start, start + len(T), t0, tuple(rows), tuple(starts), tuple(lengths))
+
+
+def dac_plan(T, rates, max_chunk_samples: int) -> list[DacChunk]:
+    """Cut the list, in order, into chunks whose packed audio rows (gaps included) stay within max_chunk_samples; an utterance that
+    alone exceeds the limit gets a chunk of its own."""
+    g0 = dac_min_gap(rates)
+    hop = 1
+    for r in rates:
+        hop *= r
+    cu = offsets(T)
+    chunks, s = [], 0
+    while s < len(T):
+        e = s + 1
+        while e < len(T) and hop * (g0 * (e - s + 2) + cu[e + 1] - cu[s]) <= max_chunk_samples:
+            e += 1
+        chunks.append(dac_pack(T[s:e], rates, g0, s, cu[s]))
+        s = e
+    return chunks
