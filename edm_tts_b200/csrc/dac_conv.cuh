@@ -1268,8 +1268,9 @@ __global__ void __launch_bounds__(256) dac_conv_last_kernel(const DacConvLastPar
   }
 }
 
-// Gap rows of the packed decoder batch (DACDecoder.forward_batch, DESIGN §4a): every producer writes bias / Snake(bias) / junk view
-// rows into the rows between utterances, and the next multi-tap conv must read them as its zero padding. A [start, end) row range of
+// Gap rows of the packed encoder and decoder batches (DACEncoder.forward_batch, DACDecoder.forward_batch, DESIGN §4a): every producer
+// writes bias / Snake(bias) / junk view rows into the rows between utterances, and the next multi-tap conv must read them as its zero
+// padding. A [start, end) row range of
 // a channel-last buffer is one contiguous span of (end - start) * pitch bytes, so this is a memset over a list of spans: blockIdx.y
 // walks the ranges, the x blocks of a range stride over its 16-byte words.
 constexpr int kZeroRowsThreads = 256;

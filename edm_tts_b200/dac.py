@@ -13,6 +13,7 @@ import os
 
 import torch
 
+from . import varlen
 from .config import DACConfig
 from .dac_decoder import DACDecoder
 from .dac_encoder import DACEncoder, code_lengths
@@ -57,6 +58,33 @@ class DAC:
         quantizer, as under the reference's autocast (dump_tokens.py:213)."""
         z = self.encoder(audio, out_dtype=torch.bfloat16)
         return self.quantizer.encode(z, n_quantizers)
+
+    @torch.no_grad()
+    def encode_to_codes_batch(self, audios, n_quantizers=None) -> list:
+        """audios: list of mono clips [1, L_i] of different lengths -> list of int64 codes [n_codebooks, T_i], T_i =
+        get_code_lengths(L_i), views of one flat buffer laid out as varlen.split_blocks (what the S2A infer_batch returns and
+        decode_from_codes_batch takes). Item i equals encode_to_codes(audios[i][None], n_quantizers)[0] bit for bit. The clips of a
+        chunk are encoded in one packed pass (DACEncoder.forward_batch) and quantized by one RVQ call over the packed z, whose gap
+        frames are dropped."""
+        T = [self.encoder.lengths(L_i)[-1] for L_i in self.encoder._check_list(audios)]
+        n = self.quantizer.n_codebooks
+        out = torch.empty(n * sum(T), device=self.device, dtype=torch.int64)
+        cu = varlen.offsets(T)
+
+        def gather(ch, z):
+            # out[n cu_i + q T_i + t] = codes[q, a_i + t] for the chunk's clips, as one index_select over the packed codes
+            codes = self.quantizer.encode(z, n_quantizers)[0]                # [n, rows], gap frames included
+            meta = torch.tensor([ch.lengths[-1], ch.starts[-1]], dtype=torch.int64).to(self.device)
+            sizes = n * meta[0]
+            m = n * (cu[ch.stop] - cu[ch.start])
+            clip = torch.repeat_interleave(torch.arange(ch.stop - ch.start, device=self.device), sizes, output_size=m)
+            within = torch.arange(m, device=self.device) - (sizes.cumsum(0) - sizes)[clip]
+            t_i = meta[0][clip]
+            idx = (within // t_i) * codes.shape[1] + meta[1][clip] + within % t_i
+            torch.index_select(codes.reshape(-1), 0, idx, out=out[n * cu[ch.start]:n * cu[ch.stop]])
+
+        self.encoder._forward_packed(audios, torch.bfloat16, gather)
+        return varlen.split_blocks(out, T, n)
 
     def preprocess(self, audio_data: torch.Tensor, sample_rate=None):
         """modeling_dac.py:75-93: resample to the model's rate when another one is given (torchaudio, as the reference), then right-pad

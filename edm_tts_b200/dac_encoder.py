@@ -13,6 +13,8 @@ import math
 import torch
 
 from . import _lib as L
+from . import varlen
+from .varlen import strided_conv_length
 
 
 _FUSED = (64, 128)   # channel counts whose ResidualUnits run as one launch (edm_dac_resunit); at 256 the two-launch form is as fast
@@ -23,12 +25,6 @@ def _fold(sd, key):
     g = sd[key + ".parametrizations.weight.original0"].float()
     v = sd[key + ".parametrizations.weight.original1"].float()
     return v * (g / v.flatten(1).norm(dim=1).view(-1, 1, 1))
-
-
-def strided_conv_length(L_in, stride: int):
-    """Output length of Conv1d(kernel 2s, stride s, padding ceil(s/2)) (encoder.py:19-25); works on ints and integer tensors. The
-    other convs of the encoder (k=7 pad 3, dilated k=7 pad 3d, k=1, k=3 pad 1) keep the length."""
-    return (L_in + 2 * math.ceil(stride / 2) - 2 * stride) // stride + 1
 
 
 def code_lengths(input_lengths, strides=(2, 4, 5, 8)):
@@ -81,6 +77,7 @@ class DACEncoder:
         self.a_last = alpha(f"{prefix}block.{n}")
         self.w_last, self.b_last = conv(f"{prefix}block.{n + 1}")
         self._ws = {}
+        self._pws = None
 
     def eval(self):
         return self
@@ -93,16 +90,8 @@ class DACEncoder:
             out.append(strided_conv_length(out[-1], s))
         return out
 
-    def _workspace(self, B: int, L_in: int):
-        key = (B, L_in)
-        ws = self._ws.get(key)
-        if ws is not None:
-            return ws
-        # keep two geometries (a batch that does not divide into equal chunks alternates between two chunk sizes; re-allocating
-        # per chunk costs more than the kernels), drop the oldest beyond that: the buffers are large
-        while len(self._ws) >= 2:
-            self._ws.pop(next(iter(self._ws)))
-        lens = self.lengths(L_in)
+    def _alloc(self, B: int, lens):
+        """Stage buffers for B sequences of lens[k] rows at stage k."""
         dev = self.device
         ws = dict(lens=lens, y=[], sx=[], sh=[], sd=[], sm=[])
         c = self.d_model
@@ -118,8 +107,31 @@ class DACEncoder:
             c *= 2
         ws["y"].append(None)
         ws["sx"].append(torch.empty(B, lens[-1], c, device=dev, dtype=torch.bfloat16))
+        return ws
+
+    def _workspace(self, B: int, L_in: int):
+        key = (B, L_in)
+        ws = self._ws.get(key)
+        if ws is not None:
+            return ws
+        # keep two geometries (a batch that does not divide into equal chunks alternates between two chunk sizes; re-allocating
+        # per chunk costs more than the kernels), drop the oldest beyond that: the buffers are large
+        while len(self._ws) >= 2:
+            self._ws.pop(next(iter(self._ws)))
+        ws = self._alloc(B, self.lengths(L_in))
         self._ws[key] = ws
         return ws
+
+    def _packed_workspace(self, rows0: int):
+        """Grow-only workspace of the packed path, sized for rows0 packed audio rows (stage k: rows0 / r_k rows). The chunks of a list
+        have different geometries; re-allocating per chunk would cost more than the kernels."""
+        if self._pws is None or self._pws["lens"][0] < rows0:
+            self._pws = None                                                     # release the smaller one first
+            lens = [rows0]
+            for s in self.strides:
+                lens.append(lens[-1] // s)
+            self._pws = self._alloc(1, lens)
+        return self._pws
 
     # ------------------------------------------------------------------ forward
     def _conv(self, a, a_rows, a_cols, w, bias, taps, step, off, rows_out, B, alpha=None, x_res=None, y=None, s_out=None,
@@ -158,14 +170,23 @@ class DACEncoder:
     def _forward_chunk(self, audio, z_out):
         B, _, L_in = audio.shape
         ws = self._workspace(B, L_in)
-        lens = ws["lens"]
+        return self._run(ws, B, ws["lens"], audio, z_out)
+
+    def _run(self, ws, B, lens, audio, z_out, clear=None):
+        """The encoder's launches over ws (stage k holds lens[k] rows per sequence; the buffers may be longer) from audio [B, ..., L]
+        into z_out [B, enc_dim, T]. clear(k, ptr, pitch_bytes, sd), when given, runs after every launch whose bf16 operand output at
+        stage k a multi-tap conv reads next; sd marks the strided conv's padded operand, whose row 0 is `pad` rows before row 0 of the
+        stage."""
         c = self.d_model
         first_alpha = self.blocks[0]["units"][0]["a_in"]
-        L.check(L.lib().edm_dac_conv_first(L.ptr(audio), B, L_in, L.ptr(self.w0), L.ptr(self.b0), L.ptr(first_alpha), c, L.ptr(ws["y"][0]),
+        L.check(L.lib().edm_dac_conv_first(L.ptr(audio), B, lens[0], L.ptr(self.w0), L.ptr(self.b0), L.ptr(first_alpha), c, L.ptr(ws["y"][0]),
                                            L.ptr(ws["sx"][0]), L.stream_ptr()), "dac_conv_first")
+        if clear:
+            clear(0, ws["sx"][0].data_ptr(), c * 2, False)
         for k, blk in enumerate(self.blocks):
             s, Lk, Ln = blk["stride"], lens[k], lens[k + 1]
-            y, sx, sh, sd = ws["y"][k], ws["sx"][k], ws["sh"][k], ws["sd"][k]
+            y, sx, sh, sd = ws["y"][k][:, :Lk], ws["sx"][k][:, :Lk], ws["sh"][k][:, :Lk], ws["sd"][k][:, :(Ln + 1) * s]
+            sm = ws["sm"][k][:, :Lk] if ws["sm"][k] is not None else None
             src = sx
             for u, ru in enumerate(blk["units"]):
                 d = 3 ** u
@@ -177,18 +198,91 @@ class DACEncoder:
                     self._resunit(src, B, Lk, c, d, ru, a_next, y, dst, dst_off, dst_rows)
                 else:
                     # dilated k=7 conv of Snake(x); epilogue applies the unit's second Snake
-                    self._conv(src, Lk, c, ru["w7"], ru["b7"], 7, d, -3 * d, Lk, B, alpha=ru["a_mid"], s_out=ws["sm"][k], s_rows=Lk)
+                    self._conv(src, Lk, c, ru["w7"], ru["b7"], 7, d, -3 * d, Lk, B, alpha=ru["a_mid"], s_out=sm, s_rows=Lk)
                     # 1x1 conv + residual add into the fp32 stream; epilogue applies the Snake in front of the next conv
-                    self._conv(ws["sm"][k], Lk, c, ru["w1"], ru["b1"], 1, 1, 0, Lk, B, alpha=a_next, x_res=y, y=y, s_out=dst,
+                    self._conv(sm, Lk, c, ru["w1"], ru["b1"], 1, 1, 0, Lk, B, alpha=a_next, x_res=y, y=y, s_out=dst,
                                s_row_off=dst_off, s_rows=dst_rows)
+                if clear:
+                    clear(k, dst.data_ptr(), c * 2, u == 2)
                 src = dst
             # strided conv on the padded operand viewed as [Ln + 1][s * c]
             nxt_alpha = self.blocks[k + 1]["units"][0]["a_in"] if k + 1 < len(self.blocks) else self.a_last
             sd_view = sd.view(B, Ln + 1, s * c)
             last = k + 1 == len(self.blocks)      # nothing reads the fp32 stream after the last strided conv
-            self._conv(sd_view, Ln + 1, s * c, blk["wd"], blk["bd"], 2, 1, 0, Ln, B, alpha=nxt_alpha, y=None if last else ws["y"][k + 1],
-                       s_out=ws["sx"][k + 1], s_rows=Ln)
+            self._conv(sd_view, Ln + 1, s * c, blk["wd"], blk["bd"], 2, 1, 0, Ln, B, alpha=nxt_alpha,
+                       y=None if last else ws["y"][k + 1][:, :Ln], s_out=ws["sx"][k + 1][:, :Ln], s_rows=Ln)
             c *= 2
+            if clear:
+                clear(k + 1, ws["sx"][k + 1].data_ptr(), c * 2, False)
         T = lens[-1]
-        self._conv(ws["sx"][-1], T, c, self.w_last, self.b_last, 3, 1, -1, T, B, zt=z_out)
+        self._conv(ws["sx"][-1][:, :T], T, c, self.w_last, self.b_last, 3, 1, -1, T, B, zt=z_out)
         return z_out
+
+    # ------------------------------------------------------------------ clips of different lengths
+    def _check_list(self, audios) -> list[int]:
+        """Samples per clip of a list of [1, L_i] clips; ValueError for anything else or a clip shorter than one frame."""
+        if not isinstance(audios, (list, tuple)) or len(audios) == 0:
+            raise ValueError("audios must be a non-empty list of [1, L_i] clips")
+        for a in audios:
+            if not torch.is_tensor(a) or a.dim() != 2 or a.shape[0] != 1:
+                raise ValueError("every clip must be a [1, L_i] tensor")
+            if self.lengths(int(a.shape[1]))[-1] <= 0:
+                raise ValueError(f"a clip of {int(a.shape[1])} samples is shorter than one frame")
+        return [int(a.shape[1]) for a in audios]
+
+    @torch.no_grad()
+    def forward_batch(self, audios, out_dtype=torch.bfloat16) -> list:
+        """List of mono clips [1, L_i] (any float dtype, converted as forward converts) -> list of z [enc_dim, T_i] (bf16 or fp32),
+        T_i = lengths(L_i)[-1], views of buffers of this call. Item i equals forward(audios[i][None])[0] bit for bit."""
+        out = []
+        self._forward_packed(audios, out_dtype, lambda ch, z: out.extend(z[0, :, a:a + n] for a, n in zip(ch.starts[-1], ch.lengths[-1])))
+        return out
+
+    def _forward_packed(self, audios, out_dtype, consume):
+        """Encodes the list chunk by chunk (varlen.enc_plan); consume(chunk, z) gets each chunk's packed z [1, enc_dim, rows[-1]], a
+        fresh tensor whose gap frames hold junk."""
+        if out_dtype not in (torch.bfloat16, torch.float32):
+            raise ValueError("out_dtype must be bfloat16 or float32")
+        lens = self._check_list(audios)
+        plan = varlen.enc_plan(lens, self.strides, self.max_chunk_samples)
+        K = len(self.strides)
+        # one upload per call: the gap ranges of every chunk and stage ((start, end) pairs); list k <= K clears the operand of stage k,
+        # list K + 1 + k the strided conv's padded operand of stage k: the same gaps `pad` rows later, the first one from row 0 (the
+        # front rows) and the last one to the end of the [Ln + 1][s C] view, rows a previous larger chunk may have written
+        host, at = [], []
+        for ch in plan:
+            at.append([])
+            lists = [ch.gaps(k) for k in range(K + 1)]
+            for k, s in enumerate(self.strides):
+                pad = math.ceil(s / 2)
+                g = [(b + pad, e + pad) for b, e in ch.gaps(k)]
+                g[0], g[-1] = (0, g[0][1]), (g[-1][0], ch.rows[k] + s)
+                lists.append(g)
+            for g in lists:
+                at[-1].append((len(host), len(g), max(e - b for b, e in g)))
+                host += g
+        dev_buf = torch.tensor([v for g in host for v in g], dtype=torch.int32).to(self.device)
+        # the packed audio of every chunk in one copy: clips at their packed rows, zeros in between
+        clips = [a.to(self.device, torch.float32).reshape(-1) for a in audios]
+        zeros = torch.zeros(max(e - b for ch in plan for b, e in ch.gaps(0)), device=self.device)
+        pieces = []
+        for ch in plan:
+            for (b, e), i in zip(ch.gaps(0), range(ch.start, ch.stop + 1)):
+                pieces.append(zeros[:e - b])
+                if i < ch.stop:
+                    pieces.append(clips[i])
+        packed = torch.cat(pieces)
+        ws = self._packed_workspace(max(ch.rows[0] for ch in plan))
+        o0 = 0
+        for ch, at_ch in zip(plan, at):
+            def clear(k, ptr, pitch, sd, at_ch=at_ch):
+                first, n, widest = at_ch[K + 1 + k if sd else k]
+                self._zero_rows(ptr, pitch, dev_buf.data_ptr() + 8 * first, n, widest)
+
+            z = torch.empty(1, self.enc_dim, ch.rows[-1], device=self.device, dtype=out_dtype)
+            self._run(ws, 1, ch.rows, packed[o0:o0 + ch.rows[0]], z, clear)
+            o0 += ch.rows[0]
+            consume(ch, z)
+
+    def _zero_rows(self, ptr, pitch, ranges_ptr, n, widest):
+        L.check(L.lib().edm_dac_zero_rows(ptr, pitch, ranges_ptr, n, widest, L.stream_ptr()), "dac_zero_rows")

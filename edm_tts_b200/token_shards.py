@@ -37,18 +37,29 @@ class TokenShardWriter:
         return os.path.join(self.output_dir, f"{self.rank}_{self._index}.pt")
 
     def add_batch(self, ids, acoustic_codes, semantic_codes, code_lengths=None, **optional):
-        """One tokenizer batch. code_lengths[i] trims the padded tail (dump_tokens.py:201-222); optional per-utterance lists
-        are stored under the reference's singular key names when given (plural keyword -> singular key)."""
+        """One tokenizer batch: padded tensors acoustic_codes [B, n, T] / semantic_codes [B, T], whose code_lengths[i] trims the
+        padded tail (dump_tokens.py:201-222), or per-utterance lists [n, T_i] / [T_i] (e.g. what DAC.encode_to_codes_batch returns),
+        which need no code_lengths. Optional per-utterance lists are stored under the reference's singular key names when given
+        (plural keyword -> singular key)."""
         B = len(ids)
-        if acoustic_codes.shape[0] != B or semantic_codes.shape[0] != B:
+        lists = isinstance(acoustic_codes, (list, tuple))
+        if lists != isinstance(semantic_codes, (list, tuple)):
+            raise ValueError("acoustic_codes and semantic_codes must both be lists or both be tensors")
+        if len(acoustic_codes) != B or len(semantic_codes) != B:
             raise ValueError("ids, acoustic_codes and semantic_codes must agree on the batch size")
-        if acoustic_codes.shape[-1] != semantic_codes.shape[-1]:
-            raise ValueError("acoustic and semantic codes must have the same number of frames")  # audio_tokenizer.py:56-57
-        ac = acoustic_codes.detach().to("cpu", self.dtype)
-        sc = semantic_codes.detach().to("cpu", self.dtype)
+        if lists:
+            if any(a.dim() != 2 or s.dim() != 1 or a.shape[-1] != s.shape[-1] for a, s in zip(acoustic_codes, semantic_codes)):
+                raise ValueError("every utterance needs acoustic codes [n, T_i] and semantic codes [T_i] of the same T_i")
+            ac = [a.detach().to("cpu", self.dtype) for a in acoustic_codes]
+            sc = [s.detach().to("cpu", self.dtype) for s in semantic_codes]
+        else:
+            if acoustic_codes.shape[-1] != semantic_codes.shape[-1]:
+                raise ValueError("acoustic and semantic codes must have the same number of frames")  # audio_tokenizer.py:56-57
+            ac = acoustic_codes.detach().to("cpu", self.dtype)
+            sc = semantic_codes.detach().to("cpu", self.dtype)
         for i, name in enumerate(ids):
-            n = int(code_lengths[i]) if code_lengths is not None else ac.shape[-1]
-            item = {"acoustic_codes": ac[i, :, :n].clone(), "semantic_codes": sc[i, :n].clone()}
+            n = int(code_lengths[i]) if code_lengths is not None else ac[i].shape[-1]
+            item = {"acoustic_codes": ac[i][:, :n].clone(), "semantic_codes": sc[i][:n].clone()}
             for key in OPTIONAL_KEYS:
                 vals = optional.get(key + "s", optional.get(key))
                 if vals is not None:

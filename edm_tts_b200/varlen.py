@@ -6,9 +6,11 @@ per-frame data of utterance i starts at cu_t[i] (targets) or cu_p[i] (prompt), a
 equal lengths this is the [B, ...] layout of a uniform batch.
 
 DAC decoder (DACDecoder.forward_batch): the utterances are packed along time with zero gap rows between them, see dac_pack.
+DAC encoder (DACEncoder.forward_batch): the same idea for the downsampling stack, see enc_pack.
 """
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass
 
 
@@ -93,8 +95,9 @@ def dac_min_gap(rates) -> int:
 
 @dataclass(frozen=True)
 class DacChunk:
-    """Utterances [start, stop) of the caller's list, decoded by one packed pass. rows[k] packed rows of stage k, starts[k][i] /
-    lengths[k][i] where utterance start + i sits in them; t0 is the chunk's first frame in the concatenated latent."""
+    """Utterances [start, stop) of the caller's list, run through one packed pass. rows[k] packed rows of stage k, starts[k][i] /
+    lengths[k][i] where utterance start + i sits in them; t0 is the chunk's first row in the concatenated input (latent frames for
+    the decoder, audio samples for the encoder)."""
     start: int
     stop: int
     t0: int
@@ -142,5 +145,94 @@ def dac_plan(T, rates, max_chunk_samples: int) -> list[DacChunk]:
         while e < len(T) and hop * (g0 * (e - s + 2) + cu[e + 1] - cu[s]) <= max_chunk_samples:
             e += 1
         chunks.append(dac_pack(T[s:e], rates, g0, s, cu[s]))
+        s = e
+    return chunks
+
+
+# ---------------------------------------------------------------------------------------------------------------------------------
+# DAC encoder batches: clips packed along time with zero gap rows, for the downsampling stack (DESIGN §4a). Stage 0 is the audio (and
+# the first conv's output, same rows); stage k follows the k-th strided conv (kernel 2s, stride s, padding ceil(s/2)), which reads its
+# operand through a [rows / s][s C] view: a clip's output lands at its packed place only if its start is a multiple of s at every stage,
+# so in audio rows every clip starts at a multiple of the hop. Clip i takes a slot of ceil(L_i / hop) + G latent frames behind G frames
+# in front of the first clip; at stage k (cumulative stride r_k) it starts at a[0][i] / r_k and has the single-path length chain
+# L[k][i] = strided_conv_length(L[k-1][i], s_k).
+
+ENC_FIRST_READ = 3      # first conv k=7 (reads the packed audio)
+ENC_UNIT_READ = 27      # dilation-9 k=7 conv of the last ResidualUnit of every stage before a strided conv
+ENC_LAST_READ = 1       # last conv k=3 (reads the latent)
+
+
+def strided_conv_length(L_in, stride: int):
+    """Output length of Conv1d(kernel 2s, stride s, padding ceil(s/2)) (encoder.py:19-25); works on ints and integer tensors. The
+    other convs of the encoder (k=7 pad 3, dilated k=7 pad 3d, k=1, k=3 pad 1) keep the length."""
+    return (L_in + 2 * math.ceil(stride / 2) - 2 * stride) // stride + 1
+
+
+def enc_stage_reads(rates) -> list[int]:
+    """Widest one-sided read into each stage's operand: the ResidualUnits and the strided conv (ceil(s/2) rows on either side) read
+    stages 0 .. K-1 (the first conv reads the audio at stage 0), the last conv reads the latent (stage K)."""
+    return ([max(ENC_FIRST_READ, ENC_UNIT_READ, math.ceil(rates[0] / 2))] + [max(ENC_UNIT_READ, math.ceil(s / 2)) for s in rates[1:]]
+            + [ENC_LAST_READ])
+
+
+def enc_stage_gaps(g: int, rates) -> list[int]:
+    """Narrowest gap at each stage for a latent gap of g frames: (hop / r_k) g rows, reached when the clip in front of it is a
+    multiple of the hop long (a shorter clip leaves more)."""
+    out = [int(g) * math.prod(rates)]
+    for s in rates:
+        out.append(out[-1] // s)
+    return out
+
+
+def enc_min_gap(rates) -> int:
+    """Smallest latent gap G whose gaps cover every stage's widest one-sided read."""
+    if not rates or any(int(s) < 2 for s in rates):
+        raise ValueError(f"strides must be >= 2 (a stride-1 conv of kernel 2 lengthens the clip into its gap), got {tuple(rates)}")
+    need = enc_stage_reads(rates)
+    g = 1
+    while any(x < n for x, n in zip(enc_stage_gaps(g, rates), need)):
+        g += 1
+    return g
+
+
+def enc_rows(frames: int) -> int:
+    """Packed latent rows for `frames` latent frames of gaps and slots: rounded up to a multiple of 8 by lengthening the tail gap, so
+    bf16 z rows are 16-byte multiples, as the RVQ's TMA maps read them."""
+    return (frames + 7) // 8 * 8
+
+
+def enc_slot(L_i: int, hop: int, g: int) -> int:
+    """Latent frames of clip i's slot: ceil(L_i / hop) frames for the clip, then a gap of g."""
+    return -(-int(L_i) // hop) + g
+
+
+def enc_pack(L, rates, g: int, start: int = 0, t0: int = 0) -> DacChunk:
+    """Packed geometry of clips with L[i] audio samples (stage 0 = audio, stage K = latent)."""
+    hop = math.prod(rates)
+    a, pos = [], g
+    for x in L:
+        a.append(hop * pos)
+        pos += enc_slot(x, hop, g)
+    rows, starts, lengths = [hop * enc_rows(pos)], [tuple(a)], [tuple(int(x) for x in L)]
+    for s in rates:
+        rows.append(rows[-1] // s)
+        starts.append(tuple(x // s for x in starts[-1]))
+        lengths.append(tuple(strided_conv_length(x, s) for x in lengths[-1]))
+    return DacChunk(start, start + len(L), t0, tuple(rows), tuple(starts), tuple(lengths))
+
+
+def enc_plan(L, rates, max_chunk_samples: int) -> list[DacChunk]:
+    """Cut the list, in order, into chunks whose packed audio rows (gaps included) stay within max_chunk_samples; a clip that alone
+    exceeds the limit gets a chunk of its own."""
+    g = enc_min_gap(rates)
+    hop = math.prod(rates)
+    cu = offsets(L)
+    chunks, s = [], 0
+    while s < len(L):
+        e, frames = s + 1, g + enc_slot(L[s], hop, g)
+        while e < len(L) and hop * enc_rows(frames + enc_slot(L[e], hop, g)) <= max_chunk_samples:
+            frames += enc_slot(L[e], hop, g)
+            e += 1
+        chunks.append(enc_pack(L[s:e], rates, g, s, cu[s]))
         s = e
     return chunks

@@ -155,9 +155,9 @@ int edm_dac_resunit(const void* a, long long a_batch_stride, int B, int rows, in
 int edm_dac_conv_last(const void* a, long long a_batch_stride, int B, int rows, int c_pad, const float* w, float bias, float* out,
                       int apply_tanh, void* stream);
 
-/* Clears row ranges of a channel-last buffer in one launch (16-byte stores): the gap rows of a packed decoder batch
- * (DACDecoder.forward_batch), which every conv producer overwrites with bias / Snake(bias) and which the next multi-tap conv must read
- * as its zero padding. buf: row 0 of the buffer, 16-byte aligned; row_pitch_bytes: bytes per row, a multiple of 16; ranges: device
+/* Clears row ranges of a channel-last buffer in one launch (16-byte stores): the gap rows of a packed encoder or decoder batch
+ * (DACEncoder.forward_batch, DACDecoder.forward_batch), which every conv producer overwrites with bias / Snake(bias) and which the
+ * next multi-tap conv must read as its zero padding. buf: row 0 of the buffer, 16-byte aligned; row_pitch_bytes: bytes per row, a multiple of 16; ranges: device
  * array of n_ranges int pairs (start, end), 0 <= start <= end rows, each [start, end) cleared; max_range_rows >= the longest
  * end - start (sizes the grid only). */
 int edm_dac_zero_rows(void* buf, long long row_pitch_bytes, const int* ranges, int n_ranges, int max_range_rows, void* stream);
