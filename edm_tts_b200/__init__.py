@@ -22,4 +22,7 @@ def __getattr__(name):
     if name == "DACEncoder":
         from .dac_encoder import DACEncoder
         return DACEncoder
+    if name in ("HubertFeatures", "SemanticTokenizer"):
+        from . import hubert
+        return getattr(hubert, name)
     raise AttributeError(name)

@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(_HERE, "libedm_s2a.so")
 
 EPI_BF16, EPI_SWISH_BF16, EPI_QKV_ROPE, EPI_RESID_F32, EPI_F32, EPI_GLU_BF16 = range(6)
 EPI_ARGMAX = 10
+EPI_GELU_BF16 = 11
 
 
 class S2AConfig(C.Structure):
@@ -60,6 +61,10 @@ _SIGNATURES = {
     "edm_dac_resunit": (_i, [_vp, _ll, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _ll, _i, _i, _vp]),
     "edm_dac_conv_first": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "edm_dac_zero_rows": (_i, [_vp, _ll, _vp, _i, _i, _vp]),
+    "edm_hubert_conv0": (_i, [_vp, _ll, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "edm_hubert_ln512": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp]),
+    "edm_hubert_pad_rows": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "edm_hubert_pos_conv": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "edm_codes_to_features": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "edm_s2a_num_weights": (_i, [C.POINTER(S2AConfig)]),
     "edm_s2a_weight_name": (C.c_char_p, [C.POINTER(S2AConfig), _i]),

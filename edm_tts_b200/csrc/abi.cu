@@ -274,6 +274,8 @@ int launch_gemm_t(const CUtensorMap& ma, const WMap& wm, const GemmParams& p_in,
       EDM_CUDA(cudaFuncSetAttribute(gemm_bf16_tn_pair_kernel<EPI_RESID_TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPairSmemBytes));
     if (EPI == EPI_SWISH_BF16)
       EDM_CUDA(cudaFuncSetAttribute(gemm_bf16_tn_pair_kernel<EPI_SWISH_TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPairSmemBytes));
+    if (EPI == EPI_GELU_BF16)
+      EDM_CUDA(cudaFuncSetAttribute(gemm_bf16_tn_pair_kernel<EPI_GELU_TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPairSmemBytes));
     if (EPI == EPI_QKV_ROPE)
       EDM_CUDA(cudaFuncSetAttribute(gemm_bf16_tn_pair_kernel<EPI_ROPE_TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPairSmemBytes));
     if (EPI == EPI_F32)
@@ -306,12 +308,15 @@ int launch_gemm_t(const CUtensorMap& ma, const WMap& wm, const GemmParams& p_in,
     CUtensorMap mc;  // fp32 logits leave as 32 x 32 TMA store boxes
     if (int rc = make_tmap_f32_2d(&mc, p.out, p.M, p.N, p.ldo, 32, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
     launch_pdl(gemm_bf16_tn_pair_kernel<EPI_F32_TMA>, dim3(2 * pairs), dim3(kGemmThreads), kPairSmemBytes, st, ma, mb, mc, p);
-  } else if ((EPI == EPI_SWISH_BF16 || EPI == EPI_QKV_ROPE) && gemm_out_tma() && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0 && (p.ldo * 2) % 16 == 0) {
+  } else if ((EPI == EPI_SWISH_BF16 || EPI == EPI_GELU_BF16 || EPI == EPI_QKV_ROPE) && gemm_out_tma() && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0 &&
+             (p.ldo * 2) % 16 == 0) {
     // bf16 tiles leave as TMA store boxes (whole 128-byte lines) instead of 16-byte stores from registers
     CUtensorMap mc;
     if (int rc = make_tmap_2d(&mc, p.out, p.M, p.N, p.ldo, 32)) return rc;
     if (EPI == EPI_SWISH_BF16)
       launch_pdl(gemm_bf16_tn_pair_kernel<EPI_SWISH_TMA>, dim3(2 * pairs), dim3(kGemmThreads), kPairSmemBytes, st, ma, mb, mc, p);
+    else if (EPI == EPI_GELU_BF16)
+      launch_pdl(gemm_bf16_tn_pair_kernel<EPI_GELU_TMA>, dim3(2 * pairs), dim3(kGemmThreads), kPairSmemBytes, st, ma, mb, mc, p);
     else
       launch_pdl(gemm_bf16_tn_pair_kernel<EPI_ROPE_TMA>, dim3(2 * pairs), dim3(kGemmThreads), kPairSmemBytes, st, ma, mb, mc, p);
   } else {
@@ -330,6 +335,7 @@ int launch_gemm(int epi, const CUtensorMap& ma, const WMap& mb, const GemmParams
     case EPI_F32: return launch_gemm_t<EPI_F32>(ma, mb, p, st);
     case EPI_GLU_BF16: return launch_gemm_t<EPI_GLU_BF16>(ma, mb, p, st);
     case EPI_ARGMAX: return launch_gemm_t<EPI_ARGMAX>(ma, mb, p, st);
+    case EPI_GELU_BF16: return launch_gemm_t<EPI_GELU_BF16>(ma, mb, p, st);
   }
   return fail(EDM_ERR_INVALID, "unknown epilogue %d", epi);
 }
@@ -2399,4 +2405,66 @@ extern "C" int edm_t2s_decode_batch(edm_t2s_ctx* c, int n_seq, const int* text_t
   if (pred_iters < 1) return fail(EDM_ERR_INVALID, "pred_iters must be >= 1");
   if (int rc = edm_t2s_begin_batch(c, n_seq, text_tokens, n_text_host, length_host, stream)) return rc;
   return t2s_iterate(c, pred_iters, temperature, seed, cat_noise, remask_noise, forced_ids, forced_masks, tokens_out, stream);
+}
+
+// ================================================================================================ HuBERT feature extractor
+#include "hubert.cuh"
+
+extern "C" int edm_hubert_conv0(const float* audio, long long n_samples, int rows, const float* w, const float* bias, const float* ln_w,
+                                const float* ln_b, void* out, void* stream) {
+  if (int rc = check_arch()) return rc;
+  if (rows <= 0) return 0;
+  if (!audio || !w || !bias || !ln_w || !ln_b || !out || n_samples <= 0) return fail(EDM_ERR_INVALID, "hubert_conv0: null argument");
+  HbConv0Params p;
+  p.audio = audio; p.n_samples = n_samples; p.rows = rows; p.w = w; p.bias = bias; p.ln_w = ln_w; p.ln_b = ln_b;
+  p.out = static_cast<__nv_bfloat16*>(out);
+  const long long blocks = (static_cast<long long>(rows) + 7) / 8;
+  hubert_conv0_kernel<<<static_cast<int>(blocks < 8LL * num_sms() ? blocks : 8LL * num_sms()), 256, 0, static_cast<cudaStream_t>(stream)>>>(p);
+  EDM_LAUNCH_CHECK("hubert_conv0");
+  return 0;
+}
+
+extern "C" int edm_hubert_ln512(const void* in, const int* gather, int rows, const float* w, const float* b, int gelu, void* out, void* stream) {
+  if (int rc = check_arch()) return rc;
+  if (rows <= 0) return 0;
+  if (!in || !w || !b || !out) return fail(EDM_ERR_INVALID, "hubert_ln512: null argument");
+  if (gather != nullptr && in == out) return fail(EDM_ERR_INVALID, "hubert_ln512: a gathering call cannot run in place");
+  HbLnParams p;
+  p.in = static_cast<const __nv_bfloat16*>(in); p.gather = gather; p.rows = rows; p.w = w; p.b = b; p.gelu = gelu;
+  p.out = static_cast<__nv_bfloat16*>(out);
+  hubert_ln512_kernel<<<(rows + 7) / 8, 256, 0, static_cast<cudaStream_t>(stream)>>>(p);
+  EDM_LAUNCH_CHECK("hubert_ln512");
+  return 0;
+}
+
+extern "C" int edm_hubert_pad_rows(const float* x, const int* map, int rows, void* out, void* stream) {
+  if (int rc = check_arch()) return rc;
+  if (rows <= 0) return 0;
+  if (!x || !map || !out) return fail(EDM_ERR_INVALID, "hubert_pad_rows: null argument");
+  hubert_pad_rows_kernel<<<(rows + 7) / 8, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, map, rows, static_cast<__nv_bfloat16*>(out));
+  EDM_LAUNCH_CHECK("hubert_pad_rows");
+  return 0;
+}
+
+extern "C" int edm_hubert_pos_conv(const void* xp, const int* map, int rows, const void* w, const float* bias, float* x, void* stream) {
+  if (int rc = check_arch()) return rc;
+  if (rows <= 0) return 0;
+  if (!xp || !map || !w || !bias || !x) return fail(EDM_ERR_INVALID, "hubert_pos_conv: null argument");
+  if ((reinterpret_cast<uintptr_t>(x) & 15) != 0) return fail(EDM_ERR_INVALID, "hubert_pos_conv: x must be 16-byte aligned");
+  static DeviceOnce attr_once;
+  if (attr_once.needed()) {
+    EDM_CUDA(cudaFuncSetAttribute(hubert_pos_conv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPcSmemBytes));
+    attr_once.done();
+  }
+  CUtensorMap ma, mw;
+  if (int rc = make_tmap_2d(&ma, xp, rows, kD, kD, 128)) return rc;
+  if (int rc = make_tmap_2d(&mw, w, kD, 64ull * kPcTaps, 64ull * kPcTaps, 64)) return rc;
+  HbPosConvParams p;
+  p.rows = rows; p.bias = bias; p.map = map; p.x = x;
+  const long long tiles = (static_cast<long long>(rows) + 127) / 128 * 16;
+  if (tiles > 0x7fffffffLL) return fail(EDM_ERR_INVALID, "hubert_pos_conv: too many rows");
+  ProfScope prof(PK_CONV, 2.0 * rows * kD * 64 * kPcTaps, static_cast<cudaStream_t>(stream));
+  hubert_pos_conv_kernel<<<static_cast<int>(tiles < num_sms() ? tiles : num_sms()), kPcThreads, kPcSmemBytes, static_cast<cudaStream_t>(stream)>>>(ma, mw, p);
+  EDM_LAUNCH_CHECK("hubert_pos_conv");
+  return 0;
 }

@@ -35,7 +35,12 @@ enum EpiKind : int {
   EPI_SWISH_TMA = 7,   // EPI_SWISH_BF16 with the tile leaving as TMA store boxes (pair kernel only; launcher's choice)
   EPI_RESID_TMA = 6,   // EPI_RESID_F32 with the add carried out as TMA reduce-add boxes (pair kernel only; chosen by the
                        // launcher, not part of the ABI): 128 B rows reach L2 as whole lines instead of 16 B reductions
+  EPI_GELU_BF16 = 11,  // h = bf16(acc + bias); out_bf16 = bf16(GELU_erf(h))                       (HuBERT FeedForward up-proj)
+  EPI_GELU_TMA = 12,   // EPI_GELU_BF16 with TMA store boxes (pair kernel only; launcher's choice)
 };
+
+// exact (erf) GELU, nn.GELU() / ACT2FN["gelu"]
+__device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.0f + erff(x * 0.7071067811865476f)); }
 
 struct GemmParams {
   int M, N, K;
@@ -98,6 +103,9 @@ __device__ __forceinline__ void gemm_store_32(const GemmParams& p, int row, int 
         const uint32_t s2 = pack_bf16x2(sigmoid_tanh(bf16lo(h2)), sigmoid_tanh(bf16hi(h2)));
         w[i] = bf16x2_mul(h2, s2);
       }
+    } else if constexpr (EPI == EPI_GELU_BF16) {
+#pragma unroll
+      for (int i = 0; i < 16; ++i) w[i] = pack_bf16x2(gelu_erf(bf16_round(v[2 * i])), gelu_erf(bf16_round(v[2 * i + 1])));
     } else {
 #pragma unroll
       for (int i = 0; i < 16; ++i) w[i] = pack_bf16x2(v[2 * i], v[2 * i + 1]);
@@ -441,7 +449,7 @@ template <int EPI>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kGemmThreads, 1)
 gemm_bf16_tn_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                          const __grid_constant__ CUtensorMap tma_c, const GemmParams p) {
-  constexpr bool kTmaOut = EPI == EPI_RESID_TMA || EPI == EPI_SWISH_TMA || EPI == EPI_ROPE_TMA || EPI == EPI_F32_TMA;
+  constexpr bool kTmaOut = EPI == EPI_RESID_TMA || EPI == EPI_SWISH_TMA || EPI == EPI_GELU_TMA || EPI == EPI_ROPE_TMA || EPI == EPI_F32_TMA;
   constexpr bool kRope = EPI == EPI_QKV_ROPE || EPI == EPI_ROPE_TMA;
   constexpr int kSt = pair_stages(kTmaOut, kRope);
   constexpr uint32_t kStagingOffset = kSt * kPairStageBytes;
@@ -590,6 +598,35 @@ gemm_bf16_tn_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid
         if (lane == 0) bulk_wait_group_read0();
         __syncwarp();
         gemm_epilogue_rope64(p, row, col0, r0, r1, rope_tile ? smem_u32(s_rope) + tr * 256 : 0u, tr & 7, smem_u32(stg) + lane * 128);
+        fence_proxy_async_smem();
+        __syncwarp();
+        if (lane == 0) {
+          tma_store_2d(&tma_c, stg, col0, m_blk * 2 * kGemmBM + static_cast<int>(rank) * kGemmBM + quad * 32);
+          bulk_commit_group();
+        }
+        continue;
+      }
+      if constexpr (EPI == EPI_GELU_TMA) {
+        // as EPI_SWISH_TMA below, but each 16-byte chunk goes to the staging box as soon as it is computed (erf is long: fewer live
+        // registers than converting the whole slice first)
+        uint8_t* stg = smem + kStagingOffset + (warp - 2) * kPairStagingBytes;
+        const uint32_t stg_row = smem_u32(stg) + lane * 128;
+        const int sw = lane & 7;
+        if (lane == 0) bulk_wait_group_read0();
+        __syncwarp();
+#pragma unroll
+        for (int c = 0; c < 8; ++c) {
+          const uint32_t* r = c < 4 ? r0 : r1;
+          const int q = (c & 3) * 8;
+          uint32_t w[4];
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float4 b = bias4((q + 2 * e) / 4 + 8 * (c >> 2));
+            const float b0 = (e & 1) ? b.z : b.x, b1 = (e & 1) ? b.w : b.y;
+            w[e] = pack_bf16x2(gelu_erf(bf16_round(__uint_as_float(r[q + 2 * e]) + b0)), gelu_erf(bf16_round(__uint_as_float(r[q + 2 * e + 1]) + b1)));
+          }
+          sts128(stg_row + ((c ^ sw) << 4), make_float4(__uint_as_float(w[0]), __uint_as_float(w[1]), __uint_as_float(w[2]), __uint_as_float(w[3])));
+        }
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) {

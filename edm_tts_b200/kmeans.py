@@ -3,7 +3,7 @@
 Mirrors the tail of SemanticModelHuBERT.encode / encode_batch
 (edm_tts/models/audio_tokenizer/semantic_tokenizer_hubert/semantic_tokenizer_hubert.py:74-90):
     dists = -torch.cdist(embed, cluster_centers, p=2); clusters = dists.argmax(dim=-1)
-The HuBERT backbone itself stays a third-party model; this replaces the distance + arg-max step only.
+This replaces the distance + arg-max step; the HuBERT backbone in front of it is `hubert.HubertFeatures` (`hubert.SemanticTokenizer` chains the two).
 """
 from __future__ import annotations
 

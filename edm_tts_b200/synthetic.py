@@ -294,3 +294,26 @@ def make_inputs(B: int, T: int, P: int, steps: int, cfg: OracleConfig, seed: int
     u = torch.rand(n, B, T, generator=g).clamp_(1e-10, 1 - 1e-7)
     out["remask_gumbel"] = -torch.log(-torch.log(u))       # noise of random_topk_mask
     return out
+
+
+def hubert_config(**overrides):
+    """transformers HubertConfig of hubert-large (the semantic tokenizer's backbone): every field the kernels depend on set explicitly,
+    the rest at transformers' defaults."""
+    from transformers import HubertConfig
+
+    kw = dict(hidden_size=1024, num_hidden_layers=24, num_attention_heads=16, intermediate_size=4096, feat_extract_norm="layer",
+              do_stable_layer_norm=True, conv_bias=True)
+    kw.update(overrides)
+    return HubertConfig(**kw)
+
+
+def make_hubert_state_dict(seed: int = 0, config=None) -> dict:
+    """A HubertModel(config).state_dict() with transformers' own random initialisation, seeded (hubert_config() by default)."""
+    from transformers import HubertModel
+
+    cfg = config if config is not None else hubert_config()
+    devnull = torch.random.fork_rng(devices=[])
+    with devnull:
+        torch.manual_seed(seed)
+        model = HubertModel(cfg)
+    return {k: v.detach().clone() for k, v in model.state_dict().items()}

@@ -36,6 +36,7 @@ enum edm_epilogue {
   EDM_EPI_RESID_F32 = 3,   /* conformer.py:222-233       x += scale * (Linear(...)) on the fp32 residual stream */
   EDM_EPI_F32 = 4,         /* injection_conformer_wrapper.py:56-63   logits head */
   EDM_EPI_GLU_BF16 = 5,    /* conformer.py:59-66,170-171  pointwise conv + GLU; weight rows interleaved 32 value | 32 gate */
+  EDM_EPI_GELU_BF16 = 11,  /* transformers HubertFeedForward: intermediate_dense -> GELU (erf); out_bf16 = GELU(bf16(acc + bias)) */
   EDM_EPI_ARGMAX = 10      /* logits head followed by argmax(-1) (wrapper :119-121, modeling :228): out = float2 [M, ldo] partials,
                               out[r, c / 64] = (max, first arg-max as int bits) of logits[r, c .. c + 64); N % 64 == 0 */
 };
@@ -166,6 +167,32 @@ int edm_dac_zero_rows(void* buf, long long row_pitch_bytes, const int* ranges, i
  * y fp32 [B][L][c0] and s_out bf16 = Snake_alpha(y). w fp32 [c0][7]; c0 % 64 == 0. */
 int edm_dac_conv_first(const float* audio, int B, int L, const float* w, const float* bias, const float* alpha, int c0, float* y,
                        void* s_out, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * HuBERT-large backbone of the semantic tokenizer (semantic_tokenizer_hubert.py:74-90: transformers HubertModel, layer-norm
+ * feature extractor, stable-layer-norm encoder, features = hidden_states[output_layer]). The transformer layers are edm_layernorm,
+ * edm_gemm_bf16 (EDM_EPI_BF16 fused q|k|v, EDM_EPI_RESID_F32 out_proj / output_dense, EDM_EPI_GELU_BF16 intermediate_dense) and
+ * edm_attention_varlen (scale 1/8 = 64^-1/2); the strided convs 1-6 of the feature extractor are edm_dac_conv on the [rows / 2][1024]
+ * view of their 512-channel input. The calls below are the rest. Clips are packed as described in csrc/hubert.cuh. */
+
+/* HubertLayerNormConvLayer 0 (conv_layers[0]: Conv1d(1, 512, k 10, s 5) -> LayerNorm(512) -> GELU): audio fp32 [n_samples] ->
+ * out bf16 [rows][512], frame f reading samples 5f .. 5f + 9 (zero at or past n_samples). w fp32 [10][512] (tap-major). */
+int edm_hubert_conv0(const float* audio, long long n_samples, int rows, const float* w, const float* bias, const float* ln_w,
+                     const float* ln_b, void* out, void* stream);
+
+/* LayerNorm(512, eps 1e-5) on bf16 rows, then GELU (erf) when gelu != 0: out[r] = act(LN(in[gather ? gather[r] : r])). Replaces the
+ * LayerNorm + GELU of HubertLayerNormConvLayer 1-6 (in place, gather NULL) and the LayerNorm of HubertFeatureProjection (gathering the
+ * valid frames of the packed conv output). */
+int edm_hubert_ln512(const void* in, const int* gather, int rows, const float* w, const float* b, int gelu, void* out, void* stream);
+
+/* Operand of the positional conv: out bf16 [rows][1024], row r = bf16(x[map[r]]) or zeros when map[r] < 0 (x fp32 [N][1024]). */
+int edm_hubert_pad_rows(const float* x, const int* map, int rows, void* out, void* stream);
+
+/* HubertPositionalConvEmbedding + residual add (HubertEncoderStableLayerNorm.forward: x = x + GELU(SamePad(conv(x)))), grouped conv
+ * k 128, padding 64, 16 groups of 64 channels, tcgen05 implicit GEMM: x[map[t]] += bf16(GELU(bf16(conv(xp)[t] + bias))) for every padded
+ * row t with map[t] >= 0, where xp is edm_hubert_pad_rows' output with >= 64 zero rows on both sides of every sequence. w bf16
+ * [1024][128 * 64] (row 64 g + n, column 64 j + c = weight-normed weight[64 g + n, c, j]). */
+int edm_hubert_pos_conv(const void* xp, const int* map, int rows, const void* w, const float* bias, float* x, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * S2A decoder context: InjectionConformerModel.infer_special, modeling_injection_conformer.py:130-230, and
