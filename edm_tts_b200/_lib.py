@@ -56,6 +56,8 @@ _SIGNATURES = {
     "edm_remask": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _f, _f, _ull, _u, _vp]),
     "edm_rvq_encode_tc": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "edm_kmeans_assign": (_i, [_vp, _ll, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "edm_kmeans_update_workspace_bytes": (_sz, [_ll, _i, _i]),
+    "edm_kmeans_update": (_i, [_vp, _ll, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "edm_dac_conv": (_i, [_vp, _ll, _i, _ll, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _ll, _vp, _ll, _i, _i, _vp, _i, _vp]),
     "edm_dac_conv_last": (_i, [_vp, _ll, _i, _i, _i, _vp, C.c_float, _vp, _i, _vp]),
     "edm_dac_resunit": (_i, [_vp, _ll, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _ll, _i, _i, _vp]),

@@ -888,6 +888,37 @@ extern "C" int edm_kmeans_assign(const float* x, long long n_frames, int dim, co
   return 0;
 }
 
+extern "C" size_t edm_kmeans_update_workspace_bytes(long long n, int dim, int n_centroids) {
+  if (n < 0 || dim <= 0 || n_centroids <= 0) return 0;
+  return static_cast<size_t>(n_centroids + (n + kKmUpdRows - 1) / kKmUpdRows) * static_cast<size_t>(dim) * sizeof(double);
+}
+
+extern "C" int edm_kmeans_update(const float* x, long long n, int dim, const long long* idx, const long long* perm, const long long* offsets,
+                                 int n_centroids, double* partials, float* centroids, double* sums_out, void* stream) {
+  if (int rc = check_arch()) return rc;
+  if (dim <= 0 || dim % kKmKc != 0 || n_centroids <= 0 || n_centroids > kKmMaxCentroids || n < 0 || n > 0x7fffffffLL)
+    return fail(EDM_ERR_INVALID, "kmeans_update shape n=%lld dim=%d centroids=%d unsupported (dim %% 32, 1 <= centroids <= 4096)", n, dim, n_centroids);
+  if ((reinterpret_cast<uintptr_t>(x) & 15) != 0 || (reinterpret_cast<uintptr_t>(partials) & 15) != 0)
+    return fail(EDM_ERR_INVALID, "kmeans_update: x and partials must be 16-byte aligned");
+  if (n == 0) {
+    if (sums_out != nullptr) EDM_CUDA(cudaMemsetAsync(sums_out, 0, static_cast<size_t>(n_centroids) * dim * sizeof(double), static_cast<cudaStream_t>(stream)));
+    return 0;
+  }
+  KmeansUpdateParams p;
+  p.x = x; p.idx = idx; p.perm = perm; p.offsets = offsets; p.partials = partials; p.centroids = centroids; p.sums = sums_out;
+  p.n = n; p.dim = dim; p.n_centroids = n_centroids;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int d4 = dim / 4;
+  const int t1 = d4 < kKmUpdThreads ? (d4 + 31) / 32 * 32 : kKmUpdThreads;
+  const dim3 g1(static_cast<unsigned>((n + kKmUpdRows - 1) / kKmUpdRows), (d4 + t1 - 1) / t1);
+  kmeans_update_partial_kernel<<<g1, t1, 0, st>>>(p);
+  EDM_LAUNCH_CHECK("kmeans_update_partial");
+  const int t2 = dim < kKmUpdThreads ? dim : kKmUpdThreads;
+  kmeans_update_finalize_kernel<<<dim3(n_centroids, (dim + t2 - 1) / t2), t2, 0, st>>>(p);
+  EDM_LAUNCH_CHECK("kmeans_update_finalize");
+  return 0;
+}
+
 // ---------------------------------------------------------------------------------------------- DAC encoder convolutions
 namespace {
 // bf16 operand [B][rows][cols] with an explicit batch stride (elements): box = 64 channels x 128 rows x 1 batch; rows outside

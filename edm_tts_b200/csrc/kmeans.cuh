@@ -186,4 +186,92 @@ kmeans_assign_kernel(const __grid_constant__ CUtensorMap tma_x, const __grid_con
   if (warp == 1) tmem_dealloc<512>(tmem_base);
 }
 
+// ---------------------------------------------------------------------------------------------- centroid update (one Lloyd step)
+// centroid[c] = (sum of the rows assigned to c) / count_c, accumulated in fp64 and rounded once to fp32; empty clusters are left as
+// they are. The rows are read through perm, which lists them cluster by cluster (offsets[c] .. offsets[c + 1] are c's positions).
+//   pass 1 (kmeans_update_partial_kernel): item = (segment j of kKmUpdRows consecutive perm positions, column slice). The item walks
+//          its positions one cluster run at a time and writes one fp64 partial sum per (cluster c, segment j) to slot c + j. Along
+//          perm, c + j strictly increases from one run to the next (the next non-empty cluster c' > c starts in the segment where c
+//          ends or later), so slots never collide: at most n_centroids + ceil(n / kKmUpdRows) of them.
+//   pass 2 (kmeans_update_finalize_kernel): item = (cluster, column slice): the cluster's partials in segment order, / count; the
+//          fp64 sums themselves on request (the fit takes the objective of the assignment from them).
+// Segments are fixed by kKmUpdRows and n alone, never by the grid, so every launch on every device adds the same numbers in the same
+// order: the centroids are the same bits from run to run. A cluster holding most rows spreads over many pass-1 items.
+constexpr int kKmUpdRows = 256;        // perm positions per pass-1 segment
+constexpr int kKmUpdThreads = 128;
+// Rows per unrolled group. ptxas interleaves a group's adds with its loads (2-3 rows in flight per thread). At 32 registers an SM
+// holds 2048 threads, so that is ~80 KB of loads in flight per SM, about twice HBM latency x bandwidth / 148 SMs.
+constexpr int kKmUpdUnroll = 8;
+
+struct KmeansUpdateParams {
+  const float* x;                      // [n, dim]
+  const long long* idx;                // [n] cluster of each row
+  const long long* perm;               // [n] rows cluster by cluster
+  const long long* offsets;            // [n_centroids + 1] first perm position of each cluster, offsets[n_centroids] = n
+  double* partials;                    // [n_centroids + ceil(n / kKmUpdRows)][dim]
+  float* centroids;                    // [n_centroids, dim], rewritten for non-empty clusters
+  double* sums;                        // [n_centroids, dim] the fp64 sums of the clusters (0 for empty ones), or nullptr
+  long long n;
+  int dim, n_centroids;
+};
+
+__device__ __forceinline__ void acc4(double (&a)[4], const float4 v) {
+  a[0] += v.x; a[1] += v.y; a[2] += v.z; a[3] += v.w;
+}
+
+// grid (ceil(n / kKmUpdRows), ceil(dim / 4 / blockDim.x)); thread <-> 4 consecutive columns
+__global__ void __launch_bounds__(kKmUpdThreads) kmeans_update_partial_kernel(const KmeansUpdateParams p) {
+  __shared__ long long s_row[kKmUpdRows];
+  const long long seg = blockIdx.x;
+  const long long pos0 = seg * kKmUpdRows;
+  const int rows = static_cast<int>(min(static_cast<long long>(kKmUpdRows), p.n - pos0));
+  for (int i = threadIdx.x; i < rows; i += blockDim.x) s_row[i] = __ldg(p.perm + pos0 + i);
+  __syncthreads();
+  const int d4 = p.dim / 4;
+  const int q = blockIdx.y * blockDim.x + threadIdx.x;
+  const bool active = q < d4;
+  const float4* x4 = reinterpret_cast<const float4*>(p.x) + q;
+  int i = 0;
+  while (i < rows) {   // block-uniform: one cluster run of the segment per trip
+    const long long c = __ldg(p.idx + s_row[i]);
+    if (c < 0 || c >= p.n_centroids) break;                          // inconsistent idx / offsets: stop rather than run away
+    const int end = static_cast<int>(min(static_cast<long long>(rows), __ldg(p.offsets + c + 1) - pos0));
+    if (end <= i) break;
+    if (active) {
+      double a[4] = {0.0, 0.0, 0.0, 0.0};
+      int r = i;
+      for (; r + kKmUpdUnroll <= end; r += kKmUpdUnroll) {
+        float4 v[kKmUpdUnroll];
+#pragma unroll
+        for (int u = 0; u < kKmUpdUnroll; ++u) v[u] = __ldg(x4 + s_row[r + u] * d4);
+#pragma unroll
+        for (int u = 0; u < kKmUpdUnroll; ++u) acc4(a, v[u]);
+      }
+      for (; r < end; ++r) acc4(a, __ldg(x4 + s_row[r] * d4));
+      double2* dst = reinterpret_cast<double2*>(p.partials + (c + seg) * p.dim) + 2 * q;
+      dst[0] = make_double2(a[0], a[1]);
+      dst[1] = make_double2(a[2], a[3]);
+    }
+    i = end;
+  }
+}
+
+// grid (n_centroids, ceil(dim / blockDim.x)); thread <-> column
+__global__ void __launch_bounds__(kKmUpdThreads) kmeans_update_finalize_kernel(const KmeansUpdateParams p) {
+  const int c = blockIdx.x;
+  const int col = blockIdx.y * blockDim.x + threadIdx.x;
+  if (col >= p.dim) return;
+  const long long a = __ldg(p.offsets + c), b = __ldg(p.offsets + c + 1);
+  const long long o = static_cast<long long>(c) * p.dim + col;
+  double s = 0.0;
+  if (b > a) {
+    const long long j0 = a / kKmUpdRows, j1 = (b - 1) / kKmUpdRows;
+    const double* src = p.partials + (c + j0) * p.dim + col;
+#pragma unroll 4
+    for (long long j = j0; j <= j1; ++j, src += p.dim) s += *src;
+    p.centroids[o] = __double2float_rn(s / static_cast<double>(b - a));
+  }
+  if (p.sums != nullptr) p.sums[o] = s;
+}
+
 }  // namespace edm

@@ -325,6 +325,19 @@ def normalize_clip(x: torch.Tensor) -> torch.Tensor:
     return (x - x.mean()) / torch.sqrt(x.var(unbiased=False) + 1e-7)
 
 
+def _prep_clip(clip: torch.Tensor, device, normalize: bool) -> torch.Tensor:
+    clip = clip.to(device, torch.float32)
+    return normalize_clip(clip) if normalize else clip
+
+
+def _check_clips(clips) -> None:
+    if not isinstance(clips, (list, tuple)) or len(clips) == 0:
+        raise ValueError("clips must be a non-empty list of [L_i] tensors")
+    for c in clips:
+        if not torch.is_tensor(c) or c.dim() != 1:
+            raise ValueError("every clip must be a 1-D [L_i] tensor")
+
+
 class SemanticTokenizer:
     """Semantic tokens of the reference's tokenizer (semantic_tokenizer_hubert.py encode / encode_batch): HuBERT features of
     `hubert.output_layer` followed by the nearest k-means centroid (KMeansAssigner, edm_kmeans_assign).
@@ -340,9 +353,24 @@ class SemanticTokenizer:
         self.normalize = bool(normalize)
         self.assigner = KMeansAssigner(cluster_centers, device=hubert.device)
 
+    @classmethod
+    @torch.no_grad()
+    def fit(cls, hubert: HubertFeatures, clips, n_centroids: int = 1024, normalize: bool = True, **fit_kw):
+        """Fit the k-means centroids on the HuBERT features of `clips` ([L_i] at 16 kHz) and build a tokenizer on them; replaces the
+        reference's offline step (utility_scripts/hubert_kmeans/: features dumped to .npy, then faiss k-means). The clips get the same
+        normalisation as encode_batch; their features stay on the device and never go to disk: 4 KB of fp32 per 20 ms frame, so about
+        4 GB per million frames (5.6 h of audio), held twice while they are concatenated. fit_kw go to kmeans.fit_kmeans (niter, seed,
+        max_points_per_centroid, init). Returns (SemanticTokenizer, KMeansFit)."""
+        from .kmeans import fit_kmeans
+
+        _check_clips(clips)
+        feats = hubert.forward_batch([_prep_clip(c, hubert.device, normalize) for c in clips])
+        feats = torch.cat(feats)
+        fit = fit_kmeans(feats, n_centroids=n_centroids, device=hubert.device, **fit_kw)
+        return cls(hubert, fit.centroids, normalize=normalize), fit
+
     def _prep(self, clip):
-        clip = clip.to(self.hubert.device, torch.float32)
-        return normalize_clip(clip) if self.normalize else clip
+        return _prep_clip(clip, self.hubert.device, self.normalize)
 
     @torch.no_grad()
     def encode(self, audio: torch.Tensor) -> torch.Tensor:
@@ -355,11 +383,7 @@ class SemanticTokenizer:
     @torch.no_grad()
     def encode_batch(self, clips) -> list:
         """List of [L_i] clips at 16 kHz -> list of int64 [T_i] cluster ids (views of one buffer); item i equals encode(clips[i][None])[0]."""
-        if not isinstance(clips, (list, tuple)) or len(clips) == 0:
-            raise ValueError("clips must be a non-empty list of [L_i] tensors")
-        for c in clips:
-            if not torch.is_tensor(c) or c.dim() != 1:
-                raise ValueError("every clip must be a 1-D [L_i] tensor")
+        _check_clips(clips)
         feats = self.hubert.forward_batch([self._prep(c) for c in clips])
         ids = self.assigner.assign(torch.cat(feats))
         return list(torch.split(ids, [f.shape[0] for f in feats]))

@@ -123,6 +123,19 @@ int edm_codes_to_features(const long long* codes, const float* proj, float* out,
 int edm_kmeans_assign(const float* x, long long n_frames, int dim, const float* c_hi, const float* c_lo,
                       const float* half_neg_norm, int n_centroids, long long* idx_out, float* score_out, void* stream);
 
+/* Centroid update of one Lloyd iteration (the k-means fit of the semantic tokenizer; the reference fits offline with faiss,
+ * utility_scripts/hubert_kmeans/): centroids[c] = (sum of rows x[r] with idx[r] == c) / count_c, accumulated in fp64 and rounded once
+ * to fp32, written in place; clusters with count 0 keep their row. perm [n] lists the rows cluster by cluster (e.g. the indices of
+ * a stable sort of idx), offsets [n_centroids + 1] the first position of each cluster in perm (offsets[n_centroids] = n). Every idx
+ * must lie in [0, n_centroids): for an id outside it nothing is read or written out of bounds, but a segment stops summing there, so
+ * the centroids of the clusters after it in that segment are wrong (edm_tts_b200/kmeans.py checks the ids first). The sum of
+ * each cluster is taken in a fixed order that depends on n only, so the result is the same bits for any device and run.
+ * partials: fp64 scratch of edm_kmeans_update_workspace_bytes(n, dim, n_centroids) bytes. sums_out (nullable) [n_centroids, dim]
+ * receives the fp64 sums of the clusters (0 for empty ones). dim % 32 == 0, 1 <= n_centroids <= 4096; x and partials 16-byte aligned. */
+size_t edm_kmeans_update_workspace_bytes(long long n, int dim, int n_centroids);
+int edm_kmeans_update(const float* x, long long n, int dim, const long long* idx, const long long* perm, const long long* offsets,
+                      int n_centroids, double* partials, float* centroids, double* sums_out, void* stream);
+
 /* One convolution of the DAC encoder as an implicit GEMM on tcgen05 (bf16 operands, fp32 accumulate), channel-last activations.
  * Replaces each WNConv1d (+ the Snake1d in front of the NEXT conv, + the ResidualUnit add) of edm_tts/models/dac/encoder.py:11-58 /
  * nn_layers.py:8-47 (run under bf16 autocast by utility_scripts/dump_tokens/dump_tokens.py:213).
