@@ -76,6 +76,7 @@ _SIGNATURES = {
     "edm_s2a_bind": (_i, [_vp, _vp, _sz, _i, _i, _i]),
     "edm_s2a_workspace_bytes_varlen": (_sz, [_vp, _i, _vp, _vp]),
     "edm_s2a_bind_varlen": (_i, [_vp, _vp, _sz, _i, _vp, _vp, _vp]),
+    "edm_s2a_bind_masked": (_i, [_vp, _vp, _sz, _i, _vp, _vp, _vp]),
     "edm_s2a_buffer": (_vp, [_vp, C.c_char_p, C.POINTER(_sz)]),
     "edm_s2a_set_batch_offset": (_i, [_vp, _ll]),
     "edm_s2a_set_seed_buffer": (_i, [_vp, _vp]),

@@ -1183,12 +1183,13 @@ struct edm_s2a_ctx {
   bool bound = false;
   int B = 0, T = 0, P = 0, N = 0, M = 0, Mt = 0, Mp = 0, max_n = 0, min_t = 0;
   bool varlen = false;
+  bool masked = false;             // edm_s2a_bind_masked: varlen, with the known rows anywhere in their sequence (lay.tgt_enc / lay.enc_slot)
   SeqLayout lay;                   // where the sequences are (device arrays in the workspace after a varlen bind)
   const int* pairs = nullptr;      // varlen: attention (sequence, query pair) list in the workspace, longest first
   int n_pairs = 0;
   double attn_flops = 0.0;
   ConvRuns conv_runs;              // varlen: runs of the streaming conv kernel
-  int* layout_dev = nullptr;       // varlen: the layout arrays in the workspace (cu_n | cu_t | cu_runs | pairs)
+  int* layout_dev = nullptr;       // varlen: the layout arrays in the workspace (cu_n | cu_t | cu_runs | pairs [| tgt_enc | enc_slot])
   std::vector<int> host_layout;    // varlen: their host image
   uint8_t* ws = nullptr;
   size_t ws_bytes = 0;
@@ -1199,7 +1200,7 @@ struct edm_s2a_ctx {
   __nv_bfloat16 *z, *h, *qkv, *g, *zt, *fine_h, *fine_z;
   int *ids, *ids_raw, *pred_codes, *pred_raw, *fine_codes, *sem_tokens, *sem_prompt, *ac_prompt;
   uint8_t *mask_a, *mask_b, *mask_raw;
-  const float* prompt_proj = nullptr;            // optional caller-projected prompt injections [n_inj, B*P, 1024] (edm_s2a_set_prompt_injections)
+  const float* prompt_proj = nullptr;            // optional caller-projected prompt injections [n_inj, sum P_s, 1024] (edm_s2a_set_prompt_injections)
   const unsigned long long* seed_dev = nullptr;  // optional device-resident seed offset (edm_s2a_set_seed_buffer)
   int ac_levels = 0;
   long long batch_offset = 0;  // global index of this context's first sequence (Philox counters)
@@ -1431,6 +1432,10 @@ int varlen_shape(const edm_s2a_ctx* c, int n_seq, const int* T, const int* P, si
   *M = m; *Mt = mt; *Mp = mp; *n_pairs = static_cast<int>(pairs);
   return 0;
 }
+
+// ints of the layout arrays of a varlen or masked bind: cu_n | cu_t | cu_runs [n_seq + 1 each] | attention pairs | tgt_enc [Mt] |
+// enc_slot [M]. A varlen bind leaves the two row maps unused, so both binds need the same workspace for the same T_s / P_s.
+size_t varlen_layout_ints(int n_seq, size_t M, size_t Mt, int n_pairs) { return 3 * (static_cast<size_t>(n_seq) + 1) + n_pairs + Mt + M; }
 }  // namespace
 
 extern "C" size_t edm_s2a_workspace_bytes(const edm_s2a_ctx* ctx, int B, int T, int P) {
@@ -1443,7 +1448,7 @@ extern "C" size_t edm_s2a_workspace_bytes_varlen(const edm_s2a_ctx* ctx, int n_s
   size_t M, Mt, Mp;
   int n_pairs;
   if (varlen_shape(ctx, n_seq, T, P, &M, &Mt, &Mp, &n_pairs)) return 0;
-  return carve(const_cast<edm_s2a_ctx*>(ctx), nullptr, n_seq, M, Mt, Mp, 3 * (static_cast<size_t>(n_seq) + 1) + n_pairs, false);
+  return carve(const_cast<edm_s2a_ctx*>(ctx), nullptr, n_seq, M, Mt, Mp, varlen_layout_ints(n_seq, M, Mt, n_pairs), false);
 }
 
 extern "C" int edm_s2a_bind(edm_s2a_ctx* c, void* workspace, size_t bytes, int B, int T, int P) {
@@ -1457,7 +1462,7 @@ extern "C" int edm_s2a_bind(edm_s2a_ctx* c, void* workspace, size_t bytes, int B
   carve(c, static_cast<uint8_t*>(workspace), B, B * N, static_cast<size_t>(B) * T, static_cast<size_t>(B) * P, 0, true);
   c->ws = static_cast<uint8_t*>(workspace); c->ws_bytes = bytes;
   c->B = B; c->T = T; c->P = P; c->N = P + T; c->M = B * (P + T); c->Mt = B * T; c->Mp = B * P; c->max_n = P + T; c->min_t = T;
-  c->varlen = false; c->lay = uniform_layout(B, P + T, T); c->pairs = nullptr; c->n_pairs = 0; c->conv_runs = ConvRuns();
+  c->varlen = false; c->masked = false; c->lay = uniform_layout(B, P + T, T); c->pairs = nullptr; c->n_pairs = 0; c->conv_runs = ConvRuns();
   c->attn_flops = 4.0 * B * 16 * static_cast<double>(c->N) * c->N * 64;
   c->host_layout.clear();
   c->prompt_proj = nullptr;
@@ -1473,19 +1478,22 @@ extern "C" int edm_s2a_bind(edm_s2a_ctx* c, void* workspace, size_t bytes, int B
   return 0;
 }
 
-extern "C" int edm_s2a_bind_varlen(edm_s2a_ctx* c, void* workspace, size_t bytes, int n_seq, const int* T, const int* P, void* stream) {
+namespace {
+// edm_s2a_bind_varlen (target == nullptr: the P_s prompt rows lead each sequence) and edm_s2a_bind_masked (target[row] != 0 marks the
+// target rows, the others are the known rows): the host image of every layout array goes to the workspace in one copy on `stream`.
+int bind_packed(edm_s2a_ctx* c, void* workspace, size_t bytes, int n_seq, const int* T, const int* P, const unsigned char* target, void* stream) {
   if (c == nullptr || workspace == nullptr) return fail(EDM_ERR_INVALID, "bind arguments");
   if ((reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) return fail(EDM_ERR_INVALID, "workspace must be 1024-byte aligned");
   size_t M, Mt, Mp;
   int n_pairs;
   if (int rc = varlen_shape(c, n_seq, T, P, &M, &Mt, &Mp, &n_pairs)) return rc;
-  const size_t n1 = static_cast<size_t>(n_seq) + 1, layout_ints = 3 * n1 + n_pairs;
+  const size_t n1 = static_cast<size_t>(n_seq) + 1, layout_ints = varlen_layout_ints(n_seq, M, Mt, n_pairs);
   const size_t need = carve(c, nullptr, n_seq, M, Mt, Mp, layout_ints, false);
   if (bytes < need) return fail(EDM_ERR_INVALID, "workspace too small: %zu < %zu", bytes, need);
   c->bound = false;
   carve(c, static_cast<uint8_t*>(workspace), n_seq, M, Mt, Mp, layout_ints, true);
   int* dev = c->layout_dev;
-  // host image of the layout arrays: cu_n | cu_t | cu_runs | pairs
+  // host image of the layout arrays: cu_n | cu_t | cu_runs | pairs | tgt_enc | enc_slot
   std::vector<int> lens(n_seq);
   std::vector<int>& h = c->host_layout;
   h.assign(3 * n1, 0);
@@ -1503,12 +1511,33 @@ extern "C" int edm_s2a_bind_varlen(edm_s2a_ctx* c, void* workspace, size_t bytes
   const int run_len = conv_run_len(n_seq, lens.data(), 0, num_sms());
   for (int i = 0; i < n_seq; ++i) h[2 * n1 + i + 1] = h[2 * n1 + i] + (lens[i] + run_len - 1) / run_len;
   append_attention_pairs(lens, &h);
-  EDM_CUDA(cudaMemcpyAsync(dev, h.data(), layout_ints * sizeof(int), cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream)));
+  const size_t maps = h.size();  // tgt_enc starts here, enc_slot Mt ints later
+  if (target != nullptr) {
+    h.resize(layout_ints, 0);
+    int* tgt_enc = h.data() + maps;
+    int* enc_slot = tgt_enc + Mt;
+    int r = 0;
+    for (int i = 0; i < n_seq; ++i) {
+      int t = 0, k = 0;
+      for (int row = h[i]; row < h[i + 1]; ++row) {
+        if (target[row]) {
+          tgt_enc[r++] = row;
+          enc_slot[row] = t++;
+        } else {
+          enc_slot[row] = -1 - k++;
+        }
+      }
+    }
+  }
+  EDM_CUDA(cudaMemcpyAsync(dev, h.data(), (target != nullptr ? layout_ints : maps) * sizeof(int), cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream)));
   c->ws = static_cast<uint8_t*>(workspace); c->ws_bytes = bytes;
   c->B = n_seq; c->T = 0; c->P = 0; c->N = 0;
   c->M = static_cast<int>(M); c->Mt = static_cast<int>(Mt); c->Mp = static_cast<int>(Mp); c->max_n = max_n; c->min_t = min_t;
   c->varlen = true;
+  c->masked = target != nullptr;
   c->lay.n_seq = n_seq; c->lay.N = 0; c->lay.T = 0; c->lay.cu_n = dev; c->lay.cu_t = dev + n1; c->lay.rows = c->M; c->lay.t_rows = c->Mt;
+  c->lay.tgt_enc = c->masked ? dev + maps : nullptr;
+  c->lay.enc_slot = c->masked ? dev + maps + Mt : nullptr;
   c->conv_runs.run_len = run_len; c->conv_runs.cu_runs = dev + 2 * n1; c->conv_runs.num_units = h[2 * n1 + n_seq];
   c->pairs = dev + 3 * n1; c->n_pairs = n_pairs;
   c->attn_flops = flops;
@@ -1524,6 +1553,27 @@ extern "C" int edm_s2a_bind_varlen(edm_s2a_ctx* c, void* workspace, size_t bytes
   c->bound = true;
   return 0;
 }
+}  // namespace
+
+extern "C" int edm_s2a_bind_varlen(edm_s2a_ctx* c, void* workspace, size_t bytes, int n_seq, const int* T, const int* P, void* stream) {
+  return bind_packed(c, workspace, bytes, n_seq, T, P, nullptr, stream);
+}
+
+extern "C" int edm_s2a_bind_masked(edm_s2a_ctx* c, void* workspace, size_t bytes, int n_seq, const int* N, const unsigned char* target, void* stream) {
+  if (c == nullptr || n_seq <= 0 || n_seq >= (1 << 15) || N == nullptr || target == nullptr) return fail(EDM_ERR_INVALID, "bind_masked arguments (n_seq=%d)", n_seq);
+  std::vector<int> T(n_seq), P(n_seq);
+  size_t row = 0;
+  for (int i = 0; i < n_seq; ++i) {
+    if (N[i] <= 0 || N[i] > c->cfg.max_positions) return fail(EDM_ERR_INVALID, "sequence %d: N=%d outside [1, %d]", i, N[i], c->cfg.max_positions);
+    int t = 0;
+    for (int n = 0; n < N[i]; ++n) t += target[row + n] != 0;
+    row += N[i];
+    if (t == 0) return fail(EDM_ERR_INVALID, "sequence %d: no target row", i);
+    T[i] = t;
+    P[i] = N[i] - t;
+  }
+  return bind_packed(c, workspace, bytes, n_seq, T.data(), P.data(), target, stream);
+}
 
 extern "C" void* edm_s2a_buffer(edm_s2a_ctx* c, const char* name, size_t* bytes) {
   if (c == nullptr || !c->bound || name == nullptr) return nullptr;
@@ -1536,7 +1586,8 @@ extern "C" void* edm_s2a_buffer(edm_s2a_ctx* c, const char* name, size_t* bytes)
       {"logits", c->logits, Mt * 1024 * 4}, {"coarse_logits", c->coarse_logits, c->keep_logits ? 4 * Mt * 1024 * 4 : 0},
       {"fine_logits", c->fine_logits, c->keep_logits ? Mt * c->n_fine * 1024 * 4 : 0}, {"logp", c->logp, Mt * 4}, {"ids", c->ids, Mt * 4},
       {"ids_raw", c->ids_raw, Mt * 4}, {"pred_codes", c->pred_codes, Mt * 16}, {"pred_raw", c->pred_raw, Mt * 16},
-      {"fine_codes", c->fine_codes, Mt * c->n_fine * 4}, {"mask", c->mask_cur(), Mt}, {"mask_raw", c->mask_raw, Mt}};
+      {"fine_codes", c->fine_codes, Mt * c->n_fine * 4}, {"mask", c->mask_cur(), Mt}, {"mask_raw", c->mask_raw, Mt},
+      {"tgt_enc", const_cast<int*>(c->lay.tgt_enc), c->masked ? Mt * 4 : 0}, {"enc_slot", const_cast<int*>(c->lay.enc_slot), c->masked ? M * 4 : 0}};
   for (auto& e : tab)
     if (strcmp(e.n, name) == 0) {
       if (bytes) *bytes = e.b;
@@ -1608,7 +1659,7 @@ extern "C" int edm_s2a_set_low_latency(edm_s2a_ctx* c, int on) {
 
 extern "C" int edm_s2a_set_prompt_injections(edm_s2a_ctx* c, const float* proj) {
   if (c == nullptr) return fail(EDM_ERR_INVALID, "null context");
-  if (c->varlen && proj != nullptr) return fail(EDM_ERR_STATE, "feature-valued prompt injections need a uniform bind (edm_s2a_bind)");
+  if (c->varlen && !c->masked && proj != nullptr) return fail(EDM_ERR_STATE, "feature-valued prompt injections need a uniform or masked bind");
   c->prompt_proj = proj;
   return 0;
 }

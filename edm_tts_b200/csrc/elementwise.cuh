@@ -128,7 +128,7 @@ struct LnParams {
   const float *w1, *b1, *w2, *b2;
   float* y_out;           // nullable
   __nv_bfloat16* z_out;   // nullable
-  SeqLayout lay;          // compact != 0: the bf16 store keeps only target rows, encoder row of (s, P_s + t) -> target row of (s, t)
+  SeqLayout lay;          // compact != 0: the bf16 store keeps only target rows, encoder row of target t of s -> target row of (s, t)
   int compact;
   float eps;
   int reverse;            // 1: rows are walked from the last to the first (L2 reuse of the producer's most recent output)
@@ -173,9 +173,9 @@ __global__ void __launch_bounds__(256, 3) layernorm_kernel(const LnParams p) {
     if (p.compact) {
       int s, n;
       p.lay.enc_pos(row, s, n);
-      const int np = p.lay.p_len(s);
-      if (n < np) return;
-      zrow = p.lay.t_start(s) + (n - np);
+      const int t = p.lay.slot(row, s, n);
+      if (t < 0) return;
+      zrow = p.lay.t_start(s) + t;
     }
     if (p.w2 != nullptr) row_layernorm(v, p.w2, p.b2, lane, p.eps);
     row_store_bf16(p.z_out + zrow * kD, lane, v);
@@ -239,9 +239,9 @@ __global__ void __launch_bounds__(256) layernorm_splitk_kernel(const LnParams p)
     if (p.compact) {
       int s, n;
       p.lay.enc_pos(row, s, n);
-      const int np = p.lay.p_len(s);
-      if (n < np) return;
-      zrow = p.lay.t_start(s) + (n - np);
+      const int t = p.lay.slot(row, s, n);
+      if (t < 0) return;
+      zrow = p.lay.t_start(s) + t;
     }
     if (p.w2 != nullptr) row_layernorm(v, p.w2, p.b2, lane, p.eps);
     row_store_bf16(p.z_out + zrow * kD, lane, v);
@@ -445,17 +445,18 @@ __global__ void __launch_bounds__(256) build_input_kernel(const BuildInputParams
   if (row >= p.rows) return;
   int b, n;
   p.lay.enc_pos(row, b, n);
-  const int np = p.lay.p_len(b);
+  const int t = p.lay.slot(row, b, n);
   float v[32];
-  if (n < np) {
+  if (t < 0) {
+    const int k = -1 - t;  // k-th known row of sequence b
     const long long pb = p.lay.p_start(b);
-    const int code = clamp_index(p.ac_prompt[static_cast<long long>(p.ac_prompt_levels) * pb + n], kV);  // level 0
+    const int code = clamp_index(p.ac_prompt[static_cast<long long>(p.ac_prompt_levels) * pb + k], kV);  // level 0
     row_load_f32_ldg(p.feat_table + static_cast<long long>(code) * kD, lane, v);
     row_add_f32_ldg(p.feat_const, lane, v);
     row_layernorm(v, p.fp_ln_w, p.fp_ln_b, lane, p.eps);
-    row_add_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_prompt[pb + n], p.num_semantic)) * kD, lane, v);
+    row_add_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_prompt[pb + k], p.num_semantic)) * kD, lane, v);
   } else {
-    row_load_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_tokens[p.lay.t_start(b) + (n - np)], p.num_semantic)) * kD, lane, v);
+    row_load_f32_ldg(p.sem_emb + static_cast<long long>(clamp_index(p.sem_tokens[p.lay.t_start(b) + t], p.num_semantic)) * kD, lane, v);
     row_add_f32_ldg(p.mask_token, lane, v);
   }
   row_store_f32(p.x + static_cast<long long>(row) * kD, lane, v);
@@ -507,7 +508,7 @@ __global__ void __launch_bounds__(256) update_input_kernel(const UpdateInputPara
 // Reference: injection_conformer_wrapper.py:107-129. At injection layer k (level k):
 //   inj = LN_k(Linear_k(sum_{i<=k} W_out_i codebook_i[code_i] + b_out_i)) = LN_k(sum_i inj_table[k][i][code_i] + inj_const[k])
 //   x   = block_out + inj + (k > 0 ? previous coarse block_out : 0)
-// code_i comes from the arg-max of this pass for target rows and from the acoustic prompt for prompt rows.
+// code_i comes from the arg-max of this pass for target rows and from the acoustic prompt for prompt (known) rows.
 struct InjectParams {
   float* x;                 // out: encoder rows [sum N_s, 1024]
   const float* cur_out;     // block output at this injection layer (coarse_out[k])
@@ -532,18 +533,18 @@ __global__ void __launch_bounds__(256) inject_kernel(const InjectParams p) {
   if (row >= p.rows) return;
   int b, n;
   p.lay.enc_pos(static_cast<int>(row), b, n);
-  const int np = p.lay.p_len(b);
+  const int t = p.lay.slot(static_cast<int>(row), b, n);
   float v[32];
-  if (n < np && p.prompt_proj != nullptr) {
-    row_load_f32_ldg(p.prompt_proj + (p.lay.p_start(b) + static_cast<long long>(n)) * kD, lane, v);
+  if (t < 0 && p.prompt_proj != nullptr) {
+    row_load_f32_ldg(p.prompt_proj + (p.lay.p_start(b) + static_cast<long long>(-1 - t)) * kD, lane, v);
   } else {
     row_load_f32_ldg(p.inj_const, lane, v);
     for (int i = 0; i <= p.level; ++i) {
       int code;
-      if (n < np)
-        code = p.ac_prompt[static_cast<long long>(p.ac_prompt_levels) * p.lay.p_start(b) + static_cast<long long>(i) * np + n];
+      if (t < 0)
+        code = p.ac_prompt[static_cast<long long>(p.ac_prompt_levels) * p.lay.p_start(b) + static_cast<long long>(i) * p.lay.p_len(b) + (-1 - t)];
       else
-        code = p.pred_codes[p.lay.out_offset(b, i, 4, n - np)];
+        code = p.pred_codes[p.lay.out_offset(b, i, 4, t)];
       row_add_f32_ldg(p.tables[i] + static_cast<long long>(clamp_index(code, kV)) * kD, lane, v);
     }
   }

@@ -7,6 +7,11 @@
 //   [Q, T_s] blocks (codes, coarse ids)   sequence s starts at Q * cu_t[s]
 // A uniform batch (every sequence N rows, T of them targets) is the same layout with cu_n[s] = s N and cu_t[s] = s T; it is
 // described without arrays (cu_n == nullptr) and the helpers reduce to those closed forms.
+// Masked layout (edm_s2a_bind_masked, speech editing): the P_s prompt ("known") rows of a sequence may sit anywhere among its N_s rows,
+// not only in front. Two more arrays say where: tgt_enc maps target row -> encoder row, enc_slot maps encoder row -> target index t
+// (>= 0) or -1 - k for the sequence's k-th known row in time order; per-sequence prompt data (tokens, codes, projected injections) keeps
+// the known rows in that order. Without these arrays (every other bind) the known rows are the prefix and the helpers keep their
+// closed forms.
 #pragma once
 
 namespace edm {
@@ -17,6 +22,8 @@ struct SeqLayout {
   const int* cu_n;   // [n_seq + 1] first encoder row of each sequence, cu_n[n_seq] = total rows; nullptr: uniform
   const int* cu_t;   // [n_seq + 1] first target row of each sequence
   int rows, t_rows;  // totals (sum N_s, sum T_s), for the host side of a launch
+  const int* tgt_enc = nullptr;   // [t_rows] encoder row of every target row; nullptr: target t of sequence s is row n_start(s) + p_len(s) + t
+  const int* enc_slot = nullptr;  // [rows] target index, or -1 - (index among the sequence's known rows); nullptr: the known rows are the prefix
 
   __device__ __forceinline__ bool packed() const { return cu_n != nullptr; }
   __device__ __forceinline__ int n_start(int s) const { return packed() ? __ldg(cu_n + s) : s * N; }
@@ -55,7 +62,17 @@ struct SeqLayout {
       t = r - s * T;
     }
   }
-  __device__ __forceinline__ long long enc_row(int s, int t) const { return static_cast<long long>(n_start(s)) + p_len(s) + t; }
+  __device__ __forceinline__ long long enc_row(int s, int t) const {
+    if (tgt_enc != nullptr) return __ldg(tgt_enc + t_start(s) + t);
+    return static_cast<long long>(n_start(s)) + p_len(s) + t;
+  }
+  // encoder row `row` (position n of sequence s, from enc_pos) -> its target index t >= 0, or -1 - k when it is the sequence's k-th
+  // known row (prompt data of sequence s at p_start(s) + k)
+  __device__ __forceinline__ int slot(int row, int s, int n) const {
+    if (enc_slot != nullptr) return __ldg(enc_slot + row);
+    const int np = p_len(s);
+    return n < np ? -1 - n : n - np;
+  }
   // element (q, t) of sequence s in a buffer of per-sequence [Q, T_s] blocks
   __device__ __forceinline__ long long out_offset(int s, int q, int Q, int t) const {
     return static_cast<long long>(Q) * t_start(s) + static_cast<long long>(q) * t_len(s) + t;

@@ -107,15 +107,24 @@ class _Encoder:
         self._m = model
 
     @staticmethod
-    def _prompt_len(x, mask_time_indices):
+    def _layout(x, mask_time_indices):
+        """-> (P, target): a common suffix [:, P:] of target rows (mask None: P = 0) runs on the uniform bind (target None); any other
+        boolean mask with the same count in every row (the reference's .view(b, ...)) on the masked bind (target: the mask on the host)."""
+        B, N = x.shape[:2]
         if mask_time_indices is None:
-            return 0
-        first = mask_time_indices[0].to(torch.int64).argmax().item() if mask_time_indices[0].any() else x.shape[1]
-        expect = torch.zeros_like(mask_time_indices)
-        expect[:, first:] = True
-        if not torch.equal(expect, mask_time_indices):
-            raise ValueError("mask_time_indices must select a common suffix [:, P:] of every sequence (as infer_special builds it)")
-        return int(first)
+            return 0, None
+        m = mask_time_indices.to("cpu", torch.bool)
+        if tuple(m.shape) != (B, N):
+            raise ValueError(f"mask_time_indices must be [b, n] = {(B, N)}, got {tuple(m.shape)}")
+        counts = m.sum(1)
+        if not bool((counts == counts[0]).all()):
+            raise ValueError("mask_time_indices must select the same number of positions in every sequence")
+        T = int(counts[0])
+        if T == 0:
+            raise ValueError("mask_time_indices selects no position")
+        if bool(m[:, N - T:].all()):
+            return N - T, None
+        return N - T, m
 
     @_on_device
     def forward_first_level(self, x, mask=None, mask_time_indices=None):
@@ -127,8 +136,11 @@ class _Encoder:
         if B > MAX_CHUNK:
             return torch.cat([self.forward_first_level(x[i:i + MAX_CHUNK], None, None if mask_time_indices is None else mask_time_indices[i:i + MAX_CHUNK])
                               for i in range(0, B, MAX_CHUNK)])
-        P = self._prompt_len(x, mask_time_indices)
-        m._bind(B, N - P, P)
+        P, target = self._layout(x, mask_time_indices)
+        if target is None:
+            m._bind(B, N - P, P)
+        else:
+            m._bind_masked([N] * B, target)
         xf = x.float().contiguous()
         L.check(L.lib().edm_s2a_first_level(m._ctx, L.ptr(xf), L.stream_ptr()), "first_level")
         return m._view("logits", (B, 1, N - P, m.num_codevectors), torch.float32).clone()
@@ -137,29 +149,33 @@ class _Encoder:
     def forward(self, x, mask=None, injections=None, acoustic_model=None, mask_time_indices=None, *, prompt_codes=None,
                 forced_coarse=None):
         """injection_conformer_wrapper.py:92-150 in eval mode -> logits [b, q, t, codes] (fp32).
-        Prompt rows are injected either from `injections` -- the reference's argument: one feature tensor [b, n, 1024] per injection
-        layer (cumulative DAC features of the prompt, zeros on the target rows), projected here with project_injection[k].0 on the
-        tensor cores -- or from the acoustic prompt *codes* (prompt_codes [b, >=4, P]) through the folded tables, which is what
-        infer_special does. `acoustic_model` is accepted for signature compatibility (the model's own folded tables are used)."""
+        Prompt rows (the rows mask_time_indices leaves out: a prefix, or any rows with the same count per sequence) are injected either
+        from `injections` -- the reference's argument: one feature tensor [b, n, 1024] per injection layer (cumulative DAC features of
+        the prompt, zeros on the target rows), projected here with project_injection[k].0 on the tensor cores -- or from the acoustic
+        prompt *codes* (prompt_codes [b, >=4, P], the prompt rows in time order) through the folded tables, which is what infer_special
+        does. `acoustic_model` is accepted for signature compatibility (the model's own folded tables are used)."""
         assert mask is None, "the S2A decode path never passes a padding mask"
         m = self._m
         x = x.to(m.device)
         B, N, _ = x.shape
         if B > MAX_CHUNK:
             raise ValueError(f"encoder.forward takes at most {MAX_CHUNK} sequences per call (infer_special chunks larger batches itself)")
-        P = self._prompt_len(x, mask_time_indices)
+        P, target = self._layout(x, mask_time_indices)
         n_inj = len(m.injection_layers)
         if P > 0 and prompt_codes is None and injections is None:
-            raise ValueError("a prompt prefix needs its injections: pass injections=[features per injection layer] or prompt_codes=<acoustic prompt tokens>")
-        m._bind(B, N - P, P, keep_logits=True)
+            raise ValueError("prompt rows need their injections: pass injections=[features per injection layer] or prompt_codes=<acoustic prompt tokens>")
+        if target is None:
+            m._bind(B, N - P, P, keep_logits=True)
+        else:
+            m._bind_masked([N] * B, target, keep_logits=True)
         L.check(L.lib().edm_s2a_set_prompt_injections(m._ctx, None), "set_prompt_injections")
         keep = None
         if P > 0 and prompt_codes is not None:
-            m._load_prompt_codes(prompt_codes)
+            m._load_prompt_codes(prompt_codes, B * (N - P), B * P)
         elif P > 0:
             if len(injections) < n_inj:
                 raise IndexError("one injection tensor per injection layer is required")   # reference: list index out of range
-            m._load_prompt_codes(torch.zeros(B, n_inj, P, dtype=torch.int64))
+            m._load_prompt_codes(torch.zeros(B, n_inj, P, dtype=torch.int64), B * (N - P), B * P)
             # project_injection[k].0 on the prompt rows (bf16 operands as under autocast, fp32 accumulate + bias), LayerNorm in the kernel
             w = m._w
             keep = torch.empty(n_inj, B * P, 1024, device=m.device, dtype=torch.float32)
@@ -167,7 +183,7 @@ class _Encoder:
                 inj = injections[k].to(m.device)
                 if tuple(inj.shape) != (B, N, 1024):
                     raise ValueError(f"injections[{k}] must be [b, n, 1024], got {tuple(inj.shape)}")
-                a = inj[:, :P].reshape(B * P, 1024).to(torch.bfloat16).contiguous()
+                a = (inj[:, :P] if target is None else inj[~target.to(m.device)]).reshape(B * P, 1024).to(torch.bfloat16).contiguous()
                 L.check(L.lib().edm_gemm_bf16(L.ptr(a), 1024, L.ptr(w["inj_w"][k]), 1024, B * P, 1024, 1024, L.EPI_F32, L.ptr(w["inj_b"][k]),
                                               L.ptr(keep[k]), 1024, 1.0, None, None, 1, 0, L.stream_ptr()), "gemm")
                 del a
@@ -374,6 +390,29 @@ class InjectionConformerModel:
         L.check(lib.edm_s2a_bind_varlen(self._ctx, self._ws.data_ptr(), self._ws.numel(), n, t_arr, p_arr, L.stream_ptr()), "bind_varlen")
         self._bound = key
 
+    def _bind_masked(self, N, target, keep_logits=False):
+        """Packed workspace for utterances of N[i] frames whose targets are marked in `target` (host bool, all utterances
+        concatenated; edm_s2a_bind_masked)."""
+        tb = target.to("cpu", torch.uint8).contiguous().reshape(-1).numpy().tobytes()
+        key = ("masked", tuple(N), tb, bool(keep_logits))
+        if self._bound == key:
+            return
+        lib = L.lib()
+        L.check(lib.edm_s2a_set_keep_logits(self._ctx, int(bool(keep_logits))), "set_keep_logits")
+        n, cu = len(N), varlen.offsets(N)
+        T = [tb[cu[i]:cu[i + 1]].count(1) for i in range(n)]
+        t_arr, p_arr, n_arr = (C.c_int * n)(*T), (C.c_int * n)(*[a - b for a, b in zip(N, T)]), (C.c_int * n)(*N)
+        need = lib.edm_s2a_workspace_bytes_varlen(self._ctx, n, t_arr, p_arr)
+        if need == 0:
+            raise ValueError("invalid infill batch: " + lib.edm_last_error().decode("utf-8", "replace"))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = None
+            self._ws = torch.empty(need, device=self.device, dtype=torch.uint8)
+        self._bound = None
+        tgt = (C.c_ubyte * len(tb)).from_buffer_copy(tb)
+        L.check(lib.edm_s2a_bind_masked(self._ctx, self._ws.data_ptr(), self._ws.numel(), n, n_arr, tgt, L.stream_ptr()), "bind_masked")
+        self._bound = key
+
     def _view(self, name, shape, dtype):
         nbytes = C.c_size_t(0)
         p = L.lib().edm_s2a_buffer(self._ctx, name.encode(), C.byref(nbytes))
@@ -387,11 +426,10 @@ class InjectionConformerModel:
         assert numel * esz <= nbytes.value, (name, shape, nbytes.value)
         return self._ws[off:off + numel * esz].view(dtype).view(*shape)
 
-    def _load_prompt_codes(self, prompt_codes):
-        B, T, P = self._bound[:3]
+    def _load_prompt_codes(self, prompt_codes, n_target, n_prompt):
         pc = prompt_codes.to(self.device, torch.int32).contiguous()
-        dummy_sem = torch.zeros(B, T, device=self.device, dtype=torch.int32)
-        dummy_sp = torch.zeros(B, P, device=self.device, dtype=torch.int32)
+        dummy_sem = torch.zeros(n_target, device=self.device, dtype=torch.int32)
+        dummy_sp = torch.zeros(n_prompt, device=self.device, dtype=torch.int32)
         L.check(L.lib().edm_s2a_build_input(self._ctx, L.ptr(dummy_sem), L.ptr(dummy_sp), L.ptr(pc), pc.shape[1], L.stream_ptr()), "build_input")
 
     def set_low_latency(self, on=True):
@@ -465,7 +503,6 @@ class InjectionConformerModel:
         infer_special(semantic_tokens[i][None], ..., batch_offset=batch_offset + i)[0] (outside low-latency mode). The keyword extras
         are per-utterance lists shaped as infer_special's extras for one utterance: cat_gumbel[i] [S-1, T_i, codes], remask_gumbel[i]
         [S-1, 1, T_i], forced_ids[i] [S, 1, T_i], forced_masks[i] [S-1, 1, T_i], forced_coarse[i] [1, 4, T_i]."""
-        dev, lib = self.device, L.lib()
         if not isinstance(semantic_tokens, (list, tuple)) or len(semantic_tokens) == 0:
             raise ValueError("semantic_tokens must be a non-empty list of [T_i] tensors")
         n = len(semantic_tokens)
@@ -497,25 +534,36 @@ class InjectionConformerModel:
                 _check_range(a, self.num_codevectors, "acoustic_prompt_tokens")
                 _check_range(x, self.config.num_semantic_tokens, "semantic_prompt_tokens")
             P = [int(x.shape[0]) for x in sp]
-        S = int(steps)
+        self._check_extras(T, int(steps), cat_gumbel=cat_gumbel, remask_gumbel=remask_gumbel, forced_ids=forced_ids, forced_masks=forced_masks,
+                           forced_coarse=forced_coarse)
+        q = int(acoustic_prompt_tokens[0].shape[0]) if has_prompt else 0
+        return self._decode_packed(T, P, semantic_tokens, semantic_prompt_tokens if has_prompt else None,
+                                   acoustic_prompt_tokens if has_prompt else None, q, None, int(steps), temperature, seed, batch_offset,
+                                   cat_gumbel, remask_gumbel, forced_ids, forced_masks, forced_coarse)
+
+    def _check_extras(self, T, S, **extras):
+        """The per-utterance parity extras of infer_batch / infill_batch: shapes as infer_special's for one utterance of T[i] targets."""
         V = self.num_codevectors
-        extras = dict(cat_gumbel=(cat_gumbel, lambda t: (S - 1, t, V)), remask_gumbel=(remask_gumbel, lambda t: (S - 1, 1, t)),
-                      forced_ids=(forced_ids, lambda t: (S, 1, t)), forced_masks=(forced_masks, lambda t: (S - 1, 1, t)),
-                      forced_coarse=(forced_coarse, lambda t: (1, 4, t)))
-        for name, (lst, shape) in extras.items():
+        shapes = dict(cat_gumbel=lambda t: (S - 1, t, V), remask_gumbel=lambda t: (S - 1, 1, t), forced_ids=lambda t: (S, 1, t),
+                      forced_masks=lambda t: (S - 1, 1, t), forced_coarse=lambda t: (1, 4, t))
+        for name, lst in extras.items():
             if lst is None:
                 continue
-            if not isinstance(lst, (list, tuple)) or len(lst) != n:
+            if not isinstance(lst, (list, tuple)) or len(lst) != len(T):
                 raise ValueError(f"{name} must be a list with one entry per utterance")
             for i, x in enumerate(lst):
-                if tuple(x.shape) != shape(T[i]):
-                    raise ValueError(f"{name}[{i}] must be {shape(T[i])}, got {tuple(x.shape)}")
-        if forced_ids is not None:
-            for x in forced_ids:
-                _check_range(x, V, "forced_ids")
-        if forced_coarse is not None:
-            for x in forced_coarse:
-                _check_range(x, V, "forced_coarse")
+                if tuple(x.shape) != shapes[name](T[i]):
+                    raise ValueError(f"{name}[{i}] must be {shapes[name](T[i])}, got {tuple(x.shape)}")
+        for name in ("forced_ids", "forced_coarse"):
+            for x in extras.get(name) or ():
+                _check_range(x, V, name)
+
+    def _decode_packed(self, T, P, sem_target, sem_known, codes_known, q, target, S, temperature, seed, batch_offset, cat_gumbel,
+                       remask_gumbel, forced_ids, forced_masks, forced_coarse):
+        """Chunks of MAX_CHUNK utterances through one packed bind each: the varlen bind (target None: the P[i] prompt frames lead), or
+        the masked bind (target: per-utterance bool masks). Per-target inputs are lists over the targets of each utterance, per-known
+        inputs (sem_known [P_i], codes_known [q, P_i]) over its prompt / known frames, both in time order."""
+        dev, lib = self.device, L.lib()
         Q = self.num_quantizers
         out = torch.empty(Q * sum(T), device=dev, dtype=torch.int64)
 
@@ -524,10 +572,14 @@ class InjectionConformerModel:
 
         for ch in varlen.plan(T, P, MAX_CHUNK, batch_offset):
             sl = slice(ch.start, ch.stop)
-            self._bind_varlen(ch.T, ch.P)
-            sem = cat(semantic_tokens, sl, 0, torch.int32)
-            spc = cat(semantic_prompt_tokens, sl, 0, torch.int32) if has_prompt else None
-            apc = torch.cat([a.to(dev).reshape(-1) for a in acoustic_prompt_tokens[sl]]).to(torch.int32).contiguous() if has_prompt else None
+            if target is None:
+                self._bind_varlen(ch.T, ch.P)
+            else:
+                self._bind_masked([t + p for t, p in zip(ch.T, ch.P)], torch.cat(target[sl]))
+            known = codes_known is not None and sum(ch.P) > 0
+            sem = cat(sem_target, sl, 0, torch.int32)
+            spc = cat(sem_known, sl, 0, torch.int32) if known else None
+            apc = torch.cat([a.to(dev).reshape(-1) for a in codes_known[sl]]).to(torch.int32).contiguous() if known else None
             cg = cat(cat_gumbel, sl, 1, torch.float32)
             rg = cat(remask_gumbel, sl, 2, torch.float32)
             fi = cat(forced_ids, sl, 2, torch.int32)
@@ -535,10 +587,36 @@ class InjectionConformerModel:
             fc = None if forced_coarse is None else torch.cat([x.to(dev).reshape(-1) for x in forced_coarse[sl]]).to(torch.int32).contiguous()
             codes = out[Q * ch.t0:Q * (ch.t0 + sum(ch.T))]
             L.check(lib.edm_s2a_set_batch_offset(self._ctx, ch.batch_offset), "set_batch_offset")
-            L.check(lib.edm_s2a_decode(self._ctx, L.ptr(sem), L.ptr(spc), L.ptr(apc), int(acoustic_prompt_tokens[0].shape[0]) if has_prompt else 0,
+            L.check(lib.edm_s2a_decode(self._ctx, L.ptr(sem), L.ptr(spc), L.ptr(apc), q if codes_known is not None else 0,
                                        S, float(temperature), int(seed), L.ptr(cg), L.ptr(rg), L.ptr(fi), L.ptr(fm), L.ptr(fc), L.ptr(codes),
                                        L.stream_ptr()), "decode")
         return varlen.split_blocks(out, T, Q)
+
+    @torch.no_grad()
+    @_on_device
+    def infill_batch(self, semantic_tokens, acoustic_tokens, regenerate, steps=8, temperature=1.0, *, seed=0, batch_offset=0,
+                     cat_gumbel=None, remask_gumbel=None, forced_ids=None, forced_masks=None, forced_coarse=None):
+        """Speech editing: regenerate the chosen frames of each utterance given the others (the S2A model's training objective,
+        modeling_injection_conformer.py:96-102, at inference). semantic_tokens: list of [N_i]; acoustic_tokens: list of [q, N_i] codes
+        (one q in [1, 12]; the values at regenerated frames are ignored); regenerate: list of bool [N_i], at least one True each.
+        The other frames are known and treated exactly as prompt frames (input sem + LN(Linear(feat_0)), never sampled or re-masked,
+        injected with the cumulative ground-truth features of their first min(4, q) levels; q must cover every injection layer when
+        any frame is known). Returns a list of LongTensor [12, T_i] (T_i = regenerate[i].sum()): the codes of the regenerated frames in
+        time order, views of one packed output. With the known frames in front this is infer_batch with them as prompts, bit for bit;
+        target t of utterance i draws Philox counter (batch_offset + i) T_i + t. Chunks of 64 utterances at batch offsets
+        batch_offset + 64 c. The keyword extras are per-utterance lists shaped as infer_batch's for T_i targets."""
+        sp = varlen.infill_split(semantic_tokens, acoustic_tokens, regenerate, self.num_codevectors, self.config.num_semantic_tokens,
+                                 self.num_quantizers)
+        T, P = list(sp.T), list(sp.P)
+        if steps > 1 and min(T) < 2:
+            raise IndexError("re-masking needs at least 2 frames to regenerate (the reference's take_along_dim is out of range for T = 1 with steps > 1)")
+        q = int(acoustic_tokens[0].shape[0])
+        if sum(P) > 0 and q < len(self.injection_layers):
+            raise IndexError("known frames need at least one code level per injection layer")  # reference: list index out of range
+        self._check_extras(T, int(steps), cat_gumbel=cat_gumbel, remask_gumbel=remask_gumbel, forced_ids=forced_ids, forced_masks=forced_masks,
+                           forced_coarse=forced_coarse)
+        return self._decode_packed(T, P, sp.sem_target, sp.sem_known, sp.codes_known, q, sp.target, int(steps), temperature, seed,
+                                   batch_offset, cat_gumbel, remask_gumbel, forced_ids, forced_masks, forced_coarse)
 
     @torch.no_grad()
     @_on_device

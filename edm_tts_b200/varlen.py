@@ -5,6 +5,8 @@ S2A (edm_s2a_bind_varlen): utterance i has T_i target and P_i prompt frames. Pac
 per-frame data of utterance i starts at cu_t[i] (targets) or cu_p[i] (prompt), a per-utterance [Q, T_i] block at Q * cu_t[i]. With
 equal lengths this is the [B, ...] layout of a uniform batch.
 
+S2A infilling (edm_s2a_bind_masked): the same with the known (prompt) frames anywhere in their utterance, see infill_split.
+
 DAC decoder (DACDecoder.forward_batch): the utterances are packed along time with zero gap rows between them, see dac_pack.
 DAC encoder (DACEncoder.forward_batch): the same idea for the downsampling stack, see enc_pack.
 """
@@ -46,6 +48,90 @@ def split_blocks(packed, T, Q: int) -> list:
     """Views [Q, T_i] of a flat packed buffer of per-utterance [Q, T_i] blocks."""
     cu = offsets(T)
     return [packed[Q * cu[i]:Q * cu[i + 1]].view(Q, T[i]) for i in range(len(T))]
+
+
+# ---------------------------------------------------------------------------------------------------------------------------------
+# S2A infilling (edm_s2a_bind_masked): utterance i has N_i frames, T_i >= 1 of them marked to regenerate (targets), the other
+# P_i = N_i - T_i known. Per-target data is packed as a varlen batch with T_i targets, per-known data as its prompt of P_i frames, both
+# in time order; the encoder rows keep the utterance's own frame order.
+
+
+@dataclass(frozen=True)
+class Infill:
+    """An infill batch split into what the masked bind takes: per utterance the frame count, the target / known counts, the
+    semantic tokens of the targets and of the known frames, the codes [q, P_i] of the known frames and the bool target mask."""
+    N: tuple
+    T: tuple
+    P: tuple
+    sem_target: list
+    sem_known: list
+    codes_known: list
+    target: list
+
+
+def infill_split(semantic_tokens, acoustic_tokens, regenerate, num_codes: int, num_semantic: int, max_levels: int = 12) -> Infill:
+    """Checks an infill batch (lists of semantic tokens [N_i], acoustic codes [q, N_i] with one q in [1, max_levels], bool masks [N_i]
+    of the frames to regenerate) and splits it into targets and known frames. Malformed lists or shapes and an utterance with no frame
+    to regenerate raise ValueError; a semantic token or a known frame's code out of range raises IndexError (the codes at regenerated
+    frames are ignored)."""
+    import torch
+
+    lists = (semantic_tokens, acoustic_tokens, regenerate)
+    if any(not isinstance(x, (list, tuple)) for x in lists) or len(semantic_tokens) == 0:
+        raise ValueError("semantic_tokens, acoustic_tokens and regenerate must be non-empty lists")
+    n = len(semantic_tokens)
+    if len(acoustic_tokens) != n or len(regenerate) != n:
+        raise ValueError(f"{n} semantic token lists, {len(acoustic_tokens)} acoustic and {len(regenerate)} regenerate masks")
+    if any(not torch.is_tensor(x) for lst in lists for x in lst):
+        raise ValueError("every entry must be a tensor")
+    q = int(acoustic_tokens[0].shape[0]) if acoustic_tokens[0].dim() == 2 else -1
+    N, T = [], []
+    for i, (st, ac, rg) in enumerate(zip(*lists)):
+        if st.dim() != 1 or ac.dim() != 2 or rg.dim() != 1:
+            raise ValueError(f"utterance {i}: expected semantic [N], acoustic [q, N] and regenerate [N] tensors")
+        if int(ac.shape[0]) != q or not 1 <= q <= max_levels:
+            raise ValueError(f"utterance {i}: every acoustic entry needs the same number of levels q in [1, {max_levels}]")
+        if ac.shape[1] != st.shape[0] or rg.shape[0] != st.shape[0]:
+            raise ValueError(f"utterance {i}: {st.shape[0]} semantic tokens, {ac.shape[1]} acoustic frames, {rg.shape[0]} mask entries")
+        if rg.dtype != torch.bool:
+            raise ValueError(f"regenerate[{i}] must be a bool tensor")
+        t = int(rg.sum())
+        if t < 1:
+            raise ValueError(f"utterance {i} has no frame to regenerate")
+        N.append(int(st.shape[0]))
+        T.append(t)
+    sem_t, sem_k, codes_k, tgt = [], [], [], []
+    for i, (st, ac, rg) in enumerate(zip(*lists)):
+        rg = rg.to(st.device)
+        if st.numel() and (int(st.min()) < 0 or int(st.max()) >= num_semantic):
+            raise IndexError(f"semantic_tokens[{i}]: index out of range [0, {num_semantic})")
+        known = ac[:, ~rg.to(ac.device)]
+        if known.numel() and (int(known.min()) < 0 or int(known.max()) >= num_codes):
+            raise IndexError(f"acoustic_tokens[{i}]: a known frame's code is out of range [0, {num_codes})")
+        sem_t.append(st[rg])
+        sem_k.append(st[~rg])
+        codes_k.append(known)
+        tgt.append(rg)
+    return Infill(tuple(N), tuple(T), tuple(a - b for a, b in zip(N, T)), sem_t, sem_k, codes_k, tgt)
+
+
+def infill_rows(target) -> tuple[list[int], list[int]]:
+    """Row maps of a masked bind for the bool masks `target` [N_i] of its utterances (what edm_s2a_bind_masked builds on the host):
+    tgt_enc[r] = packed encoder row of packed target row r; enc_slot[row] = target index t inside the utterance, or -1 - k for its
+    k-th known frame."""
+    tgt_enc, enc_slot, row = [], [], 0
+    for m in target:
+        t = k = 0
+        for v in (bool(x) for x in m):
+            if v:
+                tgt_enc.append(row)
+                enc_slot.append(t)
+                t += 1
+            else:
+                enc_slot.append(-1 - k)
+                k += 1
+            row += 1
+    return tgt_enc, enc_slot
 
 
 # ---------------------------------------------------------------------------------------------------------------------------------

@@ -248,11 +248,23 @@ int edm_s2a_bind(edm_s2a_ctx* ctx, void* workspace, size_t bytes, int B, int T, 
  * With equal lengths this is byte for byte the layout of edm_s2a_bind. Row t of utterance i draws the Philox counter
  * (batch_offset + i) * T_i + t, what a single-utterance call with batch offset batch_offset + i draws, so utterance i decodes to the
  * same bits as edm_s2a_bind(1, T_i, P_i) with that offset (outside low-latency mode). Copies the layout arrays into the workspace
- * on `stream`. edm_s2a_set_prompt_injections(non-NULL) is refused (EDM_ERR_STATE) under this bind. */
+ * on `stream`. edm_s2a_set_prompt_injections(non-NULL) is refused (EDM_ERR_STATE) under this bind (edm_s2a_bind_masked takes it). */
 size_t edm_s2a_workspace_bytes_varlen(const edm_s2a_ctx* ctx, int n_seq, const int* T, const int* P);
 int edm_s2a_bind_varlen(edm_s2a_ctx* ctx, void* workspace, size_t bytes, int n_seq, const int* T, const int* P, void* stream);
 
-/* named views into the bound workspace (for parity tests / the Python mirror): returns device pointer or NULL */
+/* Masked bind (speech editing: regenerate any chosen frames of an utterance given the others). Sequence i has N[i] encoder rows
+ * packed back to back; target[row] != 0 (host array, sum N[i] bytes) marks the T_i >= 1 rows to regenerate, the other
+ * P_i = N[i] - T_i rows are known rows and are treated exactly as prompt rows: input sem + LN(Linear(feat_0(code))), never sampled or
+ * re-masked, injected with the cumulative ground-truth features of their levels. Everything per target row (semantic tokens, noise,
+ * forced ids and masks, output codes) is laid out as under edm_s2a_bind_varlen with T_i targets, in time order; everything per known row
+ * (semantic prompt tokens, [q, P_i] acoustic codes, edm_s2a_set_prompt_injections rows) as its prompt of P_i frames, in time order.
+ * The Philox counter of target t is (batch_offset + i) * T_i + t, so with the known rows in front this is edm_s2a_bind_varlen with
+ * P = N - T, bit for bit. The workspace is edm_s2a_workspace_bytes_varlen(n_seq, T, P = N - T). Sequences with no target row or with
+ * N[i] > max_positions are refused. Copies the layout arrays into the workspace on `stream`. */
+int edm_s2a_bind_masked(edm_s2a_ctx* ctx, void* workspace, size_t bytes, int n_seq, const int* N, const unsigned char* target, void* stream);
+
+/* named views into the bound workspace (for parity tests / the Python mirror): returns device pointer or NULL. "tgt_enc" / "enc_slot"
+ * are the row maps of a masked bind (target row -> encoder row; encoder row -> target index t, or -1 - k for the k-th known row). */
 void* edm_s2a_buffer(edm_s2a_ctx* ctx, const char* name, size_t* bytes);
 
 /* Global index of this context's first sequence inside the caller's whole batch. The in-kernel Philox counters are
