@@ -121,9 +121,7 @@ class DAC:
     @torch.no_grad()
     def decode(self, z: torch.Tensor, length=None) -> dict:
         """z [B, D, T] -> {"audio": [B, 1, length]} (modeling_dac.py:141-161)."""
-        if self.decoder is None:
-            raise RuntimeError("this DAC was built without decoder weights")
-        x = self.decoder(z)
+        x = self._decoder_or_raise()(z)
         return {"audio": x[..., :length]}
 
     def decode_from_codes(self, codes: torch.Tensor, length=None) -> torch.Tensor:

@@ -12,7 +12,8 @@ a few guard rows in front and behind for the rows of the view that fall outside 
 
 forward_batch decodes latents of different lengths together: they are packed along time with zero gap rows between them
 (varlen.dac_pack), the same launches run with B = 1 over the packed rows, and edm_dac_zero_rows clears the gap rows of every bf16
-operand a multi-tap conv reads next, so each utterance sees exactly the zero padding it sees when decoded alone.
+operand a multi-tap conv reads next, so each utterance sees exactly the zero padding it sees when decoded alone. Weight packing,
+workspaces, launch wrappers and the gap clears are shared with the encoder (dac_stack.py).
 """
 from __future__ import annotations
 
@@ -22,7 +23,7 @@ import torch
 
 from . import _lib as L
 from . import varlen
-from .dac_encoder import _fold
+from .dac_stack import ConvStack, _fold, pack_alpha, pack_conv, padded
 from .varlen import conv_transpose_length
 
 _G = 8          # guard rows in front of every stage buffer (>= the largest transposed-conv padding)
@@ -44,34 +45,17 @@ def pack_conv_transpose(wt: torch.Tensor, stride: int, c_out_pad: int) -> torch.
     return wp.reshape(stride * c_out_pad, 2 * c_in)
 
 
-class DACDecoder:
+class DACDecoder(ConvStack):
     def __init__(self, state_dict: dict, input_channel: int = 1024, channels: int = 1536, rates=(8, 5, 4, 2), prefix: str = "",
                  device="cuda", max_chunk_samples: int = 1 << 21):
-        if not torch.cuda.is_available():
-            raise L.EdmError("edm_tts_b200 needs a CUDA device (sm_100); there is no CPU fallback")
+        super().__init__(device, max_chunk_samples)
         if input_channel % 64 != 0 or channels % 64 != 0 or channels > 1536 or max(rates) // 2 > _G:
             raise ValueError("the conv kernels need input / first-stage channel counts that are multiples of 64 (first stage <= 1536)")
-        self.device = dev = torch.device(device)
         self.input_channel, self.channels, self.rates = input_channel, channels, tuple(rates)
         self.hop_length = math.prod(rates)
-        self.max_chunk_samples = max_chunk_samples
         sd = {k: v.detach().to("cpu") for k, v in state_dict.items() if k.startswith(prefix)}
-
-        def padded(v, n, fill=0.0):
-            out = torch.full((n,), fill, dtype=torch.float32)
-            out[: v.numel()] = v.float().reshape(-1)
-            return out.to(dev).contiguous()
-
-        def conv(key, c_in_p, c_out_p):
-            w = _fold(sd, key)                                                   # [c_out, c_in, k]
-            wp = torch.zeros(c_out_p, w.shape[2], c_in_p)
-            wp[: w.shape[0], :, : w.shape[1]] = w.permute(0, 2, 1)               # K index = tap * c_in_p + channel
-            return wp.reshape(c_out_p, -1).to(dev, torch.bfloat16).contiguous(), padded(sd[key + ".bias"], c_out_p)
-
-        def alpha(key, n):
-            return padded(sd[key + ".alpha"], n, 1.0)
-
-        self.w_first, self.b_first = conv(f"{prefix}model.0", input_channel, channels)
+        dev = self.device
+        self.w_first, self.b_first = pack_conv(sd, f"{prefix}model.0", input_channel, channels, dev)
         self.blocks = []
         c_in = channels
         n = 1
@@ -84,25 +68,20 @@ class DACDecoder:
             units = []
             for u in range(3):
                 ru = f"{blk}{2 + u}.block."
-                w7, b7 = conv(ru + "1", cp, cp)
-                w1, b1 = conv(ru + "3", cp, cp)
-                units.append(dict(a_in=alpha(ru + "0", cp), w7=w7, b7=b7, a_mid=alpha(ru + "2", cp), w1=w1, b1=b1))
-            self.blocks.append(dict(stride=s, c_in=c_in, c=cp, a_up=alpha(blk + "0", c_in), wt=wp.to(dev, torch.bfloat16).contiguous(),
-                                    bt=padded(sd[blk + "1.bias"], cp), units=units))
+                w7, b7 = pack_conv(sd, ru + "1", cp, cp, dev)
+                w1, b1 = pack_conv(sd, ru + "3", cp, cp, dev)
+                units.append(dict(a_in=pack_alpha(sd, ru + "0", cp, dev), w7=w7, b7=b7, a_mid=pack_alpha(sd, ru + "2", cp, dev), w1=w1, b1=b1))
+            self.blocks.append(dict(stride=s, c_in=c_in, c=cp, a_up=pack_alpha(sd, blk + "0", c_in, dev), wt=wp.to(dev, torch.bfloat16).contiguous(),
+                                    bt=padded(sd[blk + "1.bias"], cp, 0.0, dev), units=units))
             c_in = cp
             n += 1
         c_last = channels // 2 ** len(self.rates)
-        self.a_last = alpha(f"{prefix}model.{n}", c_in)
+        self.a_last = pack_alpha(sd, f"{prefix}model.{n}", c_in, dev)
         w_last = _fold(sd, f"{prefix}model.{n + 1}")                             # [1, c_last, 7]
         wl = torch.zeros(7, c_in)
         wl[:, :c_last] = w_last[0].t()
         self.w_last = wl.to(dev).contiguous()
         self.b_last = float(sd[f"{prefix}model.{n + 1}.bias"].reshape(-1)[0])
-        self._ws = {}
-        self._pws = None
-
-    def eval(self):
-        return self
 
     # ------------------------------------------------------------------ geometry / workspace
     def lengths(self, T: int):
@@ -129,41 +108,7 @@ class DACDecoder:
         ws["audio"] = torch.empty(B, lens[-1], device=dev, dtype=torch.float32)
         return ws
 
-    def _workspace(self, B: int, T: int):
-        key = (B, T)
-        ws = self._ws.get(key)
-        if ws is not None:
-            return ws
-        # keep two geometries (a batch that does not divide into equal chunks alternates between two chunk sizes; re-allocating
-        # per chunk costs more than the kernels), drop the oldest beyond that: the buffers are large
-        while len(self._ws) >= 2:
-            self._ws.pop(next(iter(self._ws)))
-        ws = self._alloc(B, self.lengths(T))
-        self._ws[key] = ws
-        return ws
-
-    def _packed_workspace(self, rows0: int):
-        """Grow-only workspace of the packed path, sized for rows0 packed latent rows (stage k: rows0 * r_1 ... r_k rows). The chunks
-        of a list have different geometries; re-allocating per chunk would cost more than the kernels."""
-        if self._pws is None or self._pws["lens"][0] < rows0:
-            self._pws = None                                                     # release the smaller one first
-            lens = [rows0]
-            for s in self.rates:
-                lens.append(lens[-1] * s)
-            self._pws = self._alloc(1, lens)
-        return self._pws
-
-    # ------------------------------------------------------------------ launches (raw addresses: the stage buffers are used through
-    # views that start at a guard-row offset)
-    def _conv(self, a_ptr, a_rows, a_cols, a_bs, w, bias, taps, step, off, rows_out, B, alpha=None, period=0, x_res=None, y=None, y_bs=0,
-              s_out=None, s_bs=0, s_rows=0):
-        L.check(L.lib().edm_dac_conv(a_ptr, a_rows, a_cols, a_bs, B, L.ptr(w), w.shape[0], taps, step, off, rows_out, L.ptr(bias), L.ptr(alpha),
-                                     period, x_res, y, y_bs, s_out, s_bs, 0, s_rows, None, 0, L.stream_ptr()), "dac_conv")
-
-    def _resunit(self, a_ptr, a_bs, B, rows, c, dilation, ru, a_next, y_ptr, y_bs, s_ptr, s_bs):
-        L.check(L.lib().edm_dac_resunit(a_ptr, a_bs, B, rows, c, dilation, L.ptr(ru["w7"]), L.ptr(ru["w1"]), L.ptr(ru["b7"]), L.ptr(ru["a_mid"]),
-                                        L.ptr(ru["b1"]), L.ptr(a_next), y_ptr, y_bs, s_ptr, s_bs, 0, rows, L.stream_ptr()), "dac_resunit")
-
+    # ------------------------------------------------------------------ forward
     @torch.no_grad()
     def forward(self, z: torch.Tensor) -> torch.Tensor:
         """z [B, input_channel, T] (fp32 / bf16) -> audio fp32 [B, 1, L]."""
@@ -221,7 +166,7 @@ class DACDecoder:
                     a_next = self.blocks[k + 1]["a_up"] if k + 1 < len(self.blocks) else self.a_last
                 cur_ptr, oth_ptr = cur.data_ptr() + _G * c * 2, oth.data_ptr() + _G * c * 2
                 if c in _FUSED:
-                    self._resunit(cur_ptr, bs, B, Lk, c, d, ru, a_next, y_ptr, bs, oth_ptr, bs)
+                    self._resunit(cur_ptr, bs, B, Lk, c, d, ru, a_next, y_ptr, bs, oth_ptr, bs, 0, Lk)
                 else:
                     sm = ws["sm"][k]
                     self._conv(cur_ptr, Lk, c, bs, ru["w7"], ru["b7"], 7, d, -3 * d, Lk, B, alpha=ru["a_mid"], s_out=sm.data_ptr(), s_bs=Lk * c, s_rows=Lk)
@@ -256,26 +201,14 @@ class DACDecoder:
         """z [input_channel, sum(T)]: the latents of the list back to back -> list of [1, L_i] audio views."""
         plan = varlen.dac_plan(T, self.rates, self.max_chunk_samples)
         out = torch.empty(sum(ch.rows[-1] for ch in plan), device=self.device, dtype=torch.float32)
-        ws = self._packed_workspace(max(ch.rows[0] for ch in plan))
-        # one upload per call: the gap ranges of every chunk and stage ((start, end) pairs), then the packed row of every latent frame
-        host, at = [], []
-        for ch in plan:
-            at.append([])
-            for k in range(len(self.rates) + 1):
-                g = ch.gaps(k)
-                at[-1].append((len(host), len(g), max(e - b for b, e in g)))
-                host += g
-        n_pairs = len(host)
-        host = [v for g in host for v in g] + [a + t for ch in plan for a, n in zip(ch.starts[0], ch.lengths[0]) for t in range(n)]
-        dev_buf = torch.tensor(host, dtype=torch.int32).to(self.device)
-        rows_of_frame = dev_buf[2 * n_pairs:].long()
+        ws = self._packed_workspace(max(ch.rows for ch in plan))                # the largest chunk: rows[0] decides
+        # one upload per call: the gap ranges of every chunk and stage, then the packed row of every latent frame
+        frame_rows = [a + t for ch in plan for a, n in zip(ch.starts[0], ch.lengths[0]) for t in range(n)]
+        buf, clears = self._upload_gaps([[ch.gaps(k) for k in range(len(self.rates) + 1)] for ch in plan], frame_rows)
+        rows_of_frame = buf[buf.numel() - len(frame_rows):].long()
         zin = ws["zin"][0]
         views, o0 = [], 0
-        for ch, at_ch in zip(plan, at):
-            def clear(k, ptr, pitch, at_ch=at_ch):
-                first, n, widest = at_ch[k]
-                self._zero_rows(ptr, pitch, dev_buf.data_ptr() + 8 * first, n, widest)
-
+        for ch, clear in zip(plan, clears):
             t1 = ch.t0 + sum(ch.lengths[0])
             zin.index_copy_(0, rows_of_frame[ch.t0:t1], z[:, ch.t0:t1].t())
             clear(0, zin.data_ptr(), self.input_channel * 2)                     # latent gaps: the first conv's zero padding
@@ -283,6 +216,3 @@ class DACDecoder:
             views += [out[o0 + a:o0 + a + n].view(1, n) for a, n in zip(ch.starts[-1], ch.lengths[-1])]
             o0 += ch.rows[-1]
         return views
-
-    def _zero_rows(self, ptr, pitch, ranges_ptr, n, widest):
-        L.check(L.lib().edm_dac_zero_rows(ptr, pitch, ranges_ptr, n, widest, L.stream_ptr()), "dac_zero_rows")

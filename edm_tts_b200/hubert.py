@@ -23,6 +23,7 @@ from dataclasses import dataclass, field
 import torch
 
 from . import _lib as L
+from . import varlen
 
 HOP = 320                # samples per frame: prod(conv_stride)
 _KERNELS = (10, 3, 3, 3, 3, 2, 2)
@@ -154,25 +155,18 @@ def plan(lengths, max_chunk_samples: int) -> list:
     for n in lengths:
         if frame_count(n) <= 0:
             raise ValueError(f"a clip of {n} samples is shorter than one HuBERT frame (400 samples)")
-    slots = [-(-n // HOP) * HOP for n in lengths]
-    chunks, i = [], 0
-    while i < len(lengths):
-        j, tot = i + 1, slots[i]
-        while j < len(lengths) and tot + slots[j] <= max_chunk_samples:
-            tot += slots[j]
-            j += 1
-        starts = [sum(slots[i:k]) for k in range(i, j)]
+    cs = varlen.offsets(-(-n // HOP) * HOP for n in lengths)                    # slot starts: whole frames per clip, back to back
+    chunks = []
+    for i, j in varlen.cut(len(lengths), lambda s, e: cs[e] - cs[s], max_chunk_samples):
+        starts = [cs[k] - cs[i] for k in range(i, j)]
         frames = [frame_count(n) for n in lengths[i:j]]
-        cu = [0]
-        for t in frames:
-            cu.append(cu[-1] + t)
+        cu = varlen.offsets(frames)
         gather = [s // HOP + t for s, T in zip(starts, frames) for t in range(T)]
         pad_starts, pad_map = [], [-1] * POS_PAD
         for T, c0 in zip(frames, cu):
             pad_starts.append(len(pad_map))
             pad_map += list(range(c0, c0 + T)) + [-1] * POS_PAD
-        chunks.append(Chunk(i, j, starts, tot, frames, cu, gather, pad_starts, pad_map))
-        i = j
+        chunks.append(Chunk(i, j, starts, cs[j] - cs[i], frames, cu, gather, pad_starts, pad_map))
     return chunks
 
 
@@ -227,11 +221,7 @@ class HubertFeatures:
 
     @torch.no_grad()
     def forward_batch(self, clips) -> list:
-        if not isinstance(clips, (list, tuple)) or len(clips) == 0:
-            raise ValueError("clips must be a non-empty list of [L_i] tensors")
-        for c in clips:
-            if not torch.is_tensor(c) or c.dim() != 1:
-                raise ValueError("every clip must be a 1-D [L_i] tensor")
+        _check_clips(clips)
         out = []
         for ch in plan([c.shape[0] for c in clips], self.max_chunk_samples):
             x = self._run_chunk(ch, clips[ch.start:ch.stop])

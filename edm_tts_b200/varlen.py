@@ -44,6 +44,19 @@ def plan(T, P, max_chunk: int, batch_offset: int = 0) -> list[Chunk]:
             for s in range(0, len(T), max_chunk)]
 
 
+def cut(n: int, rows, limit: int) -> list[tuple[int, int]]:
+    """Cut items [0, n), in order, into ranges [s, e) whose packed rows rows(s, e) stay within limit; an item that alone exceeds the
+    limit gets a range of its own."""
+    out, s = [], 0
+    while s < n:
+        e = s + 1
+        while e < n and rows(s, e + 1) <= limit:
+            e += 1
+        out.append((s, e))
+        s = e
+    return out
+
+
 def split_blocks(packed, T, Q: int) -> list:
     """Views [Q, T_i] of a flat packed buffer of per-utterance [Q, T_i] blocks."""
     cu = offsets(T)
@@ -168,15 +181,19 @@ def dac_stage_gaps(g0: int, rates) -> list[int]:
     return out
 
 
+def min_gap(stage_gaps, reads) -> int:
+    """Smallest gap g >= 1 whose stage gaps stage_gaps(g) cover every stage's widest one-sided read reads[k]."""
+    g = 1
+    while any(x < n for x, n in zip(stage_gaps(g), reads)):
+        g += 1
+    return g
+
+
 def dac_min_gap(rates) -> int:
     """Smallest latent gap G0 whose gaps cover every stage's widest one-sided read."""
     if any(int(r) < 2 for r in rates):
         raise ValueError(f"transposed-conv strides must be >= 2 (output_padding s % 2 < s), got {tuple(rates)}")
-    need = dac_stage_reads(rates)
-    g0 = 1
-    while any(g < n for g, n in zip(dac_stage_gaps(g0, rates), need)):
-        g0 += 1
-    return g0
+    return min_gap(lambda g: dac_stage_gaps(g, rates), dac_stage_reads(rates))
 
 
 @dataclass(frozen=True)
@@ -221,18 +238,10 @@ def dac_plan(T, rates, max_chunk_samples: int) -> list[DacChunk]:
     """Cut the list, in order, into chunks whose packed audio rows (gaps included) stay within max_chunk_samples; an utterance that
     alone exceeds the limit gets a chunk of its own."""
     g0 = dac_min_gap(rates)
-    hop = 1
-    for r in rates:
-        hop *= r
+    hop = math.prod(rates)
     cu = offsets(T)
-    chunks, s = [], 0
-    while s < len(T):
-        e = s + 1
-        while e < len(T) and hop * (g0 * (e - s + 2) + cu[e + 1] - cu[s]) <= max_chunk_samples:
-            e += 1
-        chunks.append(dac_pack(T[s:e], rates, g0, s, cu[s]))
-        s = e
-    return chunks
+    rows = lambda s, e: hop * (g0 * (e - s + 1) + cu[e] - cu[s])               # | g0 | T_s | g0 | ... | T_e-1 | g0 | in audio rows
+    return [dac_pack(T[s:e], rates, g0, s, cu[s]) for s, e in cut(len(T), rows, max_chunk_samples)]
 
 
 # ---------------------------------------------------------------------------------------------------------------------------------
@@ -274,11 +283,7 @@ def enc_min_gap(rates) -> int:
     """Smallest latent gap G whose gaps cover every stage's widest one-sided read."""
     if not rates or any(int(s) < 2 for s in rates):
         raise ValueError(f"strides must be >= 2 (a stride-1 conv of kernel 2 lengthens the clip into its gap), got {tuple(rates)}")
-    need = enc_stage_reads(rates)
-    g = 1
-    while any(x < n for x, n in zip(enc_stage_gaps(g, rates), need)):
-        g += 1
-    return g
+    return min_gap(lambda g: enc_stage_gaps(g, rates), enc_stage_reads(rates))
 
 
 def enc_rows(frames: int) -> int:
@@ -312,13 +317,6 @@ def enc_plan(L, rates, max_chunk_samples: int) -> list[DacChunk]:
     exceeds the limit gets a chunk of its own."""
     g = enc_min_gap(rates)
     hop = math.prod(rates)
-    cu = offsets(L)
-    chunks, s = [], 0
-    while s < len(L):
-        e, frames = s + 1, g + enc_slot(L[s], hop, g)
-        while e < len(L) and hop * enc_rows(frames + enc_slot(L[e], hop, g)) <= max_chunk_samples:
-            frames += enc_slot(L[e], hop, g)
-            e += 1
-        chunks.append(enc_pack(L[s:e], rates, g, s, cu[s]))
-        s = e
-    return chunks
+    cu, cu_slot = offsets(L), offsets(enc_slot(x, hop, g) for x in L)
+    rows = lambda s, e: hop * enc_rows(g + cu_slot[e] - cu_slot[s])             # enc_pack's rows[0]
+    return [enc_pack(L[s:e], rates, g, s, cu[s]) for s, e in cut(len(L), rows, max_chunk_samples)]

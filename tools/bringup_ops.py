@@ -515,7 +515,8 @@ def test_dacenc():
     the same stack in plain torch (bf16 autocast, channels-first F.conv1d) as the GPU incumbent."""
     import math
     import torch.nn.functional as F
-    from edm_tts_b200.dac_encoder import DACEncoder, _fold
+    from edm_tts_b200.dac_encoder import DACEncoder
+    from edm_tts_b200.dac_stack import _fold
     from edm_tts_b200.synthetic import make_encoder_state_dict
     B, Ls = int(os.environ.get("DAC_B", "8")), int(os.environ.get("DAC_L", "960160"))
     sd = make_encoder_state_dict(64, (2, 4, 5, 8), 0)
@@ -530,18 +531,18 @@ def test_dacenc():
     times = []
     orig = enc._conv
 
-    def timed(a, a_rows, a_cols, w, bias, taps, step, off, rows_out, Bc, **kw):
+    def timed(a, a_rows, a_cols, a_bs, w, bias, taps, step, off, rows_out, Bc, **kw):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        orig(a, a_rows, a_cols, w, bias, taps, step, off, rows_out, Bc, **kw)
+        orig(a, a_rows, a_cols, a_bs, w, bias, taps, step, off, rows_out, Bc, **kw)
         e1.record()
         times.append((f"cin={a_cols} cout={w.shape[0]} taps={taps} step={step} rows={rows_out}", 2.0 * Bc * rows_out * w.shape[0] * w.shape[1], e0, e1))
     orig_ru = enc._resunit
 
-    def timed_ru(src, Bc, rows, c, dilation, ru, *a):
+    def timed_ru(a_ptr, a_bs, Bc, rows, c, dilation, *a):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        orig_ru(src, Bc, rows, c, dilation, ru, *a)
+        orig_ru(a_ptr, a_bs, Bc, rows, c, dilation, *a)
         e1.record()
         times.append((f"fused unit c={c} dilation={dilation} rows={rows}", 2.0 * Bc * rows * c * c * 8, e0, e1))
     enc._conv, enc._resunit = timed, timed_ru
@@ -590,7 +591,7 @@ def test_dacdec():
     stack in plain torch (bf16 autocast) as the GPU incumbent."""
     import torch.nn.functional as F
     from edm_tts_b200.dac_decoder import DACDecoder
-    from edm_tts_b200.dac_encoder import _fold
+    from edm_tts_b200.dac_stack import _fold
     from edm_tts_b200.synthetic import make_decoder_state_dict
     B, T = int(os.environ.get("DAC_B", "16")), int(os.environ.get("DAC_T", "500"))
     sd = make_decoder_state_dict(1024, 1536, (8, 5, 4, 2), 0)
