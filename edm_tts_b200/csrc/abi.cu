@@ -761,6 +761,10 @@ extern "C" int edm_sample(const float* logits, long long ld, int rows, const flo
   if (int rc = check_arch()) return rc;
   SampleParams p;
   if (T <= 0 || Q <= 0) return fail(EDM_ERR_INVALID, "sample: T=%d Q=%d", T, Q);
+  // B = rows / (T Q) sizes the [B, out_q_stride, T] id block: rows left over, or levels outside the stride, would write past it
+  if (rows < 0 || rows % (static_cast<long long>(T) * Q) != 0) return fail(EDM_ERR_INVALID, "sample: rows=%d is not a multiple of T*Q=%d*%d", rows, T, Q);
+  if (out_q0 < 0 || static_cast<long long>(out_q0) + Q > out_q_stride)
+    return fail(EDM_ERR_INVALID, "sample: levels [%d, %d) outside the id stride %d", out_q0, out_q0 + Q, out_q_stride);
   p.logits = logits; p.ld = ld; p.rows = rows; p.noise = noise; p.use_philox = use_philox; p.seed = seed; p.seed_dev = nullptr; p.step = step; p.seq0 = 0;
   p.forced_ids = forced_ids; p.ids = ids; p.ids_raw = nullptr; p.logp = logp; p.lay = uniform_layout(rows / (T * Q), T, T); p.Q = Q;
   p.out_q_stride = out_q_stride; p.out_q0 = out_q0;

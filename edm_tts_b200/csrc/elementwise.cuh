@@ -562,7 +562,8 @@ __global__ void __launch_bounds__(256) inject_kernel(const InjectParams p) {
 }
 
 // ------------------------------------------------------------------------------------------------ sampling
-// Philox4x32-10, counter = (row, column group, step, 0), key = seed.
+// Philox4x32-10, counter = (row counter low word, column group (sampling) or 0x52454d41 (re-masking), step, row counter high word),
+// key = seed (low word, high word). tests/philox_ref.py restates it on the host.
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
 #pragma unroll
   for (int r = 0; r < 10; ++r) {
@@ -574,9 +575,23 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
   }
   return ctr;
 }
+// Standard Gumbel from the top 24 bits k: u = float32(k + 1/2) 2^-24, g = -log(e) with e = -log(u).
+// __logf has an absolute error (about 2^-24 measured near 1, 2^-21.41 documented on [0.5, 2]) that is large against e when u is
+// close to 1, where g is largest and decides the sample: for u > 1 - 2^-10, e comes from v = 1 - u (exact for u >= 1/2) as
+// v + v^2/2 + v^3/3 (relative truncation below 2^-32). Below that, -__logf(u) keeps g within 5.3e-5 of -log(-log(u)) (measured
+// over every k on a B200), and those draws keep the bits the fast path has always given them.
+// k + 1/2 needs 25 bits, so k >= 2^23 rounds to even, and k = 2^24 - 1 rounds to u = 1: v is held at 2^-24 there, which is
+// u = 1 - 2^-24, the largest float below 1, instead of e = 0 and g = +inf. So u lies in [2^-25, 1 - 2^-24] and g in [-2.85, 16.64].
 __device__ __forceinline__ float gumbel_from_bits(uint32_t bits) {
-  const float u = (static_cast<float>(bits >> 8) + 0.5f) * (1.0f / 16777216.0f);  // (0, 1)
-  return -__logf(-__logf(u));
+  const float u = (static_cast<float>(bits >> 8) + 0.5f) * (1.0f / 16777216.0f);
+  float e;
+  if (u > 1.0f - 0x1p-10f) {
+    const float v = fmaxf(1.0f - u, 0x1p-24f);
+    e = v * (1.0f + v * (0.5f + v * (1.0f / 3.0f)));
+  } else {
+    e = -__logf(u);
+  }
+  return -__logf(e);
 }
 
 // One warp per row of 1024 logits. id = argmax(logit + gumbel) (first index wins ties); logp = log softmax(logits)[id].

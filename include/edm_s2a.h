@@ -91,7 +91,8 @@ int edm_conv_module_varlen(const void* in, int glu_input, void* out, const float
 
 /* Per-row arg-max / Gumbel-max sampling over 1024 logits + log-softmax of the chosen id.
  * rows = B*T*Q; ids land at ids[(b*out_q_stride + out_q0 + q)*T + t]. noise: [rows,1024] Gumbel or NULL;
- * use_philox: in-kernel noise when noise == NULL. Replaces modeling_injection_conformer.py:185,192,203-207,228. */
+ * use_philox: in-kernel noise when noise == NULL. rows must be a multiple of T*Q and 0 <= out_q0, out_q0 + Q <= out_q_stride
+ * (EDM_ERR_INVALID otherwise). Replaces modeling_injection_conformer.py:185,192,203-207,228. */
 int edm_sample(const float* logits, long long ld, int rows, const float* noise, int use_philox,
                unsigned long long seed, unsigned step, const int* forced_ids, int* ids, float* logp, int T, int Q,
                int out_q_stride, int out_q0, void* stream);
