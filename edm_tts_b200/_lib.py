@@ -103,11 +103,13 @@ _SIGNATURES = {
     "edm_t2s_predict_length_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "edm_t2s_begin": (_i, [_vp, _vp, _i, _i, _vp]),
     "edm_t2s_begin_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
+    "edm_t2s_begin_masked": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "edm_t2s_logits": (_i, [_vp, _vp, _vp]),
     "edm_t2s_step": (_i, [_vp, _i, _i, _f, _ull, _vp, _vp, _vp, _vp, _vp]),
     "edm_t2s_result": (_i, [_vp, _vp, _vp]),
     "edm_t2s_decode": (_i, [_vp, _vp, _i, _i, _i, _f, _ull, _vp, _vp, _vp, _vp, _vp, _vp]),
     "edm_t2s_decode_batch": (_i, [_vp, _i, _vp, _vp, _vp, _i, _f, _ull, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "edm_t2s_decode_masked": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _f, _ull, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -1877,7 +1877,7 @@ struct edm_t2s_ctx {
   const int* pairs = nullptr;  // attention items of a packed layout
   int n_pairs = 0, max_n = 0, out_len = 0;
   double sum_sq = 0.0;         // sum of L_s^2 (attention work)
-  const int* init_counts = nullptr;  // packed decode: length_s per sequence (re-masking)
+  const int* init_counts = nullptr;  // packed decode: length_s per sequence (re-masking), T_s under a masked begin
   float* part_use = nullptr;   // split-K partials of this pass, nullptr: the unsplit launches
   bool begun = false, mask_in_a = true;
   CUtensorMap m_z, m_h, m_att, m_g, m_zt, m_qkv;
@@ -2070,6 +2070,7 @@ int t2s_stack(edm_t2s_ctx* c, int blk0, int n, int H, int hp, const float* rope_
 void t2s_pass_single(edm_t2s_ctx* c, int rows, int n_text, int length) {
   c->seqs.lay = uniform_layout(1, rows, rows);
   c->seqs.cu_text = nullptr; c->seqs.cu_len = nullptr; c->seqs.n_text = n_text; c->seqs.length = length;
+  c->seqs.regen_slot = nullptr; c->seqs.regen_row = nullptr;
   c->pairs = nullptr; c->n_pairs = 0; c->max_n = rows; c->out_len = length;
   c->sum_sq = static_cast<double>(rows) * rows;
   c->init_counts = nullptr;
@@ -2077,9 +2078,12 @@ void t2s_pass_single(edm_t2s_ctx* c, int rows, int n_text, int length) {
 }
 
 // The current pass is n_seq packed sequences: n_text[s] + 1 rows each for the length predictor (length == nullptr), n_text[s] +
-// length[s] + 4 for the decode. Checks the lengths against the bound capacity and the rotary tables, then uploads the layout arrays
-// with one copy on `st`:  cu_n [n_seq + 1] | cu_text [n_seq + 1] | cu_len [n_seq + 1] | length [n_seq] | attention pairs.
-int t2s_pass_batch(edm_t2s_ctx* c, int n_seq, const int* n_text, const int* length, cudaStream_t st) {
+// length[s] + 4 for the decode. regen (host, sum length[s] bytes, or nullptr): a masked decode, speech position k of sequence s is
+// regenerated when regen[cu_len[s] + k] != 0, T_s >= 1 of them per sequence. Checks the lengths against the bound capacity and the
+// rotary tables, then uploads the layout arrays with one copy on `st`:
+//   cu_n [n_seq + 1] | cu_text [n_seq + 1] | cu_len [n_seq + 1] | init_counts [n_seq] | attention pairs | regen_slot | regen_row
+// init_counts[s] = length[s], or T_s when masked (the reference's initial = mask.sum()); the two maps (T2sSeqs) only when masked.
+int t2s_pass_batch(edm_t2s_ctx* c, int n_seq, const int* n_text, const int* length, const unsigned char* regen, cudaStream_t st) {
   if (n_seq < 1 || n_seq > c->max_seq) return fail(EDM_ERR_INVALID, "%d sequences for a workspace bound for %d", n_seq, c->max_seq);
   if (n_text == nullptr) return fail(EDM_ERR_INVALID, "per-sequence text lengths required");
   const size_t n1 = static_cast<size_t>(n_seq) + 1;
@@ -2087,7 +2091,7 @@ int t2s_pass_batch(edm_t2s_ctx* c, int n_seq, const int* n_text, const int* leng
   h.assign(3 * n1 + n_seq, 0);
   std::vector<int> rows(n_seq);
   long long total = 0;
-  int max_n = 0;
+  int max_n = 0, n_regen = 0;
   double sum_sq = 0.0;
   for (int s = 0; s < n_seq; ++s) {
     const int len = length != nullptr ? length[s] : 0;
@@ -2096,31 +2100,57 @@ int t2s_pass_batch(edm_t2s_ctx* c, int n_seq, const int* n_text, const int* leng
     if (r > c->cfg.max_positions) return fail(EDM_ERR_INVALID, "sequence %d of %lld tokens exceeds max_positions=%d", s, r, c->cfg.max_positions);
     total += r;
     if (total > c->max_len) return fail(EDM_ERR_INVALID, "sequences of %lld+ rows exceed the bound workspace (%d rows)", total, c->max_len);
+    int count = len;
+    if (regen != nullptr) {
+      count = 0;
+      for (int k = 0; k < len; ++k) count += regen[h[2 * n1 + s] + k] != 0;
+      if (count < 1) return fail(EDM_ERR_INVALID, "sequence %d has no speech position to regenerate", s);
+    }
     rows[s] = static_cast<int>(r);
     h[s + 1] = h[s] + rows[s];
     h[n1 + s + 1] = h[n1 + s] + n_text[s];
     h[2 * n1 + s + 1] = h[2 * n1 + s] + len;
-    h[3 * n1 + s] = len;
+    h[3 * n1 + s] = count;
+    n_regen += count;
     max_n = std::max(max_n, rows[s]);
     sum_sq += static_cast<double>(r) * r;
   }
   append_attention_pairs(rows, &h);
+  const size_t maps = h.size();
+  const int n_speech = h[3 * n1 - 1];
+  if (regen != nullptr) {
+    h.resize(maps + n_speech + n_regen);
+    int* slot = h.data() + maps;
+    int* row = slot + n_speech;
+    int j = 0;
+    for (int s = 0; s < n_seq; ++s) {
+      const int k0 = h[2 * n1 + s], row0 = h[s] + n_text[s] + 3;
+      for (int k = 0; k < length[s]; ++k) {
+        slot[k0 + k] = regen[k0 + k] != 0 ? j : -1;
+        if (regen[k0 + k] != 0) row[j++] = row0 + k;
+      }
+    }
+  }
   if (h.size() > c->layout_cap) return fail(EDM_ERR_INVALID, "layout of %zu ints exceeds the bound workspace (%zu)", h.size(), c->layout_cap);
   int* dev = c->layout_dev;
   EDM_CUDA(cudaMemcpyAsync(dev, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, st));
   SeqLayout& l = c->seqs.lay;
   l.n_seq = n_seq; l.N = 0; l.T = 0; l.cu_n = dev; l.cu_t = dev; l.rows = static_cast<int>(total); l.t_rows = l.rows;
   c->seqs.cu_text = dev + n1; c->seqs.cu_len = dev + 2 * n1; c->seqs.n_text = 0; c->seqs.length = 0;
-  c->pairs = dev + 3 * n1 + n_seq; c->n_pairs = static_cast<int>(h.size() - (3 * n1 + n_seq));
-  c->max_n = max_n; c->out_len = h[3 * n1 - 1]; c->sum_sq = sum_sq;
+  c->seqs.regen_slot = regen != nullptr ? dev + maps : nullptr;
+  c->seqs.regen_row = regen != nullptr ? dev + maps + n_speech : nullptr;
+  c->pairs = dev + 3 * n1 + n_seq; c->n_pairs = static_cast<int>(maps - (3 * n1 + n_seq));
+  c->max_n = max_n; c->out_len = n_regen; c->sum_sq = sum_sq;
   c->init_counts = dev + 3 * n1;
   c->part_use = nullptr;
   return 0;
 }
 
-// ints of the layout arrays of t2s_pass_batch for max_seq sequences of max_len rows in all: 3 (max_seq + 1) offsets, max_seq lengths
-// and at most max_len / 256 + max_seq attention pairs
-size_t t2s_layout_ints(int max_len, int max_seq) { return 4 * (static_cast<size_t>(max_seq) + 1) + static_cast<size_t>(max_len) / 256 + max_seq; }
+// ints of the layout arrays of t2s_pass_batch for max_seq sequences of max_len rows in all: 3 (max_seq + 1) offsets, max_seq counts,
+// at most max_len / 256 + max_seq attention pairs, and the two maps of a masked decode (fewer than max_len entries each)
+size_t t2s_layout_ints(int max_len, int max_seq) {
+  return 4 * (static_cast<size_t>(max_seq) + 1) + static_cast<size_t>(max_len) / 256 + max_seq + 2 * static_cast<size_t>(max_len);
+}
 
 // max_len rows, max_seq sequences; with_part: the split-K partial sums of a single-sequence bind
 size_t t2s_carve(edm_t2s_ctx* c, uint8_t* base, int max_len, int max_seq, bool with_part, bool assign) {
@@ -2337,17 +2367,19 @@ extern "C" int edm_t2s_predict_length(edm_t2s_ctx* c, const int* text_tokens, in
 extern "C" int edm_t2s_predict_length_batch(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, float* raw_out, void* stream) {
   if (c == nullptr || !c->bound) return fail(EDM_ERR_STATE, "context not bound");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (int rc = t2s_pass_batch(c, n_seq, n_text_host, nullptr, st)) return rc;
+  if (int rc = t2s_pass_batch(c, n_seq, n_text_host, nullptr, nullptr, st)) return rc;
   if (c->seqs.lay.rows > n_seq && text_tokens == nullptr) return fail(EDM_ERR_INVALID, "text tokens required");
   return t2s_length_predictor(c, text_tokens, raw_out, st);
 }
 
 namespace {
-// token sequences and mask state of the current pass (:205-222); text: the packed text tokens in c->text
-int t2s_begin_pass(edm_t2s_ctx* c, cudaStream_t st) {
+// token sequences and mask state of the current pass (:205-222); text: the packed text tokens in c->text; known: the known speech
+// tokens of a masked pass
+int t2s_begin_pass(edm_t2s_ctx* c, const int* known, cudaStream_t st) {
   c->mask_in_a = true;
   T2sBeginParams p;
   p.seqs = c->seqs; p.text_tokens = c->text; p.tok_text = 1; p.tok_sep = 3; p.tok_speech = 2; p.tok_mask = 4;
+  p.known = known; p.offset = c->cfg.num_special + c->cfg.text_vocab;
   p.input_ids = c->input_ids; p.tokens = c->tokens; p.full_mask = c->full_mask; p.mask = c->mask_a;
   launch_pdl(t2s_begin_kernel, dim3((c->seqs.lay.rows + 255) / 256), dim3(256), 0, st, p);
   EDM_LAUNCH_CHECK("t2s_begin");
@@ -2368,22 +2400,39 @@ extern "C" int edm_t2s_begin(edm_t2s_ctx* c, const int* text_tokens, int n_text,
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (n_text > 0) EDM_CUDA(cudaMemcpyAsync(c->text, text_tokens, sizeof(int) * n_text, cudaMemcpyDeviceToDevice, st));
   t2s_pass_single(c, static_cast<int>(L), n_text, length);
-  return t2s_begin_pass(c, st);
+  return t2s_begin_pass(c, nullptr, st);
 }
 
-// n_seq requests packed back to back: text s has n_text_host[s] tokens (packed in text_tokens), length_host[s] speech positions
-extern "C" int edm_t2s_begin_batch(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, void* stream) {
+namespace {
+// edm_t2s_begin_batch / edm_t2s_begin_masked (regen == nullptr: every speech position regenerated)
+int t2s_begin_packed(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, const int* known,
+                     const unsigned char* regen, cudaStream_t st) {
   if (c == nullptr || !c->bound) return fail(EDM_ERR_STATE, "context not bound");
   if (length_host == nullptr) return fail(EDM_ERR_INVALID, "per-sequence lengths required");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   c->begun = false;
-  if (int rc = t2s_pass_batch(c, n_seq, n_text_host, length_host, st)) return rc;
-  const int total_text = c->host_layout[2 * (static_cast<size_t>(n_seq) + 1) - 1];
+  if (int rc = t2s_pass_batch(c, n_seq, n_text_host, length_host, regen, st)) return rc;
+  const size_t n1 = static_cast<size_t>(n_seq) + 1;
+  if (regen != nullptr && known == nullptr && c->out_len < c->host_layout[3 * n1 - 1]) return fail(EDM_ERR_INVALID, "known tokens required");
+  const int total_text = c->host_layout[2 * n1 - 1];
   if (total_text > 0) {
     if (text_tokens == nullptr) return fail(EDM_ERR_INVALID, "text tokens required");
     EDM_CUDA(cudaMemcpyAsync(c->text, text_tokens, sizeof(int) * total_text, cudaMemcpyDeviceToDevice, st));
   }
-  return t2s_begin_pass(c, st);
+  return t2s_begin_pass(c, known, st);
+}
+}  // namespace
+
+// n_seq requests packed back to back: text s has n_text_host[s] tokens (packed in text_tokens), length_host[s] speech positions
+extern "C" int edm_t2s_begin_batch(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, void* stream) {
+  return t2s_begin_packed(c, n_seq, text_tokens, n_text_host, length_host, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+// :205-222 with some speech positions known: the reference's decode loop started from full_mask = the positions to regenerate (see
+// include/edm_s2a.h)
+extern "C" int edm_t2s_begin_masked(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host,
+                                    const int* known_tokens, const unsigned char* regenerate_host, void* stream) {
+  if (regenerate_host == nullptr) return fail(EDM_ERR_INVALID, "regenerate mask required");
+  return t2s_begin_packed(c, n_seq, text_tokens, n_text_host, length_host, known_tokens, regenerate_host, static_cast<cudaStream_t>(stream));
 }
 
 // embeddings_to_logits (:135-152, mask = None) -> buffer "logits" [rows, 1024] fp32 over the rows of what was begun. x_in: fp32
@@ -2448,7 +2497,8 @@ extern "C" int edm_t2s_step(edm_t2s_ctx* c, int iter, int iters, float temperatu
   return 0;
 }
 
-// speech_pred_tokens (:267): int64, semantic vocabulary; [length] of the one sequence, or [sum length_s] packed for a batch
+// speech_pred_tokens (:267): int64, semantic vocabulary; [length] of the one sequence, or [sum length_s] packed for a batch, or
+// [sum T_s] (the regenerated positions) after a masked begin
 extern "C" int edm_t2s_result(edm_t2s_ctx* c, long long* tokens_out, void* stream) {
   if (c == nullptr || !c->bound || !c->begun) return fail(EDM_ERR_STATE, "no sequence: call edm_t2s_begin first");
   if (tokens_out == nullptr) return fail(EDM_ERR_INVALID, "output required");
@@ -2490,6 +2540,16 @@ extern "C" int edm_t2s_decode_batch(edm_t2s_ctx* c, int n_seq, const int* text_t
                                     const int* forced_ids, const uint8_t* forced_masks, long long* tokens_out, void* stream) {
   if (pred_iters < 1) return fail(EDM_ERR_INVALID, "pred_iters must be >= 1");
   if (int rc = edm_t2s_begin_batch(c, n_seq, text_tokens, n_text_host, length_host, stream)) return rc;
+  return t2s_iterate(c, pred_iters, temperature, seed, cat_noise, remask_noise, forced_ids, forced_masks, tokens_out, stream);
+}
+
+// edm_t2s_decode_batch after edm_t2s_begin_masked: tokens_out [sum T_s], the regenerated positions in time order
+extern "C" int edm_t2s_decode_masked(edm_t2s_ctx* c, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host,
+                                     const int* known_tokens, const unsigned char* regenerate_host, int pred_iters, float temperature,
+                                     unsigned long long seed, const float* cat_noise, const float* remask_noise, const int* forced_ids,
+                                     const uint8_t* forced_masks, long long* tokens_out, void* stream) {
+  if (pred_iters < 1) return fail(EDM_ERR_INVALID, "pred_iters must be >= 1");
+  if (int rc = edm_t2s_begin_masked(c, n_seq, text_tokens, n_text_host, length_host, known_tokens, regenerate_host, stream)) return rc;
   return t2s_iterate(c, pred_iters, temperature, seed, cat_noise, remask_noise, forced_ids, forced_masks, tokens_out, stream);
 }
 

@@ -193,10 +193,15 @@ __global__ void __launch_bounds__(32) t2s_length_head_kernel(const float* x, con
 // The requests of a decode: sequence s is [text] bytes_s [sep] [speech] [mask] * length_s [sep] (:205-217), L_s = n_text_s + length_s + 4
 // rows of `lay` starting at lay.n_start(s). Its text bytes start at cu_text[s] of the packed text, its speech tokens at cu_len[s] of the
 // packed output. One sequence (cu_text == nullptr): n_text / length, both offsets 0.
+// A masked begin (edm_t2s_begin_masked: speech editing, prompted continuation) keeps some speech positions known; its two maps are
+// nullptr otherwise. regen_slot[len_start(s) + k] is the index of speech position k of sequence s among the regenerated positions of
+// the pass (its slot in the packed output), or -1 when the position is known; regen_row[j] is the row of regenerated position j.
 struct T2sSeqs {
   SeqLayout lay;
   const int* cu_text;  // [n_seq + 1] or nullptr
   const int* cu_len;   // [n_seq + 1] or nullptr
+  const int* regen_slot;  // [sum length_s] or nullptr
+  const int* regen_row;   // [sum T_s] or nullptr
   int n_text, length;  // the single sequence's
 
   __device__ __forceinline__ int text_start(int s) const { return cu_text != nullptr ? __ldg(cu_text + s) : 0; }
@@ -217,10 +222,14 @@ __global__ void t2s_lp_gather_kernel(const T2sSeqs q, const int* text_tokens, in
   gather[i] = n == 0 ? -1 : text_tokens[q.text_start(s) + n - 1];
 }
 
-// token sequences of the requests (:205-222); full_mask marks the speech positions.
+// token sequences of the requests (:205-222); full_mask marks the speech positions to decode. Under a masked begin a known speech
+// position holds known[len_start(s) + k] + offset (the token an iteration writes back for a sampled id, :256-257) with full_mask = 0:
+// like the text rows, it keeps its input id through every update and enters re-masking with confidence +inf (:250, :258).
 struct T2sBeginParams {
   T2sSeqs seqs;
   const int* text_tokens;  // packed [sum n_text_s], already shifted past the special tokens
+  const int* known;        // packed [sum length_s] semantic tokens, read at known positions only (seqs.regen_slot != nullptr)
+  int offset;              // num_special + text_vocab
   int tok_text, tok_sep, tok_speech, tok_mask;
   int* input_ids;          // [rows]
   int* tokens;             // [rows] the running "sampled_tokens"
@@ -240,7 +249,11 @@ __global__ void t2s_begin_kernel(const T2sBeginParams p) {
   else if (n <= n_text) tok = p.text_tokens[p.seqs.text_start(s) + n - 1];
   else if (n == n_text + 1) tok = p.tok_sep;
   else if (n == n_text + 2) tok = p.tok_speech;
-  else if (n < L - 1) { tok = p.tok_mask; m = 1; }
+  else if (n < L - 1) {
+    const int k = p.seqs.len_start(s) + n - n_text - 3;
+    if (p.seqs.regen_slot != nullptr && __ldg(p.seqs.regen_slot + k) < 0) tok = clamp_index(__ldg(p.known + k), kV) + p.offset;
+    else { tok = p.tok_mask; m = 1; }
+  }
   else tok = p.tok_sep;
   p.input_ids[i] = tok;
   p.tokens[i] = tok;
@@ -271,11 +284,16 @@ __global__ void t2s_update_kernel(const T2sUpdateParams p) {
   p.tokens[i] = tok;
 }
 
-// speech_pred_tokens = sampled_tokens[full_mask] (:267) of every sequence, packed: out[len_start(s) + k] = tokens[speech_start(s) + k]
+// speech_pred_tokens = sampled_tokens[full_mask] (:267) of every sequence, packed: out[len_start(s) + k] = tokens[speech_start(s) + k],
+// or, under a masked begin, only the regenerated positions: out[j] = tokens[regen_row[j]]
 __global__ void t2s_gather_out_kernel(const T2sSeqs q, const int* tokens, int total, long long* out) {
   pdl_sync();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
+  if (q.regen_row != nullptr) {
+    out[i] = tokens[__ldg(q.regen_row + i)];
+    return;
+  }
   const int s = q.cu_len != nullptr ? q.lay.search(q.cu_len, i) : 0;
   out[i] = tokens[q.speech_start(s) + (i - q.len_start(s))];
 }

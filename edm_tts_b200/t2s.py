@@ -3,7 +3,8 @@
 Mirrors edm_tts/models/text_to_semantic/modeling_text_to_semantic.py:26-267 (TextToSemanticWLen): same constructor inputs (config +
 state dict / HF directory), `infer(text, pred_iters, temperature, gt_length)` with the reference's argument meaning and return type
 (`.speech_pred_tokens`), `embeddings_to_logits`. `infer` decodes one sequence per call, as in the reference; `infer_batch` decodes
-a list of texts of different lengths together, packed back to back without padding. All arithmetic runs in the CUDA kernels; the only
+a list of texts of different lengths together, packed back to back without padding; `infill_batch` regenerates chosen semantic
+tokens of utterances given their transcripts and the other tokens (speech editing). All arithmetic runs in the CUDA kernels; the only
 host round trip is the predicted length (it fixes the shape of everything after it): one read per call, or per chunk of a batch.
 No CPU fallback.
 """
@@ -279,16 +280,26 @@ class TextToSemanticWLen:
     @torch.no_grad()
     @_on_device
     def decode_trace(self, text, pred_iters=10, temperature=1.0, gt_length=None, *, seed=0, batch_offset=0, cat_gumbel=None, remask_gumbel=None,
-                     forced_ids=None, forced_masks=None):
-        """infer run stage by stage through the entry points edm_t2s_decode composes; returns every intermediate. Parity tests only."""
+                     forced_ids=None, forced_masks=None, semantic_tokens=None, regenerate=None):
+        """infer run stage by stage through the entry points edm_t2s_decode composes; returns every intermediate. Parity tests only.
+        With semantic_tokens / regenerate ([N] each, gt_length unused) it is the infill decode of infill_batch([text], [semantic_tokens],
+        [regenerate]) instead, begun by edm_t2s_begin_masked; "tokens" then holds the regenerated positions."""
         lib, s_ = L.lib(), L.stream_ptr()
         tt = self.text_tokens(text)
-        length = int(gt_length) if gt_length is not None else self.predict_length(tt)[0]
         n_text = tt.numel()
-        Lseq = n_text + length + 4
         dev = self.device
         L.check(lib.edm_t2s_set_batch_offset(self._ctx, int(batch_offset)), "set_batch_offset")
-        L.check(lib.edm_t2s_begin(self._ctx, L.ptr(tt) if n_text else None, n_text, length, s_), "begin")
+        if regenerate is None:
+            length = int(gt_length) if gt_length is not None else self.predict_length(tt)[0]
+            n_out = length
+            L.check(lib.edm_t2s_begin(self._ctx, L.ptr(tt) if n_text else None, n_text, length, s_), "begin")
+        else:
+            sp = varlen.t2s_infill_split([n_text], [semantic_tokens], [regenerate], self.config.semantic_vocab_size, self.max_positions)
+            length, n_out = sp.N[0], sp.T[0]
+            known = sp.known.to(dev, torch.int32)
+            L.check(lib.edm_t2s_begin_masked(self._ctx, 1, L.ptr(tt) if n_text else None, (C.c_int * 1)(n_text), (C.c_int * 1)(length), L.ptr(known),
+                                             sp.regenerate.data_ptr(), s_), "begin_masked")
+        Lseq = n_text + length + 4
         tr = dict(step_logits=[], step_ids=[], step_masks=[], step_masks_raw=[], length=length,
                   input_ids=self._view("input_ids", (1, Lseq), torch.int32).clone().long(),
                   full_mask=self._view("full_mask", (1, Lseq), torch.uint8).clone().bool())
@@ -305,7 +316,7 @@ class TextToSemanticWLen:
             if not last:
                 tr["step_masks"].append(self._view("mask", (1, Lseq), torch.uint8).clone().bool())
                 tr["step_masks_raw"].append(self._view("mask_raw", (1, Lseq), torch.uint8).clone().bool())
-        out = torch.empty(length, device=dev, dtype=torch.int64)
+        out = torch.empty(n_out, device=dev, dtype=torch.int64)
         L.check(lib.edm_t2s_result(self._ctx, L.ptr(out), s_), "result")
         tr["tokens"] = out
         return tr
@@ -375,38 +386,80 @@ class TextToSemanticWLen:
                 raise ValueError(f"utterance {i}: length {ln} < 1")
             if Lseq[i] > self.max_positions:
                 raise ValueError(f"utterance {i}: sequence of {Lseq[i]} tokens exceeds max_positions={self.max_positions}")
-        V = self.config.semantic_vocab_size
-        extras = dict(cat_gumbel=(cat_gumbel, lambda l: (iters - 1, l, V)), remask_gumbel=(remask_gumbel, lambda l: (iters - 1, 1, l)),
-                      forced_ids=(forced_ids, lambda l: (iters, 1, l)), forced_masks=(forced_masks, lambda l: (iters - 1, 1, l)))
-        for name, (lst, shape) in extras.items():
+        extras = self._check_extras(iters, Lseq, cat_gumbel=cat_gumbel, remask_gumbel=remask_gumbel, forced_ids=forced_ids, forced_masks=forced_masks)
+        return self._decode_packed(toks, lengths, lengths, iters, temperature, seed, batch_offset, extras)
+
+    @torch.no_grad()
+    @_on_device
+    def infill_batch(self, texts, semantic_tokens, regenerate, pred_iters=10, temperature=1.0, *, seed=0, batch_offset=0, cat_gumbel=None,
+                     remask_gumbel=None, forced_ids=None, forced_masks=None):
+        """Regenerates chosen semantic tokens of each utterance given its transcript and the rest (speech editing; with a known prefix,
+        prompted continuation). texts: the transcript of the whole (edited) utterance, str or 1-D shifted-token tensors;
+        semantic_tokens[i]: LongTensor [N_i], the values at regenerated positions are ignored; regenerate[i]: BoolTensor [N_i], at least
+        one True. The decode is the reference's loop (:184-267) on [text] bytes [sep] [speech] s_1 .. s_N [sep] started from full_mask
+        = regenerate: known positions hold their tokens and are never sampled or re-masked, and mask_len counts only the regenerated
+        ones (edm_t2s_begin_masked). Returns a list of LongTensor [T_i] (T_i = regenerate[i].sum()), the regenerated tokens in time
+        order, views of one packed output. With every position regenerated, utterance i decodes to the bits of infer_batch(texts,
+        gt_lengths=N) at index i. Chunks of MAX_CHUNK and the parity extras are as in infer_batch, with L_i = len(text_i bytes) + N_i
+        + 4. Malformed input raises ValueError naming the utterance."""
+        toks = self._batch_tokens(texts)
+        iters = int(pred_iters)
+        if iters < 1:
+            raise ValueError(f"pred_iters must be >= 1, got {pred_iters}")
+        n_text = [t.numel() for t in toks]
+        sp = varlen.t2s_infill_split(n_text, semantic_tokens, regenerate, self.config.semantic_vocab_size, self.max_positions)
+        Lseq = [nt + n + 4 for nt, n in zip(n_text, sp.N)]
+        extras = self._check_extras(iters, Lseq, cat_gumbel=cat_gumbel, remask_gumbel=remask_gumbel, forced_ids=forced_ids, forced_masks=forced_masks)
+        return self._decode_packed(toks, list(sp.N), list(sp.T), iters, temperature, seed, batch_offset, extras, sp)
+
+    def _check_extras(self, iters, Lseq, **extras):
+        """the per-utterance parity extras of infer_batch / infill_batch: lists shaped as infer's extras, L_i positions each"""
+        V, n = self.config.semantic_vocab_size, len(Lseq)
+        shapes = dict(cat_gumbel=lambda l: (iters - 1, l, V), remask_gumbel=lambda l: (iters - 1, 1, l), forced_ids=lambda l: (iters, 1, l),
+                      forced_masks=lambda l: (iters - 1, 1, l))
+        for name, lst in extras.items():
             if lst is None:
                 continue
             if not isinstance(lst, (list, tuple)) or len(lst) != n:
                 raise ValueError(f"{name} must be a list with one entry per utterance")
             for i, x in enumerate(lst):
-                if tuple(x.shape) != shape(Lseq[i]):
-                    raise ValueError(f"{name}[{i}] must be {shape(Lseq[i])}, got {tuple(x.shape)}")
-        dev, lib = self.device, L.lib()
+                if tuple(x.shape) != shapes[name](Lseq[i]):
+                    raise ValueError(f"{name}[{i}] must be {shapes[name](Lseq[i])}, got {tuple(x.shape)}")
+        return extras
+
+    def _decode_packed(self, toks, lengths, out_lens, iters, temperature, seed, batch_offset, extras, infill=None):
+        """The packed decode of infer_batch (infill None) or infill_batch (infill: the varlen.T2sInfill) in chunks of MAX_CHUNK:
+        utterance i has toks[i] text tokens and lengths[i] speech positions, of which it returns out_lens[i]."""
+        n, dev, lib = len(toks), self.device, L.lib()
+        n_text = [t.numel() for t in toks]
+        Lseq = [nt + ln + 4 for nt, ln in zip(n_text, lengths)]
+        cu_len = varlen.offsets(lengths)
+        known = None if infill is None else infill.known.to(dev, torch.int32)
 
         def cat(lst, sl, dim, dtype):
             if lst is None or lst[sl.start].shape[0] == 0:  # the [iters - 1, ...] extras of a 1-iteration decode are empty
                 return None
             return torch.cat([x.to(dev) for x in lst[sl]], dim).to(dtype).contiguous()
 
-        out = torch.empty(sum(lengths), device=dev, dtype=torch.int64)
-        for ch in varlen.plan(lengths, [0] * n, MAX_CHUNK, batch_offset):
+        out = torch.empty(sum(out_lens), device=dev, dtype=torch.int64)
+        for ch in varlen.plan(out_lens, [0] * n, MAX_CHUNK, batch_offset):
             sl, m = slice(ch.start, ch.stop), ch.stop - ch.start
             ctx = self._bind_batch(sum(Lseq[sl]), m)
-            cg = cat(cat_gumbel, sl, 1, torch.float32)
-            rg = cat(remask_gumbel, sl, 2, torch.float32)
-            fi = cat(forced_ids, sl, 2, torch.int32)
-            fm = cat(forced_masks, sl, 2, torch.uint8)
+            cg = cat(extras["cat_gumbel"], sl, 1, torch.float32)
+            rg = cat(extras["remask_gumbel"], sl, 2, torch.float32)
+            fi = cat(extras["forced_ids"], sl, 2, torch.int32)
+            fm = cat(extras["forced_masks"], sl, 2, torch.uint8)
             tt = self._packed(toks[sl])
+            args = (iters, float(temperature), int(seed), L.ptr(cg), L.ptr(rg), L.ptr(fi), L.ptr(fm), L.ptr(out[ch.t0:ch.t0 + sum(ch.T)]), L.stream_ptr())
             L.check(lib.edm_t2s_set_batch_offset(ctx, ch.batch_offset), "set_batch_offset")
-            L.check(lib.edm_t2s_decode_batch(ctx, m, L.ptr(tt), (C.c_int * m)(*n_text[sl]), (C.c_int * m)(*ch.T), iters, float(temperature),
-                                             int(seed), L.ptr(cg), L.ptr(rg), L.ptr(fi), L.ptr(fm), L.ptr(out[ch.t0:ch.t0 + sum(ch.T)]),
-                                             L.stream_ptr()), "t2s_decode_batch")
-        return [b[0] for b in varlen.split_blocks(out, lengths, 1)]
+            if infill is None:
+                L.check(lib.edm_t2s_decode_batch(ctx, m, L.ptr(tt), (C.c_int * m)(*n_text[sl]), (C.c_int * m)(*lengths[sl]), *args), "t2s_decode_batch")
+            else:
+                a, b = cu_len[ch.start], cu_len[ch.stop]
+                flags = infill.regenerate[a:b].contiguous()   # host bytes, read by the call before it returns
+                L.check(lib.edm_t2s_decode_masked(ctx, m, L.ptr(tt), (C.c_int * m)(*n_text[sl]), (C.c_int * m)(*lengths[sl]), L.ptr(known[a:b]),
+                                                  flags.data_ptr(), *args), "t2s_decode_masked")
+        return [b[0] for b in varlen.split_blocks(out, out_lens, 1)]
 
     @torch.no_grad()
     @_on_device

@@ -6,6 +6,7 @@ per-frame data of utterance i starts at cu_t[i] (targets) or cu_p[i] (prompt), a
 equal lengths this is the [B, ...] layout of a uniform batch.
 
 S2A infilling (edm_s2a_bind_masked): the same with the known (prompt) frames anywhere in their utterance, see infill_split.
+Text-to-semantic infilling (edm_t2s_begin_masked): a text-to-semantic batch with some speech positions known, see t2s_infill_split.
 
 DAC decoder (DACDecoder.forward_batch): the utterances are packed along time with zero gap rows between them, see dac_pack.
 DAC encoder (DACEncoder.forward_batch): the same idea for the downsampling stack, see enc_pack.
@@ -145,6 +146,78 @@ def infill_rows(target) -> tuple[list[int], list[int]]:
                 k += 1
             row += 1
     return tgt_enc, enc_slot
+
+
+# ---------------------------------------------------------------------------------------------------------------------------------
+# Text-to-semantic infilling (edm_t2s_begin_masked): utterance i is a transcript of n_text_i tokens and N_i speech positions, T_i >= 1
+# of them regenerated, the others known. Its sequence has L_i = n_text_i + N_i + 4 rows, speech position k at row n_text_i + 3 + k.
+# Per-position data (known tokens, regenerate flags) is packed [sum N_i], the regenerated tokens [sum T_i], both in time order.
+
+
+@dataclass(frozen=True)
+class T2sInfill:
+    """A checked text-to-semantic infill batch: per utterance the speech positions N_i and the regenerated ones T_i; the packed
+    semantic tokens [sum N_i] (int64, on the tokens' device, 0 at regenerated positions) and regenerate flags [sum N_i] (uint8, host)."""
+    N: tuple
+    T: tuple
+    known: object
+    regenerate: object
+
+
+def t2s_infill_split(n_text, semantic_tokens, regenerate, num_semantic: int, max_positions: int) -> T2sInfill:
+    """Checks a text-to-semantic infill batch (transcript lengths n_text_i, semantic tokens [N_i], bool masks [N_i] of the positions
+    to regenerate) and packs it. Raises ValueError naming the utterance when the lists differ in length, a mask and its tokens differ
+    in length, an utterance has nothing to regenerate, a known token lies outside [0, num_semantic) (values at regenerated positions
+    are ignored), or L_i = n_text_i + N_i + 4 exceeds max_positions."""
+    import torch
+
+    if not isinstance(semantic_tokens, (list, tuple)) or not isinstance(regenerate, (list, tuple)) or len(semantic_tokens) == 0:
+        raise ValueError("semantic_tokens and regenerate must be non-empty lists")
+    n = len(semantic_tokens)
+    if len(regenerate) != n or len(n_text) != n:
+        raise ValueError(f"{len(n_text)} texts, {n} semantic token lists and {len(regenerate)} regenerate masks")
+    N, T = [], []
+    for i, (st, rg) in enumerate(zip(semantic_tokens, regenerate)):
+        if not torch.is_tensor(st) or not torch.is_tensor(rg) or st.dim() != 1 or rg.dim() != 1:
+            raise ValueError(f"utterance {i}: expected semantic_tokens [N] and regenerate [N] tensors")
+        if rg.dtype != torch.bool:
+            raise ValueError(f"utterance {i}: regenerate must be a bool tensor")
+        if rg.shape[0] != st.shape[0]:
+            raise ValueError(f"utterance {i}: {st.shape[0]} semantic tokens but {rg.shape[0]} regenerate entries")
+        t = int(rg.sum())
+        if t < 1:
+            raise ValueError(f"utterance {i} has no speech position to regenerate")
+        L = int(n_text[i]) + st.shape[0] + 4
+        if L > max_positions:
+            raise ValueError(f"utterance {i}: sequence of {L} tokens exceeds max_positions={max_positions}")
+        N.append(int(st.shape[0]))
+        T.append(t)
+    dev = semantic_tokens[0].device
+    regen = torch.cat([r.cpu() for r in regenerate])
+    known = torch.cat([s.to(dev, torch.int64) for s in semantic_tokens]).masked_fill(regen.to(dev), 0)
+    lo, hi = torch.aminmax(known)
+    if int(lo) < 0 or int(hi) >= num_semantic:
+        cu = offsets(N)
+        for i in range(n):
+            seg = known[cu[i]:cu[i + 1]]
+            if int(seg.min()) < 0 or int(seg.max()) >= num_semantic:
+                raise ValueError(f"utterance {i}: a known semantic token is out of range [0, {num_semantic})")
+    return T2sInfill(tuple(N), tuple(T), known, regen.to(torch.uint8))
+
+
+def t2s_infill_maps(n_text, regenerate) -> tuple[list[int], list[int]]:
+    """The two maps edm_t2s_begin_masked builds on the host for masks `regenerate` [N_i] of sequences with n_text_i text tokens:
+    regen_slot[cu_N[i] + k] = index of speech position k of utterance i among the regenerated positions of the batch, or -1 when it
+    is known; regen_row[j] = packed row of regenerated position j."""
+    regen_slot, regen_row, row0, j = [], [], 0, 0
+    for nt, m in zip(n_text, regenerate):
+        for k, v in enumerate(bool(x) for x in m):
+            regen_slot.append(j if v else -1)
+            if v:
+                regen_row.append(row0 + int(nt) + 3 + k)
+                j += 1
+        row0 += int(nt) + len(m) + 4
+    return regen_slot, regen_row
 
 
 # ---------------------------------------------------------------------------------------------------------------------------------

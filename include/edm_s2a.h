@@ -376,12 +376,22 @@ int edm_t2s_begin(edm_t2s_ctx* ctx, const int* text_tokens, int n_text, int leng
  * all of them: buffers and per-iteration noise / forcing by packed rows, result [sum length_s] packed. Copies the layout arrays into
  * the workspace on `stream`. */
 int edm_t2s_begin_batch(edm_t2s_ctx* ctx, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, void* stream);
+/* edm_t2s_begin_batch with known speech positions (speech editing, prompted continuation): the reference's decode loop (:205-267)
+ * started from a full_mask that holds only the positions to regenerate. Sequence s has length_host[s] = N_s speech positions;
+ * position k is regenerated when regenerate_host[cu + k] != 0 (host bytes, cu = N_0 + .. + N_{s-1}), otherwise it holds
+ * known_tokens[cu + k] (device int32, semantic vocabulary, clamped into it) + num_special + text_vocab for the whole decode: never
+ * sampled or re-masked. Every sequence needs T_s >= 1 regenerated position, and mask_len counts only those (:237-242 with
+ * initial = T_s). known_tokens may be NULL when every position is regenerated, which is edm_t2s_begin_batch. The Philox counters are
+ * those of edm_t2s_begin_batch. edm_t2s_logits / step work as after edm_t2s_begin_batch; edm_t2s_result then writes [sum T_s]
+ * regenerated tokens, in time order. Copies the layout arrays and the two position maps into the workspace on `stream`. */
+int edm_t2s_begin_masked(edm_t2s_ctx* ctx, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host,
+                         const int* known_tokens, const unsigned char* regenerate_host, void* stream);
 /* embeddings_to_logits :135-152 on the running tokens (x_in == NULL) or on given embeddings fp32 [L, hidden] -> buffer "logits". */
 int edm_t2s_logits(edm_t2s_ctx* ctx, const float* x_in, void* stream);
 /* :229-260 decisions of iteration `iter` of `iters`: sample (arg-max on the last), confidence re-masking, token update. */
 int edm_t2s_step(edm_t2s_ctx* ctx, int iter, int iters, float temperature, unsigned long long seed, const float* cat_noise,
                  const float* remask_noise, const int* forced_ids, const uint8_t* forced_mask, void* stream);
-/* :267 speech_pred_tokens int64 [length] ([sum length_s] after edm_t2s_begin_batch). */
+/* :267 speech_pred_tokens int64 [length] ([sum length_s] after edm_t2s_begin_batch, [sum T_s] after edm_t2s_begin_masked). */
 int edm_t2s_result(edm_t2s_ctx* ctx, long long* tokens_out, void* stream);
 /* begin + pred_iters x (logits, step) + result. */
 int edm_t2s_decode(edm_t2s_ctx* ctx, const int* text_tokens, int n_text, int length, int pred_iters, float temperature,
@@ -391,6 +401,12 @@ int edm_t2s_decode(edm_t2s_ctx* ctx, const int* text_tokens, int n_text, int len
 int edm_t2s_decode_batch(edm_t2s_ctx* ctx, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host, int pred_iters,
                          float temperature, unsigned long long seed, const float* cat_noise, const float* remask_noise, const int* forced_ids,
                          const uint8_t* forced_masks, long long* tokens_out, void* stream);
+/* begin_masked + pred_iters x (logits, step) + result (:184-267 from the masked start); noise / forcing arrays [iteration][sum L_s
+ * (x 1024)] or NULL, tokens_out [sum T_s]. */
+int edm_t2s_decode_masked(edm_t2s_ctx* ctx, int n_seq, const int* text_tokens, const int* n_text_host, const int* length_host,
+                          const int* known_tokens, const unsigned char* regenerate_host, int pred_iters, float temperature,
+                          unsigned long long seed, const float* cat_noise, const float* remask_noise, const int* forced_ids,
+                          const uint8_t* forced_masks, long long* tokens_out, void* stream);
 
 /* number of kernels launched by this library since load (bench.py's gpu_launches) */
 unsigned long long edm_launch_count(void);
